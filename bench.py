@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BiGCN training throughput (trees/s) on B200, the metric of BASELINE.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch: graph prep + forward + nll_loss + backward
 + Adam on a Twitter16-shaped synthetic batch of 128 reply trees per GPU (BASELINE.json
@@ -64,7 +64,26 @@ def parse():
     ap.add_argument("--cpu-sample-trees", type=int, default=TREES_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernels", action="store_true", help="skip the large-N propagate micro-benchmark")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (loss, log-probs, the parameters "
+                         "Adam wrote and the gradients it used) as DIR/<name>.npy, float32 (rank 0)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "bigcn_b200":
+        ap.error("--dump-outputs applies to --impl bigcn_b200")
+    return args
+
+
+def dump_outputs(out_dir, tr, loss):
+    """The arrays a caller of FusedTrainer.step holds after the last timed step: the loss, the batch's log-probs,
+    every parameter as Adam left it and the gradient it was updated with (about 10 MB in all)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.reshape(1), "logp": tr.last_logp}
+    arrays.update({"param." + k: v for k, v in tr.views.items()})
+    arrays.update({"grad." + k: v for k, v in tr.gviews.items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    log(f"dumped {len(arrays)} arrays to {out_dir}")
 
 
 def peaks():
@@ -326,6 +345,8 @@ def run_ours(args):
                   "captures_in_timed_region": tr.graph_captures - captures0,
                   "replays_in_timed_region": tr.graph_replays - replays0, "prefetch_next_batch": prefetch}
     log(f"resident: {ms / args.steps:.4f} ms/step, cpu enqueue {cpu_enqueue_ms:.4f} ms/step, graphs {graph_info}")
+    if args.dump_outputs and rank == 0:      # before dp_parity_check, which resets the trainer's parameters
+        dump_outputs(args.dump_outputs, tr, loss)
     dp_parity = dp_parity_check(torch, bigcn_b200, tr, dev, rank, world, args) if world > 1 else None
 
     # ---- end to end: host buffers in, loss out ---------------------------------------
