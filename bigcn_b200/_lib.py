@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "libbigcn_b200.so")
 H = 64
 FLAG_EDGE_RANGE, FLAG_BATCH_ORDER, FLAG_ROOT_RANGE = 1, 2, 4
 DEG_BY = {"target": 0, "source": 1}
-GEMM_MODE = {"fp32": 0, "tf32": 1, "tf32x3": 2, "mixed": 3, "sparse": 4, "tf32x2": 5}
+GEMM_MODE = {"fp32": 0, "tf32": 1, "tf32x3": 2, "mixed": 3, "sparse": 4, "tf32x2": 5, "bf16": 6}
 FLAG_X_NOT_SPARSE = 8
 FLAG_X_CSR_RANGE = 16
 DIR_TD, DIR_BU = 1, 2
@@ -122,6 +122,7 @@ _SIGS = {
                                                   c_ptr, c_ptr, c_ptr, c_ptr, C.c_int32, C.c_int32, c_ptr, C.c_size_t,
                                                   c_ptr]),
     "bigcn_dense_row_counts": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr]),
+    "bigcn_dense_row_counts_bf16": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr]),
     "bigcn_dense_rows_to_csr": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, C.c_int64, c_ptr, c_ptr, c_ptr, C.c_int64,
                                           c_ptr, c_ptr]),
     "bigcn_readout_backward": (C.c_int, [c_ptr, C.c_int64, c_ptr, c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr]),

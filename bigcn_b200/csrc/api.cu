@@ -106,7 +106,8 @@ int xw_dispatch(const float* x, int64_t N, int64_t K, const float* const* w, int
     if (int rc = transpose_jobs_launch(js, st)) return rc;
     return xw_fp32(x, N, K, scratch, n_out, y, ldy, st);
   }
-  BIGCN_CHECK_ARG(mode == BIGCN_GEMM_TF32 || mode == BIGCN_GEMM_TF32X3 || mode == BIGCN_GEMM_TF32X2, "xw: unknown gemm_mode %d", mode);
+  BIGCN_CHECK_ARG(mode == BIGCN_GEMM_TF32 || mode == BIGCN_GEMM_TF32X3 || mode == BIGCN_GEMM_TF32X2 || mode == BIGCN_GEMM_BF16,
+                  "xw: unknown gemm_mode %d", mode);
   return xw_tc_weights(x, N, K, w, ldw, n_out, scratch, y, ldy, mode, st);
 }
 
@@ -274,11 +275,21 @@ static int check_common(const bigcn_dims_t* dm, const bigcn_opts_t* o, const cha
   BIGCN_CHECK_ARG(o->p_drop >= 0.f && o->p_drop < 1.f, "%s: p_drop must be in [0,1)", who);
   return 0;
 }
+// BIGCN_GEMM_BF16: x is a dense bf16 matrix the TMA can address (16 B rows, 16 B aligned)
+static int check_bf16_x(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_opts_t* o, const char* who) {
+  if (o->gemm_mode != BIGCN_GEMM_BF16 || dm->N == 0) return 0;
+  BIGCN_CHECK_ARG(bt->x != nullptr, "%s: gemm_mode BF16 needs a dense bf16 x (CSR input takes gemm_mode SPARSE)", who);
+  BIGCN_CHECK_ARG(dm->K % 8 == 0, "%s: gemm_mode BF16 needs in_feats a multiple of 8 (16 B rows for TMA), got %lld", who,
+                  (long long)dm->K);
+  BIGCN_CHECK_ARG((reinterpret_cast<uintptr_t>(bt->x) & 15) == 0, "%s: gemm_mode BF16 needs x 16-byte aligned", who);
+  return 0;
+}
 
 int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_params_t* pr,
                      const bigcn_opts_t* o, float* feat, int32_t* flags, void* ws, size_t ws_bytes,
                      cudaStream_t st) {
   if (int rc = check_common(dm, o, "features_forward")) return rc;
+  if (int rc = check_bf16_x(dm, bt, o, "features_forward")) return rc;
   FeatWs w = carve_features(dm, ws, ws_bytes, bt->prepared);
   BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total, "features_forward: workspace too small (%zu < %zu)",
                   ws_bytes, w.total);
@@ -290,6 +301,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   const bool sparse = o->gemm_mode == BIGCN_GEMM_SPARSE;
   const bool dropping = o->training && o->p_drop > 0.f;
   const bool csr_in = bt->x == nullptr && N > 0;
+  const int x_bf16 = o->gemm_mode == BIGCN_GEMM_BF16;
   BIGCN_CHECK_ARG(!csr_in || (sparse && bt->x_ptr && bt->x_col && bt->x_val),
                   "features_forward: x == NULL needs gemm_mode SPARSE and x_ptr / x_col / x_val");
   if (csr_in) {
@@ -334,6 +346,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     a.x = bt->x; a.rootindex = bt->rootindex; a.batch = bt->batch;
     a.N = N; a.B = B; a.K = K; a.node_id_base = bt->node_id_base;
     a.ksplit = root_splits;
+    a.x_bf16 = x_bf16;
     for (int q = 0; q < dirs.n; ++q) {
       const int d = dirs.id[q];   // one split: straight into z (the mix kernel reads a node's R before it writes the node's z)
       a.w2bT[q] = w.w2bT[d]; a.r[q] = root_splits > 1 ? w.rootR[d] : w.z[d]; a.drop[q] = make_drop(o, d);
@@ -342,7 +355,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   }
   {
     RootNzArgs a{bt->x, bt->rootindex, N, B, K, w.rnz_cnt, w.rnz_col, w.rnz_val, flags,
-                 w.slot, w.overflow, DW2B_CAP};
+                 w.slot, w.overflow, DW2B_CAP, x_bf16};
     if (prepared) {
       // done by bigcn_batch_prepare
     } else if (csr_in) {
@@ -475,6 +488,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
 int batch_prepare(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_opts_t* o, int32_t* flags, void* prepared,
                   size_t prepared_bytes, cudaStream_t st) {
   if (int rc = check_common(dm, o, "batch_prepare")) return rc;
+  if (int rc = check_bf16_x(dm, bt, o, "batch_prepare")) return rc;
   PrepWs w = carve_prepared(dm, prepared, prepared_bytes);
   BIGCN_CHECK_ARG(prepared != nullptr && prepared_bytes >= w.total, "batch_prepare: buffer too small (%zu < %zu)",
                   prepared_bytes, w.total);
@@ -517,7 +531,8 @@ int batch_prepare(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_o
     const int64_t E[2] = {dm->E_td, dm->E_bu};
     if (int rc = graph_prep_impl(2, ei, E, N, bt->batch, B, o->deg_by, w.g, w.node_ptr, flags, w.prep_ws, w.prep_bytes, pb))
       return rc;
-    RootNzArgs a{bt->x, bt->rootindex, N, B, K, w.rnz_cnt, w.rnz_col, w.rnz_val, flags, w.slot, w.overflow, DW2B_CAP};
+    RootNzArgs a{bt->x, bt->rootindex, N, B, K, w.rnz_cnt, w.rnz_col, w.rnz_val, flags, w.slot, w.overflow, DW2B_CAP,
+                 o->gemm_mode == BIGCN_GEMM_BF16};
     if (csr_in) {
       if (int rc = root_nz_csr_launch(a, bt->x_ptr, bt->x_col, bt->x_val, pb)) return rc;
     } else {
@@ -541,6 +556,7 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
                       const bigcn_opts_t* o, const float* grad_feat, const bigcn_params_t* gr,
                       void* ws, size_t ws_bytes, cudaStream_t st) {
   if (int rc = check_common(dm, o, "features_backward")) return rc;
+  if (int rc = check_bf16_x(dm, bt, o, "features_backward")) return rc;
   FeatWs w = carve_features(dm, ws, ws_bytes, bt->prepared);
   BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total, "features_backward: workspace too small");
   const int64_t N = dm->N, B = dm->B, K = dm->K;
@@ -622,6 +638,7 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
       a.x = bt->x; a.rootindex = bt->rootindex; a.batch = bt->batch;
       a.N = N; a.B = B; a.K = K; a.ld = H + K; a.node_id_base = bt->node_id_base;
       a.nseg = dw2b_dense_segments(N, B, K);
+      a.x_bf16 = o->gemm_mode == BIGCN_GEMM_BF16;
       for (int q = 0; q < dirs.n; ++q) {
         const int d = dirs.id[q];
         a.t2[q] = t2[d]; a.part[q] = w.S[d]; a.dw2[q] = gdir_w2(gr, d); a.drop[q] = make_drop(o, d);
@@ -779,6 +796,8 @@ static void knob_defaults() {
   // which then no longer queues behind them); bit 1 = the sort's last two launches at the step stream's priority.
   // tools/stepbench.py 12:0,1,2,3 -> 0.3347 / 0.3319 / 0.3347 / 0.3328 ms per step.
   g_knob[12] = 1;
+  // knob 13: 2 = two bf16 terms of the small operand in gemm_mode BF16 instead of three (the A/B of tools/bf16bench.py;
+  // three are shipped, DESIGN.md section 8)
   if (const char* e = getenv("BIGCN_MIX_TC")) {
     if (e[0] == 'b' && e[1] == 'w') g_knob[8] = 0;        // "bwd"
     else if (e[0] == 'b') g_knob[8] = 2;                  // "both"
@@ -817,7 +836,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 100; }
+extern "C" int bigcn_version(void) { return 101; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;

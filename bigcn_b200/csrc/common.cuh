@@ -1,6 +1,7 @@
 // Shared device helpers for libbigcn_b200.so (sm_100a only).
 #pragma once
 
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -53,6 +54,10 @@ struct Carver {
 
 // ---------------------------------------------------------------- device side
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
+
+// an element of x as fp32: x is fp32, or bf16 in BIGCN_GEMM_BF16 (widened exactly)
+__device__ __forceinline__ float x_f32(float v) { return v; }
+__device__ __forceinline__ float x_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
 
 __device__ __forceinline__ float4 ldg_stream_f4(const float* p) {
   float4 r;

@@ -39,6 +39,32 @@ __global__ void __launch_bounds__(256) k_feed_count(const float* __restrict__ x,
   }
 }
 
+// the same count for a bf16 x (BIGCN_GEMM_BF16's density probe): 8 elements per 16 B load when rows allow it; a bf16
+// is zero when its bits other than the sign are (so -0 counts as zero, as -0.f != 0.f is false above)
+__device__ __forceinline__ int nz_bf16x2(uint32_t v) { return ((v & 0x7FFFu) != 0u) + ((v & 0x7FFF0000u) != 0u); }
+__global__ void __launch_bounds__(256) k_feed_count_bf16(const __nv_bfloat16* __restrict__ x, int64_t N, int64_t K,
+                                                         int32_t* __restrict__ cnt) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarp = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const bool vec = (K % 8 == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+  for (int64_t r = warp0; r < N; r += nwarp) {
+    const __nv_bfloat16* xr = x + r * K;
+    int c = 0;
+    if (vec) {
+      for (int64_t q = lane; q < K / 8; q += 32) {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(xr) + q);
+        c += nz_bf16x2(v.x) + nz_bf16x2(v.y) + nz_bf16x2(v.z) + nz_bf16x2(v.w);
+      }
+    } else {
+      for (int64_t k = lane; k < K; k += 32) c += __bfloat162float(xr[k]) != 0.f;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(FULL_MASK, c, o);
+    if (lane == 0) cnt[r] = c;
+  }
+}
+
 // second pass: (col, val) of every row in ascending column order at ptr_local[r] + base; also the
 // rows' entries of the combined row-pointer array
 __global__ void __launch_bounds__(256) k_feed_fill(const float* __restrict__ x, int64_t N, int64_t K,
@@ -120,6 +146,14 @@ extern "C" int bigcn_dense_row_counts(const float* x, int64_t N, int64_t K, int3
   if (N == 0) return 0;
   k_feed_count<<<feed_grid(N), 256, 0, (cudaStream_t)stream>>>(x, N, K, cnt);
   BIGCN_CHECK_LAUNCH("k_feed_count");
+  return 0;
+}
+
+extern "C" int bigcn_dense_row_counts_bf16(const void* x, int64_t N, int64_t K, int32_t* cnt, bigcn_stream_t stream) {
+  BIGCN_CHECK_ARG(N >= 0 && K > 0 && (N == 0 || (x && cnt)), "dense_row_counts_bf16: bad arguments");
+  if (N == 0) return 0;
+  k_feed_count_bf16<<<feed_grid(N), 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const __nv_bfloat16*>(x), N, K, cnt);
+  BIGCN_CHECK_LAUNCH("k_feed_count_bf16");
   return 0;
 }
 

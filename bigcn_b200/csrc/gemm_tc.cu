@@ -41,6 +41,38 @@ struct TcParams {
   float* partial;  // [grid.y][N][n_out] or NULL
 };
 
+// Epilogue warps 4..7 of k_xw_tc / k_xw_bf16 (q = TMEM lane quarter this warp may access): per tile, the two M = 128
+// accumulators TMEM -> registers -> y (or this split's partial), then hand TMEM back to the MMA issuer
+__device__ __forceinline__ void xw_epilogue(const TcParams& p, uint32_t tmem_base, uint32_t bar_tmem_full,
+                                            uint32_t bar_tmem_empty, int q, int lane) {
+  uint32_t tile_ph = 0;
+  for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, tile_ph ^= 1) {
+    mbar_wait(bar_tmem_full, tile_ph);
+    tc_fence_after();
+    const int64_t m0 = (int64_t)tile * TC_BLOCK_M;
+#pragma unroll 1
+    for (int a = 0; a < 2; ++a) {
+      const int64_t row = m0 + a * 128 + q * 32 + lane;
+      for (int c0 = 0; c0 < p.n_out; c0 += 32) {
+        uint32_t r[32];
+        tc_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(a * 128 + c0), r);
+        tc_wait_ld();
+        if (row < p.N) {
+          float4* dst = p.partial ? reinterpret_cast<float4*>(p.partial + ((int64_t)blockIdx.y * p.N + row) * p.n_out + c0)
+                                  : reinterpret_cast<float4*>(p.y + row * p.ldy + c0);
+#pragma unroll
+          for (int j = 0; j < 8; ++j)
+            dst[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]),
+                                 __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
+        }
+      }
+    }
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(bar_tmem_empty);
+  }
+}
+
 // NB = number of B operands per stage (1: W, 2: W and W_lo); XS: X split hi / lo in shared memory (TF32X3)
 template <int NB, bool XS>
 __global__ void __launch_bounds__(XS ? TC_THREADS_XS : TC_THREADS, 1)
@@ -164,34 +196,8 @@ k_xw_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUten
         if (++s == STAGES) { s = 0; ph ^= 1; }
       }
     }
-  } else if (warp >= 4 && warp < 8) {   // ===== epilogue: TMEM -> registers -> global =====
-    const int q = warp & 3;   // TMEM lane quarter this warp may access
-    uint32_t tile_ph = 0;
-    for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, tile_ph ^= 1) {
-      mbar_wait(smem_u32(&bar_tmem_full), tile_ph);
-      tc_fence_after();
-      const int64_t m0 = (int64_t)tile * TC_BLOCK_M;
-#pragma unroll 1
-      for (int a = 0; a < 2; ++a) {
-        const int64_t row = m0 + a * 128 + q * 32 + lane;
-        for (int c0 = 0; c0 < p.n_out; c0 += 32) {
-          uint32_t r[32];
-          tc_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(a * 128 + c0), r);
-          tc_wait_ld();
-          if (row < p.N) {
-            float4* dst = p.partial ? reinterpret_cast<float4*>(p.partial + ((int64_t)blockIdx.y * p.N + row) * p.n_out + c0)
-                                    : reinterpret_cast<float4*>(p.y + row * p.ldy + c0);
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-              dst[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]),
-                                   __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
-          }
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(smem_u32(&bar_tmem_empty));
-    }
+  } else if (warp >= 4 && warp < 8) {
+    xw_epilogue(p, tmem_base, smem_u32(&bar_tmem_full), smem_u32(&bar_tmem_empty), warp & 3, lane);
   }
   tc_fence_before();
   __syncthreads();
@@ -231,18 +237,45 @@ __global__ void k_split_hi_lo(const float* __restrict__ w, int64_t ldw, int64_t 
 
 // ---------------------------------------------------------------- host side
 bool xw_tc_available() { return encode_fn() != nullptr; }
+// BIGCN_GEMM_BF16 (bf16 x; below)
+static int xw_bf16(const void* x, int64_t N, int64_t K, const float* const* w, int64_t ldw, int n_out, float* scratch,
+                   float* y, int64_t ldy, cudaStream_t st, float* partial);
+static int dw_bf16(const void* x, int64_t N, int64_t K, const float* t, int n_out, float* scratch01, float* scratch2,
+                   float* partial, float* dw_a, int64_t ldw_a, int64_t k0_a, float* dw_b, int64_t ldw_b, int64_t k0_b,
+                   cudaStream_t st);
 
 // w[0], w[1]: the [64, K] PyG weights of the active directions (row pitch ldw); scratch:
 // 2 * n_out * K floats for the TF32X3 split (may be NULL in TF32 mode)
 size_t xw_tc_partial_floats() { return (size_t)num_sms() * TC_BLOCK_M * 128; }
 
+// few tiles (small batch): split K so that the SMs share the K blocks, at least three per CTA.  Sets p.kb_per and
+// p.partial (NULL: not split); returns the number of splits (grid.y)
+static int xw_split_k(TcParams& p, float* partial) {
+  int nsplit = 1;
+  p.kb_per = p.num_kb;
+  p.partial = nullptr;
+  if (partial != nullptr && p.num_tiles * 4 <= num_sms() && p.num_kb >= 6) {
+    int want = num_sms() / p.num_tiles;
+    const int max_by_kb = p.num_kb / 3;
+    if (want > max_by_kb) want = max_by_kb;
+    if (want > 1) {
+      p.kb_per = (int)ceil_div(p.num_kb, want);
+      nsplit = (int)ceil_div(p.num_kb, p.kb_per);
+      if (nsplit > 1) p.partial = partial;
+      else p.kb_per = p.num_kb;
+    }
+  }
+  return nsplit;
+}
+
 // partial: xw_tc_partial_floats() floats or NULL (no split-K)
 int xw_tc_weights(const float* x, int64_t N, int64_t K, const float* const* w, int64_t ldw, int n_out,
                   float* scratch, float* y, int64_t ldy, int mode, cudaStream_t st, float* partial) {
   BIGCN_CHECK_ARG(encode_fn() != nullptr, "xw_tc: cuTensorMapEncodeTiled is unavailable in this driver");
+  BIGCN_CHECK_ARG(n_out == 64 || n_out == 128, "xw_tc: n_out must be 64 or 128");
+  if (mode == BIGCN_GEMM_BF16) return xw_bf16(x, N, K, w, ldw, n_out, scratch, y, ldy, st, partial);
   BIGCN_CHECK_ARG(K % 4 == 0 && ldw % 4 == 0, "xw_tc: in_feats must be a multiple of 4 for TMA (got %lld)", (long long)K);
   BIGCN_CHECK_ARG((reinterpret_cast<uintptr_t>(x) & 15) == 0, "xw_tc: x must be 16-byte aligned");
-  BIGCN_CHECK_ARG(n_out == 64 || n_out == 128, "xw_tc: n_out must be 64 or 128");
   if (N == 0) return 0;
   const int nb = mode == BIGCN_GEMM_TF32 ? 1 : 2;
   const bool xsplit = mode == BIGCN_GEMM_TF32X3;
@@ -275,21 +308,7 @@ int xw_tc_weights(const float* x, int64_t N, int64_t K, const float* const* w, i
   const int stages = xsplit ? 2 : (nb == 1 ? 4 : 3);
   const size_t smem = (size_t)stages * stage_bytes + 1024;
   int grid_x = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
-  // few tiles (small batch): split K so that the SMs share the K blocks, at least three per CTA
-  int nsplit = 1;
-  p.kb_per = p.num_kb;
-  p.partial = nullptr;
-  if (partial != nullptr && p.num_tiles * 4 <= num_sms() && p.num_kb >= 6) {
-    int want = num_sms() / p.num_tiles;
-    const int max_by_kb = p.num_kb / 3;
-    if (want > max_by_kb) want = max_by_kb;
-    if (want > 1) {
-      p.kb_per = (int)ceil_div(p.num_kb, want);
-      nsplit = (int)ceil_div(p.num_kb, p.kb_per);
-      if (nsplit > 1) p.partial = partial;
-      else p.kb_per = p.num_kb;
-    }
-  }
+  const int nsplit = xw_split_k(p, partial);
   const dim3 grid(grid_x, nsplit);
   static bool attr = false;
   if (!attr) {
@@ -350,6 +369,35 @@ struct DwtParams {
   int rows_per_split; // multiple of DWT_BK
 };
 
+// Epilogue warps 4..7 of k_dw_tc / k_dw_bf16: the 128 x 256 accumulator (q < n_out / 32: rows of this direction set)
+// TMEM -> registers -> partial[split][col][o]; a CTA without node rows writes zeros
+__device__ __forceinline__ void dw_epilogue(const DwtParams& p, uint32_t tmem_base, uint32_t bar_tmem_full, int num_kb,
+                                            int col0, int q, int lane) {
+  float* out = p.partial + (size_t)blockIdx.y * p.K * p.n_out;
+  const int m = q * 32 + lane;
+  if (num_kb > 0) {
+    mbar_wait(bar_tmem_full, 0);
+    tc_fence_after();
+  }
+  if (q < p.n_out / 32) {
+    for (int c0 = 0; c0 < DWT_N; c0 += 32) {
+      uint32_t r[32];
+      if (num_kb > 0) {
+        tc_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
+        tc_wait_ld();
+      } else {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) r[j] = 0u;
+      }
+#pragma unroll
+      for (int j = 0; j < 32; ++j) {
+        const int64_t col = (int64_t)col0 + c0 + j;
+        if (col < p.K) out[col * p.n_out + m] = __uint_as_float(r[j]);   // 32 lanes -> 128 B
+      }
+    }
+  }
+}
+
 template <int NA, bool XS>
 __global__ void __launch_bounds__(XS ? TC_THREADS_XS : TC_THREADS, 1)
 k_dw_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_t,
@@ -389,7 +437,6 @@ k_dw_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUten
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_s;
-  const int m_blocks = p.n_out / 32;   // 4 (both directions) or 2
 
   if (warp == 0) {
     if (lane == 0) {   // ===== TMA producer =====
@@ -456,31 +503,8 @@ k_dw_tc(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUten
       if (lane == 0) mbar_arrive(smem_u32(&bar_conv[s]));
       if (++s == STAGES) { s = 0; ph ^= 1; }
     }
-  } else if (warp >= 4 && warp < 8) {   // ===== epilogue =====
-    const int q = warp & 3;
-    float* out = p.partial + (size_t)blockIdx.y * p.K * p.n_out;
-    const int m = q * 32 + lane;
-    if (num_kb > 0) {
-      mbar_wait(smem_u32(&bar_tmem_full), 0);
-      tc_fence_after();
-    }
-    if (q < m_blocks) {
-      for (int c0 = 0; c0 < DWT_N; c0 += 32) {
-        uint32_t r[32];
-        if (num_kb > 0) {
-          tc_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
-          tc_wait_ld();
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) r[j] = 0u;
-        }
-#pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          const int64_t col = (int64_t)col0 + c0 + j;
-          if (col < p.K) out[col * p.n_out + m] = __uint_as_float(r[j]);   // 32 lanes -> 128 B
-        }
-      }
-    }
+  } else if (warp >= 4 && warp < 8) {
+    dw_epilogue(p, tmem_base, smem_u32(&bar_tmem_full), num_kb, col0, warp & 3, lane);
   }
   tc_fence_before();
   __syncthreads();
@@ -506,6 +530,17 @@ static int make_map_mn(CUtensorMap* m, const float* base, int64_t rows, int64_t 
   return 0;
 }
 
+// node splits of the dW GEMMs for N > 0: one wave of (column tile x split) CTAs, at least four stages of DWT_BK rows per
+// split; *rps = rows per split (a multiple of DWT_BK)
+static int dw_node_splits(int64_t N, int tiles, int64_t* rps) {
+  int nsplit = num_sms() / tiles;
+  const int64_t max_split = ceil_div(N, 4 * DWT_BK);
+  if (nsplit > max_split) nsplit = (int)max_split;
+  if (nsplit < 1) nsplit = 1;
+  *rps = ceil_div(ceil_div(N, nsplit), DWT_BK) * DWT_BK;
+  return (int)ceil_div(N, *rps);
+}
+
 __global__ void k_split_rows_hi_lo(const float* __restrict__ t, int64_t n, float* __restrict__ hi,
                                    float* __restrict__ lo) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -524,6 +559,8 @@ int dw_tc(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, int
   BIGCN_CHECK_ARG(K % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0, "dw_tc: x must be TMA-addressable");
   BIGCN_CHECK_ARG(ldt == n_out && (n_out == 64 || n_out == 128), "dw_tc: t must be dense [N, 64|128]");
   if (K == 0) return 0;
+  if (mode == BIGCN_GEMM_BF16)
+    return dw_bf16(x, N, K, t, n_out, hi_scratch, lo_scratch, partial, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
   const int na = mode == BIGCN_GEMM_TF32 ? 1 : 2;   // TF32X2, TF32X3 and MIXED split T
   const bool xsplit = mode == BIGCN_GEMM_TF32X3;    // ... and TF32X3 splits X in shared memory as well
   const int tiles = (int)ceil_div(K, DWT_N);
@@ -531,12 +568,8 @@ int dw_tc(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, int
   if (N == 0) {
     cudaMemsetAsync(partial, 0, (size_t)K * n_out * sizeof(float), st);
   } else {
-    nsplit = num_sms() / tiles;
-    const int64_t max_split = ceil_div(N, 4 * DWT_BK);
-    if (nsplit > max_split) nsplit = (int)max_split;
-    if (nsplit < 1) nsplit = 1;
-    int64_t rps = ceil_div(ceil_div(N, nsplit), DWT_BK) * DWT_BK;
-    nsplit = (int)ceil_div(N, rps);
+    int64_t rps = 0;
+    nsplit = dw_node_splits(N, tiles, &rps);
     const float* t_hi = t;
     const float* t_lo = t;
     if (na == 2) {
@@ -567,6 +600,357 @@ int dw_tc(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, int
     else if (!xsplit) k_dw_tc<2, false><<<dim3(tiles, nsplit), TC_THREADS, smem, st>>>(mx, mt, ml, p);
     else k_dw_tc<2, true><<<dim3(tiles, nsplit), TC_THREADS_XS, smem, st>>>(mx, mt, ml, p);
     BIGCN_CHECK_LAUNCH("k_dw_tc");
+  }
+  return dw_reduce_launch(partial, nsplit, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
+}
+
+
+// =====================================================================================
+// BIGCN_GEMM_BF16: x arrives as bf16 and is read from HBM as it is (half the bytes of fp32).  A bf16 x is exact, so the
+// only rounding left is in the small operand (W forward, T backward): it is split into NT bf16 terms
+//   t0 = bf16(v), t1 = bf16(v - t0), t2 = bf16(v - t0 - t1)
+// (each difference exact in fp32) and every term takes one kind::f16 MMA against the same x tile into one fp32 TMEM
+// accumulator.  Three terms carry 24 significant bits, as many as fp32; two carry 16.  DESIGN.md section 8 has the
+// measurements behind the term count (knob 13 = 2 selects two terms for the A/B).
+template <int NT>
+__device__ __forceinline__ void bf16_terms(float v, __nv_bfloat16 (&t)[NT]) {
+  float r = v;
+#pragma unroll
+  for (int i = 0; i < NT; ++i) {
+    t[i] = __float2bfloat16_rn(r);
+    r -= __bfloat162float(t[i]);
+  }
+}
+static int bf16_nterms() { return debug_knob(13) == 2 ? 2 : 3; }
+
+// terms of the [64, K] weight w (row pitch ldw) of direction d: out[t][d * 64 + r][k], [NT][n_out][K] bf16
+template <int NT>
+__global__ void k_split_w_bf16(const float* __restrict__ w, int64_t ldw, int64_t K, int n_out, int d,
+                               __nv_bfloat16* __restrict__ out) {
+  const int64_t n = 64 * K;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / K, k = i % K;
+    __nv_bfloat16 t[NT];
+    bf16_terms<NT>(w[r * ldw + k], t);
+#pragma unroll
+    for (int j = 0; j < NT; ++j) out[((int64_t)j * n_out + d * 64 + r) * K + k] = t[j];
+  }
+}
+
+// ---- forward  Y[N, n_out] = X[N, K] * W^T  with X bf16 -------------------------------------------------------------
+// Same warp roles, 256-row tiles (two M = 128 accumulators sharing every B tile), split-K and epilogue as k_xw_tc.
+// K blocks of 32 elements = one 64 B row of the SWIZZLE_64B layout: a stage is 16 KB of X plus NT x 8 KB of W terms
+// (40 KB at NT = 3: five stages; 32 KB at NT = 2: six).  With 64-element blocks and the 128B swizzle a stage would be
+// 80 KB and only two would fit.
+constexpr int BF_BLOCK_K = 32;
+constexpr int BF_UMMA_K = 16;
+constexpr int BF_A_BYTES = TC_BLOCK_M * 64;   // 16 KB
+constexpr int BF_B_BYTES = 128 * 64;          // 8 KB: one W term, up to 128 output rows
+template <int NT>
+constexpr int bf_xw_stages() { return NT == 3 ? 5 : 6; }
+template <int NT>
+constexpr int bf_xw_smem() { return bf_xw_stages<NT>() * (BF_A_BYTES + NT * BF_B_BYTES) + 1024; }
+
+template <int NT>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+k_xw_bf16(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const TcParams p) {
+  constexpr int STAGES = bf_xw_stages<NT>();
+  constexpr int STAGE_BYTES = BF_A_BYTES + NT * BF_B_BYTES;
+  extern __shared__ __align__(1024) uint8_t tc_smem[];
+  __shared__ __align__(8) uint64_t bar_full[STAGES];
+  __shared__ __align__(8) uint64_t bar_empty[STAGES];
+  __shared__ __align__(8) uint64_t bar_tmem_full, bar_tmem_empty;
+  __shared__ uint32_t tmem_base_s;
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t smem0 = (smem_u32(tc_smem) + 1023u) & ~1023u;
+  const int kb0 = blockIdx.y * p.kb_per, kb1 = min(p.num_kb, kb0 + p.kb_per);
+
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&map_x);
+    tma_prefetch_desc(&map_w);
+    for (int s = 0; s < STAGES; ++s) {
+      mbar_init(smem_u32(&bar_full[s]), 1);
+      mbar_init(smem_u32(&bar_empty[s]), 1);
+    }
+    mbar_init(smem_u32(&bar_tmem_full), 1);
+    mbar_init(smem_u32(&bar_tmem_empty), 4);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 2) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(&tmem_base_s)));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = tmem_base_s;
+
+  if (warp == 0) {
+    if (lane == 0) {   // ===== TMA producer =====
+      int s = 0;
+      uint32_t ph = 0;
+      const uint32_t tx = (uint32_t)(BF_A_BYTES + NT * p.n_out * 64);
+      for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+        const int m0 = tile * TC_BLOCK_M;
+        for (int kb = kb0; kb < kb1; ++kb) {
+          mbar_wait(smem_u32(&bar_empty[s]), ph ^ 1);
+          const uint32_t full = smem_u32(&bar_full[s]);
+          const uint32_t sa = smem0 + s * STAGE_BYTES;
+          mbar_expect_tx(full, tx);
+          tma_load_2d(sa, &map_x, full, kb * BF_BLOCK_K, m0);
+#pragma unroll
+          for (int t = 0; t < NT; ++t) tma_load_2d(sa + BF_A_BYTES + t * BF_B_BYTES, &map_w, full, kb * BF_BLOCK_K, t * p.n_out);
+          if (++s == STAGES) { s = 0; ph ^= 1; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {   // ===== MMA issuer =====
+      const uint32_t idesc = make_idesc_bf16(128, p.n_out);
+      int s = 0;
+      uint32_t ph = 0, tile_ph = 0;
+      for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, tile_ph ^= 1) {
+        mbar_wait(smem_u32(&bar_tmem_empty), tile_ph ^ 1);
+        tc_fence_after();
+        for (int kb = kb0; kb < kb1; ++kb) {
+          mbar_wait(smem_u32(&bar_full[s]), ph);
+          tc_fence_after();
+          const uint32_t sa = smem0 + s * STAGE_BYTES;
+#pragma unroll
+          for (int k = 0; k < BF_BLOCK_K / BF_UMMA_K; ++k) {
+            const uint32_t koff = k * BF_UMMA_K * 2;         // 32 B per K step inside the 64 B row
+            const uint64_t da0 = make_desc_k_sw64(sa + koff);
+            const uint64_t da1 = make_desc_k_sw64(sa + 128 * 64 + koff);
+#pragma unroll
+            for (int t = 0; t < NT; ++t) {
+              const uint64_t db = make_desc_k_sw64(sa + BF_A_BYTES + t * BF_B_BYTES + koff);
+              const uint32_t acc = ((kb - kb0) | k | t) ? 1u : 0u;
+              tc_mma_f16(tmem_base, da0, db, idesc, acc);
+              tc_mma_f16(tmem_base + 128, da1, db, idesc, acc);
+            }
+          }
+          tc_commit(smem_u32(&bar_empty[s]));
+          if (kb == kb1 - 1) tc_commit(smem_u32(&bar_tmem_full));
+          if (++s == STAGES) { s = 0; ph ^= 1; }
+        }
+      }
+    }
+  } else if (warp >= 4) {
+    xw_epilogue(p, tmem_base, smem_u32(&bar_tmem_full), smem_u32(&bar_tmem_empty), warp & 3, lane);
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem_base));
+  }
+}
+
+// x: bf16 [N, K]; w[0], w[1]: fp32 [64, K] (row pitch ldw); scratch: at least 3 * n_out * K bf16 (the W terms)
+static int xw_bf16(const void* x, int64_t N, int64_t K, const float* const* w, int64_t ldw, int n_out, float* scratch,
+                   float* y, int64_t ldy, cudaStream_t st, float* partial) {
+  if (N == 0) return 0;
+  BIGCN_CHECK_ARG(x != nullptr, "xw (bf16): NULL x");
+  BIGCN_CHECK_ARG(K % 8 == 0, "xw (bf16): in_feats must be a multiple of 8 for TMA (16 B rows), got %lld", (long long)K);
+  BIGCN_CHECK_ARG((reinterpret_cast<uintptr_t>(x) & 15) == 0, "xw (bf16): x must be 16-byte aligned");
+  BIGCN_CHECK_ARG(scratch != nullptr, "xw (bf16): needs the weight scratch");
+  const int nt = bf16_nterms();
+  __nv_bfloat16* terms = reinterpret_cast<__nv_bfloat16*>(scratch);
+  for (int d = 0; d < n_out / 64; ++d) {
+    if (nt == 3) k_split_w_bf16<3><<<num_sms() * 2, 256, 0, st>>>(w[d], ldw, K, n_out, d, terms);
+    else k_split_w_bf16<2><<<num_sms() * 2, 256, 0, st>>>(w[d], ldw, K, n_out, d, terms);
+    BIGCN_CHECK_LAUNCH("k_split_w_bf16");
+  }
+  CUtensorMap mx, mw;
+  if (int rc = make_map_bf16(&mx, x, N, K, K, BF_BLOCK_K, TC_BLOCK_M, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
+  if (int rc = make_map_bf16(&mw, terms, (int64_t)nt * n_out, K, K, BF_BLOCK_K, n_out, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
+  TcParams p;
+  p.y = y; p.ldy = ldy; p.N = N; p.K = K; p.n_out = n_out;
+  p.num_tiles = (int)ceil_div(N, TC_BLOCK_M);
+  p.num_kb = (int)ceil_div(K, BF_BLOCK_K);
+  const int grid_x = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
+  const int nsplit = xw_split_k(p, partial);
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(k_xw_bf16<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_xw_smem<3>());
+    cudaFuncSetAttribute(k_xw_bf16<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_xw_smem<2>());
+    attr = true;
+  }
+  const dim3 grid(grid_x, nsplit);
+  if (nt == 3) k_xw_bf16<3><<<grid, TC_THREADS, bf_xw_smem<3>(), st>>>(mx, mw, p);
+  else k_xw_bf16<2><<<grid, TC_THREADS, bf_xw_smem<2>(), st>>>(mx, mw, p);
+  BIGCN_CHECK_LAUNCH("k_xw_bf16");
+  if (nsplit > 1) {
+    int rb = (int)ceil_div(N * (n_out / 4), 256);
+    if (rb > num_sms() * 4) rb = num_sms() * 4;
+    k_xw_splitk_reduce<<<rb, 256, 0, st>>>(partial, nsplit, N, n_out, y, ldy);
+    BIGCN_CHECK_LAUNCH("k_xw_splitk_reduce");
+  }
+  return 0;
+}
+
+// ---- weight gradient  dW^T[k, o] = sum_i X[i, k] * T[i, o]  with X bf16 -------------------------------------------
+// As k_dw_tc (D[128 outputs, 256 columns of X] over the node axis, one wave of (column tile x node split) CTAs, ordered
+// split-K reduce), with 16-bit MN-major operands: SWIZZLE_128B atoms of 64 elements x 8 node rows, TMA boxes of
+// 64 columns x 32 node rows.  A stage is 32 node rows (two K = 16 MMAs per term): NT x 8 KB of T terms + 16 KB of X.
+constexpr int DWB_BK = 32;
+constexpr int DWB_A_BYTES = 2 * DWB_BK * 128;   // one T term: 128 outputs = 2 blocks of 64
+constexpr int DWB_B_BYTES = 4 * DWB_BK * 128;   // 256 columns of X = 4 blocks of 64
+template <int NT>
+constexpr int bf_dw_stages() { return NT == 3 ? 5 : 6; }
+template <int NT>
+constexpr int bf_dw_smem() { return bf_dw_stages<NT>() * (NT * DWB_A_BYTES + DWB_B_BYTES) + 1024; }
+__host__ __device__ constexpr uint32_t make_idesc_bf16_mn(int m, int n) {
+  return make_idesc_bf16(m, n) | (1u << 15) | (1u << 16);   // a_major = b_major = MN
+}
+
+template <int NT>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+k_dw_bf16(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_t0,
+          const __grid_constant__ CUtensorMap map_t1, const __grid_constant__ CUtensorMap map_t2, const DwtParams p) {
+  static_assert(DWB_BK == DWT_BK, "dw_tc's node splits are multiples of DWT_BK");
+  constexpr int STAGES = bf_dw_stages<NT>();
+  constexpr int STAGE_BYTES = NT * DWB_A_BYTES + DWB_B_BYTES;   // [T0 | T1 | (T2) | X]
+  extern __shared__ __align__(1024) uint8_t tc_smem[];
+  __shared__ __align__(8) uint64_t bar_full[STAGES];
+  __shared__ __align__(8) uint64_t bar_empty[STAGES];
+  __shared__ __align__(8) uint64_t bar_tmem_full;
+  __shared__ uint32_t tmem_base_s;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t smem0 = (smem_u32(tc_smem) + 1023u) & ~1023u;
+  const int col0 = blockIdx.x * DWT_N;
+  const int64_t r_begin = (int64_t)blockIdx.y * p.rows_per_split;
+  const int64_t r_end = min(p.N, r_begin + p.rows_per_split);
+  const int num_kb = r_end > r_begin ? (int)((r_end - r_begin + DWB_BK - 1) / DWB_BK) : 0;
+
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&map_x);
+    tma_prefetch_desc(&map_t0);
+    for (int s = 0; s < STAGES; ++s) {
+      mbar_init(smem_u32(&bar_full[s]), 1);
+      mbar_init(smem_u32(&bar_empty[s]), 1);
+    }
+    mbar_init(smem_u32(&bar_tmem_full), 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 2) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(&tmem_base_s)));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = tmem_base_s;
+
+  if (warp == 0) {
+    if (lane == 0) {   // ===== TMA producer =====
+      int s = 0;
+      uint32_t ph = 0;
+      // both 64-output blocks of every term are always loaded: a block beyond n_out is out of bounds -> zero filled
+      const uint32_t tx = (uint32_t)(NT * DWB_A_BYTES + DWB_B_BYTES);
+      for (int kb = 0; kb < num_kb; ++kb) {
+        mbar_wait(smem_u32(&bar_empty[s]), ph ^ 1);
+        const uint32_t full = smem_u32(&bar_full[s]);
+        const uint32_t sa = smem0 + s * STAGE_BYTES;
+        const int row = (int)(r_begin + (int64_t)kb * DWB_BK);
+        mbar_expect_tx(full, tx);
+#pragma unroll
+        for (int mb = 0; mb < 2; ++mb) {
+          tma_load_2d(sa + mb * (DWB_BK * 128), &map_t0, full, mb * 64, row);
+          tma_load_2d(sa + DWB_A_BYTES + mb * (DWB_BK * 128), &map_t1, full, mb * 64, row);
+          if (NT == 3) tma_load_2d(sa + 2 * DWB_A_BYTES + mb * (DWB_BK * 128), &map_t2, full, mb * 64, row);
+        }
+#pragma unroll
+        for (int nb = 0; nb < 4; ++nb)
+          tma_load_2d(sa + NT * DWB_A_BYTES + nb * (DWB_BK * 128), &map_x, full, col0 + nb * 64, row);
+        if (++s == STAGES) { s = 0; ph ^= 1; }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {   // ===== MMA issuer =====
+      const uint32_t idesc = make_idesc_bf16_mn(128, DWT_N);
+      int s = 0;
+      uint32_t ph = 0;
+      for (int kb = 0; kb < num_kb; ++kb) {
+        mbar_wait(smem_u32(&bar_full[s]), ph);
+        tc_fence_after();
+        const uint32_t sa = smem0 + s * STAGE_BYTES;
+#pragma unroll
+        for (int k = 0; k < DWB_BK / BF_UMMA_K; ++k) {
+          const uint32_t koff = k * BF_UMMA_K * 128;           // 16 node rows of 128 B
+          const uint64_t db = make_desc_mn_sw128_16b(sa + NT * DWB_A_BYTES + koff, DWB_BK * 128);
+#pragma unroll
+          for (int t = 0; t < NT; ++t) {
+            const uint64_t da = make_desc_mn_sw128_16b(sa + t * DWB_A_BYTES + koff, DWB_BK * 128);
+            tc_mma_f16(tmem_base, da, db, idesc, (kb | k | t) ? 1u : 0u);
+          }
+        }
+        tc_commit(smem_u32(&bar_empty[s]));
+        if (kb == num_kb - 1) tc_commit(smem_u32(&bar_tmem_full));
+        if (++s == STAGES) { s = 0; ph ^= 1; }
+      }
+    }
+  } else if (warp >= 4) {
+    dw_epilogue(p, tmem_base, smem_u32(&bar_tmem_full), num_kb, col0, warp & 3, lane);
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem_base));
+  }
+}
+
+// terms of t [n elements]: t0 -> t01[i], t1 -> t01[n + i], t2 -> t2[i]
+template <int NT>
+__global__ void k_split_rows_bf16(const float* __restrict__ t, int64_t n, __nv_bfloat16* __restrict__ t01,
+                                  __nv_bfloat16* __restrict__ t2) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    __nv_bfloat16 v[NT];
+    bf16_terms<NT>(t[i], v);
+    t01[i] = v[0];
+    t01[n + i] = v[1];
+    if (NT == 3) t2[i] = v[NT - 1];
+  }
+}
+
+// x: bf16 [N, K]; t: fp32 [N, n_out]; scratch01: N * n_out floats (terms 0 and 1 as bf16), scratch2: N * n_out floats
+static int dw_bf16(const void* x, int64_t N, int64_t K, const float* t, int n_out, float* scratch01, float* scratch2,
+                   float* partial, float* dw_a, int64_t ldw_a, int64_t k0_a, float* dw_b, int64_t ldw_b, int64_t k0_b,
+                   cudaStream_t st) {
+  BIGCN_CHECK_ARG(N == 0 || (x != nullptr && K % 8 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0),
+                  "dw (bf16): x must be 16-byte aligned with in_feats a multiple of 8 (TMA)");
+  BIGCN_CHECK_ARG(scratch01 != nullptr && scratch2 != nullptr, "dw (bf16): needs the split scratch");
+  const int tiles = (int)ceil_div(K, DWT_N);
+  int nsplit = 1;
+  if (N == 0) {
+    cudaMemsetAsync(partial, 0, (size_t)K * n_out * sizeof(float), st);
+  } else {
+    int64_t rps = 0;
+    nsplit = dw_node_splits(N, tiles, &rps);
+    const int nt = bf16_nterms();
+    __nv_bfloat16* t01 = reinterpret_cast<__nv_bfloat16*>(scratch01);
+    __nv_bfloat16* t2 = reinterpret_cast<__nv_bfloat16*>(scratch2);
+    if (nt == 3) k_split_rows_bf16<3><<<num_sms() * 4, 256, 0, st>>>(t, N * n_out, t01, t2);
+    else k_split_rows_bf16<2><<<num_sms() * 4, 256, 0, st>>>(t, N * n_out, t01, t2);
+    BIGCN_CHECK_LAUNCH("k_split_rows_bf16");
+    CUtensorMap mx, m0, m1, m2;
+    if (int rc = make_map_bf16(&mx, x, N, K, K, 64, DWB_BK, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    if (int rc = make_map_bf16(&m0, t01, N, n_out, n_out, 64, DWB_BK, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    if (int rc = make_map_bf16(&m1, t01 + N * n_out, N, n_out, n_out, 64, DWB_BK, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    if (int rc = make_map_bf16(&m2, t2, N, n_out, n_out, 64, DWB_BK, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
+    DwtParams p;
+    p.partial = partial; p.N = N; p.K = K; p.n_out = n_out; p.rows_per_split = (int)rps;
+    static bool attr = false;
+    if (!attr) {
+      cudaFuncSetAttribute(k_dw_bf16<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_dw_smem<3>());
+      cudaFuncSetAttribute(k_dw_bf16<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_dw_smem<2>());
+      attr = true;
+    }
+    if (nt == 3) k_dw_bf16<3><<<dim3(tiles, nsplit), TC_THREADS, bf_dw_smem<3>(), st>>>(mx, m0, m1, m2, p);
+    else k_dw_bf16<2><<<dim3(tiles, nsplit), TC_THREADS, bf_dw_smem<2>(), st>>>(mx, m0, m1, m2, p);
+    BIGCN_CHECK_LAUNCH("k_dw_bf16");
   }
   return dw_reduce_launch(partial, nsplit, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
 }

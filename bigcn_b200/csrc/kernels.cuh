@@ -36,7 +36,8 @@ int dw_fp32(const float*, int64_t, int64_t, const float*, int64_t, int, float*, 
 struct PropDir { const int32_t* ptr; const int32_t* idx; const float* dis; const float* h; const float* bias; float* out; int64_t ldh, ldo; int32_t* lng; int64_t E; };
 struct PropArgs { PropDir d[2]; int64_t N; int32_t relu; int32_t cb; };
 int propagate_launch(const PropArgs&, int, cudaStream_t);
-struct RootNzArgs { const float* x; const int64_t* rootindex; int64_t N, B, K; int32_t* cnt; int32_t* col; float* val; int32_t* flags; int32_t* slot; int32_t* overflow; int32_t cap; };
+struct RootNzArgs { const float* x; const int64_t* rootindex; int64_t N, B, K; int32_t* cnt; int32_t* col; float* val; int32_t* flags; int32_t* slot; int32_t* overflow; int32_t cap;
+                    int32_t x_bf16;   /* x holds bf16 (BIGCN_GEMM_BF16) */ };
 int root_nz_launch(const RootNzArgs&, cudaStream_t);
 int root_nz_csr_launch(const RootNzArgs&, const int32_t*, const int32_t*, const float*, cudaStream_t);
 struct RootProjArgs { const int32_t* cnt; const int32_t* col; const float* val; const float* w2bT[2]; float* P[2]; int64_t B, K; };
@@ -127,6 +128,7 @@ struct RootDenseArgs {
   int32_t ksplit;         // column ranges summed by different CTAs (small batches: a CTA's chain of K / 32 chunks is the
                           // latency of the whole pass); the consumer adds the partials in split order
   DropSpec drop[2];
+  int32_t x_bf16;         // x holds bf16 (BIGCN_GEMM_BF16)
 };
 constexpr int64_t RD_CAP_ROWS = 32768;   // rows of split partials per direction the workspace holds
 int root_dense_splits(int64_t N, int64_t K);
@@ -138,6 +140,7 @@ struct Dw2bDenseArgs {
   float* part[2];         // [nseg][K][64]
   float* dw2[2];          // conv2.lin.weight gradient [64][64 + K]
   DropSpec drop[2];
+  int32_t x_bf16;         // x holds bf16 (BIGCN_GEMM_BF16)
 };
 int root_dense_forward(const RootDenseArgs&, int ndir, cudaStream_t);
 int dw2b_dense_segments(int64_t N, int64_t B, int64_t K);

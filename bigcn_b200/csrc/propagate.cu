@@ -81,6 +81,8 @@ int propagate_launch(const PropArgs& a0, int ndir, cudaStream_t st) {
 // CTA per tree: 8 warps ballot 32-column strips, a strip-count scan orders them, a second
 // pass writes (col, val) at its rank and slot[k][b] = rank for the positive columns (column-major map,
 // preset to -1, that the dW2b reduce uses to find a column's slot in each tree with coalesced loads).
+// T = float, or __nv_bfloat16 when x is bf16 (BIGCN_GEMM_BF16: the values are widened exactly).
+template <typename T>
 __global__ void __launch_bounds__(256) k_root_nz(RootNzArgs a) {
   extern __shared__ int strip[];  // [nstrips] counts -> exclusive offsets
   __shared__ int s_total;
@@ -90,10 +92,10 @@ __global__ void __launch_bounds__(256) k_root_nz(RootNzArgs a) {
   const int64_t r = a.rootindex[b];
   const bool ok = r >= 0 && r < a.N;
   if (!ok && threadIdx.x == 0) atomicOr(a.flags, BIGCN_FLAG_ROOT_RANGE);
-  const float* xr = a.x + (ok ? r : 0) * a.K;
+  const T* xr = reinterpret_cast<const T*>(a.x) + (ok ? r : 0) * a.K;
   for (int s = w; s < nstrips; s += 8) {
     const int64_t k = (int64_t)s * 32 + lane;
-    const float v = (ok && k < a.K) ? xr[k] : 0.f;
+    const float v = (ok && k < a.K) ? x_f32(xr[k]) : 0.f;
     const unsigned m = __ballot_sync(FULL_MASK, v > 0.f);
     if (lane == 0) strip[s] = __popc(m);
   }
@@ -120,7 +122,7 @@ __global__ void __launch_bounds__(256) k_root_nz(RootNzArgs a) {
   __syncthreads();
   for (int s = w; s < nstrips; s += 8) {
     const int64_t k = (int64_t)s * 32 + lane;
-    const float v = (ok && k < a.K) ? xr[k] : 0.f;
+    const float v = (ok && k < a.K) ? x_f32(xr[k]) : 0.f;
     const unsigned m = __ballot_sync(FULL_MASK, v > 0.f);
     const int pos = strip[s] + __popc(m & ((1u << lane) - 1u));
     if (v > 0.f) {
@@ -924,7 +926,8 @@ int root_nz_launch(const RootNzArgs& a, cudaStream_t st) {
   cudaMemsetAsync(a.slot, 0xFF, (size_t)a.B * a.K * sizeof(int32_t), st);   // -1: column not positive in that root
   const size_t smem = (size_t)((a.K + 31) / 32) * sizeof(int);
   BIGCN_CHECK_ARG(smem <= 48 * 1024, "root_nz: in_feats too large (%lld)", (long long)a.K);
-  k_root_nz<<<(int)a.B, 256, smem, st>>>(a);
+  if (a.x_bf16) k_root_nz<__nv_bfloat16><<<(int)a.B, 256, smem, st>>>(a);
+  else k_root_nz<float><<<(int)a.B, 256, smem, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_root_nz");
   return 0;
 }

@@ -25,15 +25,17 @@ namespace bigcn {
 constexpr int RD_KC = 32;   // columns per chunk
 
 // relu(x[root, k .. k + 3]) masked by the dropout decisions of node `node` for columns 64 + k .. 64 + k + 3 (k % 4 == 0:
-// exactly one Philox block, the block the list walk of the mix kernel draws for these columns)
+// exactly one Philox block, the block the list walk of the mix kernel draws for these columns).  T = float, or
+// __nv_bfloat16 when x is bf16 (BIGCN_GEMM_BF16: widened exactly, so the same values as from the fp32 copy)
+template <typename T>
 __device__ __forceinline__ void masked_root_quad(const float* __restrict__ x, int64_t root_row, int64_t K, int64_t k,
                                                  const DropSpec& ds, int64_t node, float out[4]) {
   out[0] = out[1] = out[2] = out[3] = 0.f;
   if (root_row < 0 || k >= K) return;
-  const float* xr = x + root_row * K + k;
+  const T* xr = reinterpret_cast<const T*>(x) + root_row * K + k;
   float v[4];
 #pragma unroll
-  for (int j = 0; j < 4; ++j) v[j] = k + j < K ? fmaxf(__ldg(xr + j), 0.f) : 0.f;
+  for (int j = 0; j < 4; ++j) v[j] = k + j < K ? fmaxf(x_f32(__ldg(xr + j)), 0.f) : 0.f;
   if ((v[0] > 0.f) | (v[1] > 0.f) | (v[2] > 0.f) | (v[3] > 0.f)) {
     const Philox4 r = drop_block(ds, node, (uint32_t)((H + k) >> 2));
     out[0] = r.x >= ds.thresh ? v[0] : 0.f;
@@ -50,7 +52,7 @@ __device__ __forceinline__ void masked_root_quad(const float* __restrict__ x, in
 // wavefronts per column and warp: NPT = 2: 2 + 8 for 8 packed fmas per thread; NPT = 4: 4 + 8 for 16 (the first
 // version -- outputs 8 q .. + 7, a two-way bank conflict on every W load -- ran at 44 % conflicted wavefronts and was
 // bound by them: profiles/r02e_prof_rootdense_*).
-template <int NPT>
+template <int NPT, typename T>
 __global__ void __launch_bounds__(256) k_root_dense(RootDenseArgs a) {
   constexpr int TN = 32 * NPT;
   __shared__ __align__(16) float sW[RD_KC][H];
@@ -79,7 +81,7 @@ __global__ void __launch_bounds__(256) k_root_dense(RootDenseArgs a) {
     for (int u = 0; u < NPT; ++u) {   // the masked root operand: TN nodes x 8 quads, consecutive lanes = consecutive nodes
       const int q = t + 256 * u, node = q % TN, kq = q / TN;
       float m[4];
-      masked_root_quad(a.x, sRoot[node], a.K, k0 + 4 * kq, ds, a.node_id_base + i0 + node, m);
+      masked_root_quad<T>(a.x, sRoot[node], a.K, k0 + 4 * kq, ds, a.node_id_base + i0 + node, m);
 #pragma unroll
       for (int j = 0; j < 4; ++j) sA[4 * kq + j][node] = k0 + 4 * kq + j < kend ? m[j] : 0.f;
     }
@@ -126,10 +128,14 @@ int root_dense_splits(int64_t N, int64_t K) {
 
 int root_dense_forward(const RootDenseArgs& a, int ndir, cudaStream_t st) {
   if (a.N == 0) return 0;
-  if (a.N * ndir * a.ksplit >= (int64_t)128 * 2 * num_sms())   // enough 128-node tiles for two waves: the leaner inner loop
-    k_root_dense<4><<<dim3((unsigned)ceil_div(a.N, 128), ndir, a.ksplit), 256, 0, st>>>(a);
-  else
-    k_root_dense<2><<<dim3((unsigned)ceil_div(a.N, 64), ndir, a.ksplit), 256, 0, st>>>(a);
+  const dim3 g4((unsigned)ceil_div(a.N, 128), ndir, a.ksplit), g2((unsigned)ceil_div(a.N, 64), ndir, a.ksplit);
+  if (a.N * ndir * a.ksplit >= (int64_t)128 * 2 * num_sms()) {   // enough 128-node tiles for two waves: the leaner inner loop
+    if (a.x_bf16) k_root_dense<4, __nv_bfloat16><<<g4, 256, 0, st>>>(a);
+    else k_root_dense<4, float><<<g4, 256, 0, st>>>(a);
+  } else {
+    if (a.x_bf16) k_root_dense<2, __nv_bfloat16><<<g2, 256, 0, st>>>(a);
+    else k_root_dense<2, float><<<g2, 256, 0, st>>>(a);
+  }
   BIGCN_CHECK_LAUNCH("k_root_dense");
   return 0;
 }
@@ -139,6 +145,7 @@ int root_dense_forward(const RootDenseArgs& a, int ndir, cudaStream_t st) {
 // the segment in tiles of 32, ascending.  The operand tile is stored [node][column]: a thread's four columns are one
 // vector load.  Per node and warp: 4 + 8 shared-memory wavefronts for 16 packed fmas per thread.
 constexpr int RD_BK = 128;   // columns per CTA
+template <typename T>
 __global__ void __launch_bounds__(256) k_dw2b_dense_part(Dw2bDenseArgs a) {
   __shared__ __align__(16) float sT[32][H];
   __shared__ __align__(16) float sA[32][RD_BK + 4];
@@ -162,7 +169,7 @@ __global__ void __launch_bounds__(256) k_dw2b_dense_part(Dw2bDenseArgs a) {
       const int q = t + 256 * u, node = q >> 5, cq = q & 31;
       const int64_t i = i0 + node;
       float m[4];
-      masked_root_quad(a.x, i < s1 ? a.rootindex[a.batch[i]] : -1, a.K, k0 + 4 * cq, ds, a.node_id_base + i, m);
+      masked_root_quad<T>(a.x, i < s1 ? a.rootindex[a.batch[i]] : -1, a.K, k0 + 4 * cq, ds, a.node_id_base + i, m);
       st4(&sA[node][4 * cq], make_float4(m[0], m[1], m[2], m[3]));
     }
     __syncthreads();
@@ -213,7 +220,9 @@ int dw2b_dense_backward(const Dw2bDenseArgs& a0, int ndir, cudaStream_t st) {
   if (a0.K == 0) return 0;
   Dw2bDenseArgs a = a0;
   a.seg_rows = ceil_div(ceil_div(a.N > 0 ? a.N : 1, a.nseg), 32) * 32;
-  k_dw2b_dense_part<<<dim3((unsigned)ceil_div(a.K, RD_BK), a.nseg, ndir), 256, 0, st>>>(a);
+  const dim3 grid((unsigned)ceil_div(a.K, RD_BK), a.nseg, ndir);
+  if (a.x_bf16) k_dw2b_dense_part<__nv_bfloat16><<<grid, 256, 0, st>>>(a);
+  else k_dw2b_dense_part<float><<<grid, 256, 0, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_dw2b_dense_part");
   k_dw2b_dense_reduce<<<dim3((unsigned)ceil_div(a.K * H, 256), ndir), 256, 0, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_dw2b_dense_reduce");

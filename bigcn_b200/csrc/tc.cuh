@@ -63,6 +63,43 @@ __host__ __device__ constexpr uint32_t make_idesc_tf32(int m, int n) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 
+// ---- kind::f16 (BIGCN_GEMM_BF16: bf16 operands, fp32 accumulator in TMEM), UMMA_K = 16
+__device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                           uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// kind::f16 instruction descriptor: c_format F32 (1) at [4,6), a/b_format BF16 (1) at [7,10)/[10,13), K-major A and B,
+// N >> 3 at [17,23), M >> 4 at [24,29)
+__host__ __device__ constexpr uint32_t make_idesc_bf16(int m, int n) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+// K-major SWIZZLE_64B descriptor: rows of 64 B (32 bf16), 8-row atoms of 512 B (SBO), LBO unused, layout 4 (SW64)
+__device__ __forceinline__ uint64_t make_desc_k_sw64(uint32_t saddr) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
+  d |= (uint64_t)1 << 16;
+  d |= (uint64_t)(512 >> 4) << 32;
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)4 << 61;
+  return d;
+}
+// MN-major SWIZZLE_128B descriptor for 16-bit operands: 128 B (64 bf16) contiguous along MN, rows of the K axis 128 B
+// apart, 8-row atoms (SBO = 1024 B), LBO = bytes between 64-element MN blocks
+__device__ __forceinline__ uint64_t make_desc_mn_sw128_16b(uint32_t saddr, uint32_t lbo_bytes) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
+  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
+  d |= (uint64_t)(1024 >> 4) << 32;
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)2 << 61;   // LayoutType::SWIZZLE_128B
+  return d;
+}
+
 // generic-proxy writes to shared memory -> visible to the async proxy (tcgen05.mma reads)
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
@@ -115,6 +152,23 @@ inline int make_map(CUtensorMap* m, const float* base, int64_t rows, int64_t col
                                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("xw_tc: cuTensorMapEncodeTiled failed (%d)", (int)r);
+    return 2;
+  }
+  return 0;
+}
+
+// 2-D bf16 row-major [rows, cols] with row pitch ld (elements); box = box_cols x box_rows with the given swizzle
+inline int make_map_bf16(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_cols,
+                         int box_rows, CUtensorMapSwizzle swizzle) {
+  const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  const cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
+  const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+  const cuuint32_t estr[2] = {1, 1};
+  const CUresult r = encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstr, box,
+                                 estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("bf16 tensor map: cuTensorMapEncodeTiled failed (%d)", (int)r);
     return 2;
   }
   return 0;

@@ -384,6 +384,7 @@ extern "C" int bigcn_gcnconv_weighted_forward(const float* x, int64_t N, int64_t
   cudaStream_t st = (cudaStream_t)stream;
   BIGCN_CHECK_ARG(N >= 0 && K > 0 && E >= 0 && w && flags && (E == 0 || (edge_index && edge_weight)),
                   "gcnconv_weighted_forward: bad arguments");
+  BIGCN_CHECK_ARG(gemm_mode != BIGCN_GEMM_BF16, "gcnconv_weighted_forward: gemm_mode BF16 is not supported here (fp32 x)");
   WConvWs cw = carve_wconv(N, E, K, workspace, workspace_bytes);
   BIGCN_CHECK_ARG(workspace && workspace_bytes >= cw.total, "gcnconv_weighted_forward: workspace too small");
   if (int rc = wnorm_run(cw.n, edge_index, E, edge_weight, N, deg_by, flags, st)) return rc;
@@ -405,6 +406,7 @@ extern "C" int bigcn_gcnconv_weighted_backward(const float* x, int64_t N, int64_
                                                bigcn_stream_t stream) {
   cudaStream_t st = (cudaStream_t)stream;
   BIGCN_CHECK_ARG(N >= 0 && K > 0 && E >= 0 && dw && db, "gcnconv_weighted_backward: bad arguments");
+  BIGCN_CHECK_ARG(gemm_mode != BIGCN_GEMM_BF16, "gcnconv_weighted_backward: gemm_mode BF16 is not supported here (fp32 x)");
   WConvWs cw = carve_wconv(N, E, K, workspace, workspace_bytes);
   BIGCN_CHECK_ARG(workspace && workspace_bytes >= cw.total, "gcnconv_weighted_backward: workspace too small");
   const WGraph& G = cw.n.G;

@@ -20,7 +20,7 @@ import ctypes as C
 import weakref
 
 from .ops import (FeaturesFunction, GCNConvFunction, GCNConvWeightedFunction, HeadFunction, raise_on_flags,
-                  capture_graph, pick_gemm_mode, _as_x, _i64, _make_structs, _p, _stream)
+                  capture_graph, pick_gemm_mode, bf16_features_dense, _as_x, _i64, _make_structs, _p, _stream)
 
 H = L.H
 
@@ -91,6 +91,7 @@ class _RumorGCN(torch.nn.Module):
         self.node_id_base = 0
         self.last_flags = None
         self._auto_mode = None
+        self._bf16_dense = None
         self.dense_roots = "auto"           # see resolved_dense_roots
 
     def resolved_gemm_mode(self, x):
@@ -108,10 +109,15 @@ class _RumorGCN(torch.nn.Module):
     def resolved_dense_roots(self, x):
         """``opts.dense_roots`` (training only): the root half of conv2.lin as a tiled masked product instead of a walk
         over each tree's positive root columns.  ``self.dense_roots`` = True / False forces it; 'auto' (default) turns
-        it on when ``gemm_mode='auto'`` measured DENSE features (PHEME's sentence embeddings) -- bag-of-words roots
-        (~20 columns) keep the list walk.  Same forward sums in the same order either way."""
+        it on when ``gemm_mode='auto'`` measured DENSE features (PHEME's sentence embeddings), or when ``gemm_mode='bf16'``
+        finds dense rows with the same probe on the bf16 values -- bag-of-words roots (~20 columns) keep the list walk.
+        Same forward sums in the same order either way."""
         if self.dense_roots != "auto":
             return bool(self.dense_roots) and isinstance(x, torch.Tensor) and x.layout == torch.strided
+        if self.gemm_mode == "bf16":
+            if self._bf16_dense is None:     # decided once, on the first feature matrix, like gemm_mode='auto'
+                self._bf16_dense = bf16_features_dense(x.detach())
+            return self._bf16_dense
         return self.gemm_mode == "auto" and self.resolved_gemm_mode(x) != "sparse"
 
     def _conv_params(self):
@@ -200,14 +206,14 @@ class BiGCN(torch.nn.Module):
     def _infer_plan(self, data):
         L.require_device()
         td, bu = self.TDrumorGCN, self.BUrumorGCN
-        x, xs = _as_x(data.x)
+        mode = td.resolved_gemm_mode(data.x)
+        x, xs = _as_x(data.x, mode)
         ei, bue, batch, root = _i64(data.edge_index), _i64(data.BU_edge_index), _i64(data.batch), _i64(data.rootindex)
         params = tuple(p.detach() for p in td._conv_params() + bu._conv_params())
         for t in (x, ei, bue, batch, root) + params:
             if t is not None and not t.is_cuda:
                 raise L.BigcnError("bigcn_b200 ops take CUDA tensors only (no CPU fallback)")
         c = self.fc.weight.shape[0]
-        mode = td.resolved_gemm_mode(data.x)
         if xs is not None and mode != "sparse":
             raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
         dims, bt, pr = _make_structs(x, ei, bue, batch, root, params, c, td.node_id_base, xs)

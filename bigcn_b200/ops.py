@@ -153,13 +153,42 @@ def host_dense_to_csr(x, n_threads=0, out=None, cap=None):
     return SparseX(ptr[:n + 1], col[:nnz], val[:nnz], (n, k))
 
 
-def _as_x(x):
-    """dense fp32 tensor | SparseX | torch sparse tensor -> (dense or None, SparseX or None)"""
+def bf16_x(x):
+    """data.x for ``gemm_mode='bf16'``: a dense, contiguous CUDA bfloat16 matrix whose rows the TMA can address,
+    passed through as it is.  Anything else raises (never a silent cast)."""
+    if not isinstance(x, torch.Tensor) or x.layout != torch.strided:
+        raise L.BigcnError("gemm_mode='bf16' needs a dense torch.bfloat16 data.x; a sparse x takes gemm_mode='sparse'")
+    if x.dtype != torch.bfloat16:
+        raise L.BigcnError(f"gemm_mode='bf16' needs data.x in torch.bfloat16, got {x.dtype}: convert the features once "
+                           "with x.to(torch.bfloat16), or keep fp32 features with gemm_mode='tf32x3'")
+    _need_cuda(x)
+    if x.dim() != 2:
+        raise L.BigcnError(f"gemm_mode='bf16': data.x must be [N, in_feats], got shape {tuple(x.shape)}")
+    if not x.is_contiguous():
+        raise L.BigcnError("gemm_mode='bf16': data.x must be contiguous (row pitch = in_feats): pass x.contiguous()")
+    if x.shape[1] % 8:
+        raise L.BigcnError(f"gemm_mode='bf16': in_feats must be a multiple of 8 (16-byte rows for TMA), got "
+                           f"{x.shape[1]}: pad the features with zero columns (and the weights to match)")
+    if x.data_ptr() % 16:
+        raise L.BigcnError("gemm_mode='bf16': data.x must start on a 16-byte boundary: pass x.clone()")
+    return x
+
+
+def _as_x(x, gemm_mode=None):
+    """dense fp32 tensor | SparseX | torch sparse tensor -> (dense or None, SparseX or None); with
+    ``gemm_mode='bf16'`` the dense bf16 x as it is (bf16_x)"""
+    if gemm_mode == "bf16":
+        return bf16_x(x), None
     if isinstance(x, SparseX):
         return None, x
     if isinstance(x, torch.Tensor) and x.layout != torch.strided:
         return None, SparseX.from_torch_csr(x)
     return _f32(x), None
+
+
+def _x_for(x, gemm_mode):
+    """a dense x for one of the ops below: bf16 as it is in ``gemm_mode='bf16'``, fp32 otherwise"""
+    return bf16_x(x) if gemm_mode == "bf16" else _f32(x)
 
 
 def pick_gemm_mode(x, sample_rows=4096):
@@ -178,11 +207,31 @@ def pick_gemm_mode(x, sample_rows=4096):
     tma_ok = k % 4 == 0 and x.data_ptr() % 16 == 0       # TMA needs 16 B aligned rows; otherwise the exact FFMA scan
     cnt = torch.empty(m, dtype=torch.int32, device=x.device)
     check(lib().bigcn_dense_row_counts(_p(x), m, k, _p(cnt), _stream()), "dense_row_counts")
-    c = cnt.cpu().numpy()
-    cap = min(int(k), 48)
-    if float(c.mean()) <= cap / 2 and int(c.max()) <= 4 * cap:
+    if _rows_look_sparse(cnt, k):
         return "sparse"
     return "tf32x3" if tma_ok else "fp32"
+
+
+def _rows_look_sparse(cnt, k):
+    """the row-density threshold of pick_gemm_mode over per-row non-zero counts (one device -> host read)"""
+    c = cnt.cpu().numpy()
+    cap = min(int(k), 48)
+    return float(c.mean()) <= cap / 2 and int(c.max()) <= 4 * cap
+
+
+def bf16_features_dense(x, sample_rows=4096):
+    """``gemm_mode='bf16'``: whether a bf16 feature matrix has dense rows (PHEME's embeddings) rather than
+    bag-of-words rows -- the same probe and threshold as pick_gemm_mode, counted on the bf16 values
+    (bigcn_dense_row_counts_bf16).  Decides ``dense_roots='auto'`` in that mode."""
+    L.require_device()
+    x = bf16_x(x)
+    n, k = x.shape
+    m = min(int(n), int(sample_rows))
+    if m == 0:
+        return False
+    cnt = torch.empty(m, dtype=torch.int32, device=x.device)
+    check(lib().bigcn_dense_row_counts_bf16(_p(x), m, k, _p(cnt), _stream()), "dense_row_counts_bf16")
+    return not _rows_look_sparse(cnt, k)
 
 
 # ----------------------------------------------------------------------------- graph prep
@@ -238,9 +287,10 @@ def transpose_weight(w, k0, k, wt, col0):
 
 
 def xw(x, weights, gemm_mode="fp32"):
-    """y[N, 64*len(weights)] = x @ cat(weights).T with one pass over x (weights: [64,K] each)."""
+    """y[N, 64*len(weights)] = x @ cat(weights).T with one pass over x (weights: [64,K] each).  ``gemm_mode='bf16'``
+    takes a bf16 x as it is; y is fp32 in every mode."""
     L.require_device()
-    x = _f32(x)
+    x = _x_for(x, gemm_mode)
     _need_cuda(x, *weights)
     n, k = x.shape
     n_out = H * len(weights)
@@ -369,7 +419,7 @@ class GCNConvFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, edge_index, weight, bias, deg_by, gemm_mode):
         L.require_device()
-        x, weight, bias = _f32(x), _f32(weight), _f32(bias)
+        x, weight, bias = _x_for(x, gemm_mode), _f32(weight), _f32(bias)
         ei = _i64(edge_index)
         _need_cuda(x, ei, weight, bias)
         n, k = x.shape
@@ -499,7 +549,7 @@ class FeaturesFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, ei, bu_ei, batch, rootindex, opts, *params):
         L.require_device()
-        x, xs = _as_x(x)
+        x, xs = _as_x(x, opts["gemm_mode"])
         if xs is not None and opts["gemm_mode"] != "sparse":
             raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
         ei, bu_ei, batch, rootindex = _i64(ei), _i64(bu_ei), _i64(batch), _i64(rootindex)

@@ -26,7 +26,7 @@ from torch.library import custom_op
 from . import _lib as L
 from . import ops
 from ._lib import H, check, lib
-from .ops import _p, _stream, _f32, _i64
+from .ops import _p, _stream, _f32, _i64, _x_for
 
 T11 = Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]
 
@@ -61,13 +61,13 @@ def xw(x: Tensor, w: Tensor, mode: str) -> Tensor:
 
 @xw.register_fake
 def _(x, w, mode):
-    return x.new_empty(x.shape[0], H)
+    return x.new_empty(x.shape[0], H, dtype=torch.float32)   # fp32 whatever x is (bf16 in mode 'bf16')
 
 
 @custom_op("bigcn_b200::xw_wgrad", mutates_args=(), device_types="cuda")
 def xw_wgrad(x: Tensor, t: Tensor, mode: str) -> Tensor:
     L.require_device()
-    x, t = _f32(x), _f32(t)
+    x, t = _x_for(x, mode), _f32(t)
     n, k = x.shape
     m = L.GEMM_MODE["fp32" if mode == "sparse" else mode]
     dw = torch.empty(H, k, dtype=torch.float32, device=x.device)
@@ -79,7 +79,7 @@ def xw_wgrad(x: Tensor, t: Tensor, mode: str) -> Tensor:
 
 @xw_wgrad.register_fake
 def _(x, t, mode):
-    return x.new_empty(H, x.shape[1])
+    return x.new_empty(H, x.shape[1], dtype=torch.float32)
 
 
 def _xw_setup(ctx, inputs, output):

@@ -164,7 +164,7 @@ class FusedTrainer:
     def _plan(self, data, b_global, node_id_base, seed):
         """Everything one step needs besides the launches: argument structs, output buffers, workspace."""
         m = self.model
-        x, xs = _as_x(data.x)
+        x, xs = _as_x(data.x, m.TDrumorGCN.resolved_gemm_mode(data.x))
         ei, bu, batch, root = _i64(data.edge_index), _i64(data.BU_edge_index), _i64(data.batch), \
             _i64(data.rootindex)
         y = _i64(data.y)
@@ -280,7 +280,7 @@ class FusedTrainer:
         need = l.bigcn_batch_prepare_bytes(C.byref(p["dims"]))
         nxt = None
         if next_data is not None:
-            nx, nxs = _as_x(next_data.x)
+            nx, nxs = _as_x(next_data.x, self.model.TDrumorGCN.resolved_gemm_mode(next_data.x))
             nd, nbt, _ = _make_structs(nx, _i64(next_data.edge_index), _i64(next_data.BU_edge_index), _i64(next_data.batch),
                                        _i64(next_data.rootindex), (None,) * 8, p["c"], 0, nxs)
             need = max(need, l.bigcn_batch_prepare_bytes(C.byref(nd)))
@@ -507,7 +507,7 @@ def launches_per_step(n_nodes: int, n_dirs: int = 2, training: bool = True, gemm
         return (bits + 7) // 8
     prep = 1 + 2 + 3 * radix_passes(n_nodes) + 1 + 1   # count, scan x2, radix passes, deg, hub lists
     sparse = gemm_mode == "sparse"
-    xw = 1 + (n_dirs if gemm_mode == "tf32x3" else 0)     # [W hi/lo split per direction], X*W
+    xw = 1 + (n_dirs if gemm_mode in ("tf32x3", "bf16") else 0)     # [W hi/lo or bf16-term split per direction], X*W
     csc = 0
     if sparse:      # row scan x2 + compaction (or CSR ingest), radix passes over the column keys, finish, hub columns
         kbits = max(1, (in_feats - 1).bit_length())
@@ -519,7 +519,7 @@ def launches_per_step(n_nodes: int, n_dirs: int = 2, training: bool = True, gemm
     if sparse:
         dw = 1                                 # sweep over the column-sorted non-zeros
     else:
-        dw = 1 + (1 if gemm_mode in ("tf32x3", "mixed") else 0) + n_dirs   # [T hi/lo split], dW GEMM/scan, reduce x dirs
+        dw = 1 + (1 if gemm_mode in ("tf32x3", "mixed", "bf16") else 0) + n_dirs   # [T split], dW GEMM/scan, reduce x dirs
     # gscale+colsum, propT(g2), outer x2, [segsum | dw2b part], dw2b reduce + dense fallback,
     # bwdmix+colsum, propT, dW
     bwd = 2 + 1 + 2 + 1 + 2 + 2 + 1 + dw

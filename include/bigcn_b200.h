@@ -69,6 +69,12 @@ extern "C" {
 /* exact fp32 scan forward that also captures the non-zeros of x; the weight gradient is a sweep
  * over the column-sorted non-zeros (no second pass over x).  For bag-of-words inputs. */
 #define BIGCN_GEMM_SPARSE 4
+/* x is a dense BF16 matrix: every `const float* x` of a call made in this mode (bigcn_batch_t.x, bigcn_xw,
+ * bigcn_xw_wgrad, bigcn_gcnconv_forward / _backward) points at bf16 rows with a pitch of K elements; K must be a
+ * multiple of 8 and x 16 B aligned (TMA).  X*W and dW1 run on tcgen05 kind::f16 with the small operand (W forward,
+ * T backward) split into three bf16 terms (24 significant bits): fp32-class relative to the fp32 widening of x.
+ * Parameters, activations and gradients stay fp32.  Not for CSR input or the edge-weighted GCNConv (error). */
+#define BIGCN_GEMM_BF16 6
 
 /* direction bits */
 #define BIGCN_DIR_TD 1
@@ -87,7 +93,7 @@ typedef struct bigcn_dims {
 
 /* The five attributes forward(data) reads (BiGCN_Twitter.py:27,45-47,78). */
 typedef struct bigcn_batch {
-  const float* x;               /* [N,K]    data.x                       */
+  const float* x;               /* [N,K]    data.x (bf16 rows in BIGCN_GEMM_BF16) */
   const int64_t* edge_index;    /* [2,E_td] data.edge_index  [parent;child] */
   const int64_t* bu_edge_index; /* [2,E_bu] data.BU_edge_index [child;parent] */
   const int64_t* batch;         /* [N]      data.batch (sorted)          */
@@ -183,14 +189,16 @@ int bigcn_graph_prep(int32_t n_dirs, const int64_t* const* edge_index, const int
  * Replaces GCNConv.lin (cuBLAS SGEMM) at BiGCN_Twitter.py:42,92.
  * y[N, 64*n_w] = x[N,K] * [w0; w1]^T with w0, w1 the [64,K] lin.weight tensors (row pitch
  * ldw) of one or two directions (w1 = NULL for one), so TD and BU share ONE pass over x.
- * gemm_mode FP32: exact-fp32 streaming scan; TF32 / TF32X3: tcgen05 + TMA + TMEM GEMM.
+ * gemm_mode FP32: exact-fp32 streaming scan; TF32 / TF32X3: tcgen05 + TMA + TMEM GEMM; BF16: x holds bf16
+ * rows (pitch K), tcgen05 kind::f16 with the weights split into bf16 terms.
  * scratch: bigcn_xw_scratch_floats(K, n_w) floats.  ldy = row pitch of y. */
 size_t bigcn_xw_scratch_floats(int64_t K, int32_t n_w);
 int bigcn_xw(const float* x, int64_t N, int64_t K, const float* w0, const float* w1, int64_t ldw,
              float* y, int64_t ldy, int32_t gemm_mode, float* scratch, bigcn_stream_t stream);
 /* The autograd transpose of the above (dW1 = T1^T X, SURVEY.md appendix B):
  * dw_d[o, k] = sum_i t[i, 64*d + o] * x[i, k] for d < n_w; t is [N, 64*n_w] dense.
- * FP32: exact streaming scan; TF32: one tcgen05 pass; TF32X3 / MIXED: T split hi + lo. */
+ * FP32: exact streaming scan; TF32: one tcgen05 pass; TF32X3 / MIXED: T split hi + lo; BF16: x holds bf16 rows,
+ * kind::f16 with t split into bf16 terms. */
 size_t bigcn_xw_wgrad_scratch_floats(int64_t N, int64_t K, int32_t n_w);
 int bigcn_xw_wgrad(const float* x, int64_t N, int64_t K, const float* t, int32_t n_w, float* dw0,
                    float* dw1, int64_t ldw, int32_t gemm_mode, float* scratch, bigcn_stream_t stream);
@@ -273,7 +281,8 @@ int bigcn_dropout_mask(uint64_t seed, int32_t stream_id, int64_t node_id_base, i
 /* ---- GCNConv on its own -------------------------------------------------
  * conv(x, edge_index) as called at explain_PHEME.py:95,132.  w is [64,K]
  * (lin.weight), bias [64]; out [N,64].  Backward returns dw, db (x is an input of the
- * path and carries no gradient, SURVEY.md appendix B). */
+ * path and carries no gradient, SURVEY.md appendix B).  gemm_mode BIGCN_GEMM_BF16: x holds bf16 rows (pitch K)
+ * in both calls. */
 size_t bigcn_gcnconv_workspace_bytes(int64_t N, int64_t E, int64_t K);
 int bigcn_gcnconv_forward(const float* x, int64_t N, int64_t K, const int64_t* edge_index,
                           int64_t E, const float* w, const float* bias, int32_t deg_by,
@@ -406,6 +415,8 @@ int bigcn_adam_step(float* param, const float* grad, float* exp_avg, float* exp_
  * row pointer stops growing and BIGCN_FLAG_X_NOT_SPARSE is set in *flags: never an out-of-bounds
  * write, never a silent wrong answer. */
 int bigcn_dense_row_counts(const float* x, int64_t N, int64_t K, int32_t* cnt, bigcn_stream_t stream);
+/* The same count for a bf16 x [N,K] (row pitch K): the density probe of BIGCN_GEMM_BF16 (dense or bag-of-words rows). */
+int bigcn_dense_row_counts_bf16(const void* x, int64_t N, int64_t K, int32_t* cnt, bigcn_stream_t stream);
 int bigcn_dense_rows_to_csr(const float* x, int64_t N, int64_t K, const int32_t* incl_counts, int64_t base,
                             int32_t* ptr_out, int32_t* col, float* val, int64_t cap, int32_t* flags,
                             bigcn_stream_t stream);
