@@ -836,7 +836,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 101; }
+extern "C" int bigcn_version(void) { return 102; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
@@ -963,6 +963,29 @@ extern "C" int bigcn_features_backward(const bigcn_dims_t* dims, const bigcn_bat
   BIGCN_CHECK_ARG(batch && params && grad_feat && grads, "features_backward: NULL argument");
   return features_backward(dims, batch, params, opts, grad_feat, grads, workspace, workspace_bytes,
                            (cudaStream_t)stream);
+}
+
+// ---- gradient w.r.t. x of the feature path: dX = T1cat [W1_d0; W1_d1] (SURVEY.md appendix B) ----------------------
+extern "C" size_t bigcn_x_dgrad_scratch_floats(int64_t N, int64_t K, int32_t n_w) { return dx_tc_scratch_floats(N, K, n_w); }
+
+extern "C" int bigcn_x_dgrad(const float* t, int32_t n_w, const float* w0, const float* w1, int64_t ldw, int64_t N,
+                             int64_t K, float* dx, void* dx_bf16, float* scratch, bigcn_stream_t stream) {
+  const float* ws[2] = {w0, w1};
+  return dx_tc(t, n_w, ws, ldw, N, K, dx, dx_bf16, scratch, (cudaStream_t)stream);
+}
+
+extern "C" int bigcn_features_x_grad(const bigcn_dims_t* dims, const bigcn_params_t* params, const bigcn_opts_t* opts,
+                                     float* dx, void* dx_bf16, float* scratch, void* workspace, size_t workspace_bytes,
+                                     bigcn_stream_t stream) {
+  if (int rc = check_common(dims, opts, "features_x_grad")) return rc;
+  BIGCN_CHECK_ARG(params != nullptr, "features_x_grad: NULL params");
+  const FeatWs w = carve_features(dims, workspace, workspace_bytes);
+  BIGCN_CHECK_ARG(workspace != nullptr && workspace_bytes >= w.total, "features_x_grad: workspace too small");
+  const Dirs dirs = active_dirs(opts->dir_mask);
+  BIGCN_CHECK_ARG(dirs.n > 0, "features_x_grad: empty dir_mask");
+  // T1 of the active directions, side by side: written by bigcn_features_backward, read by nothing after it
+  const float* ws[2] = {dir_w1(params, dirs.id[0]), dirs.n == 2 ? dir_w1(params, dirs.id[1]) : nullptr};
+  return dx_tc(w.h2[0], dirs.n, ws, dims->K, dims->N, dims->K, dx, dx_bf16, scratch, (cudaStream_t)stream);
 }
 
 extern "C" size_t bigcn_gcnconv_workspace_bytes(int64_t N, int64_t E, int64_t K) {

@@ -955,4 +955,255 @@ static int dw_bf16(const void* x, int64_t N, int64_t K, const float* t, int n_ou
   return dw_reduce_launch(partial, nsplit, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
 }
 
+
+// =====================================================================================
+// Input gradient  dX[N, K] = T[N, 64 n_w] * Wcat[64 n_w, K],  Wcat = [W_0; W_1] the [64, K] conv1.lin weights
+// (SURVEY appendix B: dX = T1 W1, summed over the directions by the reduction itself).
+// D[M = 128 rows of T, N = 256 columns of dX] with a reduction depth of only 64 n_w: both operands are small (T is
+// 16 MB, W 2.5 MB at Twitter scale) and the [N, K] output dominates the bytes.  3xTF32, T_hi W_hi + T_hi W_lo +
+// T_lo W_hi: both operands are split beforehand (k_split_rows_hi_lo, k_split_wT_hi_lo), so the MMA loop has no
+// converter warps.  W is laid out transposed as [K][64 n_w] (the forward's w1T layout): the B operand is K-major with
+// a 256 / 512 B row pitch that TMA can address whatever K is; rows >= K and >= N are zero-filled by TMA and the
+// column tail is cut in the epilogue.  Persistent CTAs walk the (row tile, column tile) pairs; the accumulator is
+// double-buffered in TMEM (2 x 256 columns), so eight epilogue warps drain tile i while the MMAs of tile i + 1 run.
+//   warp 0 : TMA producer      warp 1 : MMA issuer      warp 2 : TMEM allocator      warps 4-11 : epilogue
+// Every output element is written once by one thread from one accumulator: deterministic, no atomics.
+constexpr int DX_BM = 128;
+constexpr int DX_BN = 256;
+constexpr int DX_A_BYTES = DX_BM * 128;                             // 16 KB: 128 rows x 32 fp32
+constexpr int DX_B_BYTES = DX_BN * 128;                             // 32 KB: 256 rows x 32 fp32
+constexpr int DX_STAGE_BYTES = 2 * DX_A_BYTES + 2 * DX_B_BYTES;     // [T_hi | T_lo | W_hi | W_lo] = 96 KB
+constexpr int DX_STAGES = 2;
+constexpr int DX_THREADS = 384;
+constexpr int DX_SMEM = DX_STAGES * DX_STAGE_BYTES + 1024;
+
+struct DxParams {
+  void* dx;          // [N][K] fp32 or bf16
+  int64_t N, K;
+  int num_kb;        // 64 n_w / 32
+  int col_tiles;     // ceil(K / 256)
+  int num_tiles;     // ceil(N / 128) * col_tiles
+  int vec;           // 1: dx rows can take 16 B stores (K a multiple of 16 B, dx 16 B aligned)
+};
+
+// one thread's 32 consecutive accumulator columns of one row -> dx (fp32, or bf16 rounded to nearest even once)
+template <typename OutT>
+__device__ __forceinline__ void dx_store32(const DxParams& p, int64_t row, int64_t col, const uint32_t (&r)[32]) {
+  if (row >= p.N || col >= p.K) return;
+  OutT* dst = reinterpret_cast<OutT*>(p.dx) + row * p.K + col;
+  if (p.vec && col + 32 <= p.K) {
+    if constexpr (sizeof(OutT) == 4) {
+      float4* d4 = reinterpret_cast<float4*>(dst);
+#pragma unroll
+      for (int j = 0; j < 8; ++j)
+        d4[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
+                            __uint_as_float(r[4 * j + 3]));
+    } else {
+      uint32_t h[16];
+#pragma unroll
+      for (int j = 0; j < 16; ++j) {
+        const __nv_bfloat162 b = __floats2bfloat162_rn(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1]));
+        h[j] = *reinterpret_cast<const uint32_t*>(&b);
+      }
+      uint4* d4 = reinterpret_cast<uint4*>(dst);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) d4[j] = make_uint4(h[4 * j], h[4 * j + 1], h[4 * j + 2], h[4 * j + 3]);
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      if (col + j < p.K) {
+        if constexpr (sizeof(OutT) == 4) dst[j] = __uint_as_float(r[j]);
+        else dst[j] = __float2bfloat16_rn(__uint_as_float(r[j]));
+      }
+    }
+  }
+}
+
+template <typename OutT>
+__global__ void __launch_bounds__(DX_THREADS, 1)
+k_dx_tc(const __grid_constant__ CUtensorMap map_t, const __grid_constant__ CUtensorMap map_tlo,
+        const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_wlo, const DxParams p) {
+  extern __shared__ __align__(1024) uint8_t tc_smem[];
+  __shared__ __align__(8) uint64_t bar_full[DX_STAGES];
+  __shared__ __align__(8) uint64_t bar_empty[DX_STAGES];
+  __shared__ __align__(8) uint64_t bar_tmem_full[2];
+  __shared__ __align__(8) uint64_t bar_tmem_empty[2];
+  __shared__ uint32_t tmem_base_s;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t smem0 = (smem_u32(tc_smem) + 1023u) & ~1023u;
+
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&map_t);
+    tma_prefetch_desc(&map_tlo);
+    tma_prefetch_desc(&map_w);
+    tma_prefetch_desc(&map_wlo);
+    for (int s = 0; s < DX_STAGES; ++s) {
+      mbar_init(smem_u32(&bar_full[s]), 1);
+      mbar_init(smem_u32(&bar_empty[s]), 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(smem_u32(&bar_tmem_full[a]), 1);
+      mbar_init(smem_u32(&bar_tmem_empty[a]), 8);   // the eight epilogue warps
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 2) {   // 512 TMEM columns: two 128 x 256 fp32 accumulators
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_base_s)));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = tmem_base_s;
+
+  if (warp == 0) {
+    if (lane == 0) {   // ===== TMA producer =====
+      int s = 0;
+      uint32_t ph = 0;
+      for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
+        const int m0 = (tile / p.col_tiles) * DX_BM;
+        const int c0 = (tile % p.col_tiles) * DX_BN;
+        for (int kb = 0; kb < p.num_kb; ++kb) {
+          mbar_wait(smem_u32(&bar_empty[s]), ph ^ 1);
+          const uint32_t full = smem_u32(&bar_full[s]);
+          const uint32_t sa = smem0 + s * DX_STAGE_BYTES;
+          mbar_expect_tx(full, (uint32_t)DX_STAGE_BYTES);
+          tma_load_2d(sa, &map_t, full, kb * 32, m0);
+          tma_load_2d(sa + DX_A_BYTES, &map_tlo, full, kb * 32, m0);
+          tma_load_2d(sa + 2 * DX_A_BYTES, &map_w, full, kb * 32, c0);
+          tma_load_2d(sa + 2 * DX_A_BYTES + DX_B_BYTES, &map_wlo, full, kb * 32, c0);
+          if (++s == DX_STAGES) { s = 0; ph ^= 1; }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {   // ===== MMA issuer =====
+      const uint32_t idesc = make_idesc_tf32(DX_BM, DX_BN);
+      int s = 0;
+      uint32_t ph = 0;
+      int it = 0;
+      for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+        const int a = it & 1;
+        mbar_wait(smem_u32(&bar_tmem_empty[a]), ((it >> 1) & 1) ^ 1);   // the epilogue has drained this accumulator
+        tc_fence_after();
+        const uint32_t d = tmem_base + (uint32_t)(a * DX_BN);
+        for (int kb = 0; kb < p.num_kb; ++kb) {
+          mbar_wait(smem_u32(&bar_full[s]), ph);
+          tc_fence_after();
+          const uint32_t sa = smem0 + s * DX_STAGE_BYTES;
+#pragma unroll
+          for (int k = 0; k < 32 / TC_UMMA_K; ++k) {
+            const uint32_t koff = k * TC_UMMA_K * 4;
+            const uint64_t dt = make_desc_k_sw128(sa + koff);
+            const uint64_t dtl = make_desc_k_sw128(sa + DX_A_BYTES + koff);
+            const uint64_t dw = make_desc_k_sw128(sa + 2 * DX_A_BYTES + koff);
+            const uint64_t dwl = make_desc_k_sw128(sa + 2 * DX_A_BYTES + DX_B_BYTES + koff);
+            tc_mma_tf32(d, dt, dw, idesc, (kb | k) ? 1u : 0u);
+            tc_mma_tf32(d, dt, dwl, idesc, 1u);
+            tc_mma_tf32(d, dtl, dw, idesc, 1u);
+          }
+          tc_commit(smem_u32(&bar_empty[s]));
+          if (kb == p.num_kb - 1) tc_commit(smem_u32(&bar_tmem_full[a]));
+          if (++s == DX_STAGES) { s = 0; ph ^= 1; }
+        }
+      }
+    }
+  } else if (warp >= 4) {   // ===== epilogue: warp w reads TMEM lanes 32 (w % 4).. and one half of the 256 columns
+    const int q = warp & 3, half = (warp - 4) >> 2;
+    int it = 0;
+    for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+      const int a = it & 1;
+      mbar_wait(smem_u32(&bar_tmem_full[a]), (it >> 1) & 1);
+      tc_fence_after();
+      const int64_t row = (int64_t)(tile / p.col_tiles) * DX_BM + q * 32 + lane;
+      const int64_t col = (int64_t)(tile % p.col_tiles) * DX_BN + half * 128;
+#pragma unroll 1
+      for (int c = 0; c < 128; c += 32) {
+        uint32_t r[32];
+        tc_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(a * DX_BN + half * 128 + c), r);
+        tc_wait_ld();
+        dx_store32<OutT>(p, row, col + c, r);
+      }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(smem_u32(&bar_tmem_empty[a]));
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base));
+  }
+}
+
+// Transposed hi / lo split of one direction's [64, K] weight into columns col0..col0+63 of [K][ldo]
+__global__ void k_split_wT_hi_lo(const float* __restrict__ w, int64_t ldw, int64_t K, int ldo, int col0,
+                                 float* __restrict__ hi, float* __restrict__ lo) {
+  const int64_t n = 64 * K;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t k = i >> 6, r = i & 63;
+    const float v = w[r * ldw + k];
+    const float h = __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
+    hi[k * ldo + col0 + r] = h;
+    lo[k * ldo + col0 + r] = __uint_as_float((__float_as_uint(v - h) + 0x1000u) & 0xFFFFE000u);
+  }
+}
+
+size_t dx_tc_scratch_floats(int64_t N, int64_t K, int n_w) {
+  return (size_t)2 * H * n_w * (size_t)((N > 0 ? N : 1) + (K > 0 ? K : 1));
+}
+
+// t: [N, 64 n_w] dense; w[d]: [64, K] (row pitch ldw) for d < n_w; exactly one of dx (fp32) / dx_bf16 is set, [N, K]
+// dense; scratch: dx_tc_scratch_floats(N, K, n_w) floats, 16 B aligned
+int dx_tc(const float* t, int n_w, const float* const* w, int64_t ldw, int64_t N, int64_t K, float* dx, void* dx_bf16,
+          float* scratch, cudaStream_t st) {
+  BIGCN_CHECK_ARG(encode_fn() != nullptr, "x_dgrad: cuTensorMapEncodeTiled is unavailable in this driver");
+  BIGCN_CHECK_ARG(n_w == 1 || n_w == 2, "x_dgrad: n_w must be 1 or 2");
+  BIGCN_CHECK_ARG((dx != nullptr) != (dx_bf16 != nullptr), "x_dgrad: pass exactly one of dx / dx_bf16");
+  BIGCN_CHECK_ARG(N >= 0 && K >= 0 && ldw >= K, "x_dgrad: bad sizes");
+  if (N == 0 || K == 0) return 0;
+  BIGCN_CHECK_ARG(t != nullptr && w[0] != nullptr && (n_w == 1 || w[1] != nullptr) && scratch != nullptr,
+                  "x_dgrad: NULL argument");
+  BIGCN_CHECK_ARG((reinterpret_cast<uintptr_t>(t) & 15) == 0 && (reinterpret_cast<uintptr_t>(scratch) & 15) == 0,
+                  "x_dgrad: t and scratch must be 16-byte aligned");
+  const int nk = H * n_w;
+  float* t_hi = scratch;
+  float* t_lo = t_hi + (size_t)N * nk;
+  float* w_hi = t_lo + (size_t)N * nk;
+  float* w_lo = w_hi + (size_t)K * nk;
+  k_split_rows_hi_lo<<<num_sms() * 4, 256, 0, st>>>(t, N * nk, t_hi, t_lo);
+  BIGCN_CHECK_LAUNCH("k_split_rows_hi_lo");
+  for (int d = 0; d < n_w; ++d) {
+    k_split_wT_hi_lo<<<num_sms() * 2, 256, 0, st>>>(w[d], ldw, K, nk, d * H, w_hi, w_lo);
+    BIGCN_CHECK_LAUNCH("k_split_wT_hi_lo");
+  }
+  CUtensorMap mt, mtl, mw, mwl;
+  if (int rc = make_map(&mt, t_hi, N, nk, nk, DX_BM)) return rc;
+  if (int rc = make_map(&mtl, t_lo, N, nk, nk, DX_BM)) return rc;
+  if (int rc = make_map(&mw, w_hi, K, nk, nk, DX_BN)) return rc;
+  if (int rc = make_map(&mwl, w_lo, K, nk, nk, DX_BN)) return rc;
+  const bool bf = dx_bf16 != nullptr;
+  DxParams p;
+  p.dx = bf ? dx_bf16 : static_cast<void*>(dx);
+  p.N = N; p.K = K;
+  p.num_kb = nk / 32;
+  p.col_tiles = (int)ceil_div(K, DX_BN);
+  p.num_tiles = (int)(ceil_div(N, DX_BM) * p.col_tiles);
+  BIGCN_CHECK_ARG(ceil_div(N, DX_BM) * p.col_tiles < (int64_t)1 << 31, "x_dgrad: too many tiles");
+  p.vec = (K % (bf ? 8 : 4) == 0) && (reinterpret_cast<uintptr_t>(p.dx) & 15) == 0;
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(k_dx_tc<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, DX_SMEM);
+    cudaFuncSetAttribute(k_dx_tc<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, DX_SMEM);
+    attr = true;
+  }
+  const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
+  if (bf) k_dx_tc<__nv_bfloat16><<<grid, DX_THREADS, DX_SMEM, st>>>(mt, mtl, mw, mwl, p);
+  else k_dx_tc<float><<<grid, DX_THREADS, DX_SMEM, st>>>(mt, mtl, mw, mwl, p);
+  BIGCN_CHECK_LAUNCH("k_dx_tc");
+  return 0;
+}
+
 }  // namespace bigcn

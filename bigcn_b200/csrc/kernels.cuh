@@ -32,6 +32,9 @@ int dw_tc(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, int
           int mode, cudaStream_t st);
 int dw_fp32(const float*, int64_t, int64_t, const float*, int64_t, int, float*, float*, int64_t, int64_t,
             float*, int64_t, int64_t, cudaStream_t);
+size_t dx_tc_scratch_floats(int64_t N, int64_t K, int n_w);
+int dx_tc(const float* t, int n_w, const float* const* w, int64_t ldw, int64_t N, int64_t K, float* dx, void* dx_bf16,
+          float* scratch, cudaStream_t st);
 
 struct PropDir { const int32_t* ptr; const int32_t* idx; const float* dis; const float* h; const float* bias; float* out; int64_t ldh, ldo; int32_t* lng; int64_t E; };
 struct PropArgs { PropDir d[2]; int64_t N; int32_t relu; int32_t cb; };

@@ -305,6 +305,28 @@ def xw(x, weights, gemm_mode="fp32"):
     return y
 
 
+def x_dgrad(t, weights, out_dtype=torch.float32):
+    """dx[N,K] = t @ cat(weights) with t [N, 64*len(weights)] and weights [64,K] each: the input gradient of ``xw``
+    (tcgen05 kind::tf32, 3xTF32: fp32-class).  ``out_dtype`` float32, or bfloat16 (rounded once to nearest even)."""
+    L.require_device()
+    t = _f32(t)
+    ws = [_f32(w) for w in weights]
+    _need_cuda(t, *ws)
+    n, k = t.shape[0], ws[0].shape[1]
+    if t.shape[1] != H * len(ws) or any(w.shape != (H, k) for w in ws):
+        raise L.BigcnError(f"x_dgrad: t must be [N,{H * len(ws)}] and every weight [64,{k}]")
+    if len(ws) == 2 and ws[0].stride(0) != ws[1].stride(0):
+        raise L.BigcnError("x_dgrad: the two weight matrices must share a row pitch")
+    if out_dtype not in (torch.float32, torch.bfloat16):
+        raise L.BigcnError(f"x_dgrad: out_dtype must be float32 or bfloat16, got {out_dtype}")
+    dx = torch.empty(n, k, dtype=out_dtype, device=t.device)
+    scr = torch.empty(lib().bigcn_x_dgrad_scratch_floats(n, k, len(ws)), dtype=torch.float32, device=t.device)
+    bf = out_dtype == torch.bfloat16
+    check(lib().bigcn_x_dgrad(_p(t), len(ws), _p(ws[0]), _p(ws[1]) if len(ws) == 2 else None, ws[0].stride(0), n, k,
+                              None if bf else _p(dx), _p(dx) if bf else None, _p(scr), _stream()), "x_dgrad")
+    return dx
+
+
 class XSparseProduct:
     """y = x @ cat(weights).T through the exact scan that also captures the non-zeros of x
     (``gemm_mode='sparse'`` on its own).  ``wgrad(t)`` returns the weight gradients from the
@@ -615,7 +637,20 @@ class FeaturesFunction(torch.autograd.Function):
         check(lib().bigcn_features_backward(C.byref(dims), C.byref(bt), C.byref(pr), C.byref(ctx.o), _p(g),
                                             C.byref(gs), _p(ws), ws.numel(), _stream()),
               "features_backward")
-        return (None, None, None, None, None, None) + grads
+        dx = None
+        if ctx.needs_input_grad[0] and x is not None:
+            # only conv1 carries a gradient to x: the root-extend reads the detached copy.copy (BiGCN_Twitter.py:28).
+            # dX = T1cat [W1_TD; W1_BU], T1cat left in the workspace by features_backward.  Same dtype as the x the
+            # forward read: bf16 in gemm_mode='bf16', fp32 otherwise (autograd casts it to a widened x's dtype)
+            n, k = x.shape
+            dx = torch.empty(n, k, dtype=x.dtype, device=x.device)
+            bf = x.dtype == torch.bfloat16
+            nscr = lib().bigcn_x_dgrad_scratch_floats(n, k, bin(ctx.o.dir_mask).count("1"))
+            scr = torch.empty(nscr, dtype=torch.float32, device=x.device)
+            check(lib().bigcn_features_x_grad(C.byref(dims), C.byref(pr), C.byref(ctx.o), None if bf else _p(dx),
+                                              _p(dx) if bf else None, _p(scr), _p(ws), ws.numel(), _stream()),
+                  "features_x_grad")
+        return (dx, None, None, None, None, None) + grads
 
 
 class HeadFunction(torch.autograd.Function):

@@ -6,7 +6,8 @@ is a thin call into libbigcn_b200.so on the current stream; outputs come from to
   graph_prep(edge_index, num_nodes, batch?, num_graphs, deg_by)
         -> (in_ptr, in_idx, out_ptr, out_idx, deg, dis, rowsum, node_ptr, flags, in_long, out_long)
         gcn_norm / add_remaining_self_loops structure [torch_geometric], BiGCN_Twitter.py:42,56,92,105
-  xw(x, w, mode) -> [N,64]            GCNConv.lin;  backward: xw_wgrad(x, t, mode) -> [64,K]
+  xw(x, w, mode) -> [N,64]            GCNConv.lin;  backward: xw_wgrad(x, t, mode) -> [64,K] and, when x wants a
+        gradient, xw_dgrad(t, w, mode) -> [N,K]
   propagate(h, in_ptr, in_idx, out_ptr, out_idx, dis, num_edges, in_long?, out_long?, bias?, relu) -> [N,64]
         MessagePassing.propagate + bias (+ relu); backward: the transposed CSR for dh, column sums for dbias
   readout(h2, h1, node_ptr, rootindex, batch) -> [B,128]   second root-extend + scatter_mean (:58-65);
@@ -82,15 +83,28 @@ def _(x, t, mode):
     return x.new_empty(H, x.shape[1], dtype=torch.float32)
 
 
+@custom_op("bigcn_b200::xw_dgrad", mutates_args=(), device_types="cuda")
+def xw_dgrad(g: Tensor, w: Tensor, mode: str) -> Tensor:
+    # the input gradient g @ w of xw: bf16 in mode 'bf16' (the dtype xw reads there), fp32 otherwise
+    return ops.x_dgrad(g, [w], torch.bfloat16 if mode == "bf16" else torch.float32)
+
+
+@xw_dgrad.register_fake
+def _(g, w, mode):
+    return g.new_empty(g.shape[0], w.shape[1], dtype=torch.bfloat16 if mode == "bf16" else torch.float32)
+
+
 def _xw_setup(ctx, inputs, output):
     x, w, mode = inputs
-    ctx.save_for_backward(x)
+    ctx.save_for_backward(x, w)
     ctx.mode = mode
 
 
 def _xw_backward(ctx, g):
-    (x,) = ctx.saved_tensors
-    return None, torch.ops.bigcn_b200.xw_wgrad(x, g.contiguous(), ctx.mode), None   # x is data on this path
+    x, w = ctx.saved_tensors
+    g = g.contiguous()
+    dx = torch.ops.bigcn_b200.xw_dgrad(g, w, ctx.mode) if ctx.needs_input_grad[0] else None
+    return dx, torch.ops.bigcn_b200.xw_wgrad(x, g, ctx.mode), None
 
 
 xw.register_autograd(_xw_backward, setup_context=_xw_setup)

@@ -202,6 +202,13 @@ int bigcn_xw(const float* x, int64_t N, int64_t K, const float* w0, const float*
 size_t bigcn_xw_wgrad_scratch_floats(int64_t N, int64_t K, int32_t n_w);
 int bigcn_xw_wgrad(const float* x, int64_t N, int64_t K, const float* t, int32_t n_w, float* dw0,
                    float* dw1, int64_t ldw, int32_t gemm_mode, float* scratch, bigcn_stream_t stream);
+/* The input gradient of the above, same kernel as bigcn_features_x_grad:
+ * dx[i, k] = sum_{d < n_w} sum_o t[i, 64*d + o] * w_d[o, k]; t is [N, 64*n_w] dense, w0 / w1 the [64,K] weights
+ * (row pitch ldw; w1 = NULL for one).  Exactly one of dx (fp32) / dx_bf16 (bf16) is non-NULL, [N,K] dense; any K >= 1.
+ * scratch: bigcn_x_dgrad_scratch_floats(N, K, n_w) floats, 16 B aligned. */
+size_t bigcn_x_dgrad_scratch_floats(int64_t N, int64_t K, int32_t n_w);
+int bigcn_x_dgrad(const float* t, int32_t n_w, const float* w0, const float* w1, int64_t ldw, int64_t N, int64_t K,
+                  float* dx, void* dx_bf16, float* scratch, bigcn_stream_t stream);
 /* The same product and gradient through the row-sparse view of x (BIGCN_GEMM_SPARSE, for
  * bag-of-words inputs: Process/getTwittergraph.py:16-24 densifies `index:count` pairs).
  * bigcn_xw_sparse: exact fp32 scan that also records the non-zeros of x, then CSR
@@ -349,6 +356,16 @@ int bigcn_features_backward(const bigcn_dims_t* dims, const bigcn_batch_t* batch
                             const bigcn_params_t* params, const bigcn_opts_t* opts,
                             const float* grad_feat, const bigcn_params_t* grads,
                             void* workspace, size_t workspace_bytes, bigcn_stream_t stream);
+/* Gradient w.r.t. data.x (dense x): the reference's conv1 reads x (BiGCN_Twitter.py:42) while its root-extend reads
+ * the detached copy.copy x1 (:28,45-50), so only conv1 carries one back: dX = sum over the directions of T1_d W1_d
+ * with T1_d = A-hat_d^T G1_d, the matrix whose transpose product is dW1.  Call after bigcn_features_backward with the
+ * same dims, params, opts and workspace (it reads T1 from there; dir_mask selects the directions).
+ * Exactly one of dx (fp32 [N,K]) and dx_bf16 (bf16 [N,K], each element rounded once to nearest even) is non-NULL.
+ * tcgen05 kind::tf32 in the 3xTF32 form (T_hi W_hi + T_hi W_lo + T_lo W_hi): fp32-class; deterministic (no atomics).
+ * scratch: bigcn_x_dgrad_scratch_floats(N, K, n_w) floats, 16 B aligned. */
+int bigcn_features_x_grad(const bigcn_dims_t* dims, const bigcn_params_t* params, const bigcn_opts_t* opts,
+                          float* dx, void* dx_bf16, float* scratch, void* workspace, size_t workspace_bytes,
+                          bigcn_stream_t stream);
 
 /* ---- head ---------------------------------------------------------------
  * Replaces fc + log_softmax (BiGCN_Twitter.py:129-130). */
