@@ -110,6 +110,11 @@ _SIGS = {
     "bigcn_x_dgrad_scratch_floats": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int32]),
     "bigcn_x_dgrad": (C.c_int, [c_ptr, C.c_int32, c_ptr, c_ptr, C.c_int64, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr,
                                 c_ptr]),
+    "bigcn_features_x_grad_csr": (C.c_int, [C.POINTER(Dims), C.POINTER(BatchPtrs), C.POINTER(Opts), c_ptr, C.c_int64,
+                                            c_ptr, C.c_size_t, c_ptr]),
+    "bigcn_x_dgrad_csr_scratch_floats": (C.c_size_t, [C.c_int64, C.c_int32]),
+    "bigcn_x_dgrad_csr": (C.c_int, [c_ptr, c_ptr, C.c_int64, C.c_int64, C.c_int64, c_ptr, C.c_int32, c_ptr, c_ptr,
+                                    C.c_int64, c_ptr, c_ptr, c_ptr]),
     "bigcn_head_forward": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr, c_ptr]),
     "bigcn_head_backward_scratch_floats": (C.c_size_t, [C.c_int64, C.c_int64]),
     "bigcn_head_backward": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr,

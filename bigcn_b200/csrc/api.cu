@@ -836,7 +836,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 102; }
+extern "C" int bigcn_version(void) { return 103; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
@@ -986,6 +986,45 @@ extern "C" int bigcn_features_x_grad(const bigcn_dims_t* dims, const bigcn_param
   // T1 of the active directions, side by side: written by bigcn_features_backward, read by nothing after it
   const float* ws[2] = {dir_w1(params, dirs.id[0]), dirs.n == 2 ? dir_w1(params, dirs.id[1]) : nullptr};
   return dx_tc(w.h2[0], dirs.n, ws, dims->K, dims->N, dims->K, dx, dx_bf16, scratch, (cudaStream_t)stream);
+}
+
+// ---- ... for a CSR x: the same gradient sampled at x's stored entries (an SDDMM) ----------------------------------
+extern "C" size_t bigcn_x_dgrad_csr_scratch_floats(int64_t K, int32_t n_w) { return (size_t)(K > 0 ? K : 0) * H * n_w; }
+
+extern "C" int bigcn_x_dgrad_csr(const int32_t* ptr, const int32_t* col, int64_t N, int64_t K, int64_t nnz,
+                                 const float* t, int32_t n_w, const float* w0, const float* w1, int64_t ldw, float* dval,
+                                 float* scratch, bigcn_stream_t stream) {
+  BIGCN_CHECK_ARG(N >= 0 && K > 0 && nnz >= 0, "x_dgrad_csr: bad dims");
+  BIGCN_CHECK_ARG((n_w == 1 && w1 == nullptr) || (n_w == 2 && w1 != nullptr), "x_dgrad_csr: n_w must be 1 (w1 NULL) or 2");
+  BIGCN_CHECK_ARG(ldw >= K, "x_dgrad_csr: ldw < K");
+  if (N == 0 && nnz == 0) return 0;
+  // col and t are read only for entries below nnz: an empty CSR may pass NULL for them
+  BIGCN_CHECK_ARG(w0 && scratch && (N == 0 || ptr) && (nnz == 0 || (dval && col && t)), "x_dgrad_csr: NULL argument");
+  BIGCN_CHECK_ARG(((reinterpret_cast<uintptr_t>(t) | reinterpret_cast<uintptr_t>(scratch)) & 15) == 0,
+                  "x_dgrad_csr: t and scratch must be 16 B aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int n_out = H * n_w;
+  TransposeJobs js{};
+  js.job[js.n++] = TransposeJob{w0, ldw, 0, K, scratch, n_out, 0};
+  if (n_w == 2) js.job[js.n++] = TransposeJob{w1, ldw, 0, K, scratch, n_out, H};
+  if (int rc = transpose_jobs_launch(js, st)) return rc;
+  return dx_csr(ptr, col, N, K, nnz, t, scratch, n_out, dval, st);
+}
+
+extern "C" int bigcn_features_x_grad_csr(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts,
+                                         float* dval, int64_t nnz, void* workspace, size_t workspace_bytes,
+                                         bigcn_stream_t stream) {
+  if (int rc = check_common(dims, opts, "features_x_grad_csr")) return rc;
+  BIGCN_CHECK_ARG(batch && batch->x == nullptr && batch->x_ptr && batch->x_col,
+                  "features_x_grad_csr: needs the CSR x the forward read (x NULL, x_ptr / x_col set)");
+  BIGCN_CHECK_ARG(opts->gemm_mode == BIGCN_GEMM_SPARSE, "features_x_grad_csr: a CSR x runs in gemm_mode SPARSE");
+  BIGCN_CHECK_ARG(nnz >= 0 && (nnz == 0 || dval), "features_x_grad_csr: bad dval / nnz");
+  const FeatWs w = carve_features(dims, workspace, workspace_bytes);
+  BIGCN_CHECK_ARG(workspace != nullptr && workspace_bytes >= w.total, "features_x_grad_csr: workspace too small");
+  const int n_out = active_dirs(opts->dir_mask).n == 2 ? 2 * H : H;
+  // T1cat [N][n_out]: written by bigcn_features_backward.  W1^T [K][n_out] in the same direction order: written by
+  // bigcn_features_forward (step 2, every gemm_mode SPARSE step), and by nothing after it
+  return dx_csr(batch->x_ptr, batch->x_col, dims->N, dims->K, nnz, w.h2[0], w.w1T, n_out, dval, (cudaStream_t)stream);
 }
 
 extern "C" size_t bigcn_gcnconv_workspace_bytes(int64_t N, int64_t E, int64_t K) {

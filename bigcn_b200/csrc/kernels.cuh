@@ -196,6 +196,9 @@ int xw_fp32_capture(const float*, int64_t, int64_t, const float*, int, float*, i
 int xw_csr(const XSparse& x, const float* wt, int n_out, float* y, int64_t ldy, cudaStream_t st, bool check_state = false);
 int x_capture(const float* x, int64_t N, int64_t K, const XSparse& xs, cudaStream_t st);
 int xw_ell(const XSparse& xs, const float* x, const float* wt, int n_out, float* y, int64_t ldy, cudaStream_t st);
+// dval[e] = t[i] . wt[col[e]] for every stored entry e = (i, col[e]) of the CSR (ptr, col); 0 for e in [ptr[N], nnz)
+int dx_csr(const int32_t* ptr, const int32_t* col, int64_t N, int64_t K, int64_t nnz, const float* t, const float* wt,
+           int n_out, float* dval, cudaStream_t st);
 
 // fork / join onto the library's side stream (independent short kernels run beside the main chain)
 struct SideStream {

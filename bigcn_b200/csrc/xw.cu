@@ -451,6 +451,105 @@ int xw_csr(const XSparse& xs, const float* wt, int n_out, float* y, int64_t ldy,
   return 0;
 }
 
+// The input gradient of k_xw_csr sampled at x's stored entries (an SDDMM): for entry e = (i, k) of the CSR,
+// dval[e] = sum_o t[i][o] * wt[k][o], o < NOUT -- the dense dX = T W at the entries the forward read.
+// Work units: a row's entries up to the next multiple of DXC_SEG (one unit per row), plus, for each multiple of
+// DXC_SEG inside [0, ptr[N]), the entries from there to the next multiple in the row that crosses it (found by
+// binary search): no unit holds more than DXC_SEG entries, so a row with all K columns spreads over many warps.
+// A warp keeps its row of t in registers, takes 32 entries at a time and forms each one's dot product as lane
+// partials (fixed FMA order) plus the xor butterfly of warp_sum; one store per 32 entries.  No atomics: every
+// value is the same fixed-order sum on every run.  A column outside [0, K) gets 0 (the forward skips it), and so
+// does every e in [ptr[N], nnz).
+constexpr int DXC_SEG = 256;
+constexpr int DXC_BLOCKS_PER_SM = 6;   // 40 registers, no spills (the default bound squeezes it to 32 and spills)
+template <int NOUT>
+__global__ void __launch_bounds__(256, DXC_BLOCKS_PER_SM)
+    k_dx_csr(const int32_t* __restrict__ ptr, const int32_t* __restrict__ col, int64_t N, int64_t K, int64_t nnz,
+             const float* __restrict__ t, const float* __restrict__ wt, float* __restrict__ dval) {
+  // N < 2^30, nnz < 2^31 - DXC_SEG (checked by dx_csr): row, entry and unit indices fit int32
+  constexpr int V = NOUT / 32;
+  const int lane = threadIdx.x & 31;
+  const int tid = blockIdx.x * blockDim.x + threadIdx.x, nthr = gridDim.x * blockDim.x;
+  const int n = (int)N;
+  const int tot = n > 0 ? (int)min((int64_t)ptr[n], nnz) : 0;   // entries that belong to a row
+  for (int e = max(tot, 0) + tid; e < nnz; e += nthr) dval[e] = 0.f;
+  const int nbound = tot > 0 ? (tot - 1) / DXC_SEG : 0;         // multiples of DXC_SEG strictly inside (0, tot)
+  for (int u = tid >> 5; u < n + nbound; u += nthr >> 5) {
+    int row, s, e;
+    if (u < n) {
+      row = u;
+      s = ptr[row];
+      e = min(ptr[row + 1], (s / DXC_SEG + 1) * DXC_SEG);
+    } else {
+      s = (u - n + 1) * DXC_SEG;
+      int lo = 0, hi = n - 1;   // the last row starting at or before s
+      while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (ptr[mid] <= s) lo = mid;
+        else hi = mid - 1;
+      }
+      row = lo;
+      if (ptr[row] == s) continue;   // the row starts on the boundary: its own unit covers these entries
+      e = min(ptr[row + 1], s + DXC_SEG);
+    }
+    e = min(e, tot);
+    if (s >= e) continue;
+    float tr[V];
+    {
+      const float* tp = t + (int64_t)row * NOUT + lane * V;
+      if (V == 4) {
+        const float4 v = *reinterpret_cast<const float4*>(tp);
+        tr[0] = v.x; tr[1] = v.y; tr[2] = v.z; tr[3] = v.w;
+      } else {
+        const float2 v = *reinterpret_cast<const float2*>(tp);
+        tr[0] = v.x; tr[1] = v.y;
+      }
+    }
+    for (int p0 = s; p0 < e; p0 += 32) {
+      const int p = p0 + lane;
+      const int k = p < e ? col[p] : -1;
+      const int m = min(32, e - p0);
+      float mine = 0.f;
+      for (int l0 = 0; l0 < m; l0 += 4) {
+        float part[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {   // four independent L2 reads of wt rows in flight
+          const int kk = __shfl_sync(FULL_MASK, k, (l0 + j) & 31);
+          part[j] = 0.f;
+          if (l0 + j < m && kk >= 0 && kk < K) {   // warp-uniform
+            const float* wr = wt + (int64_t)kk * NOUT + lane * V;
+            if (V == 4) {
+              const float4 w = *reinterpret_cast<const float4*>(wr);
+              part[j] = fmaf(tr[3], w.w, fmaf(tr[2], w.z, fmaf(tr[1], w.y, tr[0] * w.x)));
+            } else {
+              const float2 w = *reinterpret_cast<const float2*>(wr);
+              part[j] = fmaf(tr[1], w.y, tr[0] * w.x);
+            }
+          }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float v = warp_sum(part[j]);
+          if (lane == l0 + j) mine = v;
+        }
+      }
+      if (p < e) dval[p] = mine;
+    }
+  }
+}
+int dx_csr(const int32_t* ptr, const int32_t* col, int64_t N, int64_t K, int64_t nnz, const float* t, const float* wt,
+           int n_out, float* dval, cudaStream_t st) {
+  BIGCN_CHECK_ARG(N >= 0 && N < (1ll << 30) && nnz >= 0 && nnz < (1ll << 31) - DXC_SEG, "x_dgrad_csr: N or nnz too large");
+  if (N == 0 && nnz == 0) return 0;
+  int64_t blocks = ceil_div(N + nnz / DXC_SEG + 1, 8);
+  const int64_t cap = (int64_t)num_sms() * DXC_BLOCKS_PER_SM;   // all resident: one wave of the grid-stride loop
+  if (blocks > cap) blocks = cap;
+  if (n_out == 128) k_dx_csr<128><<<(int)blocks, 256, 0, st>>>(ptr, col, N, K, nnz, t, wt, dval);
+  else k_dx_csr<64><<<(int)blocks, 256, 0, st>>>(ptr, col, N, K, nnz, t, wt, dval);
+  BIGCN_CHECK_LAUNCH("k_dx_csr");
+  return 0;
+}
+
 // ------------------------------------------------------------ weight transposes
 // wt[k*ldwt + col0 + o] = w[o*ldw + k0 + k], o < 64  (32 x 64 tiles through smem)
 __global__ void k_transpose_w(const float* __restrict__ w, int64_t ldw, int64_t k0, int64_t K,

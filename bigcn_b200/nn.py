@@ -20,7 +20,7 @@ import ctypes as C
 import weakref
 
 from .ops import (FeaturesFunction, GCNConvFunction, GCNConvWeightedFunction, HeadFunction, raise_on_flags,
-                  capture_graph, pick_gemm_mode, bf16_features_dense, _as_x, _i64, _make_structs, _p, _stream)
+                  capture_graph, pick_gemm_mode, bf16_features_dense, x_val, _as_x, _i64, _make_structs, _p, _stream)
 
 H = L.H
 
@@ -138,7 +138,7 @@ class _RumorGCN(torch.nn.Module):
     def forward(self, data):
         none4 = (None,) * 4
         params = self._conv_params() + none4 if self._dir == L.DIR_TD else none4 + self._conv_params()
-        feat = FeaturesFunction.apply(data.x, data.edge_index, data.BU_edge_index, data.batch,
+        feat = FeaturesFunction.apply(data.x, x_val(data.x), data.edge_index, data.BU_edge_index, data.batch,
                                       data.rootindex, self._opts(self._dir, data.x), *params)
         return feat[:, 2 * H:] if self._dir == L.DIR_TD else feat[:, :2 * H]
 
@@ -193,7 +193,7 @@ class BiGCN(torch.nn.Module):
         opts = td._opts(L.DIR_TD | L.DIR_BU, data.x)
         flags = torch.zeros(1, dtype=torch.int32, device=data.x.device)
         opts["flags"] = flags
-        feat = FeaturesFunction.apply(data.x, data.edge_index, data.BU_edge_index, data.batch,
+        feat = FeaturesFunction.apply(data.x, x_val(data.x), data.edge_index, data.BU_edge_index, data.batch,
                                       data.rootindex, opts, *td._conv_params(),
                                       *self.BUrumorGCN._conv_params())
         out = HeadFunction.apply(feat, self.fc.weight, self.fc.bias)

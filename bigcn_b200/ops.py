@@ -327,6 +327,33 @@ def x_dgrad(t, weights, out_dtype=torch.float32):
     return dx
 
 
+def x_dgrad_csr(xs, t, weights):
+    """dval[e] = t[i] . cat(weights)[:, col[e]] for every stored entry e = (i, col[e]) of the SparseX ``xs``: the input
+    gradient of ``xs @ cat(weights).T`` sampled at x's pattern (the gradient of ``xs.val``; plain fp32 FMAs,
+    deterministic).  t [N, 64*len(weights)], weights [64,K] each.  Returns fp32 [xs.val.numel()]: an entry whose column
+    is outside [0, K), and every entry past ptr[N], gets 0."""
+    L.require_device()
+    t = _f32(t)
+    ws = [_f32(w) for w in weights]
+    _need_cuda(t, xs.ptr, xs.col, *ws)
+    n, k = xs.shape
+    if t.shape != (n, H * len(ws)) or any(w.shape != (H, k) for w in ws):
+        raise L.BigcnError(f"x_dgrad_csr: t must be [{n},{H * len(ws)}] and every weight [64,{k}]")
+    if len(ws) == 2 and ws[0].stride(0) != ws[1].stride(0):
+        raise L.BigcnError("x_dgrad_csr: the two weight matrices must share a row pitch")
+    if xs.ptr.dtype != torch.int32 or xs.col.dtype != torch.int32 or xs.ptr.numel() != n + 1:
+        raise L.BigcnError("x_dgrad_csr: ptr must be int32 [N+1] and col int32")
+    nnz = xs.val.numel()
+    if xs.col.numel() < nnz:
+        raise L.BigcnError(f"x_dgrad_csr: col holds {xs.col.numel()} entries, val {nnz}")
+    dval = torch.empty(nnz, dtype=torch.float32, device=t.device)
+    scr = torch.empty(lib().bigcn_x_dgrad_csr_scratch_floats(k, len(ws)), dtype=torch.float32, device=t.device)
+    check(lib().bigcn_x_dgrad_csr(_p(xs.ptr.contiguous()), _p(xs.col.contiguous()), n, k, nnz, _p(t), len(ws),
+                                  _p(ws[0]), _p(ws[1]) if len(ws) == 2 else None, ws[0].stride(0), _p(dval), _p(scr),
+                                  _stream()), "x_dgrad_csr")
+    return dval
+
+
 class XSparseProduct:
     """y = x @ cat(weights).T through the exact scan that also captures the non-zeros of x
     (``gemm_mode='sparse'`` on its own).  ``wgrad(t)`` returns the weight gradients from the
@@ -564,13 +591,32 @@ def _make_structs(x, ei, bu_ei, batch, rootindex, params, num_classes, node_id_b
     return dims, bt, pr
 
 
+def x_val(x):
+    """The autograd input that carries a SparseX's gradient (its ``val``), None for any other data.x:
+    FeaturesFunction takes it beside x, which autograd cannot see into."""
+    return x.val if isinstance(x, SparseX) else None
+
+
 class FeaturesFunction(torch.autograd.Function):
     """TDrumorGCN / BUrumorGCN forward for the directions in dir_mask -> feat [B,256]
-    laid out [BU mean | BU root | TD mean | TD root] (cat order of BiGCN_Twitter.py:128)."""
+    laid out [BU mean | BU root | TD mean | TD root] (cat order of BiGCN_Twitter.py:128).
+
+    Gradient w.r.t. data.x (conv1's input) when it requires one: a dense x gets dX = T1cat [W1_TD; W1_BU]; a sparse
+    x gets that gradient sampled at its stored entries -- ``val`` (= ``x_val(x)``, a SparseX's values) gets fp32 [nnz],
+    a torch sparse COO x a COO gradient on ``x.coalesce()``'s indices (the ``torch.sparse.mm`` convention), a
+    torch sparse CSR x a CSR gradient on its own ``crow_indices`` / ``col_indices`` (torch's ``csr @ dense``
+    returns a dense one instead: the masked form keeps the gradient as small as x)."""
 
     @staticmethod
-    def forward(ctx, x, ei, bu_ei, batch, rootindex, opts, *params):
+    def forward(ctx, x, val, ei, bu_ei, batch, rootindex, opts, *params):
         L.require_device()
+        ctx.x_layout = x.layout if isinstance(x, torch.Tensor) else None
+        if ctx.needs_input_grad[0] and x.layout == torch.sparse_coo:
+            x = x.coalesce()     # the CSR below keeps this order: its gradient values map onto these indices
+        if ctx.needs_input_grad[0] and x.layout in (torch.sparse_coo, torch.sparse_csr):
+            ctx.x_pattern = (x.indices(),) if x.layout == torch.sparse_coo else (x.crow_indices(), x.col_indices())
+        elif ctx.needs_input_grad[0] and x.layout != torch.strided:
+            raise L.BigcnError(f"a gradient w.r.t. a {x.layout} data.x is not produced: pass it as sparse COO or CSR")
         x, xs = _as_x(x, opts["gemm_mode"])
         if xs is not None and opts["gemm_mode"] != "sparse":
             raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
@@ -637,8 +683,20 @@ class FeaturesFunction(torch.autograd.Function):
         check(lib().bigcn_features_backward(C.byref(dims), C.byref(bt), C.byref(pr), C.byref(ctx.o), _p(g),
                                             C.byref(gs), _p(ws), ws.numel(), _stream()),
               "features_backward")
-        dx = None
-        if ctx.needs_input_grad[0] and x is not None:
+        dx = dval = None
+        if (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]) and xs is not None:
+            # the dense gradient below sampled at the stored entries of x, in CSR order; T1cat and W1^T come from ws
+            nnz = xs.val.numel()
+            g = torch.empty(nnz, dtype=torch.float32, device=xs.val.device)
+            check(lib().bigcn_features_x_grad_csr(C.byref(dims), C.byref(bt), C.byref(ctx.o), _p(g), nnz, _p(ws),
+                                                  ws.numel(), _stream()), "features_x_grad_csr")
+            if ctx.needs_input_grad[1]:
+                dval = g
+            elif ctx.x_layout == torch.sparse_coo:
+                dx = torch.sparse_coo_tensor(ctx.x_pattern[0], g, xs.shape, is_coalesced=True)
+            else:
+                dx = torch.sparse_csr_tensor(*ctx.x_pattern, g, xs.shape)
+        elif ctx.needs_input_grad[0] and x is not None:
             # only conv1 carries a gradient to x: the root-extend reads the detached copy.copy (BiGCN_Twitter.py:28).
             # dX = T1cat [W1_TD; W1_BU], T1cat left in the workspace by features_backward.  Same dtype as the x the
             # forward read: bf16 in gemm_mode='bf16', fp32 otherwise (autograd casts it to a widened x's dtype)
@@ -650,7 +708,7 @@ class FeaturesFunction(torch.autograd.Function):
             check(lib().bigcn_features_x_grad(C.byref(dims), C.byref(pr), C.byref(ctx.o), None if bf else _p(dx),
                                               _p(dx) if bf else None, _p(scr), _p(ws), ws.numel(), _stream()),
                   "features_x_grad")
-        return (dx, None, None, None, None, None) + grads
+        return (dx, dval, None, None, None, None, None) + grads
 
 
 class HeadFunction(torch.autograd.Function):

@@ -209,6 +209,18 @@ int bigcn_xw_wgrad(const float* x, int64_t N, int64_t K, const float* t, int32_t
 size_t bigcn_x_dgrad_scratch_floats(int64_t N, int64_t K, int32_t n_w);
 int bigcn_x_dgrad(const float* t, int32_t n_w, const float* w0, const float* w1, int64_t ldw, int64_t N, int64_t K,
                   float* dx, void* dx_bf16, float* scratch, bigcn_stream_t stream);
+/* The same input gradient for a CSR x (ptr [N+1], col [nnz], int32), sampled at x's stored entries (an SDDMM, the
+ * convention of torch.sparse.mm's gradient): for every entry e < ptr[N] of row i,
+ *   dval[e] = sum_{d < n_w} sum_o t[i, 64*d + o] * w_d[o, col[e]]
+ * in plain fp32 FMAs (no TF32), deterministic (no atomics).  Every stored entry gets its value: explicit zeros, and
+ * each duplicate (row, col) entry in full.  An entry whose column is outside [0, K) gets 0 (the forward skips it).
+ * nnz is the length of dval: the entries in [ptr[N], nnz) are set to 0 (a CSR handed over at capacity), and
+ * nothing at or past nnz is read or written.  t is [N, 64*n_w] dense, 16 B aligned; w0 / w1 as above.
+ * scratch (W transposed): bigcn_x_dgrad_csr_scratch_floats(K, n_w) floats, 16 B aligned. */
+size_t bigcn_x_dgrad_csr_scratch_floats(int64_t K, int32_t n_w);
+int bigcn_x_dgrad_csr(const int32_t* ptr, const int32_t* col, int64_t N, int64_t K, int64_t nnz, const float* t,
+                      int32_t n_w, const float* w0, const float* w1, int64_t ldw, float* dval, float* scratch,
+                      bigcn_stream_t stream);
 /* The same product and gradient through the row-sparse view of x (BIGCN_GEMM_SPARSE, for
  * bag-of-words inputs: Process/getTwittergraph.py:16-24 densifies `index:count` pairs).
  * bigcn_xw_sparse: exact fp32 scan that also records the non-zeros of x, then CSR
@@ -366,6 +378,14 @@ int bigcn_features_backward(const bigcn_dims_t* dims, const bigcn_batch_t* batch
 int bigcn_features_x_grad(const bigcn_dims_t* dims, const bigcn_params_t* params, const bigcn_opts_t* opts,
                           float* dx, void* dx_bf16, float* scratch, void* workspace, size_t workspace_bytes,
                           bigcn_stream_t stream);
+/* Gradient w.r.t. a CSR data.x (batch->x = NULL, x_ptr / x_col / x_val, gemm_mode BIGCN_GEMM_SPARSE): the dX above
+ * sampled at x's stored entries, dval[e] = (T1cat[i] . W1cat^T[col[e]]) for entry e of row i -- the gradient of
+ * x_val.  Same kernel and conventions as bigcn_x_dgrad_csr (nnz = the length of dval; [ptr[N], nnz) set to 0).
+ * Call after bigcn_features_backward with the same dims, batch, opts and workspace: it reads T1cat, and W1^T as
+ * bigcn_features_forward laid it out, from there (dir_mask selects the directions); no scratch. */
+int bigcn_features_x_grad_csr(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts,
+                              float* dval, int64_t nnz, void* workspace, size_t workspace_bytes,
+                              bigcn_stream_t stream);
 
 /* ---- head ---------------------------------------------------------------
  * Replaces fc + log_softmax (BiGCN_Twitter.py:129-130). */
