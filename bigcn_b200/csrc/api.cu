@@ -1163,7 +1163,8 @@ extern "C" size_t bigcn_xw_wgrad_scratch_floats(int64_t N, int64_t K, int32_t n_
 extern "C" int bigcn_xw_wgrad(const float* x, int64_t N, int64_t K, const float* t, int32_t n_w, float* dw0,
                               float* dw1, int64_t ldw, int32_t gemm_mode, float* scratch,
                               bigcn_stream_t stream) {
-  BIGCN_CHECK_ARG(x && t && dw0 && scratch && (n_w == 1 || (n_w == 2 && dw1)), "xw_wgrad: bad arguments");
+  // N = 0 writes zeros; x and t may then be NULL (an empty torch tensor has no storage)
+  BIGCN_CHECK_ARG((N == 0 || (x && t)) && dw0 && scratch && (n_w == 1 || (n_w == 2 && dw1)), "xw_wgrad: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
   const int n_out = H * n_w;
   float* partial = scratch;

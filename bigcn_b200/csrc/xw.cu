@@ -836,10 +836,12 @@ int dw_fp32(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, i
             float* partial, float* dw_a, int64_t ldw_a, int64_t k0_a, float* dw_b, int64_t ldw_b,
             int64_t k0_b, cudaStream_t st) {
   if (K == 0) return 0;
-  const DwPlan p = dw_plan(N, K, x);
-  if (N == 0) {
+  if (N == 0) {   // before dw_plan, whose chunk size is 0 rows here
     cudaMemsetAsync(partial, 0, (size_t)K * n_out * sizeof(float), st);
-  } else if (p.fast) {
+    return dw_reduce_launch(partial, 1, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
+  }
+  const DwPlan p = dw_plan(N, K, x);
+  if (p.fast) {
     dim3 grid((unsigned)ceil_div(K, DW_COLS), (unsigned)p.nchunk);
     static bool attr_set = false;
     if (!attr_set) {
@@ -859,8 +861,7 @@ int dw_fp32(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, i
     else k_dw_naive<64><<<(int)ceil_div(tot, 256), 256, 0, st>>>(x, N, K, t, ldt, partial);
     BIGCN_CHECK_LAUNCH("k_dw_naive");
   }
-  const int nchunk = N == 0 ? 1 : p.nchunk;
-  return dw_reduce_launch(partial, nchunk, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
+  return dw_reduce_launch(partial, p.nchunk, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);
 }
 
 int dw_reduce_launch(const float* partial, int nchunk, int64_t K, int n_out, float* dw_a, int64_t ldw_a,

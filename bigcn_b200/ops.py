@@ -457,7 +457,7 @@ def raise_on_flags(flags: torch.Tensor):
         msgs.append("sparse data.x has a column index outside [0, in_feats)")
     if v & L.FLAG_X_NOT_SPARSE:
         msgs.append("gemm_mode='sparse' needs at most N*min(K,48) non-zeros in data.x (the conv1 weight "
-                    "gradient of this batch is NaN): use 'mixed' / 'tf32x3' / 'fp32' for dense features")
+                    "gradient of this batch is NaN): use 'tf32x3' / 'fp32' for dense features")
     raise IndexError("bigcn_b200: invalid graph input: " + "; ".join(msgs))
 
 

@@ -64,7 +64,9 @@ extern "C" {
 #define BIGCN_GEMM_TF32 1
 #define BIGCN_GEMM_TF32X3 2
 #define BIGCN_GEMM_TF32X2 5
-/* exact fp32 scan for X*W (forward), tcgen05 hi/lo-split GEMM for the weight gradient */
+/* exact fp32 scan for X*W (forward), tcgen05 hi/lo-split GEMM for the weight gradient.  The weight gradient is the
+ * TF32X2 product (T split, x as it is): like TF32X2 it is exact to ~2^-22 only when x is representable in TF32
+ * (bag-of-words counts are); on dense features it is 1e-4-class, so use TF32X3 or FP32 there. */
 #define BIGCN_GEMM_MIXED 3
 /* exact fp32 scan forward that also captures the non-zeros of x; the weight gradient is a sweep
  * over the column-sorted non-zeros (no second pass over x).  For bag-of-words inputs. */
@@ -197,8 +199,9 @@ int bigcn_xw(const float* x, int64_t N, int64_t K, const float* w0, const float*
              float* y, int64_t ldy, int32_t gemm_mode, float* scratch, bigcn_stream_t stream);
 /* The autograd transpose of the above (dW1 = T1^T X, SURVEY.md appendix B):
  * dw_d[o, k] = sum_i t[i, 64*d + o] * x[i, k] for d < n_w; t is [N, 64*n_w] dense.
- * FP32: exact streaming scan; TF32: one tcgen05 pass; TF32X3 / MIXED: T split hi + lo; BF16: x holds bf16 rows,
- * kind::f16 with t split into bf16 terms. */
+ * FP32: exact streaming scan; TF32: one tcgen05 pass; TF32X2 / MIXED: T split hi + lo (fp32-class only when x is
+ * TF32-representable); TF32X3: T and x split; BF16: x holds bf16 rows, kind::f16 with t split into bf16 terms.
+ * N = 0 writes zeros (x and t may then be NULL). */
 size_t bigcn_xw_wgrad_scratch_floats(int64_t N, int64_t K, int32_t n_w);
 int bigcn_xw_wgrad(const float* x, int64_t N, int64_t K, const float* t, int32_t n_w, float* dw0,
                    float* dw1, int64_t ldw, int32_t gemm_mode, float* scratch, bigcn_stream_t stream);
