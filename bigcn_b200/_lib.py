@@ -143,6 +143,8 @@ _SIGS = {
     "bigcn_eval_counts": (C.c_int, [c_ptr, c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr]),
     "bigcn_nll_loss": (C.c_int, [c_ptr, c_ptr, C.c_int64, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr]),
     "bigcn_assemble_batch": (C.c_int, [c_ptr] * 14 + [C.c_int64, C.c_int64, C.c_int64, C.c_uint64] + [c_ptr] * 9),
+    "bigcn_assemble_batch_dense": (C.c_int, [c_ptr] * 10 + [C.c_int64, C.c_int64, C.c_int64, C.c_uint64] + [c_ptr] * 6
+                                   + [C.c_int64, C.c_int32, c_ptr, c_ptr]),
     "bigcn_dp_slice": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "bigcn_dp_reduce_adam": (C.c_int, [C.POINTER(c_ptr), C.POINTER(c_ptr), C.c_int32, C.c_int32, c_ptr, c_ptr,
                                        C.c_int64, c_ptr, c_ptr, C.c_int32, C.c_double, C.c_double, C.c_double,

@@ -836,7 +836,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 103; }
+extern "C" int bigcn_version(void) { return 104; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;

@@ -6,10 +6,14 @@
 //     (dataset.py:68-90; random.sample -> the k smallest of per-position Philox keys);
 //   * collate: concatenate x, offset edge_index / BU_edge_index / rootindex by the cumulative
 //     node count, batch[i] = tree of node i, y.
-// The packed dataset keeps x as CSR (the `index:count` pairs getTwittergraph.py:16-24 reads,
-// never densified), so the assembled batch feeds the BIGCN_GEMM_SPARSE path directly.
+// The packed dataset keeps x either as CSR (the `index:count` pairs getTwittergraph.py:16-24 reads,
+// never densified), so the assembled batch feeds the BIGCN_GEMM_SPARSE path directly, or as dense
+// fp32 / bf16 rows (PHEME's sentence embeddings), gathered by k_asm_dense_rows into a dense [n, K] x
+// for the tensor-core modes.
 // Offsets per tree are computed by the caller on the host from the (host-known) tree sizes:
 // nothing here synchronises.
+#include <algorithm>
+
 #include "kernels.cuh"
 
 namespace bigcn {
@@ -50,6 +54,14 @@ __global__ void __launch_bounds__(256) k_asm_nodes(AsmArgs a) {
   const int64_t t = a.tree_id[b];
   const int64_t n0 = a.node_ptr[t], n = a.node_ptr[t + 1] - n0;
   const int64_t off = a.node_off[b];
+  if (a.x_ptr == nullptr) {   // dense features: k_asm_dense_rows copies the rows
+    for (int64_t i = threadIdx.x; i < n; i += blockDim.x) a.batch[off + i] = b;
+    if (threadIdx.x == 0) {
+      a.rootindex[b] = off + a.root_local[t];
+      a.y[b] = a.y_all[t];
+    }
+    return;
+  }
   const int64_t z0 = a.x_ptr[n0], nz = a.x_ptr[n0 + n] - z0;
   const int64_t zoff = a.nnz_off[b];
   for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
@@ -169,6 +181,93 @@ __global__ void __launch_bounds__(128) k_asm_edges(AsmArgs a) {
   }
 }
 
+// Dense feature rows.  Tree b's rows [node_ptr[tree_id[b]], +n_b) of x_all go to rows [node_off[b], +n_b) of ox,
+// every row K * elem_bytes bytes; the batch's x is the concatenation of B byte ranges.
+//   * Work split: the batch's units, in chunks of DR_THREADS * DR_UNROLL, are dealt out in contiguous runs to a grid
+//     sized to the machine -- not a CTA per tree, since a PHEME batch mixes single-node trees with 300-node ones, and
+//     one such tree is 118 MB in bf16 at K = 196,608.
+//   * Offsets: tree_id / node_off usually sit in pinned host memory, a PCIe round trip per read.  Each CTA stages the
+//     (source - destination) row delta of the trees its run touches into shared memory once, read by parallel threads;
+//     a row's tree comes from the batch vector k_asm_nodes has just written to device memory.  No device scratch
+//     array is needed, and no per-chunk search through host memory.  When node_off is pinned host memory, the host
+//     reads the row count at launch: the grid is sized to the chunks (a 24-tree PHEME batch needs ~45 CTAs, not 4 per
+//     SM, each of which would otherwise wait on the same PCIe read before it knows it has nothing to do).
+//   * Units: 16 bytes (LDG.128 / STG.128) when the row bytes and both pointers allow it, else 4 or 2; integers
+//     throughout, so every bit pattern (NaN payloads, -0.0) is copied as it is.  DR_UNROLL loads in flight per thread.
+//   * Unit indices are 64-bit; the row / column split of a unit uses a 32-bit multiply-shift division by the row's
+//     unit count on offsets below 2^31 (row_units < 2^30, so row remainder + chunk stays below that).
+constexpr int DR_THREADS = 256, DR_UNROLL = 8, DR_TREES = 512;
+
+struct DenseRowArgs {
+  const int64_t* node_ptr;
+  const int64_t* tree_id;
+  const int64_t* node_off;
+  const int64_t* batch;    // [N] tree of each batch row, written by k_asm_nodes
+  const void* x;           // [N_all, K]
+  void* ox;                // [N, K]
+  int64_t B;
+  int64_t n;               // rows of the batch (node_off[B]) when the host could read it, else -1
+  uint32_t row_units;      // units per row
+  uint32_t mul, shift;     // v / row_units == (umulhi(v, mul) + v) >> shift for every 32-bit v
+};
+
+__device__ __forceinline__ uint32_t dr_div(const DenseRowArgs& a, uint32_t v) {
+  return (uint32_t)(((uint64_t)__umulhi(v, a.mul) + v) >> a.shift);
+}
+
+template <typename U>
+__global__ void __launch_bounds__(DR_THREADS) k_asm_dense_rows(DenseRowArgs a) {
+  __shared__ int64_t s_delta[DR_TREES];
+  __shared__ int64_t s_n, s_row0, s_row1;
+  const U* __restrict__ src = static_cast<const U*>(a.x);
+  U* __restrict__ dst = static_cast<U*>(a.ox);
+  const int64_t ru = a.row_units;
+  if (threadIdx.x == 0) s_n = a.n >= 0 ? a.n : a.node_off[a.B];
+  __syncthreads();
+  constexpr int64_t CH = (int64_t)DR_THREADS * DR_UNROLL;
+  const int64_t total = s_n * ru;
+  const int64_t per = ((total + CH - 1) / CH + gridDim.x - 1) / gridDim.x;     // chunks per CTA
+  const int64_t lo = min(total, (int64_t)blockIdx.x * per * CH), hi = min(total, lo + per * CH);
+  if (lo >= hi) return;
+  const int64_t b_lo = a.batch[lo / ru], b_hi = a.batch[(hi - 1) / ru] + 1;
+  for (int64_t b0 = b_lo; b0 < b_hi; b0 += DR_TREES) {
+    const int nb = (int)min((int64_t)DR_TREES, b_hi - b0);
+    __syncthreads();   // the previous round is done with s_delta / s_row*
+    for (int j = threadIdx.x; j < nb; j += DR_THREADS) {
+      const int64_t off = a.node_off[b0 + j];
+      s_delta[j] = a.node_ptr[a.tree_id[b0 + j]] - off;
+      if (j == 0) s_row0 = off;
+    }
+    if (threadIdx.x == 0) s_row1 = a.node_off[b0 + nb];
+    __syncthreads();
+    const int64_t u0 = max(lo, s_row0 * ru), u1 = min(hi, s_row1 * ru);
+    if (u0 >= u1) continue;
+    int64_t row = u0 / ru;
+    uint32_t rem = (uint32_t)(u0 - row * ru);      // unit u0 + c sits at (row, rem + c) with rem + c < 2^31
+    for (int64_t u = u0; u < u1; u += CH) {
+      U v[DR_UNROLL];
+#pragma unroll
+      for (int i = 0; i < DR_UNROLL; ++i) {
+        const uint32_t c = (uint32_t)(i * DR_THREADS) + threadIdx.x;
+        if (u + c < u1) {
+          const uint32_t q = dr_div(a, rem + c);
+          const int64_t r = row + q;
+          const int64_t j = __ldg(a.batch + r) - b0;
+          v[i] = __ldg(src + (r + s_delta[j]) * ru + (rem + c - q * a.row_units));
+        }
+      }
+#pragma unroll
+      for (int i = 0; i < DR_UNROLL; ++i) {
+        const uint32_t c = (uint32_t)(i * DR_THREADS) + threadIdx.x;
+        if (u + c < u1) dst[u + c] = v[i];
+      }
+      const uint32_t q = dr_div(a, rem + (uint32_t)CH);
+      row += q;
+      rem = rem + (uint32_t)CH - q * a.row_units;
+    }
+  }
+}
+
 }  // namespace bigcn
 
 using namespace bigcn;
@@ -197,6 +296,67 @@ extern "C" int bigcn_assemble_batch(const int64_t* node_ptr, const int64_t* edge
   cudaStream_t st = (cudaStream_t)stream;
   k_asm_nodes<<<(unsigned)B, 256, 0, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_asm_nodes");
+  k_asm_edges<<<(unsigned)(2 * B), 128, 0, st>>>(a);
+  BIGCN_CHECK_LAUNCH("k_asm_edges");
+  return 0;
+}
+
+extern "C" int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                                          const int32_t* edge_dst, const int32_t* root_local, const int64_t* y_all,
+                                          const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                                          const int64_t* bu_off, int64_t B, int64_t E_td, int64_t E_bu, uint64_t seed,
+                                          int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch,
+                                          int64_t* rootindex, int64_t* y, const void* x_all, int64_t K,
+                                          int32_t elem_bytes, void* ox, bigcn_stream_t stream) {
+  BIGCN_CHECK_ARG(B >= 0 && E_td >= 0 && E_bu >= 0, "assemble_batch_dense: bad sizes");
+  BIGCN_CHECK_ARG(elem_bytes == 2 || elem_bytes == 4,
+                  "assemble_batch_dense: elem_bytes must be 2 (bf16) or 4 (fp32), got %d", (int)elem_bytes);
+  BIGCN_CHECK_ARG(K >= 1 && K * elem_bytes < (1ll << 30),
+                  "assemble_batch_dense: K = %lld (rows of 1 .. 2^30 - 1 bytes)", (long long)K);
+  if (B == 0) return 0;
+  BIGCN_CHECK_ARG(node_ptr && edge_ptr && root_local && y_all && tree_id && node_off && td_off && bu_off && batch &&
+                      rootindex && y && x_all && ox,
+                  "assemble_batch_dense: NULL argument");
+  BIGCN_CHECK_ARG(((uintptr_t)x_all | (uintptr_t)ox) % (uintptr_t)elem_bytes == 0,
+                  "assemble_batch_dense: x_all and ox must be aligned to elem_bytes (%d)", (int)elem_bytes);
+  AsmArgs a{};
+  a.node_ptr = node_ptr; a.edge_ptr = edge_ptr; a.edge_src = edge_src; a.edge_dst = edge_dst;
+  a.root_local = root_local; a.y_all = y_all;
+  a.tree_id = tree_id; a.node_off = node_off; a.td_off = td_off; a.bu_off = bu_off;
+  a.B = B; a.E_td = E_td; a.E_bu = E_bu;
+  a.k0 = (uint32_t)(seed & 0xffffffffull); a.k1 = (uint32_t)(seed >> 32);
+  a.edge_index = edge_index; a.bu_edge_index = bu_edge_index; a.batch = batch; a.rootindex = rootindex; a.y = y;
+  // the largest unit (16, 4 or 2 bytes) that divides the row bytes and both base addresses
+  const uint64_t row_bytes = (uint64_t)K * (uint64_t)elem_bytes;
+  const uint64_t align = row_bytes | (uint64_t)(uintptr_t)x_all | (uint64_t)(uintptr_t)ox;
+  const int unit = align % 16 == 0 ? 16 : align % 4 == 0 ? 4 : 2;
+  DenseRowArgs d{};
+  d.node_ptr = node_ptr; d.tree_id = tree_id; d.node_off = node_off; d.batch = batch;
+  d.x = x_all; d.ox = ox; d.B = B;
+  d.row_units = (uint32_t)(row_bytes / unit);
+  uint32_t l = 0;
+  while ((1ull << l) < d.row_units) ++l;
+  d.shift = l;
+  d.mul = (uint32_t)((((1ull << l) - d.row_units) << 32) / d.row_units + 1);
+  cudaStream_t st = (cudaStream_t)stream;
+  k_asm_nodes<<<(unsigned)B, 256, 0, st>>>(a);
+  BIGCN_CHECK_LAUNCH("k_asm_nodes");
+  // the caller wrote node_off before this call; when it is pinned host memory its last entry is readable here
+  d.n = -1;
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, node_off) == cudaSuccess && pa.type == cudaMemoryTypeHost && pa.hostPointer)
+    d.n = static_cast<const int64_t*>(pa.hostPointer)[B];
+  else
+    (void)cudaGetLastError();   // device memory, or a pointer CUDA does not know: the kernel reads node_off[B]
+  int64_t grid64 = 4ll * num_sms();
+  if (d.n >= 0) grid64 = std::min(grid64, (d.n * (int64_t)d.row_units + DR_THREADS * DR_UNROLL - 1) / (DR_THREADS * DR_UNROLL));
+  const unsigned grid = (unsigned)grid64;
+  if (grid > 0) {
+    if (unit == 16) k_asm_dense_rows<uint4><<<grid, DR_THREADS, 0, st>>>(d);
+    else if (unit == 4) k_asm_dense_rows<uint32_t><<<grid, DR_THREADS, 0, st>>>(d);
+    else k_asm_dense_rows<uint16_t><<<grid, DR_THREADS, 0, st>>>(d);
+    BIGCN_CHECK_LAUNCH("k_asm_dense_rows");
+  }
   k_asm_edges<<<(unsigned)(2 * B), 128, 0, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_asm_edges");
   return 0;

@@ -4,8 +4,10 @@ Stands in for ``BiGraphDataset`` (/root/reference/Process/dataset.py:45-99: one 
 loaded per epoch, DropEdge per direction) plus PyG's ``DataLoader`` collate
 (/root/reference/model/Twitter/BiGCN_Twitter.py:162-169) when the whole dataset fits in HBM --
 at ~14 non-zeros per node even the 1 M-tree synthetic scale-out config does.  Trees are packed
-once (features as CSR, never densified); ``batch(ids)`` builds the batch on the device with one
-call into libbigcn_b200.so and hands ``forward(data)`` a sparse ``data.x``.
+once, with the features in one of two forms: CSR (bag-of-words rows, never densified; ``data.x`` is a
+SparseX for ``gemm_mode='sparse'``) or dense fp32 / bf16 rows (PHEME's sentence embeddings; ``data.x``
+is a dense tensor for the tensor-core modes).  ``batch(ids)`` builds the batch on the device with one
+call into libbigcn_b200.so.
 """
 from __future__ import annotations
 
@@ -15,22 +17,46 @@ import torch
 from . import _lib as L
 from ._lib import check, lib
 from .data import Batch
-from .ops import SparseX, _p, _stream
+from .ops import SparseX, _p, _stream, check_bf16_width
+
+
+def _dense_storage(x, n, k):
+    """dense feature rows kept as they are: [n, k], fp32 or bf16, contiguous, on a CUDA device"""
+    if not isinstance(x, torch.Tensor) or x.layout != torch.strided or x.dtype not in (torch.float32, torch.bfloat16):
+        raise L.BigcnError(f"DeviceForest: dense features must be a torch.float32 or torch.bfloat16 tensor, got "
+                           f"{getattr(x, 'dtype', type(x))}")
+    if tuple(x.shape) != (n, k):
+        raise L.BigcnError(f"DeviceForest: dense features must be [{n}, {k}] (all nodes x in_feats), got {tuple(x.shape)}")
+    if x.dtype == torch.bfloat16:
+        check_bf16_width(k)
+    if not x.is_cuda:
+        raise L.BigcnError("DeviceForest: dense features must be on the CUDA device")
+    return x.contiguous()
 
 
 class DeviceForest:
-    def __init__(self, node_ptr, edge_ptr, edge_src, edge_dst, x_ptr, x_col, x_val, root_local, y, in_feats, device):
+    def __init__(self, node_ptr, edge_ptr, edge_src, edge_dst, x_ptr, x_col, x_val, root_local, y, in_feats, device,
+                 x=None):
+        """Trees packed back to back: node_ptr / edge_ptr [T+1], the local edge lists edge_src / edge_dst
+        ([parent; child]), root_local and y per tree, and the features of all nodes, either as CSR (x_ptr [N_all+1],
+        x_col, x_val) or -- ``x`` given, the CSR arguments None -- as dense rows [N_all, in_feats] of torch.float32
+        or torch.bfloat16 on the device, which ``batch()`` gathers into a dense ``data.x`` of the same dtype."""
         # host copies of the (small) size arrays: batch offsets are computed without touching the device
         self.h_node_ptr = np.asarray(node_ptr, np.int64)
         self.h_edge_ptr = np.asarray(edge_ptr, np.int64)
-        self.h_x_ptr_at_tree = np.asarray(x_ptr, np.int64)[self.h_node_ptr]   # nnz offset of each tree's first node
         self.in_feats = int(in_feats)
         self.device = torch.device(device)
         dev = self.device
         t = lambda a, dt: torch.as_tensor(np.ascontiguousarray(a), dtype=dt).to(dev)  # noqa: E731
         self.node_ptr, self.edge_ptr = t(node_ptr, torch.int64), t(edge_ptr, torch.int64)
         self.edge_src, self.edge_dst = t(edge_src, torch.int32), t(edge_dst, torch.int32)
-        self.x_ptr, self.x_col, self.x_val = t(x_ptr, torch.int64), t(x_col, torch.int32), t(x_val, torch.float32)
+        if x is None:
+            self.h_x_ptr_at_tree = np.asarray(x_ptr, np.int64)[self.h_node_ptr]   # nnz offset of each tree's first node
+            self.x_ptr, self.x_col, self.x_val = t(x_ptr, torch.int64), t(x_col, torch.int32), t(x_val, torch.float32)
+            self.x = None
+        else:
+            self.x_ptr = self.x_col = self.x_val = None
+            self.x = _dense_storage(x, int(self.h_node_ptr[-1]), self.in_feats)
         self.root_local, self.y = t(root_local, torch.int32), t(y, torch.int64)
         self.num_trees = len(self.h_node_ptr) - 1
         self._stage, self._turn = None, 0
@@ -38,23 +64,29 @@ class DeviceForest:
 
     def _cache_ptrs(self):
         # the dataset arrays never move: their addresses are looked up once, not on every batch
-        for k in ("node_ptr", "edge_ptr", "edge_src", "edge_dst", "x_ptr", "x_col", "x_val", "root_local", "y"):
+        for k in ("node_ptr", "edge_ptr", "edge_src", "edge_dst", "x_ptr", "x_col", "x_val", "x", "root_local", "y"):
             setattr(self, "_p_" + k, _p(getattr(self, k)))
 
     @staticmethod
     def from_device_arrays(f):
-        """From ``data.synth_forest_device`` (sparse features): everything already sits on the device; only the
-        size arrays live on the host."""
+        """From ``data.synth_forest_device``: everything already sits on the device; only the size arrays live on the
+        host.  Features stay in the form ``f`` holds them: dense rows when it has ``"x"`` (PHEME; fp32, or bf16 after
+        ``f["x"] = f["x"].to(torch.bfloat16)``), CSR otherwise."""
         self = DeviceForest.__new__(DeviceForest)
         dev = f["edge_src"].device
         self.h_node_ptr = np.asarray(f["node_ptr"], np.int64)
         self.h_edge_ptr = np.asarray(f["edge_ptr"], np.int64)
         self.node_ptr = torch.from_numpy(self.h_node_ptr).to(dev)
         self.edge_ptr = torch.from_numpy(self.h_edge_ptr).to(dev)
-        self.h_x_ptr_at_tree = f["x_ptr"][self.node_ptr].cpu().numpy()
         self.in_feats, self.device = int(f["in_feats"]), dev
         self.edge_src, self.edge_dst = f["edge_src"], f["edge_dst"]
-        self.x_ptr, self.x_col, self.x_val = f["x_ptr"], f["x_col"], f["x_val"]
+        if "x" in f:
+            self.x_ptr = self.x_col = self.x_val = None
+            self.x = _dense_storage(f["x"], int(self.h_node_ptr[-1]), self.in_feats)
+        else:
+            self.h_x_ptr_at_tree = f["x_ptr"][self.node_ptr].cpu().numpy()
+            self.x_ptr, self.x_col, self.x_val = f["x_ptr"], f["x_col"], f["x_val"]
+            self.x = None
         self.root_local, self.y = f["root_local"], f["y"].to(torch.int64)
         self.num_trees = len(self.h_node_ptr) - 1
         self._stage, self._turn = None, 0
@@ -62,15 +94,29 @@ class DeviceForest:
         return self
 
     @staticmethod
-    def from_data_list(trees, device):
+    def from_data_list(trees, device, features="csr", dtype=torch.float32):
         """Pack ``Data`` objects with the attribute layout of dataset.py:91-98 (x dense or SparseX,
-        edge_index [2,e] = [parent; child] WITHOUT DropEdge, rootindex, y)."""
+        edge_index [2,e] = [parent; child] WITHOUT DropEdge, rootindex, y).  ``features``: 'csr' keeps the non-zeros
+        of every row (bag-of-words features; ``data.x`` of a batch is a SparseX); 'dense' keeps the rows as they are,
+        in ``dtype`` (torch.float32 or torch.bfloat16; a SparseX tree is densified here, once), and a batch's
+        ``data.x`` is a dense tensor of that dtype."""
+        if features not in ("csr", "dense"):
+            raise L.BigcnError(f"DeviceForest: features must be 'csr' or 'dense', got {features!r}")
+        dense = features == "dense"
+        if dense and dtype not in (torch.float32, torch.bfloat16):
+            raise L.BigcnError(f"DeviceForest: dense features are stored as torch.float32 or torch.bfloat16, got {dtype}")
         node_ptr, edge_ptr, x_ptr = [0], [0], [0]
-        es, ed, xc, xv, roots, ys = [], [], [], [], [], []
+        es, ed, xc, xv, xd, roots, ys = [], [], [], [], [], [], []
         k = None
         for d in trees:
             x = d.x
-            if isinstance(x, SparseX):
+            if dense:
+                xn = (x.to_dense() if isinstance(x, SparseX) else x).to(dtype)
+                n, k = xn.shape
+                if dtype == torch.bfloat16:
+                    check_bf16_width(k)      # before anything is copied to the device
+                xd.append(xn)
+            elif isinstance(x, SparseX):
                 ptr, col, val, n = x.ptr.numpy().astype(np.int64), x.col.numpy(), x.val.numpy(), x.shape[0]
                 k = x.shape[1]
             else:
@@ -81,23 +127,28 @@ class DeviceForest:
                 ptr = np.concatenate([[0], np.cumsum(np.bincount(r, minlength=n))]).astype(np.int64)
             ei = d.edge_index.numpy()
             es.append(ei[0].astype(np.int32)); ed.append(ei[1].astype(np.int32))
-            xc.append(col); xv.append(val)
-            x_ptr.extend((x_ptr[-1] + ptr[1:]).tolist())
+            if not dense:
+                xc.append(col); xv.append(val)
+                x_ptr.extend((x_ptr[-1] + ptr[1:]).tolist())
             node_ptr.append(node_ptr[-1] + n)
             edge_ptr.append(edge_ptr[-1] + ei.shape[1])
             roots.append(int(d.rootindex)); ys.append(int(d.y))
         cat = lambda xs, dt: np.concatenate(xs).astype(dt) if xs else np.zeros(0, dt)  # noqa: E731
+        if dense:
+            return DeviceForest(node_ptr, edge_ptr, cat(es, np.int32), cat(ed, np.int32), None, None, None, roots, ys, k,
+                                device, x=torch.cat(xd).to(device))
         return DeviceForest(node_ptr, edge_ptr, cat(es, np.int32), cat(ed, np.int32), x_ptr, cat(xc, np.int32),
                             cat(xv, np.float32), roots, ys, k, device)
 
     @staticmethod
-    def from_npz_dir(fold_x, data_path, device, treeDic=None, lower=2, upper=100000):
+    def from_npz_dir(fold_x, data_path, device, treeDic=None, lower=2, upper=100000, features="csr",
+                     dtype=torch.float32):
         """Pack the reference's preprocessed dataset: one ``<id>.npz`` per tree under ``data_path`` with ``x`` [n, K],
         ``edgeindex`` [2, e] = [parent; child], ``rootindex`` and ``y`` (written by Process/getTwittergraph.py:67-72,
         read per item and per epoch by ``BiGraphDataset.__getitem__``, Process/dataset.py:64-99 -- here once).  The id
         filter is ``BiGraphDataset.__init__``'s (dataset.py:48-59): PHEME paths take ``fold_x`` as is, the others keep
         the ids found in ``treeDic`` whose tree has ``lower .. upper`` nodes.  ``self.ids`` holds the kept ids in
-        order: tree t of the forest is ``ids[t]``."""
+        order: tree t of the forest is ``ids[t]``.  ``features`` / ``dtype``: as in ``from_data_list``."""
         import os
         from .data import Data
         if str(data_path).find("PHEME") == -1 and treeDic is not None:
@@ -108,7 +159,7 @@ class DeviceForest:
             ei = np.asarray(z["edgeindex"], np.int64).reshape(2, -1)
             trees.append(Data(x=torch.tensor(np.asarray(z["x"]), dtype=torch.float32), edge_index=torch.from_numpy(ei),
                               rootindex=torch.tensor([int(z["rootindex"])]), y=torch.tensor([int(z["y"])])))
-        forest = DeviceForest.from_data_list(trees, device)
+        forest = DeviceForest.from_data_list(trees, device, features, dtype)
         forest.ids = list(fold_x)
         return forest
 
@@ -127,11 +178,14 @@ class DeviceForest:
 
     def batch(self, tree_ids, td_droprate=0.0, bu_droprate=0.0, seed=0) -> Batch:
         """The collated batch of ``tree_ids`` (host sequence, in batch order) with DropEdge at the
-        given rates, on the device; ``data.x`` is a SparseX."""
+        given rates, on the device; ``data.x`` is a SparseX for CSR storage, a fresh contiguous [n, in_feats] tensor
+        of the storage dtype for dense storage.  DropEdge draws depend only on the seed, the tree id, the direction and
+        the edge position: both storage forms give the same edges for the same ids and seed."""
         L.require_device()
         ids = np.asarray(tree_ids, np.int64)
         b = len(ids)
         dev = self.device
+        dense = self.x is not None
         # The per-tree offsets live in a ring of pinned staging buffers which the assembly kernels read IN PLACE
         # (pinned memory is device-addressable: 5 (b + 1) int64 cross PCIe inside the kernels, no copy, no device
         # buffer).  A slot is rewritten only after the kernels that last read it have completed: the epoch loop never
@@ -159,9 +213,13 @@ class DeviceForest:
         # int(length * (1 - droprate)), dataset.py:72,84 (Python float arithmetic = IEEE double)
         for row, rate in ((2, td_droprate), (3, bu_droprate)):
             np.cumsum(e_t if rate <= 0 else np.floor(e_t.astype(np.float64) * (1.0 - rate)).astype(np.int64), out=offs[row, 1:])
-        np.cumsum(self.h_x_ptr_at_tree[ids1] - self.h_x_ptr_at_tree[ids], out=offs[4, 1:])
+        if dense:
+            offs[4, 1:] = 0
+        else:
+            np.cumsum(self.h_x_ptr_at_tree[ids1] - self.h_x_ptr_at_tree[ids], out=offs[4, 1:])
         n, e_td, e_bu, nnz = (int(v) for v in offs[1:, b])
         # one int64 block [edge_index | BU_edge_index | batch | rootindex | y], one 32-bit block [x ptr | x col | x val]
+        # (CSR) or a dense x of its own
         blk = torch.empty(2 * e_td + 2 * e_bu + n + 2 * b, dtype=torch.int64, device=dev)
         o = 0
         ei = blk[o:o + 2 * e_td].view(2, e_td); o += 2 * e_td
@@ -169,20 +227,29 @@ class DeviceForest:
         batch = blk[o:o + n]; o += n
         root = blk[o:o + b]; o += b
         y = blk[o:o + b]
-        iblk = torch.empty(n + 1 + 2 * nnz, dtype=torch.int32, device=dev)
-        if b == 0:
-            iblk.zero_()
-        ox_ptr, ox_col = iblk[:n + 1], iblk[n + 1:n + 1 + nnz]
-        ox_val = iblk[n + 1 + nnz:].view(torch.float32)
         cur = torch.cuda.current_stream(dev)
         base, pitch = slot[0].data_ptr(), 8 * (b + 1)
-        check(lib().bigcn_assemble_batch(self._p_node_ptr, self._p_edge_ptr, self._p_edge_src, self._p_edge_dst,
-                                         self._p_x_ptr, self._p_x_col, self._p_x_val, self._p_root_local, self._p_y,
-                                         base, base + pitch, base + 2 * pitch, base + 3 * pitch, base + 4 * pitch,
-                                         b, e_td, e_bu, int(seed) & ((1 << 64) - 1), _p(ei), _p(bu), _p(batch), _p(root),
-                                         _p(y), _p(ox_ptr), _p(ox_col), _p(ox_val), cur.cuda_stream), "assemble_batch")
+        seed = int(seed) & ((1 << 64) - 1)
+        if dense:
+            x = torch.empty(n, self.in_feats, dtype=self.x.dtype, device=dev)
+            check(lib().bigcn_assemble_batch_dense(self._p_node_ptr, self._p_edge_ptr, self._p_edge_src,
+                                                   self._p_edge_dst, self._p_root_local, self._p_y, base, base + pitch,
+                                                   base + 2 * pitch, base + 3 * pitch, b, e_td, e_bu, seed, _p(ei),
+                                                   _p(bu), _p(batch), _p(root), _p(y), self._p_x, self.in_feats,
+                                                   self.x.element_size(), _p(x), cur.cuda_stream), "assemble_batch_dense")
+        else:
+            iblk = torch.empty(n + 1 + 2 * nnz, dtype=torch.int32, device=dev)
+            if b == 0:
+                iblk.zero_()
+            ox_ptr, ox_col = iblk[:n + 1], iblk[n + 1:n + 1 + nnz]
+            ox_val = iblk[n + 1 + nnz:].view(torch.float32)
+            check(lib().bigcn_assemble_batch(self._p_node_ptr, self._p_edge_ptr, self._p_edge_src, self._p_edge_dst,
+                                             self._p_x_ptr, self._p_x_col, self._p_x_val, self._p_root_local, self._p_y,
+                                             base, base + pitch, base + 2 * pitch, base + 3 * pitch, base + 4 * pitch,
+                                             b, e_td, e_bu, seed, _p(ei), _p(bu), _p(batch), _p(root),
+                                             _p(y), _p(ox_ptr), _p(ox_col), _p(ox_val), cur.cuda_stream), "assemble_batch")
+            x = SparseX(ox_ptr, ox_col, ox_val, (n, self.in_feats))
         if slot[1] is None:
             slot[1] = torch.cuda.Event()
         slot[1].record(cur)
-        return Batch(x=SparseX(ox_ptr, ox_col, ox_val, (n, self.in_feats)), edge_index=ei, BU_edge_index=bu,
-                     batch=batch, rootindex=root, y=y)
+        return Batch(x=x, edge_index=ei, BU_edge_index=bu, batch=batch, rootindex=root, y=y)

@@ -153,6 +153,13 @@ def host_dense_to_csr(x, n_threads=0, out=None, cap=None):
     return SparseX(ptr[:n + 1], col[:nnz], val[:nnz], (n, k))
 
 
+def check_bf16_width(k):
+    """bf16 features reach the tensor cores through TMA, which needs 16-byte rows"""
+    if k % 8:
+        raise L.BigcnError(f"gemm_mode='bf16': in_feats must be a multiple of 8 (16-byte rows for TMA), got "
+                           f"{k}: pad the features with zero columns (and the weights to match)")
+
+
 def bf16_x(x):
     """data.x for ``gemm_mode='bf16'``: a dense, contiguous CUDA bfloat16 matrix whose rows the TMA can address,
     passed through as it is.  Anything else raises (never a silent cast)."""
@@ -166,9 +173,7 @@ def bf16_x(x):
         raise L.BigcnError(f"gemm_mode='bf16': data.x must be [N, in_feats], got shape {tuple(x.shape)}")
     if not x.is_contiguous():
         raise L.BigcnError("gemm_mode='bf16': data.x must be contiguous (row pitch = in_feats): pass x.contiguous()")
-    if x.shape[1] % 8:
-        raise L.BigcnError(f"gemm_mode='bf16': in_feats must be a multiple of 8 (16-byte rows for TMA), got "
-                           f"{x.shape[1]}: pad the features with zero columns (and the weights to match)")
+    check_bf16_width(x.shape[1])
     if x.data_ptr() % 16:
         raise L.BigcnError("gemm_mode='bf16': data.x must start on a 16-byte boundary: pass x.clone()")
     return x

@@ -480,6 +480,19 @@ int bigcn_assemble_batch(const int64_t* node_ptr, const int64_t* edge_ptr, const
                          int64_t E_bu, uint64_t seed, int64_t* edge_index, int64_t* bu_edge_index,
                          int64_t* batch, int64_t* rootindex, int64_t* y, int32_t* ox_ptr, int32_t* ox_col,
                          float* ox_val, bigcn_stream_t stream);
+/* The same batch from a dataset whose features are DENSE rows: x_all [N_all, K] of elem_bytes = 4 (fp32) or 2 (bf16)
+ * per element, row pitch K.  The same tree, edge and offset arguments and the same pinned-memory rule as
+ * bigcn_assemble_batch (no x_ptr / x_col / x_val / nnz_off); ox [N, K] of the same element type receives tree
+ * tree_id[b]'s rows at row node_off[b], copied bit for bit (no conversion).  16-byte loads and stores when K * elem_bytes
+ * and both addresses are multiples of 16.  B = 0 returns 0; K < 1, K * elem_bytes >= 2^30, another elem_bytes or an
+ * x_all / ox not aligned to elem_bytes fail. */
+int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                               const int32_t* edge_dst, const int32_t* root_local, const int64_t* y_all,
+                               const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                               const int64_t* bu_off, int64_t B, int64_t E_td, int64_t E_bu, uint64_t seed,
+                               int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch, int64_t* rootindex,
+                               int64_t* y, const void* x_all, int64_t K, int32_t elem_bytes, void* ox,
+                               bigcn_stream_t stream);
 
 /* ---- data-parallel optimiser step over peer memory (SURVEY.md 8e) -----------------------------
  * One kernel instead of "NCCL all-reduce of the flat gradient + Adam on every rank": grads[q] /
