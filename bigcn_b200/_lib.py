@@ -18,6 +18,7 @@ DEG_BY = {"target": 0, "source": 1}
 GEMM_MODE = {"fp32": 0, "tf32": 1, "tf32x3": 2, "mixed": 3, "sparse": 4, "tf32x2": 5, "bf16": 6}
 FLAG_X_NOT_SPARSE = 8
 FLAG_X_CSR_RANGE = 16
+FLAG_EDGE_WEIGHT = 32
 DIR_TD, DIR_BU = 1, 2
 
 c_f32p = C.c_void_p  # device pointers travel as integers
@@ -32,7 +33,8 @@ class Dims(C.Structure):
 class BatchPtrs(C.Structure):
     _fields_ = [("x", c_ptr), ("edge_index", c_ptr), ("bu_edge_index", c_ptr), ("batch", c_ptr),
                 ("rootindex", c_ptr), ("node_id_base", C.c_int64),
-                ("x_ptr", c_ptr), ("x_col", c_ptr), ("x_val", c_ptr), ("prepared", c_ptr)]
+                ("x_ptr", c_ptr), ("x_col", c_ptr), ("x_val", c_ptr), ("prepared", c_ptr),
+                ("td_edge_weight", c_ptr), ("bu_edge_weight", c_ptr)]
 
 
 class Params(C.Structure):
@@ -49,7 +51,7 @@ class Opts(C.Structure):
     _fields_ = [("training", C.c_int32), ("p_drop", C.c_float), ("seed", C.c_uint64),
                 ("deg_by", C.c_int32), ("gemm_mode", C.c_int32), ("dir_mask", C.c_int32),
                 ("bwd_phase", C.c_int32), ("skip_wgrad_prep", C.c_int32), ("fused_tail", C.c_int32),
-                ("seed_dev", c_ptr), ("dense_roots", C.c_int32)]
+                ("seed_dev", c_ptr), ("dense_roots", C.c_int32), ("edge_grad", C.c_int32)]
 
 
 class BigcnError(RuntimeError):
@@ -105,6 +107,9 @@ _SIGS = {
     "bigcn_features_backward": (C.c_int, [C.POINTER(Dims), C.POINTER(BatchPtrs), C.POINTER(Params),
                                           C.POINTER(Opts), c_ptr, C.POINTER(Params), c_ptr, C.c_size_t,
                                           c_ptr]),
+    "bigcn_features_edge_workspace_bytes": (C.c_size_t, [C.POINTER(Dims), C.c_int32]),
+    "bigcn_features_edge_grad": (C.c_int, [C.POINTER(Dims), C.POINTER(BatchPtrs), C.POINTER(Opts), c_ptr, c_ptr, c_ptr,
+                                           C.c_size_t, c_ptr]),
     "bigcn_features_x_grad": (C.c_int, [C.POINTER(Dims), C.POINTER(Params), C.POINTER(Opts), c_ptr, c_ptr, c_ptr,
                                         c_ptr, C.c_size_t, c_ptr]),
     "bigcn_x_dgrad_scratch_floats": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int32]),

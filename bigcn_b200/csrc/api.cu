@@ -243,6 +243,55 @@ static FeatWs carve_features(const bigcn_dims_t* dm, void* ws, size_t bytes, voi
   return w;
 }
 
+// An edge-weighted batch: the weighted normalisation of both directions (weighted.cu), laid out after the features
+// workspace; with opts.edge_grad also the buffers that keep XW and Z alive through the backward and the per-edge
+// products of the edge gradient.
+struct WFeatWs {
+  WGraph G[2];
+  float* in_w[2];           // [E] normalised weight per by-target entry (forward sweeps)
+  float* out_w[2];          // [E] ... per by-source entry (A-hat^T sweeps)
+  float* ones;              // [Emax] the weights of a direction the caller gave none
+  float* t2;                // edge_grad: [2][N][64] T2, instead of over XW
+  float* g1;                // edge_grad: [2][N][64] G1, instead of over Z
+  float* a_e[2];            // edge_grad: [E] dL/dnorm per edge id
+  float* a_self[2];         // edge_grad: [N] ... per self-loop
+  float* ddeg[2];           // edge_grad: [N]
+  size_t total;
+};
+static WFeatWs carve_wfeat(const bigcn_dims_t* dm, void* base, bool edge_grad) {
+  WFeatWs w{};
+  Carver c(base, 0);
+  const int64_t N = dm->N;
+  const int64_t E[2] = {dm->E_td, dm->E_bu};
+  const size_t n1 = (size_t)(N > 0 ? N : 1);
+  for (int d = 0; d < 2; ++d) {
+    const size_t e1 = (size_t)(E[d] > 0 ? E[d] : 1);
+    w.G[d].in_eid = c.take<int32_t>(e1);
+    w.G[d].out_eid = c.take<int32_t>(e1);
+    w.G[d].loop_eid = c.take<int32_t>(n1);
+    w.G[d].self_w = c.take<float>(n1);
+    w.G[d].dis = c.take<float>(n1);
+    w.G[d].norm_e = c.take<float>(e1);
+    w.G[d].norm_self = c.take<float>(n1);
+    w.in_w[d] = c.take<float>(e1);
+    w.out_w[d] = c.take<float>(e1);
+  }
+  w.ones = c.take<float>((size_t)(E[0] > E[1] ? E[0] : E[1]) + 1);
+  if (edge_grad) {
+    w.t2 = c.take<float>(2 * n1 * H);
+    w.g1 = c.take<float>(2 * n1 * H);
+    for (int d = 0; d < 2; ++d) {
+      w.a_e[d] = c.take<float>((size_t)(E[d] > 0 ? E[d] : 1));
+      w.a_self[d] = c.take<float>(n1);
+      w.ddeg[d] = c.take<float>(n1);
+    }
+  }
+  w.total = align_up(c.off, 256);
+  return w;
+}
+static bool batch_weighted(const bigcn_batch_t* bt) { return bt->td_edge_weight != nullptr || bt->bu_edge_weight != nullptr; }
+static const float* dir_edge_weight(const bigcn_batch_t* bt, int d) { return d == 0 ? bt->td_edge_weight : bt->bu_edge_weight; }
+
 int batch_prepare_join(cudaStream_t st);
 
 // active directions: order TD (0), BU (1); feat base: BU -> 0, TD -> 128 (cat order of :128)
@@ -291,8 +340,13 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   if (int rc = check_common(dm, o, "features_forward")) return rc;
   if (int rc = check_bf16_x(dm, bt, o, "features_forward")) return rc;
   FeatWs w = carve_features(dm, ws, ws_bytes, bt->prepared);
-  BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total, "features_forward: workspace too small (%zu < %zu)",
-                  ws_bytes, w.total);
+  const bool weighted = batch_weighted(bt);
+  const WFeatWs wf = weighted ? carve_wfeat(dm, ws ? reinterpret_cast<char*>(ws) + w.total : nullptr, o->edge_grad != 0)
+                              : WFeatWs{};
+  BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total + wf.total, "features_forward: workspace too small (%zu < %zu)",
+                  ws_bytes, w.total + wf.total);
+  BIGCN_CHECK_ARG(!weighted || bt->prepared == nullptr,
+                  "features_forward: an edge-weighted batch takes no prepared buffer (bigcn_batch_prepare carries no weights)");
   const bool prepared = bt->prepared != nullptr;   // graph structure, root columns, CSR / CSC of x: already there
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const Dirs dirs = active_dirs(o->dir_mask);
@@ -318,9 +372,21 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   if (!prepared) {
     const int64_t* ei[2] = {bt->edge_index, bt->bu_edge_index};
     const int64_t E[2] = {dm->E_td, dm->E_bu};
+    int32_t* const eids[4] = {wf.G[0].in_eid, wf.G[0].out_eid, wf.G[1].in_eid, wf.G[1].out_eid};
     if (int rc = graph_prep_impl(2, ei, E, N, bt->batch, B, o->deg_by, w.g, w.node_ptr, flags, w.prep_ws,
-                                 w.prep_bytes, ss))
+                                 w.prep_bytes, ss, weighted ? eids : nullptr))
       return rc;
+    if (weighted) {   // the weighted normalisation of the active directions (a direction without weights: all ones)
+      if (int rc = wfeat_ones(wf.ones, E[0] > E[1] ? E[0] : E[1], ss)) return rc;
+      for (int q = 0; q < dirs.n; ++q) {
+        const int d = dirs.id[q];
+        WGraph G = wf.G[d];
+        G.g = w.g[d];
+        const float* ew = dir_edge_weight(bt, d);
+        if (int rc = wfeat_prep(G, ei[d], E[d], ew ? ew : wf.ones, N, o->deg_by, wf.in_w[d], wf.out_w[d], flags, ss))
+          return rc;
+      }
+    }
   }
   // 2. weights in the layouts the kernels stream
   const int n_out = dirs.n == 2 ? 128 : 64;
@@ -418,6 +484,10 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
       side_busy = sc != nullptr;
     }
   }
+  // edge-weighted batch: the sweeps read the normalised weight of every entry, and dis stands for the self-loop weights
+  EntryW ew_in{};
+  for (int q = 0; q < dirs.n; ++q) ew_in.w[q] = wf.in_w[dirs.id[q]];
+  const float* self_w[2] = {weighted ? wf.G[0].norm_self : w.g[0].dis, weighted ? wf.G[1].norm_self : w.g[1].dis};
   // 5. conv1 propagate + relu/dropout + conv2 lin
   {
     MixArgs a{};
@@ -426,7 +496,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     for (int q = 0; q < dirs.n; ++q) {
       const int d = dirs.id[q];
       MixDir& m = a.d[q];
-      m.ptr = w.g[d].in_ptr; m.idx = w.g[d].in_idx; m.dis = w.g[d].dis;
+      m.ptr = w.g[d].in_ptr; m.idx = w.g[d].in_idx; m.dis = self_w[d];
       m.lng = w.g[d].in_long; m.E = d == 0 ? dm->E_td : dm->E_bu;
       m.xw = w.xw + q * H; m.b1 = dir_b1(pr, d);
       m.w2aT = w.w2aT[d]; m.w2bT = w.w2bT[d]; m.P = w.P[d];
@@ -438,10 +508,10 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     for (int q = 0; q < dirs.n; ++q) a.root_r[q] = root_splits > 1 ? w.rootR[dirs.id[q]] : w.z[dirs.id[q]];
     // the tcgen05 form of the forward product (sweep + activate, then k_h64_tc) is measured slower than the fused
     // sweep at these sizes (DESIGN.md): kept behind a knob for the A/B
-    if (mix_tc_available() && !dense_roots && (debug_knob(8) == 2 || debug_knob(8) == 3)) {
+    if (mix_tc_available() && !dense_roots && !weighted && (debug_knob(8) == 2 || debug_knob(8) == 3)) {
       if (int rc = mix_tc_forward(a, dirs.n, w.w2a_split, st)) return rc;
     } else {
-      if (int rc = prop1_mix_launch(a, dirs.n, st)) return rc;
+      if (int rc = prop1_mix_launch(a, dirs.n, st, weighted ? &ew_in : nullptr)) return rc;
     }
   }
   // 6. conv2 propagate + bias + relu
@@ -450,10 +520,10 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     a.N = N; a.relu = 1;
     for (int q = 0; q < dirs.n; ++q) {
       const int d = dirs.id[q];
-      a.d[q] = PropDir{w.g[d].in_ptr, w.g[d].in_idx, w.g[d].dis, w.z[d], dir_b2(pr, d), w.h2[d], H, H,
+      a.d[q] = PropDir{w.g[d].in_ptr, w.g[d].in_idx, self_w[d], w.z[d], dir_b2(pr, d), w.h2[d], H, H,
                        w.g[d].in_long, d == 0 ? dm->E_td : dm->E_bu};
     }
-    if (int rc = propagate_launch(a, dirs.n, st)) return rc;
+    if (int rc = propagate_launch(a, dirs.n, st, weighted ? &ew_in : nullptr)) return rc;
   }
   // 7. readout
   {
@@ -489,6 +559,8 @@ int batch_prepare(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_o
                   size_t prepared_bytes, cudaStream_t st) {
   if (int rc = check_common(dm, o, "batch_prepare")) return rc;
   if (int rc = check_bf16_x(dm, bt, o, "batch_prepare")) return rc;
+  BIGCN_CHECK_ARG(!batch_weighted(bt), "batch_prepare: an edge-weighted batch is not prepared ahead (the prepared "
+                                       "buffer carries no weights): pass it to features_forward without one");
   PrepWs w = carve_prepared(dm, prepared, prepared_bytes);
   BIGCN_CHECK_ARG(prepared != nullptr && prepared_bytes >= w.total, "batch_prepare: buffer too small (%zu < %zu)",
                   prepared_bytes, w.total);
@@ -558,14 +630,23 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
   if (int rc = check_common(dm, o, "features_backward")) return rc;
   if (int rc = check_bf16_x(dm, bt, o, "features_backward")) return rc;
   FeatWs w = carve_features(dm, ws, ws_bytes, bt->prepared);
-  BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total, "features_backward: workspace too small");
+  const bool weighted = batch_weighted(bt);
+  const bool edge_grad = weighted && o->edge_grad != 0;
+  const WFeatWs wf = weighted ? carve_wfeat(dm, ws ? reinterpret_cast<char*>(ws) + w.total : nullptr, edge_grad)
+                              : WFeatWs{};
+  BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total + wf.total, "features_backward: workspace too small");
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const Dirs dirs = active_dirs(o->dir_mask);
   const int n_out = dirs.n == 2 ? 128 : 64;
   const bool dropping = o->training && o->p_drop > 0.f;
   const size_t nh = (size_t)(N > 0 ? N : 1) * H;
-  float* t2[2] = {w.xw, w.xw + nh};      // XW is dead after forward
-  float* g1[2] = {w.z[0], w.z[1]};       // Z is dead after forward
+  // XW and Z are dead after forward -- unless the edge gradient reads them (after G1 is formed): T2 and G1 then go
+  // to buffers of their own
+  float* t2[2] = {edge_grad ? wf.t2 : w.xw, (edge_grad ? wf.t2 : w.xw) + nh};
+  float* g1[2] = {edge_grad ? wf.g1 : w.z[0], edge_grad ? wf.g1 + nh : w.z[1]};
+  EntryW ew_out{};
+  const float* self_w[2] = {weighted ? wf.G[0].norm_self : w.g[0].dis, weighted ? wf.G[1].norm_self : w.g[1].dis};
+  for (int q = 0; q < dirs.n; ++q) ew_out.w[q] = wf.out_w[dirs.id[q]];
   float* t1cat = w.h2[0];                // H2 is dead once T2 exists
   // bwd_phase: 0 = everything, 1 = all but dW1, 2 = dW1 only (lets the caller all-reduce the
   // other gradients while the second X stream runs)
@@ -600,10 +681,10 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
     a.N = N; a.batch = bt->batch;
     for (int q = 0; q < dirs.n; ++q) {
       const int d = dirs.id[q];
-      a.d[q] = PropG2Dir{w.g[d].out_ptr, w.g[d].out_idx, w.g[d].dis, w.h2[d], w.gs[d], t2[d],
+      a.d[q] = PropG2Dir{w.g[d].out_ptr, w.g[d].out_idx, self_w[d], w.h2[d], w.gs[d], t2[d],
                          w.g[d].out_long, d == 0 ? dm->E_td : dm->E_bu};
     }
-    if (int rc = propagate_g2_launch(a, dirs.n, st)) return rc;
+    if (int rc = propagate_g2_launch(a, dirs.n, st, weighted ? &ew_out : nullptr)) return rc;
   }
   // 3./4. on the two side streams, beside the G1 -> T1 -> dW1 chain: db2 and dW2a = T2^T A1 on one,
   //       dW2b on the other (both read T2 only)
@@ -676,16 +757,29 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
     if (sc) stream_after(sc, 2, st, ss);           // db1: ordered sum of the partials, beside T1
     if (int rc = colsum_reduce_launch(c, dirs.n, ss)) return rc;
   }
+  // 5b. edge gradient: the per-edge products of both convs while XW, Z (conv2's input M), G1 and H2 are all alive
+  if (edge_grad) {
+    EdgeDotArgs a{};
+    a.N = N; a.batch = bt->batch;
+    const int64_t* ei[2] = {bt->edge_index, bt->bu_edge_index};
+    for (int q = 0; q < dirs.n; ++q) {
+      const int d = dirs.id[q];
+      if (dir_edge_weight(bt, d) == nullptr) continue;   // no weights, no gradient: a_e stays NULL
+      a.d[q] = EdgeDotDir{ei[d], d == 0 ? dm->E_td : dm->E_bu, w.xw + q * H, n_out, g1[d], w.z[d], w.h2[d], w.gs[d],
+                          wf.a_e[d], wf.a_self[d]};
+    }
+    if (int rc = wfeat_edge_dot(a, dirs.n, st)) return rc;
+  }
   // 6. T1 = A-hat^T G1, both directions side by side in one [N][n_out] matrix
   {
     PropArgs a{};
     a.N = N; a.relu = 0;
     for (int q = 0; q < dirs.n; ++q) {
       const int d = dirs.id[q];
-      a.d[q] = PropDir{w.g[d].out_ptr, w.g[d].out_idx, w.g[d].dis, g1[d], nullptr, t1cat + q * H, H, n_out,
+      a.d[q] = PropDir{w.g[d].out_ptr, w.g[d].out_idx, self_w[d], g1[d], nullptr, t1cat + q * H, H, n_out,
                        w.g[d].out_long, d == 0 ? dm->E_td : dm->E_bu};
     }
-    if (int rc = propagate_launch(a, dirs.n, st)) return rc;
+    if (int rc = propagate_launch(a, dirs.n, st, weighted ? &ew_out : nullptr)) return rc;
   }
   // bwd_phase 1 (the caller reduces these gradients while dW1 runs): everything but dW1 is complete at return
   if (sc && !join_late) {
@@ -704,7 +798,8 @@ dw1_only:
       if (int rc = dw_sparse(w.xs, t1cat, n_out, n_out, da, db, K, st)) return rc;
     } else if (o->gemm_mode == BIGCN_GEMM_FP32) {
       if (int rc = dw_fp32(bt->x, N, K, t1cat, n_out, n_out, w.dw_part, da, K, 0, db, K, 0, st)) return rc;
-    } else {   // G1 (w.z) and H1 are dead here: they hold the TF32 hi / lo split of T1 (T2 is still being read by the dW2 chains)
+    } else {   // Z (G1, or M with an edge gradient) and H1 are dead here: they hold the TF32 hi / lo split of T1 (T2 is still
+               // being read by the dW2 chains)
       if (int rc = dw_tc(bt->x, N, K, t1cat, n_out, n_out, w.z[0], w.h1[0], w.dw_part, da, K, 0, db, K, 0,
                          o->gemm_mode, st))
         return rc;
@@ -836,7 +931,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 104; }
+extern "C" int bigcn_version(void) { return 105; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
@@ -908,6 +1003,42 @@ extern "C" int bigcn_dropout_mask(uint64_t seed, int32_t stream_id, int64_t node
 extern "C" size_t bigcn_features_workspace_bytes(const bigcn_dims_t* dims) {
   if (!dims) return 0;
   return carve_features(dims, nullptr, 0).total;
+}
+
+extern "C" size_t bigcn_features_edge_workspace_bytes(const bigcn_dims_t* dims, int32_t edge_grad) {
+  if (!dims) return 0;
+  return carve_features(dims, nullptr, 0).total + carve_wfeat(dims, nullptr, edge_grad != 0).total;
+}
+
+extern "C" int bigcn_features_edge_grad(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts,
+                                        float* d_td_w, float* d_bu_w, void* workspace, size_t workspace_bytes,
+                                        bigcn_stream_t stream) {
+  if (int rc = check_common(dims, opts, "features_edge_grad")) return rc;
+  BIGCN_CHECK_ARG(batch != nullptr, "features_edge_grad: NULL batch");
+  BIGCN_CHECK_ARG(opts->edge_grad != 0, "features_edge_grad: needs opts.edge_grad = 1 in the forward and backward calls");
+  const FeatWs w = carve_features(dims, workspace, workspace_bytes);
+  const WFeatWs wf = carve_wfeat(dims, workspace ? reinterpret_cast<char*>(workspace) + w.total : nullptr, true);
+  BIGCN_CHECK_ARG(workspace != nullptr && workspace_bytes >= w.total + wf.total,
+                  "features_edge_grad: workspace too small (bigcn_features_edge_workspace_bytes(dims, 1))");
+  float* out[2] = {d_td_w, d_bu_w};
+  const int64_t* ei[2] = {batch->edge_index, batch->bu_edge_index};
+  const int64_t E[2] = {dims->E_td, dims->E_bu};
+  for (int d = 0; d < 2; ++d) {
+    if (out[d] == nullptr) continue;
+    BIGCN_CHECK_ARG(dir_edge_weight(batch, d) != nullptr && ((opts->dir_mask >> d) & 1),
+                    "features_edge_grad: the %s gradient needs that direction active and its weights in the batch",
+                    d == 0 ? "TD" : "BU");
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  for (int d = 0; d < 2; ++d) {
+    if (out[d] == nullptr) continue;
+    WGraph G = wf.G[d];
+    G.g = w.g[d];
+    if (int rc = wfeat_edge_grad(G, ei[d], E[d], dir_edge_weight(batch, d), dims->N, opts->deg_by, wf.a_e[d],
+                                 wf.a_self[d], wf.ddeg[d], out[d], st))
+      return rc;
+  }
+  return 0;
 }
 
 extern "C" size_t bigcn_batch_prepare_bytes(const bigcn_dims_t* dims) {

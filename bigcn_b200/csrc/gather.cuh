@@ -1,6 +1,7 @@
 // CSR row sweep shared by every A-hat / A-hat^T kernel (k_propagate, k_propagate_g2, k_prop1_mix).
 //
 //   out[i] = post( sum_{e in ptr[i]..ptr[i+1]} (dis[idx[e]] * dis[i]) * val(idx[e])  +  dis[i]^2 * val(i) )
+//   (or, edge-weighted, the precomputed normalised weight of each entry and of the self-loop: WtEntry)
 //
 // replaces MessagePassing.propagate of torch_geometric's GCNConv (index_select, broadcast
 // multiply, atomic scatter_add) reached from BiGCN_Twitter.py:42,56,92,105 and its autograd
@@ -101,12 +102,24 @@ struct Csr {
   int64_t E;      // edge capacity the hub-row list was laid out for
 };
 
-// edge weights.  GCN: w(e: j -> i) = dis[j] * dis[i], plus the self-loop dis[i]^2.
+// edge weights.  row(i) is read once per row; the self-loop term of row i is self(row(i)).
+// GCN: w(e: j -> i) = dis[j] * dis[i], plus the self-loop dis[i]^2.
 struct WtGcn {
   const float* dis;
   static constexpr bool kSelf = true;
   __device__ __forceinline__ float row(int i) const { return dis[i]; }
   __device__ __forceinline__ float edge(int, int j, float drow) const { return __fmul_rn(dis[j], drow); }
+  __device__ __forceinline__ float self(float drow) const { return __fmul_rn(drow, drow); }
+};
+// edge-weighted GCN: the normalised weight of every CSR entry and of every self-loop, precomputed
+// (weighted.cu, (dis[j] * w_e) * dis[i] as gcn_norm forms it) and read as they are
+struct WtEntry {
+  const float* val;    // [E] per CSR entry, in the order of the CSR being swept
+  const float* slf;    // [N] per node
+  static constexpr bool kSelf = true;
+  __device__ __forceinline__ float row(int i) const { return slf[i]; }
+  __device__ __forceinline__ float edge(int e, int, float) const { return val[e]; }
+  __device__ __forceinline__ float self(float s) const { return s; }
 };
 // explicit per-entry weights, no self term (column-sorted X for the weight gradient)
 struct WtVal {
@@ -114,6 +127,7 @@ struct WtVal {
   static constexpr bool kSelf = false;
   __device__ __forceinline__ float row(int) const { return 0.f; }
   __device__ __forceinline__ float edge(int e, int, float) const { return val[e]; }
+  __device__ __forceinline__ float self(float) const { return 0.f; }
 };
 
 // Post functors: operator()(row, sum, sub, half mask, scratch) finishes one row; kPairs = true
@@ -225,8 +239,7 @@ __device__ __forceinline__ void csr_sweep(const Csr g, const Wt wt, const int n,
     // finished row: add the self-loop term and park the sum in the row's own stage slot
     auto flush = [&](int u) {
       if (Wt::kSelf) {
-        const float d = sd[u];
-        acc_add<EXACT>(acc, __fmul_rn(d, d), val.value(st + u * H, sa[Q + u], sub));
+        acc_add<EXACT>(acc, wt.self(sd[u]), val.value(st + u * H, sa[Q + u], sub));
       }
       if constexpr (Post::kInline) post(i0 + u, acc, sub, hm, nullptr);   // light epilogue: finish the row right here
       else st4(st + u * H + 4 * sub, acc);
@@ -284,8 +297,7 @@ __device__ __forceinline__ void csr_sweep(const Csr g, const Wt wt, const int n,
       } else {
         v = make_float4(0.f, 0.f, 0.f, 0.f);
         if (Wt::kSelf) {
-          const float d = sd[u];
-          acc_add<EXACT>(v, __fmul_rn(d, d), val.value(st + u * H, sa[Q + u], sub));
+          acc_add<EXACT>(v, wt.self(sd[u]), val.value(st + u * H, sa[Q + u], sub));
         }
       }
       return v;
@@ -372,7 +384,7 @@ __device__ __forceinline__ void csr_sweep(const Csr g, const Wt wt, const int n,
       }
       cp_async_commit_wait_all();
       __syncwarp(hm);
-      if (Wt::kSelf) acc_add<EXACT>(tot, __fmul_rn(d, d), val.value(st, sa[Q], sub));
+      if (Wt::kSelf) acc_add<EXACT>(tot, wt.self(d), val.value(st, sa[Q], sub));
       if (sub == 0) L.done[slot] = 0;   // ready for the next launch over this CSR
       post(row, tot, sub, hm, st + R * H);
     }

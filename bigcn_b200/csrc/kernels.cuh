@@ -36,9 +36,34 @@ size_t dx_tc_scratch_floats(int64_t N, int64_t K, int n_w);
 int dx_tc(const float* t, int n_w, const float* const* w, int64_t ldw, int64_t N, int64_t K, float* dx, void* dx_bf16,
           float* scratch, cudaStream_t st);
 
+// gcn_norm with edge weights (weighted.cu): the structure of one direction and its normalisation
+struct WGraph {
+  bigcn_graph_t g;        // in/out CSR (deg / dis of the unweighted prep are scratch here)
+  int32_t* in_eid;        // [E] edge id of every by-target CSR entry
+  int32_t* out_eid;       // [E] edge id of every by-source CSR entry
+  int32_t* loop_eid;      // [N] last self-loop edge on the node, or -1
+  float* self_w;          // [N]
+  float* dis;             // [N] weighted deg^-1/2
+  float* norm_e;          // [E] per edge id (0 for self-loop / out-of-range edges)
+  float* norm_self;       // [N]
+};
+// edge-weighted batch: the normalised weight of every entry of the CSR a sweep walks, per direction (weighted.cu);
+// the launchers take NULL for the unweighted form
+struct EntryW { const float* w[2]; };
+// per direction of an edge-weighted feature path (weighted.cu): gcn_norm with weights on top of the feature path's
+// graph prep, the normalised weights in both CSR orders, NaN / negative-degree checks (BIGCN_FLAG_EDGE_WEIGHT)
+int wfeat_ones(float* ones, int64_t n, cudaStream_t st);
+int wfeat_prep(const WGraph& G, const int64_t* ei, int64_t E, const float* w, int64_t N, int32_t deg_by, float* in_w,
+               float* out_w, int32_t* flags, cudaStream_t st);
+struct EdgeDotDir { const int64_t* ei; int64_t E; const float* xw; int64_t ldxw; const float* g1; const float* m;
+                    const float* h2; const float* gs; float* a_e; float* a_self; };
+struct EdgeDotArgs { EdgeDotDir d[2]; int64_t N; const int64_t* batch; };
+int wfeat_edge_dot(const EdgeDotArgs& a, int ndir, cudaStream_t st);
+int wfeat_edge_grad(const WGraph& G, const int64_t* ei, int64_t E, const float* w, int64_t N, int32_t deg_by,
+                    const float* a_e, const float* a_self, float* ddeg, float* dw, cudaStream_t st);
 struct PropDir { const int32_t* ptr; const int32_t* idx; const float* dis; const float* h; const float* bias; float* out; int64_t ldh, ldo; int32_t* lng; int64_t E; };
 struct PropArgs { PropDir d[2]; int64_t N; int32_t relu; int32_t cb; };
-int propagate_launch(const PropArgs&, int, cudaStream_t);
+int propagate_launch(const PropArgs&, int, cudaStream_t, const EntryW* ew = nullptr);
 struct RootNzArgs { const float* x; const int64_t* rootindex; int64_t N, B, K; int32_t* cnt; int32_t* col; float* val; int32_t* flags; int32_t* slot; int32_t* overflow; int32_t cap;
                     int32_t x_bf16;   /* x holds bf16 (BIGCN_GEMM_BF16) */ };
 int root_nz_launch(const RootNzArgs&, cudaStream_t);
@@ -50,7 +75,7 @@ struct MixArgs { MixDir d[2]; int64_t N, K, ldxw; int32_t cb; int64_t node_id_ba
                  int32_t root_splits;    /* training, dense roots (rootdense.cu): > 0 = the root half comes as this many
                                             partial sums root_r[d] + s * N * 64, added in order; the list walk is skipped */
                  const float* root_r[2]; };
-int prop1_mix_launch(const MixArgs&, int, cudaStream_t);
+int prop1_mix_launch(const MixArgs&, int, cudaStream_t, const EntryW* ew = nullptr);
 // tcgen05 form (mix_tc.cu): sweep + activate, then the 64 x 64 product on the tensor cores with the root part in the epilogue
 bool mix_tc_available();
 size_t mix_tc_scratch_floats();
@@ -107,7 +132,7 @@ int train_tail_run(TailArgs ta, const float* feat, const int64_t* y, int64_t B, 
                    size_t scratch_floats, cudaStream_t st);
 struct PropG2Dir { const int32_t* ptr; const int32_t* idx; const float* dis; const float* h2; const float* gs; float* out; int32_t* lng; int64_t E; };
 struct PropG2Args { PropG2Dir d[2]; int64_t N; const int64_t* batch; int32_t cb; };
-int propagate_g2_launch(const PropG2Args&, int, cudaStream_t);
+int propagate_g2_launch(const PropG2Args&, int, cudaStream_t, const EntryW* ew = nullptr);
 struct ColsumArgs { const float* part[4]; float* out[4]; int nchunk; };
 int colsum_reduce_launch(const ColsumArgs&, int, cudaStream_t);
 struct BwdMixDir { const float* t2; const float* h1 /* A1 = dropout(relu(H1)): > 0 where kept and positive */; const float* w2; float* g1; float* part; DropSpec drop; };

@@ -43,14 +43,24 @@ struct PostBiasRelu {
   }
 };
 
-__global__ void __launch_bounds__(256, 3) k_propagate(PropArgs a) {
-  extern __shared__ __align__(128) float sweep_smem[];
-  const PropDir p = a.d[blockIdx.y];
+template <class Wt>
+__device__ __forceinline__ void propagate_dir(const PropArgs& a, const PropDir& p, const Wt& wt, float* sweep_smem) {
   const int sub = threadIdx.x & 15;
   PostBiasRelu post{p.bias, p.out, p.ldo, a.relu, make_float4(0.f, 0.f, 0.f, 0.f)};
   if (p.bias) post.b = ld4(p.bias + 4 * sub);
-  csr_sweep<PROP_R, PROP_Q, true>(Csr{p.ptr, p.idx, p.lng, p.E}, WtGcn{p.dis}, (int)a.N, a.cb, sweep_smem,
-                                  ValRow{p.h, p.ldh}, post);
+  csr_sweep<PROP_R, PROP_Q, true>(Csr{p.ptr, p.idx, p.lng, p.E}, wt, (int)a.N, a.cb, sweep_smem, ValRow{p.h, p.ldh}, post);
+}
+__global__ void __launch_bounds__(256, 3) k_propagate(PropArgs a) {
+  extern __shared__ __align__(128) float sweep_smem[];
+  const PropDir p = a.d[blockIdx.y];
+  propagate_dir(a, p, WtGcn{p.dis}, sweep_smem);
+}
+// edge-weighted batch: p.dis holds the normalised self-loop weights, ew.w[d] the normalised weight of every entry of
+// the CSR being swept (EntryW, weighted.cu)
+__global__ void __launch_bounds__(256, 3) k_propagate_w(PropArgs a, EntryW ew) {
+  extern __shared__ __align__(128) float sweep_smem[];
+  const PropDir p = a.d[blockIdx.y];
+  propagate_dir(a, p, WtEntry{ew.w[blockIdx.y], p.dis}, sweep_smem);
 }
 
 template <class K>
@@ -58,18 +68,25 @@ static void sweep_attr(K kernel, int smem) {
   cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
 }
 
-int propagate_launch(const PropArgs& a0, int ndir, cudaStream_t st) {
+int propagate_launch(const PropArgs& a0, int ndir, cudaStream_t st, const EntryW* ew) {
   if (a0.N == 0) return 0;
   constexpr int smem = SweepSmem<PROP_R, PROP_Q>::kBytes;
   static bool attr = false;
   if (!attr) {
     sweep_attr(k_propagate, smem);
+    sweep_attr(k_propagate_w, smem);
     attr = true;
   }
   PropArgs a = a0;
   const int max_ctas = num_sms() * 3;
   a.cb = sweep_cb(a.N, PROP_R, max_ctas);
-  k_propagate<<<dim3(sweep_grid(a.N, PROP_R, a.cb, max_ctas), ndir), 256, smem, st>>>(a);
+  const dim3 grid(sweep_grid(a.N, PROP_R, a.cb, max_ctas), ndir);
+  if (ew) {
+    k_propagate_w<<<grid, 256, smem, st>>>(a, *ew);
+    BIGCN_CHECK_LAUNCH("k_propagate_w");
+    return 0;
+  }
+  k_propagate<<<grid, 256, smem, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_propagate");
   return 0;
 }
@@ -382,18 +399,29 @@ struct PostMix {
   }
 };
 
-template <int R, int Q, int MINB>
-__global__ void __launch_bounds__(256, MINB) k_prop1_mix(MixArgs a) {
-  extern __shared__ __align__(128) float sweep_smem[];
-  __shared__ __align__(16) float sW[H * H];
-  const MixDir p = a.d[blockIdx.y];
+template <int R, int Q, class Wt>
+__device__ __forceinline__ void prop1_mix_dir(const MixArgs& a, const MixDir& p, const Wt& wt, float* sweep_smem,
+                                              float* sW) {
   for (int i = threadIdx.x; i < H * H; i += blockDim.x) sW[i] = p.w2aT[i];
   // csr_sweep starts with a __syncthreads()
   const int sub = threadIdx.x & 15;
   PostMix post{p, sW, a.batch, a.rnz_cnt, a.rnz_col, a.rnz_val, a.K, a.node_id_base, ld4(p.b1 + 4 * sub), a.root_splits,
                a.root_r[blockIdx.y], a.N * H};
-  csr_sweep<R, Q, true>(Csr{p.ptr, p.idx, p.lng, p.E}, WtGcn{p.dis}, (int)a.N, a.cb, sweep_smem,
-                        ValRow{p.xw, a.ldxw}, post);
+  csr_sweep<R, Q, true>(Csr{p.ptr, p.idx, p.lng, p.E}, wt, (int)a.N, a.cb, sweep_smem, ValRow{p.xw, a.ldxw}, post);
+}
+template <int R, int Q, int MINB>
+__global__ void __launch_bounds__(256, MINB) k_prop1_mix(MixArgs a) {
+  extern __shared__ __align__(128) float sweep_smem[];
+  __shared__ __align__(16) float sW[H * H];
+  const MixDir p = a.d[blockIdx.y];
+  prop1_mix_dir<R, Q>(a, p, WtGcn{p.dis}, sweep_smem, sW);
+}
+// edge-weighted batch (see k_propagate_w): p.dis holds the self-loop weights
+__global__ void __launch_bounds__(256, 4) k_prop1_mix_w(MixArgs a, EntryW ew) {
+  extern __shared__ __align__(128) float sweep_smem[];
+  __shared__ __align__(16) float sW[H * H];
+  const MixDir p = a.d[blockIdx.y];
+  prop1_mix_dir<MIX_R, MIX_Q>(a, p, WtEntry{ew.w[blockIdx.y], p.dis}, sweep_smem, sW);
 }
 
 
@@ -543,11 +571,21 @@ struct PostStore {
     st4(out + (int64_t)i * H + 4 * sub, v);
   }
 };
+template <class Wt>
+__device__ __forceinline__ void propagate_g2_dir(const PropG2Args& a, const PropG2Dir& p, const Wt& wt, float* sweep_smem) {
+  csr_sweep<PROP_R, PROP_Q, false>(Csr{p.ptr, p.idx, p.lng, p.E}, wt, (int)a.N, a.cb, sweep_smem,
+                                   ValG2{p.h2, p.gs, a.batch}, PostStore{p.out});
+}
 __global__ void __launch_bounds__(256, 3) k_propagate_g2(PropG2Args a) {
   extern __shared__ __align__(128) float sweep_smem[];
   const PropG2Dir p = a.d[blockIdx.y];
-  csr_sweep<PROP_R, PROP_Q, false>(Csr{p.ptr, p.idx, p.lng, p.E}, WtGcn{p.dis}, (int)a.N, a.cb, sweep_smem,
-                                   ValG2{p.h2, p.gs, a.batch}, PostStore{p.out});
+  propagate_g2_dir(a, p, WtGcn{p.dis}, sweep_smem);
+}
+// edge-weighted batch (see k_propagate_w): by-source CSR, its own per-entry weights
+__global__ void __launch_bounds__(256, 3) k_propagate_g2_w(PropG2Args a, EntryW ew) {
+  extern __shared__ __align__(128) float sweep_smem[];
+  const PropG2Dir p = a.d[blockIdx.y];
+  propagate_g2_dir(a, p, WtEntry{ew.w[blockIdx.y], p.dis}, sweep_smem);
 }
 
 // out[f] = sum_chunk part[chunk][f]: 4 strided groups, fixed-order combine
@@ -952,8 +990,22 @@ static int mix_launch(const MixArgs& a0, int ndir, cudaStream_t st) {
   BIGCN_CHECK_LAUNCH("k_prop1_mix");
   return 0;
 }
-int prop1_mix_launch(const MixArgs& a, int ndir, cudaStream_t st) {
+int prop1_mix_launch(const MixArgs& a, int ndir, cudaStream_t st, const EntryW* ew) {
   if (a.N == 0) return 0;
+  if (ew) {   // one configuration, the default one
+    constexpr int smem = SweepSmem<MIX_R, MIX_Q>::kBytes;
+    static bool attr = false;
+    if (!attr) {
+      sweep_attr(k_prop1_mix_w, smem);
+      attr = true;
+    }
+    MixArgs m = a;
+    const int max_ctas = num_sms() * 4;
+    m.cb = sweep_cb(m.N, MIX_R, max_ctas);
+    k_prop1_mix_w<<<dim3(sweep_grid(m.N, MIX_R, m.cb, max_ctas), ndir), 256, smem, st>>>(m, *ew);
+    BIGCN_CHECK_LAUNCH("k_prop1_mix_w");
+    return 0;
+  }
   switch (debug_knob(2)) {
     case 1: return mix_launch<4, 4, 4>(a, ndir, st);
     case 2: return mix_launch<2, 8, 4>(a, ndir, st);
@@ -990,18 +1042,25 @@ int gscale_launch(const GScaleArgs& a, int ndir, cudaStream_t st) {
   BIGCN_CHECK_LAUNCH("k_gscale");
   return 0;
 }
-int propagate_g2_launch(const PropG2Args& a0, int ndir, cudaStream_t st) {
+int propagate_g2_launch(const PropG2Args& a0, int ndir, cudaStream_t st, const EntryW* ew) {
   if (a0.N == 0) return 0;
   constexpr int smem = SweepSmem<PROP_R, PROP_Q>::kBytes;
   static bool attr = false;
   if (!attr) {
     sweep_attr(k_propagate_g2, smem);
+    sweep_attr(k_propagate_g2_w, smem);
     attr = true;
   }
   PropG2Args a = a0;
   const int max_ctas = num_sms() * 3;
   a.cb = sweep_cb(a.N, PROP_R, max_ctas);
-  k_propagate_g2<<<dim3(sweep_grid(a.N, PROP_R, a.cb, max_ctas), ndir), 256, smem, st>>>(a);
+  const dim3 grid(sweep_grid(a.N, PROP_R, a.cb, max_ctas), ndir);
+  if (ew) {
+    k_propagate_g2_w<<<grid, 256, smem, st>>>(a, *ew);
+    BIGCN_CHECK_LAUNCH("k_propagate_g2_w");
+    return 0;
+  }
+  k_propagate_g2<<<grid, 256, smem, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_propagate_g2");
   return 0;
 }

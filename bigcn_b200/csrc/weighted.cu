@@ -24,17 +24,6 @@
 
 namespace bigcn {
 
-struct WGraph {
-  bigcn_graph_t g;        // in/out CSR (deg / dis of the unweighted prep are scratch here)
-  int32_t* in_eid;        // [E] edge id of every by-target CSR entry
-  int32_t* out_eid;       // [E] edge id of every by-source CSR entry
-  int32_t* loop_eid;      // [N] last self-loop edge on the node, or -1
-  float* self_w;          // [N]
-  float* dis;             // [N] weighted deg^-1/2
-  float* norm_e;          // [E] per edge id (0 for self-loop / out-of-range edges)
-  float* norm_self;       // [N]
-};
-
 // ---- pass 1: which edge supplies a node's self-loop weight ----------------------------------
 __global__ void k_w_loops(const int64_t* __restrict__ ei, int64_t E, int64_t N, int32_t* loop_eid) {
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < E; e += (int64_t)gridDim.x * blockDim.x) {
@@ -344,6 +333,124 @@ static WConvWs carve_wconv(int64_t N, int64_t E, int64_t K, void* ws, size_t byt
   w.dw_part = c.take<float>(dw_partial_floats(N, K, 64));
   w.total = align_up(c.off, 256);
   return w;
+}
+
+// ---- the two-direction feature path on an edge-weighted batch (api.cu) -------------------------------------------
+// The feature path's own graph prep runs with the edge id as the sort payload; on top of it, per direction, the
+// normalisation above (k_w_loops, k_w_deg, k_w_norm) and then the normalised weights laid out in both CSR orders for
+// the tuned sweeps of gather.cuh (WtEntry): in_w[k] = norm_e[in_eid[k]] (A-hat), out_w[k] = norm_e[out_eid[k]]
+// (A-hat^T); the self-loop weights are norm_self.  With every weight 1 these are (dis[j] * 1) * dis[i] = dis[j] * dis[i]
+// and (dis[i] * 1) * dis[i], and the degree is a float sum of ones: the unweighted values, bit for bit.
+__global__ void k_wf_entries(WGraph G, const float* __restrict__ w, int64_t E, int64_t N, float* __restrict__ in_w,
+                             float* __restrict__ out_w, int32_t* flags) {
+  bool bad = false;
+  const int64_t n = E > N ? E : N;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) {
+    if (t < E) {
+      in_w[t] = G.norm_e[G.in_eid[t]];
+      out_w[t] = G.norm_e[G.out_eid[t]];
+      bad |= !isfinite(w[t]);
+    }
+    if (t < N) bad |= isnan(G.dis[t]);   // a negative weighted degree
+  }
+  if (bad) atomicOr(flags, BIGCN_FLAG_EDGE_WEIGHT);
+}
+
+__global__ void k_wf_fill(float* __restrict__ p, int64_t n, float v) {
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) p[t] = v;
+}
+
+int wfeat_ones(float* ones, int64_t n, cudaStream_t st) {
+  if (n <= 0) return 0;
+  k_wf_fill<<<grid_for(n, 256), 256, 0, st>>>(ones, n, 1.0f);
+  BIGCN_CHECK_LAUNCH("k_wf_fill");
+  return 0;
+}
+
+int wfeat_prep(const WGraph& G, const int64_t* ei, int64_t E, const float* w, int64_t N, int32_t deg_by, float* in_w,
+               float* out_w, int32_t* flags, cudaStream_t st) {
+  if (N == 0) return 0;
+  cudaMemsetAsync(G.loop_eid, 0xFF, (size_t)N * sizeof(int32_t), st);
+  if (E > 0) {
+    k_w_loops<<<grid_for(E, 256), 256, 0, st>>>(ei, E, N, G.loop_eid);
+    BIGCN_CHECK_LAUNCH("k_w_loops");
+  }
+  k_w_deg<<<grid_for(N, 8), 256, 0, st>>>(G, w, N, deg_by == BIGCN_DEG_BY_SOURCE);
+  BIGCN_CHECK_LAUNCH("k_w_deg");
+  if (E > 0) {
+    k_w_norm<<<grid_for(E, 256), 256, 0, st>>>(G, ei, w, E, N);
+    BIGCN_CHECK_LAUNCH("k_w_norm");
+  }
+  k_wf_entries<<<grid_for(E > N ? E : N, 256), 256, 0, st>>>(G, w, E, N, in_w, out_w, flags);
+  BIGCN_CHECK_LAUNCH("k_wf_entries");
+  return 0;
+}
+
+// ---- edge gradient of the feature path: both convs of a direction share the edge list, so
+//   a_e    = <G1[c], XW[r]> + <G2[c], M[r]>   for edge e = (r -> c), 0 for self-loop / out-of-range edges
+//   a_self = the same with r = c = i
+// with G1 the gradient at conv1's output, XW conv1's propagate input, M conv2's (the mix kernel's z) and
+// G2[c] = [H2[c] > 0] * gs[batch[c]] formed here as k_propagate_g2 forms it.  The rest of the chain (through dis and
+// the self-loop weights) is k_w_ddeg / k_w_dweight above.  Half-warp per item, each lane adds its four conv1 products,
+// then its four conv2 products, then the two; a fixed xor tree across the 16 lanes: deterministic, no atomics.
+__global__ void __launch_bounds__(256) k_wf_edge_dot(EdgeDotArgs a) {
+  const EdgeDotDir& p = a.d[blockIdx.y];
+  if (p.a_e == nullptr) return;
+  const int hl = threadIdx.x & 15;
+  const int64_t N = a.N, E = p.E;
+  const int64_t item0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+  const int64_t nitem = ((int64_t)gridDim.x * blockDim.x) >> 4;
+  const int64_t total = (E + N + 1) / 2 * 2;   // both halves of a warp stay in the loop together
+  for (int64_t it = item0; it < total; it += nitem) {
+    int64_t r = -1, c = -1;
+    if (it < E) {
+      r = p.ei[it];
+      c = p.ei[E + it];
+      if (r == c || r < 0 || r >= N || c < 0 || c >= N) r = c = -1;
+    } else if (it < E + N) {
+      r = c = it - E;
+    }
+    float d = 0.f;
+    if (r >= 0) {
+      const float4 g1 = *reinterpret_cast<const float4*>(p.g1 + c * H + 4 * hl);
+      const float4 xw = *reinterpret_cast<const float4*>(p.xw + r * p.ldxw + 4 * hl);
+      const float4 h2 = *reinterpret_cast<const float4*>(p.h2 + c * H + 4 * hl);
+      const float4 gs = *reinterpret_cast<const float4*>(p.gs + a.batch[c] * H + 4 * hl);
+      const float4 m = *reinterpret_cast<const float4*>(p.m + r * H + 4 * hl);
+      const float d1 = g1.x * xw.x + g1.y * xw.y + g1.z * xw.z + g1.w * xw.w;
+      const float d2 = (h2.x > 0.f ? gs.x : 0.f) * m.x + (h2.y > 0.f ? gs.y : 0.f) * m.y +
+                       (h2.z > 0.f ? gs.z : 0.f) * m.z + (h2.w > 0.f ? gs.w : 0.f) * m.w;
+      d = d1 + d2;
+    }
+#pragma unroll
+    for (int o = 8; o > 0; o >>= 1) d += __shfl_xor_sync(FULL_MASK, d, o);
+    if (hl == 0) {
+      if (it < E) p.a_e[it] = d;
+      else if (it < E + N) p.a_self[it - E] = d;
+    }
+  }
+}
+
+int wfeat_edge_dot(const EdgeDotArgs& a, int ndir, cudaStream_t st) {
+  int64_t m = 0;
+  for (int q = 0; q < ndir; ++q)
+    if (a.d[q].a_e && a.d[q].E + a.N > m) m = a.d[q].E + a.N;
+  if (m == 0) return 0;
+  k_wf_edge_dot<<<dim3(grid_for(m, 16), ndir), 256, 0, st>>>(a);
+  BIGCN_CHECK_LAUNCH("k_wf_edge_dot");
+  return 0;
+}
+
+int wfeat_edge_grad(const WGraph& G, const int64_t* ei, int64_t E, const float* w, int64_t N, int32_t deg_by,
+                    const float* a_e, const float* a_self, float* ddeg, float* dw, cudaStream_t st) {
+  if (E == 0) return 0;
+  if (N > 0) {
+    k_w_ddeg<<<grid_for(N, 8), 256, 0, st>>>(G, w, a_e, a_self, ddeg, N);
+    BIGCN_CHECK_LAUNCH("k_w_ddeg");
+  }
+  k_w_dweight<<<grid_for(E, 256), 256, 0, st>>>(G, ei, E, N, a_e, a_self, ddeg, deg_by == BIGCN_DEG_BY_SOURCE, dw);
+  BIGCN_CHECK_LAUNCH("k_w_dweight");
+  return 0;
 }
 
 int xw_dispatch(const float* x, int64_t N, int64_t K, const float* const* w, int n_w, int64_t ldw, float* scratch,

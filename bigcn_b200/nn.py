@@ -6,7 +6,8 @@ Same class names, constructor signatures, sub-module names and state_dict keys a
 ``GCNConv`` that stands in for ``torch_geometric.nn.GCNConv`` on this path
 (``conv(x, edge_index)`` as called at explain_PHEME.py:95,132).  ``forward(data)``
 is duck-typed on ``data.x, data.edge_index, data.BU_edge_index, data.batch,
-data.rootindex``.  All arithmetic runs in libbigcn_b200.so; nothing here falls back
+data.rootindex`` and the optional ``data.edge_weight`` / ``data.BU_edge_weight`` (the edge weights of
+both convs of that direction, as ``GCNConv(x, edge_index, edge_weight)``).  All arithmetic runs in libbigcn_b200.so; nothing here falls back
 to PyTorch or the CPU.
 """
 from __future__ import annotations
@@ -20,7 +21,8 @@ import ctypes as C
 import weakref
 
 from .ops import (FeaturesFunction, GCNConvFunction, GCNConvWeightedFunction, HeadFunction, raise_on_flags,
-                  capture_graph, pick_gemm_mode, bf16_features_dense, x_val, _as_x, _i64, _make_structs, _p, _stream)
+                  capture_graph, pick_gemm_mode, bf16_features_dense, edge_weight, x_val, _as_x, _i64, _make_structs, _p,
+                  _stream)
 
 H = L.H
 
@@ -137,9 +139,11 @@ class _RumorGCN(torch.nn.Module):
 
     def forward(self, data):
         none4 = (None,) * 4
-        params = self._conv_params() + none4 if self._dir == L.DIR_TD else none4 + self._conv_params()
+        td = self._dir == L.DIR_TD
+        params = self._conv_params() + none4 if td else none4 + self._conv_params()
+        ew = (getattr(data, "edge_weight", None), None) if td else (None, getattr(data, "BU_edge_weight", None))
         feat = FeaturesFunction.apply(data.x, x_val(data.x), data.edge_index, data.BU_edge_index, data.batch,
-                                      data.rootindex, self._opts(self._dir, data.x), *params)
+                                      data.rootindex, *ew, self._opts(self._dir, data.x), *params)
         return feat[:, 2 * H:] if self._dir == L.DIR_TD else feat[:, :2 * H]
 
 
@@ -194,7 +198,8 @@ class BiGCN(torch.nn.Module):
         flags = torch.zeros(1, dtype=torch.int32, device=data.x.device)
         opts["flags"] = flags
         feat = FeaturesFunction.apply(data.x, x_val(data.x), data.edge_index, data.BU_edge_index, data.batch,
-                                      data.rootindex, opts, *td._conv_params(),
+                                      data.rootindex, getattr(data, "edge_weight", None),
+                                      getattr(data, "BU_edge_weight", None), opts, *td._conv_params(),
                                       *self.BUrumorGCN._conv_params())
         out = HeadFunction.apply(feat, self.fc.weight, self.fc.bias)
         self.last_flags = flags
@@ -216,14 +221,18 @@ class BiGCN(torch.nn.Module):
         c = self.fc.weight.shape[0]
         if xs is not None and mode != "sparse":
             raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
-        dims, bt, pr = _make_structs(x, ei, bue, batch, root, params, c, td.node_id_base, xs)
+        ew = (edge_weight(getattr(data, "edge_weight", None), int(ei.shape[1]), "edge_weight"),
+              edge_weight(getattr(data, "BU_edge_weight", None), int(bue.shape[1]), "BU_edge_weight"))
+        dims, bt, pr = _make_structs(x, ei, bue, batch, root, params, c, td.node_id_base, xs, ew)
         opts = td._opts(L.DIR_TD | L.DIR_BU, data.x)
         o = L.Opts(training=int(self.training), p_drop=float(td.p), seed=int(opts["seed"]), deg_by=L.DEG_BY[td.deg_by],
                    gemm_mode=L.GEMM_MODE[mode], dir_mask=L.DIR_TD | L.DIR_BU, skip_wgrad_prep=1)
         dev = xs.device if xs is not None else x.device
-        ws = torch.empty(L.lib().bigcn_features_workspace_bytes(C.byref(dims)), dtype=torch.uint8, device=dev)
+        nbytes = L.lib().bigcn_features_workspace_bytes(C.byref(dims)) if ew == (None, None) else \
+            L.lib().bigcn_features_edge_workspace_bytes(C.byref(dims), 0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         return {"dims": dims, "bt": bt, "pr": pr, "o": o, "ws": ws, "c": c,
-                "keep": (x, xs, ei, bue, batch, root, params, self.fc.weight, self.fc.bias),
+                "keep": (x, xs, ei, bue, batch, root, params, ew, self.fc.weight, self.fc.bias),
                 "flags": torch.zeros(1, dtype=torch.int32, device=dev),
                 "feat": torch.empty(dims.B, 4 * H, dtype=torch.float32, device=dev),
                 "logp": torch.empty(dims.B, c, dtype=torch.float32, device=dev)}
@@ -244,8 +253,10 @@ class BiGCN(torch.nn.Module):
             x = data.x
             xk = (x.ptr.data_ptr(), x.col.data_ptr(), x.val.data_ptr(), x.shape) if hasattr(x, "ptr") else \
                 (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
+            ews = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
             key = (id(data), xk, tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
                              (data.edge_index, data.BU_edge_index, data.batch, data.rootindex)),
+                   tuple(None if t is None else (t.data_ptr(), tuple(t.shape), t.dtype) for t in ews),
                    tuple(q.data_ptr() for q in self.parameters()), self.training, self.TDrumorGCN.deg_by,
                    self.TDrumorGCN.gemm_mode)
             p = self._graphs.get(key)

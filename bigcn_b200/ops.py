@@ -458,6 +458,8 @@ def raise_on_flags(flags: torch.Tensor):
         msgs.append("data.batch is not sorted ascending within [0, B)")
     if v & L.FLAG_ROOT_RANGE:
         msgs.append("data.rootindex has an entry outside [0, N)")
+    if v & L.FLAG_EDGE_WEIGHT:
+        msgs.append("an edge weight is not finite, or a node's weighted degree is negative")
     if v & L.FLAG_X_CSR_RANGE:
         msgs.append("sparse data.x has a column index outside [0, in_feats)")
     if v & L.FLAG_X_NOT_SPARSE:
@@ -582,7 +584,24 @@ def gcn_norm(edge_index, edge_weight=None, num_nodes=None, improved=False, add_s
 _PNAMES = ("td_w1", "td_b1", "td_w2", "td_b2", "bu_w1", "bu_b1", "bu_w2", "bu_b2")
 
 
-def _make_structs(x, ei, bu_ei, batch, rootindex, params, num_classes, node_id_base, xs=None):
+def edge_weight(w, e, name):
+    """A BiGCN edge weight checked and laid out for the library: None stays None; otherwise a CUDA tensor of shape
+    [e] with a floating dtype, returned as contiguous fp32.  A non-finite value is reported by the device flags
+    (raise_on_flags), with a negative weighted degree."""
+    if w is None:
+        return None
+    if not torch.is_tensor(w):
+        raise L.BigcnError(f"{name} must be a tensor, got {type(w).__name__}")
+    if not w.is_cuda:
+        raise L.BigcnError(f"{name}: bigcn_b200 ops take CUDA tensors only (no CPU fallback)")
+    if not w.is_floating_point():
+        raise L.BigcnError(f"{name} must have a floating dtype, got {w.dtype}")
+    if tuple(w.shape) != (e,):
+        raise L.BigcnError(f"{name} must be [{e}] (one weight per column of its edge index), got {tuple(w.shape)}")
+    return w.to(torch.float32).contiguous()
+
+
+def _make_structs(x, ei, bu_ei, batch, rootindex, params, num_classes, node_id_base, xs=None, ew=(None, None)):
     n, k = xs.shape if xs is not None else x.shape
     dims = Dims(N=n, B=int(rootindex.numel()), K=k, C=num_classes, E_td=int(ei.shape[1]),
                 E_bu=int(bu_ei.shape[1]))
@@ -590,6 +609,7 @@ def _make_structs(x, ei, bu_ei, batch, rootindex, params, num_classes, node_id_b
                    rootindex=_p(rootindex), node_id_base=int(node_id_base))
     if xs is not None:
         bt.x_ptr, bt.x_col, bt.x_val = _p(xs.ptr), _p(xs.col), _p(xs.val)
+    bt.td_edge_weight, bt.bu_edge_weight = _p(ew[0]), _p(ew[1])
     pr = Params()
     for name, t in zip(_PNAMES, params):
         setattr(pr, name, _p(t))
@@ -610,10 +630,13 @@ class FeaturesFunction(torch.autograd.Function):
     x gets that gradient sampled at its stored entries -- ``val`` (= ``x_val(x)``, a SparseX's values) gets fp32 [nnz],
     a torch sparse COO x a COO gradient on ``x.coalesce()``'s indices (the ``torch.sparse.mm`` convention), a
     torch sparse CSR x a CSR gradient on its own ``crow_indices`` / ``col_indices`` (torch's ``csr @ dense``
-    returns a dense one instead: the masked form keeps the gradient as small as x)."""
+    returns a dense one instead: the masked form keeps the gradient as small as x).
+
+    ``td_ew`` / ``bu_ew`` (None, or [E_td] / [E_bu]): edge weights of both convs of that direction, as
+    ``GCNConv(x, edge_index, edge_weight)``; their gradients are formed only when they require one."""
 
     @staticmethod
-    def forward(ctx, x, val, ei, bu_ei, batch, rootindex, opts, *params):
+    def forward(ctx, x, val, ei, bu_ei, batch, rootindex, td_ew, bu_ew, opts, *params):
         L.require_device()
         ctx.x_layout = x.layout if isinstance(x, torch.Tensor) else None
         if ctx.needs_input_grad[0] and x.layout == torch.sparse_coo:
@@ -638,13 +661,19 @@ class FeaturesFunction(torch.autograd.Function):
             want = {"w1": (H, k), "b1": (H,), "w2": (H, H + k), "b2": (H,)}[name[3:]]
             if tuple(p.shape) != want:
                 raise L.BigcnError(f"{name}: expected shape {want} (hid_feats = out_feats = 64), got {tuple(p.shape)}")
-        dims, bt, pr = _make_structs(x, ei, bu_ei, batch, rootindex, params, 0, opts["node_id_base"], xs)
+        ew = (edge_weight(td_ew, int(ei.shape[1]), "edge_weight"), edge_weight(bu_ew, int(bu_ei.shape[1]), "BU_edge_weight"))
+        want_grad = opts.get("want_grad", True)
+        edge_grad = want_grad and (ctx.needs_input_grad[6] or ctx.needs_input_grad[7])
+        dims, bt, pr = _make_structs(x, ei, bu_ei, batch, rootindex, params, 0, opts["node_id_base"], xs, ew)
         o = Opts(training=int(opts["training"]), p_drop=float(opts["p"]), seed=int(opts["seed"]),
                  deg_by=L.DEG_BY[opts["deg_by"]], gemm_mode=L.GEMM_MODE[opts["gemm_mode"]],
                  dir_mask=int(opts["dir_mask"]), dense_roots=int(bool(opts.get("dense_roots", False))),
                  # inference (torch.no_grad() or no parameter wants a gradient): no column sort of x
-                 skip_wgrad_prep=int(not (opts.get("want_grad", True) and any(ctx.needs_input_grad))))
-        ws_bytes = lib().bigcn_features_workspace_bytes(C.byref(dims))
+                 skip_wgrad_prep=int(not (want_grad and any(ctx.needs_input_grad))), edge_grad=int(edge_grad))
+        if ew == (None, None):
+            ws_bytes = lib().bigcn_features_workspace_bytes(C.byref(dims))
+        else:
+            ws_bytes = lib().bigcn_features_edge_workspace_bytes(C.byref(dims), o.edge_grad)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         flags = opts.get("flags")
         if flags is None:
@@ -665,6 +694,7 @@ class FeaturesFunction(torch.autograd.Function):
         ctx.save_for_backward(*xt, ei, bu_ei, batch, rootindex, ws, *[p for p in params if p is not None])
         ctx.present = [p is not None for p in params]
         ctx.o = o
+        ctx.ew = ew
         ctx.node_id_base = opts["node_id_base"]
         ctx.flags = flags
         return feat
@@ -679,7 +709,7 @@ class FeaturesFunction(torch.autograd.Function):
         ei, bu_ei, batch, rootindex, ws = saved[1:6]
         it = iter(saved[6:])
         params = tuple(next(it) if pres else None for pres in ctx.present)
-        dims, bt, pr = _make_structs(x, ei, bu_ei, batch, rootindex, params, 0, ctx.node_id_base, xs)
+        dims, bt, pr = _make_structs(x, ei, bu_ei, batch, rootindex, params, 0, ctx.node_id_base, xs, ctx.ew)
         grads = tuple(None if p is None else torch.empty_like(p) for p in params)
         gs = Params()
         for name, t in zip(_PNAMES, grads):
@@ -688,6 +718,14 @@ class FeaturesFunction(torch.autograd.Function):
         check(lib().bigcn_features_backward(C.byref(dims), C.byref(bt), C.byref(pr), C.byref(ctx.o), _p(g),
                                             C.byref(gs), _p(ws), ws.numel(), _stream()),
               "features_backward")
+        dew = [None, None]
+        if ctx.o.edge_grad:
+            # dL/dnorm of every edge was taken by the backward; the chain through the normalisation runs here
+            for q, e in ((0, dims.E_td), (1, dims.E_bu)):
+                if ctx.needs_input_grad[6 + q] and ctx.ew[q] is not None:
+                    dew[q] = torch.empty(e, dtype=torch.float32, device=ctx.ew[q].device)
+            check(lib().bigcn_features_edge_grad(C.byref(dims), C.byref(bt), C.byref(ctx.o), _p(dew[0]), _p(dew[1]),
+                                                 _p(ws), ws.numel(), _stream()), "features_edge_grad")
         dx = dval = None
         if (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]) and xs is not None:
             # the dense gradient below sampled at the stored entries of x, in CSR order; T1cat and W1^T come from ws
@@ -713,7 +751,7 @@ class FeaturesFunction(torch.autograd.Function):
             check(lib().bigcn_features_x_grad(C.byref(dims), C.byref(pr), C.byref(ctx.o), None if bf else _p(dx),
                                               _p(dx) if bf else None, _p(scr), _p(ws), ws.numel(), _stream()),
                   "features_x_grad")
-        return (dx, dval, None, None, None, None, None) + grads
+        return (dx, dval, None, None, None, None, dew[0], dew[1], None) + grads
 
 
 class HeadFunction(torch.autograd.Function):

@@ -339,6 +339,11 @@ class FusedTrainer:
         memory) has its whole step captured into a CUDA graph: ~45 launches over four streams become one
         ``cudaGraphLaunch``, and every later step on it is a replay.  The dropout seed of a replay comes
         from the device-side calls counter, so replays draw fresh masks exactly as enqueued steps do."""
+        for d in (data, next_data):
+            if d is not None and (getattr(d, "edge_weight", None) is not None or
+                                  getattr(d, "BU_edge_weight", None) is not None):
+                raise L.BigcnError("FusedTrainer does not take edge-weighted batches (data.edge_weight / "
+                                   "data.BU_edge_weight): train them through the modules (BiGCN(data))")
         self._calls += 1
         use_graph = self.graphs and seed is None and not self.validate
         pk_any = next_data is not None or (self._prep_buf is not None and any(

@@ -48,6 +48,8 @@ extern "C" {
 #define BIGCN_FLAG_X_NOT_SPARSE 8 /* BIGCN_GEMM_SPARSE on a batch with more non-zeros than N*min(K,48):
                                      the conv1 weight gradient is NaN, use a dense gemm_mode          */
 
+#define BIGCN_FLAG_EDGE_WEIGHT 32  /* edge-weighted batch: a weight is not finite, or a node's weighted degree is
+                                      negative (its deg^-1/2 would be NaN) */
 #define BIGCN_FLAG_X_CSR_RANGE 16  /* sparse input: a column index of x is outside [0,K) (entry ignored) */
 
 /* degree convention of gcn_norm: PyG 2.x sums at the target (col); the
@@ -112,6 +114,13 @@ typedef struct bigcn_batch {
    * bigcn_train_tail / features_backward then skip graph prep, the root columns and -- BIGCN_GEMM_SPARSE -- the pass
    * over x (the product becomes a sweep over the prepared CSR, bit-identical to the fused scan). */
   void* prepared;
+  /* NULL, or the weight of every edge of the direction ([E_td] / [E_bu] fp32, aligned with edge_index /
+   * bu_edge_index): both convs of that direction then run GCNConv(x, edge_index, edge_weight) -- gcn_norm with weights
+   * (a self-loop edge in the list hands its weight to the node's loop, the last one wins; fill 1 otherwise; degree =
+   * the weighted sum).  NULL = the unweighted path, unchanged.  Needs a workspace of
+   * bigcn_features_edge_workspace_bytes and no `prepared` buffer. */
+  const float* td_edge_weight;
+  const float* bu_edge_weight;
 } bigcn_batch_t;
 
 /* Parameters in PyG-2.x state_dict layout (SURVEY.md 8b):
@@ -157,6 +166,8 @@ typedef struct bigcn_opts {
                           conv2.lin (BiGCN_Twitter.py:45-56) and its weight gradient run as tiled masked products
                           instead of walks over each tree's list of positive root columns; needs a dense x.  Same
                           forward sums in the same order either way; 0 suits bag-of-words roots */
+  int32_t edge_grad;   /* edge-weighted batch: 1 = features_backward keeps what bigcn_features_edge_grad reads (the
+                          workspace must be bigcn_features_edge_workspace_bytes(dims, 1) bytes); 0 otherwise */
 } bigcn_opts_t;
 
 const char* bigcn_last_error(void);
@@ -360,7 +371,8 @@ int bigcn_features_forward(const bigcn_dims_t* dims, const bigcn_batch_t* batch,
  * `stream` at the call.  Call it for batch i+1 right before enqueuing step i and bigcn_batch_prepare_join(stream)
  * right after step i: the HBM-bound pass over the next x then overlaps the latency-bound kernels of the current
  * step (the role of the reference's DataLoader worker processes, BiGCN_Twitter.py:168).  Capturable: fork and join
- * sit on `stream`.  Then pass the buffer as batch->prepared to the three calls of step i+1. */
+ * sit on `stream`.  Then pass the buffer as batch->prepared to the three calls of step i+1.  An edge-weighted batch
+ * (td_edge_weight / bu_edge_weight set) is refused: the buffer carries no weights. */
 size_t bigcn_batch_prepare_bytes(const bigcn_dims_t* dims);
 int bigcn_batch_prepare(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts, int32_t* flags,
                         void* prepared, size_t prepared_bytes, bigcn_stream_t stream);
@@ -371,6 +383,19 @@ int bigcn_features_backward(const bigcn_dims_t* dims, const bigcn_batch_t* batch
                             const bigcn_params_t* params, const bigcn_opts_t* opts,
                             const float* grad_feat, const bigcn_params_t* grads,
                             void* workspace, size_t workspace_bytes, bigcn_stream_t stream);
+/* Workspace of the three calls above for a batch with td_edge_weight / bu_edge_weight: the unweighted workspace, then
+ * the weighted normalisation of both directions; edge_grad = 1 adds room for the products the edge gradient reads
+ * (4 * N * 64 floats more: backward then writes T2 and G1 beside X W1^T and conv2's input instead of over them). */
+size_t bigcn_features_edge_workspace_bytes(const bigcn_dims_t* dims, int32_t edge_grad);
+/* Gradient w.r.t. the edge weights: d_td_w [E_td] / d_bu_w [E_bu] (either may be NULL; the batch must carry that
+ * direction's weights).  Call after bigcn_features_backward with the same dims, batch, opts (edge_grad = 1) and
+ * workspace.  Per direction it sums over conv1 and conv2 dL/dnorm_e = <G1[c], XW[r]> + <G2[c], M[r]> (taken by the
+ * backward) and carries it through the normalisation: dis_r dis_c dL/dnorm_e + dL/ddeg of the degree node; a self-loop
+ * edge of the list gets its node's loop gradient (every such edge, as autograd of the reference's index_put gives).
+ * Deterministic, no floating-point atomics. */
+int bigcn_features_edge_grad(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts,
+                             float* d_td_w, float* d_bu_w, void* workspace, size_t workspace_bytes,
+                             bigcn_stream_t stream);
 /* Gradient w.r.t. data.x (dense x): the reference's conv1 reads x (BiGCN_Twitter.py:42) while its root-extend reads
  * the detached copy.copy x1 (:28,45-50), so only conv1 carries one back: dX = sum over the directions of T1_d W1_d
  * with T1_d = A-hat_d^T G1_d, the matrix whose transpose product is dW1.  Call after bigcn_features_backward with the
