@@ -54,6 +54,10 @@ class Opts(C.Structure):
                 ("seed_dev", c_ptr), ("dense_roots", C.c_int32), ("edge_grad", C.c_int32)]
 
 
+class AsmWeights(C.Structure):
+    _fields_ = [(n, c_ptr) for n in ("td_weight", "bu_weight", "edge_weight", "bu_edge_weight")]
+
+
 class BigcnError(RuntimeError):
     pass
 
@@ -100,6 +104,7 @@ _SIGS = {
                                          C.c_int32, c_ptr, C.c_size_t, c_ptr]),
     "bigcn_features_workspace_bytes": (C.c_size_t, [C.POINTER(Dims)]),
     "bigcn_batch_prepare_bytes": (C.c_size_t, [C.POINTER(Dims)]),
+    "bigcn_batch_prepare_edge_bytes": (C.c_size_t, [C.POINTER(Dims)]),
     "bigcn_batch_prepare": (C.c_int, [C.POINTER(Dims), C.POINTER(BatchPtrs), C.POINTER(Opts), c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "bigcn_batch_prepare_join": (C.c_int, [c_ptr]),
     "bigcn_features_forward": (C.c_int, [C.POINTER(Dims), C.POINTER(BatchPtrs), C.POINTER(Params),
@@ -150,6 +155,10 @@ _SIGS = {
     "bigcn_assemble_batch": (C.c_int, [c_ptr] * 14 + [C.c_int64, C.c_int64, C.c_int64, C.c_uint64] + [c_ptr] * 9),
     "bigcn_assemble_batch_dense": (C.c_int, [c_ptr] * 10 + [C.c_int64, C.c_int64, C.c_int64, C.c_uint64] + [c_ptr] * 6
                                    + [C.c_int64, C.c_int32, c_ptr, c_ptr]),
+    "bigcn_assemble_batch_weighted": (C.c_int, [c_ptr] * 14 + [C.c_int64, C.c_int64, C.c_int64, C.c_uint64]
+                                      + [c_ptr] * 8 + [C.POINTER(AsmWeights), c_ptr]),
+    "bigcn_assemble_batch_dense_weighted": (C.c_int, [c_ptr] * 10 + [C.c_int64, C.c_int64, C.c_int64, C.c_uint64]
+                                            + [c_ptr] * 6 + [C.c_int64, C.c_int32, c_ptr, C.POINTER(AsmWeights), c_ptr]),
     "bigcn_dp_slice": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "bigcn_dp_reduce_adam": (C.c_int, [C.POINTER(c_ptr), C.POINTER(c_ptr), C.c_int32, C.c_int32, c_ptr, c_ptr,
                                        C.c_int64, c_ptr, c_ptr, C.c_int32, C.c_double, C.c_double, C.c_double,

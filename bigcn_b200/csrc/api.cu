@@ -291,6 +291,42 @@ static WFeatWs carve_wfeat(const bigcn_dims_t* dm, void* base, bool edge_grad) {
 }
 static bool batch_weighted(const bigcn_batch_t* bt) { return bt->td_edge_weight != nullptr || bt->bu_edge_weight != nullptr; }
 static const float* dir_edge_weight(const bigcn_batch_t* bt, int d) { return d == 0 ? bt->td_edge_weight : bt->bu_edge_weight; }
+// A weighted batch prepared ahead: bigcn_batch_prepare writes the normalisation right after the unweighted layout
+static WFeatWs carve_prepared_wfeat(const bigcn_dims_t* dm, void* prepared) {
+  const size_t base = carve_prepared(dm, nullptr, 0).total;
+  return carve_wfeat(dm, prepared ? reinterpret_cast<char*>(prepared) + base : nullptr, false);
+}
+// The weighted section a step reads: the workspace's own (features_forward fills it), with the normalisation taken from
+// the prepared buffer instead when the batch came prepared (the edge-gradient buffers stay in the workspace)
+static WFeatWs step_wfeat(const bigcn_dims_t* dm, const bigcn_batch_t* bt, void* ws, size_t feat_total, bool edge_grad) {
+  WFeatWs wf = carve_wfeat(dm, ws ? reinterpret_cast<char*>(ws) + feat_total : nullptr, edge_grad);
+  if (bt->prepared != nullptr) {
+    const WFeatWs pw = carve_prepared_wfeat(dm, bt->prepared);
+    for (int d = 0; d < 2; ++d) {
+      wf.G[d] = pw.G[d];
+      wf.in_w[d] = pw.in_w[d];
+      wf.out_w[d] = pw.out_w[d];
+    }
+    wf.ones = pw.ones;
+  }
+  return wf;
+}
+// the weighted normalisation of the active directions on top of graph prep (a direction without weights: all ones)
+static int wfeat_prep_dirs(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_opts_t* o, const WFeatWs& wf,
+                           const bigcn_graph_t* g, int32_t* flags, cudaStream_t st) {
+  const int64_t* ei[2] = {bt->edge_index, bt->bu_edge_index};
+  const int64_t E[2] = {dm->E_td, dm->E_bu};
+  if (int rc = wfeat_ones(wf.ones, E[0] > E[1] ? E[0] : E[1], st)) return rc;
+  for (int d = 0; d < 2; ++d) {
+    if (!((o->dir_mask >> d) & 1)) continue;
+    WGraph G = wf.G[d];
+    G.g = g[d];
+    const float* ew = dir_edge_weight(bt, d);
+    if (int rc = wfeat_prep(G, ei[d], E[d], ew ? ew : wf.ones, dm->N, o->deg_by, wf.in_w[d], wf.out_w[d], flags, st))
+      return rc;
+  }
+  return 0;
+}
 
 int batch_prepare_join(cudaStream_t st);
 
@@ -341,12 +377,11 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   if (int rc = check_bf16_x(dm, bt, o, "features_forward")) return rc;
   FeatWs w = carve_features(dm, ws, ws_bytes, bt->prepared);
   const bool weighted = batch_weighted(bt);
-  const WFeatWs wf = weighted ? carve_wfeat(dm, ws ? reinterpret_cast<char*>(ws) + w.total : nullptr, o->edge_grad != 0)
-                              : WFeatWs{};
+  const WFeatWs wf = weighted ? step_wfeat(dm, bt, ws, w.total, o->edge_grad != 0) : WFeatWs{};
   BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total + wf.total, "features_forward: workspace too small (%zu < %zu)",
                   ws_bytes, w.total + wf.total);
-  BIGCN_CHECK_ARG(!weighted || bt->prepared == nullptr,
-                  "features_forward: an edge-weighted batch takes no prepared buffer (bigcn_batch_prepare carries no weights)");
+  BIGCN_CHECK_ARG(!weighted || !o->edge_grad || bt->prepared == nullptr,
+                  "features_forward: opts.edge_grad takes no prepared buffer (the edge gradient runs graph prep inline)");
   const bool prepared = bt->prepared != nullptr;   // graph structure, root columns, CSR / CSC of x: already there
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const Dirs dirs = active_dirs(o->dir_mask);
@@ -376,17 +411,8 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     if (int rc = graph_prep_impl(2, ei, E, N, bt->batch, B, o->deg_by, w.g, w.node_ptr, flags, w.prep_ws,
                                  w.prep_bytes, ss, weighted ? eids : nullptr))
       return rc;
-    if (weighted) {   // the weighted normalisation of the active directions (a direction without weights: all ones)
-      if (int rc = wfeat_ones(wf.ones, E[0] > E[1] ? E[0] : E[1], ss)) return rc;
-      for (int q = 0; q < dirs.n; ++q) {
-        const int d = dirs.id[q];
-        WGraph G = wf.G[d];
-        G.g = w.g[d];
-        const float* ew = dir_edge_weight(bt, d);
-        if (int rc = wfeat_prep(G, ei[d], E[d], ew ? ew : wf.ones, N, o->deg_by, wf.in_w[d], wf.out_w[d], flags, ss))
-          return rc;
-      }
-    }
+    if (weighted)
+      if (int rc = wfeat_prep_dirs(dm, bt, o, wf, w.g, flags, ss)) return rc;
   }
   // 2. weights in the layouts the kernels stream
   const int n_out = dirs.n == 2 ? 128 : 64;
@@ -559,11 +585,12 @@ int batch_prepare(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_o
                   size_t prepared_bytes, cudaStream_t st) {
   if (int rc = check_common(dm, o, "batch_prepare")) return rc;
   if (int rc = check_bf16_x(dm, bt, o, "batch_prepare")) return rc;
-  BIGCN_CHECK_ARG(!batch_weighted(bt), "batch_prepare: an edge-weighted batch is not prepared ahead (the prepared "
-                                       "buffer carries no weights): pass it to features_forward without one");
   PrepWs w = carve_prepared(dm, prepared, prepared_bytes);
-  BIGCN_CHECK_ARG(prepared != nullptr && prepared_bytes >= w.total, "batch_prepare: buffer too small (%zu < %zu)",
-                  prepared_bytes, w.total);
+  const bool weighted = batch_weighted(bt);
+  const WFeatWs wf = weighted ? carve_prepared_wfeat(dm, prepared) : WFeatWs{};
+  BIGCN_CHECK_ARG(prepared != nullptr && prepared_bytes >= w.total + wf.total,
+                  "batch_prepare: buffer too small (%zu < %zu%s)", prepared_bytes, w.total + wf.total,
+                  weighted ? ": bigcn_batch_prepare_edge_bytes" : "");
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const bool sparse = o->gemm_mode == BIGCN_GEMM_SPARSE;
   const bool csr_in = bt->x == nullptr && N > 0;
@@ -597,12 +624,17 @@ int batch_prepare(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigcn_o
       }
     }
   }
-  // stream B: structure of both directions, then the root columns
+  // stream B: structure of both directions (an edge-weighted batch: with the edge ids, then its normalisation), then
+  // the root columns
   {
     const int64_t* ei[2] = {bt->edge_index, bt->bu_edge_index};
     const int64_t E[2] = {dm->E_td, dm->E_bu};
-    if (int rc = graph_prep_impl(2, ei, E, N, bt->batch, B, o->deg_by, w.g, w.node_ptr, flags, w.prep_ws, w.prep_bytes, pb))
+    int32_t* const eids[4] = {wf.G[0].in_eid, wf.G[0].out_eid, wf.G[1].in_eid, wf.G[1].out_eid};
+    if (int rc = graph_prep_impl(2, ei, E, N, bt->batch, B, o->deg_by, w.g, w.node_ptr, flags, w.prep_ws, w.prep_bytes, pb,
+                                 weighted ? eids : nullptr))
       return rc;
+    if (weighted)
+      if (int rc = wfeat_prep_dirs(dm, bt, o, wf, w.g, flags, pb)) return rc;
     RootNzArgs a{bt->x, bt->rootindex, N, B, K, w.rnz_cnt, w.rnz_col, w.rnz_val, flags, w.slot, w.overflow, DW2B_CAP,
                  o->gemm_mode == BIGCN_GEMM_BF16};
     if (csr_in) {
@@ -632,9 +664,9 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
   FeatWs w = carve_features(dm, ws, ws_bytes, bt->prepared);
   const bool weighted = batch_weighted(bt);
   const bool edge_grad = weighted && o->edge_grad != 0;
-  const WFeatWs wf = weighted ? carve_wfeat(dm, ws ? reinterpret_cast<char*>(ws) + w.total : nullptr, edge_grad)
-                              : WFeatWs{};
+  const WFeatWs wf = weighted ? step_wfeat(dm, bt, ws, w.total, edge_grad) : WFeatWs{};
   BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total + wf.total, "features_backward: workspace too small");
+  BIGCN_CHECK_ARG(!edge_grad || bt->prepared == nullptr, "features_backward: opts.edge_grad takes no prepared buffer");
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const Dirs dirs = active_dirs(o->dir_mask);
   const int n_out = dirs.n == 2 ? 128 : 64;
@@ -931,7 +963,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 105; }
+extern "C" int bigcn_version(void) { return 106; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
@@ -1016,6 +1048,7 @@ extern "C" int bigcn_features_edge_grad(const bigcn_dims_t* dims, const bigcn_ba
   if (int rc = check_common(dims, opts, "features_edge_grad")) return rc;
   BIGCN_CHECK_ARG(batch != nullptr, "features_edge_grad: NULL batch");
   BIGCN_CHECK_ARG(opts->edge_grad != 0, "features_edge_grad: needs opts.edge_grad = 1 in the forward and backward calls");
+  BIGCN_CHECK_ARG(batch->prepared == nullptr, "features_edge_grad: opts.edge_grad takes no prepared buffer");
   const FeatWs w = carve_features(dims, workspace, workspace_bytes);
   const WFeatWs wf = carve_wfeat(dims, workspace ? reinterpret_cast<char*>(workspace) + w.total : nullptr, true);
   BIGCN_CHECK_ARG(workspace != nullptr && workspace_bytes >= w.total + wf.total,
@@ -1044,6 +1077,10 @@ extern "C" int bigcn_features_edge_grad(const bigcn_dims_t* dims, const bigcn_ba
 extern "C" size_t bigcn_batch_prepare_bytes(const bigcn_dims_t* dims) {
   if (!dims) return 0;
   return carve_prepared(dims, nullptr, 0).total;
+}
+extern "C" size_t bigcn_batch_prepare_edge_bytes(const bigcn_dims_t* dims) {
+  if (!dims) return 0;
+  return carve_prepared(dims, nullptr, 0).total + carve_prepared_wfeat(dims, nullptr).total;
 }
 extern "C" int bigcn_batch_prepare(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts,
                                    int32_t* flags, void* prepared, size_t prepared_bytes, bigcn_stream_t stream) {

@@ -46,6 +46,9 @@ struct AsmArgs {
   int32_t* ox_ptr;           // [N+1]
   int32_t* ox_col;
   float* ox_val;
+  // edge weights (k_asm_edges<true> only), as bit patterns: copied, never converted
+  const uint32_t* ew_all[2]; // [E_all] per tree edge: TD, BU
+  uint32_t* ew[2];           // [E_td], [E_bu] per kept edge, aligned with edge_index / bu_edge_index
 };
 
 // nodes, features, labels: CTA per tree
@@ -85,6 +88,7 @@ __global__ void __launch_bounds__(256) k_asm_nodes(AsmArgs a) {
 // the k-th smallest key v; positions with key < v are kept, plus the first ones with key == v
 // until k are kept (ties, ~e^2 / 2^33 likely, resolved by position); an ordered block scan
 // compacts the kept edges.  Every k-subset is equally likely (up to those ties).
+// Weighted (W): the kept edge's weight goes to the same output position as the edge, in the same launch.
 constexpr int DE_MAX = 8192;   // edges per tree handled in shared memory (32 KB of keys)
 
 __device__ __forceinline__ uint32_t edge_key(const AsmArgs& a, int64_t t, int dir, int64_t i) {
@@ -103,6 +107,7 @@ __device__ __forceinline__ int block_sum128(int v, int* red) {   // 128 threads,
   return red[0] + red[1] + red[2] + red[3];
 }
 
+template <bool W>
 __global__ void __launch_bounds__(128) k_asm_edges(AsmArgs a) {
   __shared__ uint32_t key[DE_MAX];
   __shared__ int red[4];
@@ -122,6 +127,7 @@ __global__ void __launch_bounds__(128) k_asm_edges(AsmArgs a) {
     const int64_t s = a.edge_src[e0 + i] + noff, d = a.edge_dst[e0 + i] + noff;
     out[o0 + pos] = dir ? d : s;
     out[E + o0 + pos] = dir ? s : d;
+    if constexpr (W) a.ew[dir][o0 + pos] = a.ew_all[dir][e0 + i];
   };
   if (k >= e) {   // rate 0 (or nothing to drop): plain offset copy
     for (int i = threadIdx.x; i < e; i += 128) emit(i, i);
@@ -272,14 +278,30 @@ __global__ void __launch_bounds__(DR_THREADS) k_asm_dense_rows(DenseRowArgs a) {
 
 using namespace bigcn;
 
-extern "C" int bigcn_assemble_batch(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
-                                    const int32_t* edge_dst, const int64_t* x_ptr, const int32_t* x_col,
-                                    const float* x_val, const int32_t* root_local, const int64_t* y_all,
-                                    const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
-                                    const int64_t* bu_off, const int64_t* nnz_off, int64_t B, int64_t E_td,
-                                    int64_t E_bu, uint64_t seed, int64_t* edge_index, int64_t* bu_edge_index,
-                                    int64_t* batch, int64_t* rootindex, int64_t* y, int32_t* ox_ptr, int32_t* ox_col,
-                                    float* ox_val, bigcn_stream_t stream) {
+// weights (NULL = unweighted): checked, then laid into the assembly arguments
+static int asm_weights(AsmArgs& a, const bigcn_asm_weights_t* w, const char* who) {
+  if (w == nullptr) return 0;
+  BIGCN_CHECK_ARG(w->td_weight && (a.E_td == 0 || w->edge_weight) && (a.E_bu == 0 || w->bu_edge_weight),
+                  "%s: NULL weight array (td_weight, and an output for every non-empty direction)", who);
+  a.ew_all[0] = reinterpret_cast<const uint32_t*>(w->td_weight);
+  a.ew_all[1] = reinterpret_cast<const uint32_t*>(w->bu_weight ? w->bu_weight : w->td_weight);
+  a.ew[0] = reinterpret_cast<uint32_t*>(w->edge_weight);
+  a.ew[1] = reinterpret_cast<uint32_t*>(w->bu_edge_weight);
+  return 0;
+}
+static void asm_edges_launch(const AsmArgs& a, bool weighted, cudaStream_t st) {
+  if (weighted) k_asm_edges<true><<<(unsigned)(2 * a.B), 128, 0, st>>>(a);
+  else k_asm_edges<false><<<(unsigned)(2 * a.B), 128, 0, st>>>(a);
+}
+
+static int assemble_csr(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                        const int32_t* edge_dst, const int64_t* x_ptr, const int32_t* x_col,
+                        const float* x_val, const int32_t* root_local, const int64_t* y_all,
+                        const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                        const int64_t* bu_off, const int64_t* nnz_off, int64_t B, int64_t E_td,
+                        int64_t E_bu, uint64_t seed, int64_t* edge_index, int64_t* bu_edge_index,
+                        int64_t* batch, int64_t* rootindex, int64_t* y, int32_t* ox_ptr, int32_t* ox_col,
+                        float* ox_val, const bigcn_asm_weights_t* w, bigcn_stream_t stream) {
   BIGCN_CHECK_ARG(B >= 0 && E_td >= 0 && E_bu >= 0, "assemble_batch: bad sizes");
   if (B == 0) return 0;
   BIGCN_CHECK_ARG(node_ptr && edge_ptr && x_ptr && root_local && y_all && tree_id && node_off && td_off && bu_off &&
@@ -293,21 +315,22 @@ extern "C" int bigcn_assemble_batch(const int64_t* node_ptr, const int64_t* edge
   a.k0 = (uint32_t)(seed & 0xffffffffull); a.k1 = (uint32_t)(seed >> 32);
   a.edge_index = edge_index; a.bu_edge_index = bu_edge_index; a.batch = batch; a.rootindex = rootindex; a.y = y;
   a.ox_ptr = ox_ptr; a.ox_col = ox_col; a.ox_val = ox_val;
+  if (int rc = asm_weights(a, w, "assemble_batch")) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   k_asm_nodes<<<(unsigned)B, 256, 0, st>>>(a);
   BIGCN_CHECK_LAUNCH("k_asm_nodes");
-  k_asm_edges<<<(unsigned)(2 * B), 128, 0, st>>>(a);
+  asm_edges_launch(a, w != nullptr, st);
   BIGCN_CHECK_LAUNCH("k_asm_edges");
   return 0;
 }
 
-extern "C" int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
-                                          const int32_t* edge_dst, const int32_t* root_local, const int64_t* y_all,
-                                          const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
-                                          const int64_t* bu_off, int64_t B, int64_t E_td, int64_t E_bu, uint64_t seed,
-                                          int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch,
-                                          int64_t* rootindex, int64_t* y, const void* x_all, int64_t K,
-                                          int32_t elem_bytes, void* ox, bigcn_stream_t stream) {
+static int assemble_dense(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                          const int32_t* edge_dst, const int32_t* root_local, const int64_t* y_all,
+                          const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                          const int64_t* bu_off, int64_t B, int64_t E_td, int64_t E_bu, uint64_t seed,
+                          int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch,
+                          int64_t* rootindex, int64_t* y, const void* x_all, int64_t K,
+                          int32_t elem_bytes, void* ox, const bigcn_asm_weights_t* w, bigcn_stream_t stream) {
   BIGCN_CHECK_ARG(B >= 0 && E_td >= 0 && E_bu >= 0, "assemble_batch_dense: bad sizes");
   BIGCN_CHECK_ARG(elem_bytes == 2 || elem_bytes == 4,
                   "assemble_batch_dense: elem_bytes must be 2 (bf16) or 4 (fp32), got %d", (int)elem_bytes);
@@ -326,6 +349,7 @@ extern "C" int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t
   a.B = B; a.E_td = E_td; a.E_bu = E_bu;
   a.k0 = (uint32_t)(seed & 0xffffffffull); a.k1 = (uint32_t)(seed >> 32);
   a.edge_index = edge_index; a.bu_edge_index = bu_edge_index; a.batch = batch; a.rootindex = rootindex; a.y = y;
+  if (int rc = asm_weights(a, w, "assemble_batch_dense")) return rc;
   // the largest unit (16, 4 or 2 bytes) that divides the row bytes and both base addresses
   const uint64_t row_bytes = (uint64_t)K * (uint64_t)elem_bytes;
   const uint64_t align = row_bytes | (uint64_t)(uintptr_t)x_all | (uint64_t)(uintptr_t)ox;
@@ -357,7 +381,62 @@ extern "C" int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t
     else k_asm_dense_rows<uint16_t><<<grid, DR_THREADS, 0, st>>>(d);
     BIGCN_CHECK_LAUNCH("k_asm_dense_rows");
   }
-  k_asm_edges<<<(unsigned)(2 * B), 128, 0, st>>>(a);
+  asm_edges_launch(a, w != nullptr, st);
   BIGCN_CHECK_LAUNCH("k_asm_edges");
   return 0;
+}
+
+extern "C" int bigcn_assemble_batch(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                                    const int32_t* edge_dst, const int64_t* x_ptr, const int32_t* x_col,
+                                    const float* x_val, const int32_t* root_local, const int64_t* y_all,
+                                    const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                                    const int64_t* bu_off, const int64_t* nnz_off, int64_t B, int64_t E_td,
+                                    int64_t E_bu, uint64_t seed, int64_t* edge_index, int64_t* bu_edge_index,
+                                    int64_t* batch, int64_t* rootindex, int64_t* y, int32_t* ox_ptr, int32_t* ox_col,
+                                    float* ox_val, bigcn_stream_t stream) {
+  return assemble_csr(node_ptr, edge_ptr, edge_src, edge_dst, x_ptr, x_col, x_val, root_local, y_all, tree_id, node_off,
+                      td_off, bu_off, nnz_off, B, E_td, E_bu, seed, edge_index, bu_edge_index, batch, rootindex, y, ox_ptr,
+                      ox_col, ox_val, nullptr, stream);
+}
+
+extern "C" int bigcn_assemble_batch_weighted(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                                             const int32_t* edge_dst, const int64_t* x_ptr, const int32_t* x_col,
+                                             const float* x_val, const int32_t* root_local, const int64_t* y_all,
+                                             const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                                             const int64_t* bu_off, const int64_t* nnz_off, int64_t B, int64_t E_td,
+                                             int64_t E_bu, uint64_t seed, int64_t* edge_index, int64_t* bu_edge_index,
+                                             int64_t* batch, int64_t* rootindex, int64_t* y, int32_t* ox_ptr,
+                                             int32_t* ox_col, float* ox_val, const bigcn_asm_weights_t* weights,
+                                             bigcn_stream_t stream) {
+  BIGCN_CHECK_ARG(weights != nullptr, "assemble_batch_weighted: NULL weights (bigcn_assemble_batch takes none)");
+  return assemble_csr(node_ptr, edge_ptr, edge_src, edge_dst, x_ptr, x_col, x_val, root_local, y_all, tree_id, node_off,
+                      td_off, bu_off, nnz_off, B, E_td, E_bu, seed, edge_index, bu_edge_index, batch, rootindex, y, ox_ptr,
+                      ox_col, ox_val, weights, stream);
+}
+
+extern "C" int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                                          const int32_t* edge_dst, const int32_t* root_local, const int64_t* y_all,
+                                          const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                                          const int64_t* bu_off, int64_t B, int64_t E_td, int64_t E_bu, uint64_t seed,
+                                          int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch,
+                                          int64_t* rootindex, int64_t* y, const void* x_all, int64_t K,
+                                          int32_t elem_bytes, void* ox, bigcn_stream_t stream) {
+  return assemble_dense(node_ptr, edge_ptr, edge_src, edge_dst, root_local, y_all, tree_id, node_off, td_off, bu_off, B,
+                        E_td, E_bu, seed, edge_index, bu_edge_index, batch, rootindex, y, x_all, K, elem_bytes, ox, nullptr,
+                        stream);
+}
+
+extern "C" int bigcn_assemble_batch_dense_weighted(const int64_t* node_ptr, const int64_t* edge_ptr,
+                                                   const int32_t* edge_src, const int32_t* edge_dst,
+                                                   const int32_t* root_local, const int64_t* y_all,
+                                                   const int64_t* tree_id, const int64_t* node_off,
+                                                   const int64_t* td_off, const int64_t* bu_off, int64_t B, int64_t E_td,
+                                                   int64_t E_bu, uint64_t seed, int64_t* edge_index,
+                                                   int64_t* bu_edge_index, int64_t* batch, int64_t* rootindex,
+                                                   int64_t* y, const void* x_all, int64_t K, int32_t elem_bytes,
+                                                   void* ox, const bigcn_asm_weights_t* weights, bigcn_stream_t stream) {
+  BIGCN_CHECK_ARG(weights != nullptr, "assemble_batch_dense_weighted: NULL weights (bigcn_assemble_batch_dense takes none)");
+  return assemble_dense(node_ptr, edge_ptr, edge_src, edge_dst, root_local, y_all, tree_id, node_off, td_off, bu_off, B,
+                        E_td, E_bu, seed, edge_index, bu_edge_index, batch, rootindex, y, x_all, K, elem_bytes, ox, weights,
+                        stream);
 }

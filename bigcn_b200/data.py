@@ -267,7 +267,7 @@ def make_device_forest(n_trees: int, nodes_per_tree: int, device, seed: int = 0,
 
 
 def synth_forest_device(shape: str, n_trees: int, device, seed: int = 0, in_feats: int | None = None,
-                        num_classes: int | None = None):
+                        num_classes: int | None = None, edge_weights: bool = False):
     """A whole synthetic DATASET generated on the device in a few vectorised passes (the per-tree Python
     generators above take minutes for Weibo's 3.7 M nodes or the 1 M-tree scale-out config): tree sizes of
     SURVEY.md 8(d), hub-heavy random recursive topology (parent of local node i = floor(u^2 * i)), the root at a
@@ -275,7 +275,8 @@ def synth_forest_device(shape: str, n_trees: int, device, seed: int = 0, in_feat
     (parent, child), BoW rows of 1+Poisson(12) distinct Zipf-ish columns with counts 1..3 (kept as CSR) or,
     for PHEME, dense tanh(N(0,1)) rows.  Returns a dict of device tensors + host size arrays:
     node_ptr / edge_ptr (host int64 [T+1]), edge_src / edge_dst (int32, local ids), root_local, y, and either
-    x_ptr / x_col / x_val (CSR over all nodes) or x (dense [N, K])."""
+    x_ptr / x_col / x_val (CSR over all nodes) or x (dense [N, K]).  ``edge_weights``: also ``edge_weight``, one fp32
+    weight in (0, 1] per tree edge (drawn after everything else: the other arrays are those of the unweighted call)."""
     spec = SHAPES[shape]
     k = spec["in_feats"] if in_feats is None else in_feats
     c = spec["num_classes"] if num_classes is None else num_classes
@@ -308,7 +309,7 @@ def synth_forest_device(shape: str, n_trees: int, device, seed: int = 0, in_feat
                in_feats=k, num_classes=c, sizes=sizes)
     if shape == "pheme":
         out["x"] = torch.tanh(torch.randn(n, k, device=device, generator=g))
-        return out
+        return _synth_edge_weights(out, g, device) if edge_weights else out
     nnz = 1 + torch.poisson(torch.full((n,), 12.0, device=device), generator=g).to(torch.int64)
     rows = torch.repeat_interleave(torch.arange(n, device=device), nnz)
     uz = torch.rand(rows.numel(), device=device, generator=g, dtype=torch.float64).clamp_(min=1e-12)
@@ -320,12 +321,19 @@ def synth_forest_device(shape: str, n_trees: int, device, seed: int = 0, in_feat
     x_ptr[1:] = torch.cumsum(torch.bincount(rows, minlength=n), 0)
     out.update(x_ptr=x_ptr, x_col=cols.to(torch.int32),
                x_val=torch.randint(1, 4, (cols.numel(),), device=device, generator=g).to(torch.float32))
+    return _synth_edge_weights(out, g, device) if edge_weights else out
+
+
+def _synth_edge_weights(out, g, device):
+    e_all = int(out["edge_ptr"][-1])
+    out["edge_weight"] = 1.0 - torch.rand(e_all, device=device, generator=g)     # (0, 1]
     return out
 
 
 def forest_slice_batch(f: dict, t0: int, t1: int) -> Batch:
     """Trees [t0, t1) of a ``synth_forest_device`` dataset with DENSE features as one collated batch on the device
-    (no DropEdge: the test split of Process/process.py:63); x is a view of the dataset's rows."""
+    (no DropEdge: the test split of Process/process.py:63); x is a view of the dataset's rows.  A weighted dataset's
+    batch carries the trees' ``edge_weight`` (a view) on both directions."""
     node_ptr, edge_ptr = f["node_ptr"], f["edge_ptr"]
     n0, n1, e0, e1 = int(node_ptr[t0]), int(node_ptr[t1]), int(edge_ptr[t0]), int(edge_ptr[t1])
     dev = f["edge_src"].device
@@ -334,6 +342,9 @@ def forest_slice_batch(f: dict, t0: int, t1: int) -> Batch:
     etree = torch.repeat_interleave(torch.arange(t1 - t0, device=dev), torch.clamp(sizes - 1, min=0))
     off = starts[etree]
     ei = torch.stack([f["edge_src"][e0:e1].to(torch.int64) + off, f["edge_dst"][e0:e1].to(torch.int64) + off])
+    extra = {}
+    if "edge_weight" in f:
+        extra = {"edge_weight": f["edge_weight"][e0:e1], "BU_edge_weight": f["edge_weight"][e0:e1]}
     return Batch(x=f["x"][n0:n1], edge_index=ei, BU_edge_index=ei.flip(0).contiguous(),
                  batch=torch.repeat_interleave(torch.arange(t1 - t0, device=dev), sizes),
-                 rootindex=starts + f["root_local"][t0:t1].to(torch.int64), y=f["y"][t0:t1])
+                 rootindex=starts + f["root_local"][t0:t1].to(torch.int64), y=f["y"][t0:t1], **extra)

@@ -11,6 +11,8 @@ call into libbigcn_b200.so.
 """
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
 import torch
 
@@ -34,13 +36,27 @@ def _dense_storage(x, n, k):
     return x.contiguous()
 
 
+def _weight_storage(w, e_all, name, dev):
+    """per-tree-edge weights kept as they are: fp32 [e_all] on the device, or None"""
+    if w is None:
+        return None
+    w = torch.as_tensor(w)
+    if w.dtype != torch.float32 or tuple(w.shape) != (e_all,):
+        raise L.BigcnError(f"DeviceForest: {name} must be torch.float32 [{e_all}] (one weight per tree edge), got "
+                           f"{w.dtype} {tuple(w.shape)}")
+    return w.to(dev).contiguous()
+
+
 class DeviceForest:
     def __init__(self, node_ptr, edge_ptr, edge_src, edge_dst, x_ptr, x_col, x_val, root_local, y, in_feats, device,
-                 x=None):
+                 x=None, edge_weight=None, bu_edge_weight=None):
         """Trees packed back to back: node_ptr / edge_ptr [T+1], the local edge lists edge_src / edge_dst
         ([parent; child]), root_local and y per tree, and the features of all nodes, either as CSR (x_ptr [N_all+1],
         x_col, x_val) or -- ``x`` given, the CSR arguments None -- as dense rows [N_all, in_feats] of torch.float32
-        or torch.bfloat16 on the device, which ``batch()`` gathers into a dense ``data.x`` of the same dtype."""
+        or torch.bfloat16 on the device, which ``batch()`` gathers into a dense ``data.x`` of the same dtype.
+        ``edge_weight``: None, or one torch.float32 weight per tree edge [E_all], aligned with edge_src / edge_dst; a
+        batch then carries ``edge_weight`` / ``BU_edge_weight`` for the edges each direction kept.  ``bu_edge_weight``:
+        the BU list's own weights for the same tree edges (default: ``edge_weight``, one weight seen from either end)."""
         # host copies of the (small) size arrays: batch offsets are computed without touching the device
         self.h_node_ptr = np.asarray(node_ptr, np.int64)
         self.h_edge_ptr = np.asarray(edge_ptr, np.int64)
@@ -59,19 +75,29 @@ class DeviceForest:
             self.x = _dense_storage(x, int(self.h_node_ptr[-1]), self.in_feats)
         self.root_local, self.y = t(root_local, torch.int32), t(y, torch.int64)
         self.num_trees = len(self.h_node_ptr) - 1
+        self._set_weights(edge_weight, bu_edge_weight)
         self._stage, self._turn = None, 0
         self._cache_ptrs()
 
+    def _set_weights(self, edge_weight, bu_edge_weight):
+        e_all = int(self.h_edge_ptr[-1])
+        self.edge_weight = _weight_storage(edge_weight, e_all, "edge_weight", self.device)
+        self.bu_edge_weight = _weight_storage(bu_edge_weight, e_all, "bu_edge_weight", self.device)
+        if self.edge_weight is None and self.bu_edge_weight is not None:
+            raise L.BigcnError("DeviceForest: bu_edge_weight needs edge_weight (the TD weights of the same edges)")
+
     def _cache_ptrs(self):
         # the dataset arrays never move: their addresses are looked up once, not on every batch
-        for k in ("node_ptr", "edge_ptr", "edge_src", "edge_dst", "x_ptr", "x_col", "x_val", "x", "root_local", "y"):
+        for k in ("node_ptr", "edge_ptr", "edge_src", "edge_dst", "x_ptr", "x_col", "x_val", "x", "root_local", "y",
+                  "edge_weight", "bu_edge_weight"):
             setattr(self, "_p_" + k, _p(getattr(self, k)))
 
     @staticmethod
     def from_device_arrays(f):
         """From ``data.synth_forest_device``: everything already sits on the device; only the size arrays live on the
         host.  Features stay in the form ``f`` holds them: dense rows when it has ``"x"`` (PHEME; fp32, or bf16 after
-        ``f["x"] = f["x"].to(torch.bfloat16)``), CSR otherwise."""
+        ``f["x"] = f["x"].to(torch.bfloat16)``), CSR otherwise.  ``f["edge_weight"]`` (optional): the per-tree-edge
+        weights (``synth_forest_device(..., edge_weights=True)``)."""
         self = DeviceForest.__new__(DeviceForest)
         dev = f["edge_src"].device
         self.h_node_ptr = np.asarray(f["node_ptr"], np.int64)
@@ -89,6 +115,7 @@ class DeviceForest:
             self.x = None
         self.root_local, self.y = f["root_local"], f["y"].to(torch.int64)
         self.num_trees = len(self.h_node_ptr) - 1
+        self._set_weights(f.get("edge_weight"), None)
         self._stage, self._turn = None, 0
         self._cache_ptrs()
         return self
@@ -99,7 +126,8 @@ class DeviceForest:
         edge_index [2,e] = [parent; child] WITHOUT DropEdge, rootindex, y).  ``features``: 'csr' keeps the non-zeros
         of every row (bag-of-words features; ``data.x`` of a batch is a SparseX); 'dense' keeps the rows as they are,
         in ``dtype`` (torch.float32 or torch.bfloat16; a SparseX tree is densified here, once), and a batch's
-        ``data.x`` is a dense tensor of that dtype."""
+        ``data.x`` is a dense tensor of that dtype.  ``d.edge_weight`` (one weight per column of ``d.edge_index``), on
+        every tree or on none, is kept as the forest's ``edge_weight``."""
         if features not in ("csr", "dense"):
             raise L.BigcnError(f"DeviceForest: features must be 'csr' or 'dense', got {features!r}")
         dense = features == "dense"
@@ -107,6 +135,17 @@ class DeviceForest:
             raise L.BigcnError(f"DeviceForest: dense features are stored as torch.float32 or torch.bfloat16, got {dtype}")
         node_ptr, edge_ptr, x_ptr = [0], [0], [0]
         es, ed, xc, xv, xd, roots, ys = [], [], [], [], [], [], []
+        trees = list(trees)
+        ws = [getattr(d, "edge_weight", None) for d in trees]
+        weighted = any(w is not None for w in ws)
+        if weighted and any(w is None for w in ws):
+            raise L.BigcnError("DeviceForest: edge_weight must be given on every tree or on none")
+        for i, (d, w) in enumerate(zip(trees, ws)):
+            if weighted and tuple(torch.as_tensor(w).shape) != (int(d.edge_index.shape[1]),):
+                raise L.BigcnError(f"DeviceForest: tree {i}: edge_weight must be [{int(d.edge_index.shape[1])}] (one weight "
+                                   f"per edge), got {tuple(torch.as_tensor(w).shape)}")
+        ew = torch.cat([torch.as_tensor(w).detach().cpu().to(torch.float32).reshape(-1) for w in ws]) \
+            if weighted and trees else (torch.zeros(0, dtype=torch.float32) if weighted else None)
         k = None
         for d in trees:
             x = d.x
@@ -136,9 +175,9 @@ class DeviceForest:
         cat = lambda xs, dt: np.concatenate(xs).astype(dt) if xs else np.zeros(0, dt)  # noqa: E731
         if dense:
             return DeviceForest(node_ptr, edge_ptr, cat(es, np.int32), cat(ed, np.int32), None, None, None, roots, ys, k,
-                                device, x=torch.cat(xd).to(device))
+                                device, x=torch.cat(xd).to(device), edge_weight=ew)
         return DeviceForest(node_ptr, edge_ptr, cat(es, np.int32), cat(ed, np.int32), x_ptr, cat(xc, np.int32),
-                            cat(xv, np.float32), roots, ys, k, device)
+                            cat(xv, np.float32), roots, ys, k, device, edge_weight=ew)
 
     @staticmethod
     def from_npz_dir(fold_x, data_path, device, treeDic=None, lower=2, upper=100000, features="csr",
@@ -180,7 +219,8 @@ class DeviceForest:
         """The collated batch of ``tree_ids`` (host sequence, in batch order) with DropEdge at the
         given rates, on the device; ``data.x`` is a SparseX for CSR storage, a fresh contiguous [n, in_feats] tensor
         of the storage dtype for dense storage.  DropEdge draws depend only on the seed, the tree id, the direction and
-        the edge position: both storage forms give the same edges for the same ids and seed."""
+        the edge position: both storage forms give the same edges for the same ids and seed, and so does a weighted
+        forest, whose batches also carry ``edge_weight`` / ``BU_edge_weight`` (fp32, the kept edges' weights in order)."""
         L.require_device()
         ids = np.asarray(tree_ids, np.int64)
         b = len(ids)
@@ -230,26 +270,39 @@ class DeviceForest:
         cur = torch.cuda.current_stream(dev)
         base, pitch = slot[0].data_ptr(), 8 * (b + 1)
         seed = int(seed) & ((1 << 64) - 1)
+        extra = {}
+        aw = None
+        if self.edge_weight is not None:      # the kept edges' weights: one fp32 block [TD | BU]
+            wblk = torch.empty(e_td + e_bu, dtype=torch.float32, device=dev)
+            extra = {"edge_weight": wblk[:e_td], "BU_edge_weight": wblk[e_td:]}
+            aw = L.AsmWeights(td_weight=self._p_edge_weight, bu_weight=self._p_bu_edge_weight,
+                              edge_weight=_p(extra["edge_weight"]), bu_edge_weight=_p(extra["BU_edge_weight"]))
         if dense:
             x = torch.empty(n, self.in_feats, dtype=self.x.dtype, device=dev)
-            check(lib().bigcn_assemble_batch_dense(self._p_node_ptr, self._p_edge_ptr, self._p_edge_src,
-                                                   self._p_edge_dst, self._p_root_local, self._p_y, base, base + pitch,
-                                                   base + 2 * pitch, base + 3 * pitch, b, e_td, e_bu, seed, _p(ei),
-                                                   _p(bu), _p(batch), _p(root), _p(y), self._p_x, self.in_feats,
-                                                   self.x.element_size(), _p(x), cur.cuda_stream), "assemble_batch_dense")
+            args = (self._p_node_ptr, self._p_edge_ptr, self._p_edge_src, self._p_edge_dst, self._p_root_local, self._p_y,
+                    base, base + pitch, base + 2 * pitch, base + 3 * pitch, b, e_td, e_bu, seed, _p(ei), _p(bu), _p(batch),
+                    _p(root), _p(y), self._p_x, self.in_feats, self.x.element_size(), _p(x))
+            if aw is None:
+                check(lib().bigcn_assemble_batch_dense(*args, cur.cuda_stream), "assemble_batch_dense")
+            else:
+                check(lib().bigcn_assemble_batch_dense_weighted(*args, C.byref(aw), cur.cuda_stream),
+                      "assemble_batch_dense_weighted")
         else:
             iblk = torch.empty(n + 1 + 2 * nnz, dtype=torch.int32, device=dev)
             if b == 0:
                 iblk.zero_()
             ox_ptr, ox_col = iblk[:n + 1], iblk[n + 1:n + 1 + nnz]
             ox_val = iblk[n + 1 + nnz:].view(torch.float32)
-            check(lib().bigcn_assemble_batch(self._p_node_ptr, self._p_edge_ptr, self._p_edge_src, self._p_edge_dst,
-                                             self._p_x_ptr, self._p_x_col, self._p_x_val, self._p_root_local, self._p_y,
-                                             base, base + pitch, base + 2 * pitch, base + 3 * pitch, base + 4 * pitch,
-                                             b, e_td, e_bu, seed, _p(ei), _p(bu), _p(batch), _p(root),
-                                             _p(y), _p(ox_ptr), _p(ox_col), _p(ox_val), cur.cuda_stream), "assemble_batch")
+            args = (self._p_node_ptr, self._p_edge_ptr, self._p_edge_src, self._p_edge_dst, self._p_x_ptr, self._p_x_col,
+                    self._p_x_val, self._p_root_local, self._p_y, base, base + pitch, base + 2 * pitch, base + 3 * pitch,
+                    base + 4 * pitch, b, e_td, e_bu, seed, _p(ei), _p(bu), _p(batch), _p(root), _p(y), _p(ox_ptr),
+                    _p(ox_col), _p(ox_val))
+            if aw is None:
+                check(lib().bigcn_assemble_batch(*args, cur.cuda_stream), "assemble_batch")
+            else:
+                check(lib().bigcn_assemble_batch_weighted(*args, C.byref(aw), cur.cuda_stream), "assemble_batch_weighted")
             x = SparseX(ox_ptr, ox_col, ox_val, (n, self.in_feats))
         if slot[1] is None:
             slot[1] = torch.cuda.Event()
         slot[1].record(cur)
-        return Batch(x=x, edge_index=ei, BU_edge_index=bu, batch=batch, rootindex=root, y=y)
+        return Batch(x=x, edge_index=ei, BU_edge_index=bu, batch=batch, rootindex=root, y=y, **extra)

@@ -15,7 +15,7 @@ import torch
 
 from . import _lib as L
 from ._lib import H, Opts, Params, check, lib
-from .ops import _make_structs, _p, _stream, _i64, _f32, _as_x, capture_graph, raise_on_flags, step_stream
+from .ops import _make_structs, _p, _stream, _i64, _f32, _as_x, capture_graph, edge_weight, raise_on_flags, step_stream
 
 # flat layout: the two conv1 weights (the gradients the second X stream produces LAST) first, so
 # the gradient splits into two contiguous all-reduce buckets: [W1_td | W1_bu] and [everything else]
@@ -35,7 +35,7 @@ class FusedTrainer:
 
     def __init__(self, model, lr=5e-4, weight_decay=1e-4, betas=(0.9, 0.999), eps=1e-8,
                  process_group=None, world_size=1, validate=False, comm="auto", graphs="auto", max_graphs=16,
-                 fused_sync=True, dp_push=True):
+                 fused_sync=True, dp_push=True, edge_weights=False):
         """``comm`` (world_size > 1): "symm" = one fused kernel over NVLink peer memory
         (reduce-scatter of the gradients in rank order + Adam on the owned shard + all-gather of
         the parameters, bigcn_dp_reduce_adam) between two symmetric-memory barriers; "nccl" = two
@@ -45,12 +45,17 @@ class FusedTrainer:
         "auto" = on for a single GPU and for comm="symm", off for the NCCL path whose collectives
         run on NCCL's own stream); at most ``max_graphs`` batches are kept captured.
         ``fused_sync`` (comm="symm"): the two cross-rank barriers around the optimiser kernel happen inside it
-        (release / acquire on signal words in symmetric memory) instead of as two more launches."""
+        (release / acquire on signal words in symmetric memory) instead of as two more launches.
+        ``edge_weights``: True = ``step`` takes batches that carry ``data.edge_weight`` (TD) and / or
+        ``data.BU_edge_weight`` (BU), both convs of a direction weighted as ``GCNConv(x, edge_index, edge_weight)``; their
+        normalisation is prepared a step ahead with the rest of ``next_data``.  The weights get no gradient here (one that
+        requires grad is refused: train it through the modules).  False = such a batch is refused."""
         L.require_device()
         self.model = model
         self.lr, self.wd, self.betas, self.eps = lr, weight_decay, betas, eps
         self.pg, self.world = process_group, world_size
         self.validate = validate
+        self.edge_weights = bool(edge_weights)
         self.fused_sync = bool(fused_sync)     # comm="symm": cross-rank barriers inside the optimiser kernel
         self.dp_push = bool(dp_push)           # ... and gradient slices pushed to their owners (peer stores) instead of pulled
         self.raise_priority = False            # enqueued (not replayed) steps without a prepared batch: stay on the caller's stream
@@ -154,8 +159,9 @@ class FusedTrainer:
                 self._stage, self._hst = stage, hst
                 self._stptrs = (C.c_void_p * self.world)(*[int(p) for p in hst.buffer_ptrs])
 
-    def _workspace(self, dims, dev):
-        need = lib().bigcn_features_workspace_bytes(C.byref(dims))
+    def _workspace(self, dims, dev, weighted=False):
+        need = lib().bigcn_features_edge_workspace_bytes(C.byref(dims), 0) if weighted else \
+            lib().bigcn_features_workspace_bytes(C.byref(dims))
         if self._ws is None or self._ws.numel() < need:
             # head room: captured graphs hold pointers into the workspace, a slightly larger batch should not move it
             self._ws = torch.empty(need + need // 4 if self.graphs else need, dtype=torch.uint8, device=dev)
@@ -170,7 +176,8 @@ class FusedTrainer:
         y = _i64(data.y)
         td = m.TDrumorGCN
         c = m.fc.weight.shape[0]
-        dims, bt, _ = _make_structs(x, ei, bu, batch, root, (None,) * 8, c, node_id_base, xs)
+        ew = self._weights(data, ei, bu)
+        dims, bt, _ = _make_structs(x, ei, bu, batch, root, (None,) * 8, c, node_id_base, xs, ew)
         # seed=None: the module's seed plus the device-side calls counter (step_count[2], advanced by the
         # optimiser kernel) -- the same value whether the step is enqueued or replayed from a CUDA graph
         o = Opts(training=int(m.training), p_drop=float(td.p), seed=int(td.seed if seed is None else seed) & ((1 << 64) - 1),
@@ -180,7 +187,7 @@ class FusedTrainer:
         dev = xs.device if xs is not None else x.device
         b = dims.B
         p = {"dims": dims, "bt": bt, "o": o, "b": b, "c": c, "dev": dev, "y": y, "b_global": int(b_global or b),
-             "keep": (x, xs, ei, bu, batch, root, y),
+             "keep": (x, xs, ei, bu, batch, root, y, ew), "weighted": any(w is not None for w in ew),
              "feat": torch.empty(b, 4 * H, dtype=torch.float32, device=dev),
              "logp": torch.empty(b, c, dtype=torch.float32, device=dev),
              "gfeat": torch.empty(b, 4 * H, dtype=torch.float32, device=dev),
@@ -270,21 +277,26 @@ class FusedTrainer:
             (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
         small = tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
                       (data.edge_index, data.BU_edge_index, data.batch, data.rootindex))
-        return (id(data), xk, small, td.deg_by, td.resolved_gemm_mode(data.x))
+        return (id(data), xk, small, self._weight_key(data), td.deg_by, td.resolved_gemm_mode(data.x))
 
     def _prep_setup(self, p, data, next_data, node_id_base):
         """Decide which prepared buffer this step reads (or prepares inline) and which one the next batch's
         preparation writes; returns the part of the CUDA-graph key that pins those decisions."""
         l = lib()
         pk = self._prep_key(data)
-        need = l.bigcn_batch_prepare_bytes(C.byref(p["dims"]))
+
+        def prep_bytes(dims, weighted):
+            return (l.bigcn_batch_prepare_edge_bytes if weighted else l.bigcn_batch_prepare_bytes)(C.byref(dims))
+        need = prep_bytes(p["dims"], p["weighted"])
         nxt = None
         if next_data is not None:
             nx, nxs = _as_x(next_data.x, self.model.TDrumorGCN.resolved_gemm_mode(next_data.x))
-            nd, nbt, _ = _make_structs(nx, _i64(next_data.edge_index), _i64(next_data.BU_edge_index), _i64(next_data.batch),
-                                       _i64(next_data.rootindex), (None,) * 8, p["c"], 0, nxs)
-            need = max(need, l.bigcn_batch_prepare_bytes(C.byref(nd)))
-            nxt = {"dims": nd, "bt": nbt, "keep": (nx, nxs, next_data), "key": self._prep_key(next_data)}
+            nei, nbu = _i64(next_data.edge_index), _i64(next_data.BU_edge_index)
+            new = self._weights(next_data, nei, nbu)
+            nd, nbt, _ = _make_structs(nx, nei, nbu, _i64(next_data.batch), _i64(next_data.rootindex), (None,) * 8, p["c"],
+                                       0, nxs, new)
+            need = max(need, prep_bytes(nd, any(w is not None for w in new)))
+            nxt = {"dims": nd, "bt": nbt, "keep": (nx, nxs, nei, nbu, new, next_data), "key": self._prep_key(next_data)}
         if self._prep_buf is None or self._prep_buf[0].numel() < need:
             self._prep_buf = [torch.empty(need + need // 4, dtype=torch.uint8, device=p["dev"]) for _ in range(2)]
             self._prep_owner = [None, None]
@@ -323,7 +335,37 @@ class FusedTrainer:
             (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
         small = tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
                       (data.edge_index, data.BU_edge_index, data.batch, data.rootindex, data.y))
-        return (id(data), xk, small, b_global, node_id_base, m.training, td.p, td.deg_by, td.gemm_mode, td.dense_roots, td.seed)
+        return (id(data), xk, small, self._weight_key(data), b_global, node_id_base, m.training, td.p, td.deg_by,
+                td.gemm_mode, td.dense_roots, td.seed)
+
+    # ---- edge weights (edge_weights=True) ------------------------------------------------------------------
+    @staticmethod
+    def _weight_key(data):
+        """what a captured step or a prepared buffer read of the batch's weights: the tensors, not their values"""
+        ws = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
+        return tuple((w.data_ptr(), tuple(w.shape), w.dtype) if torch.is_tensor(w) else id(w) for w in ws)
+
+    def _check_weights(self, data):
+        ws = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
+        if all(w is None for w in ws):
+            return
+        if not self.edge_weights:
+            raise L.BigcnError("FusedTrainer does not take edge-weighted batches (data.edge_weight / data.BU_edge_weight) "
+                               "unless built with edge_weights=True; or train them through the modules (BiGCN(data))")
+        if any(torch.is_tensor(w) and w.requires_grad for w in ws):
+            raise L.BigcnError("FusedTrainer forms no edge-weight gradient: a weight that requires grad trains through "
+                               "the modules (BiGCN(data)); pass it detached here")
+
+    @staticmethod
+    def _weights_copied(data):
+        return any(torch.is_tensor(w) and (w.dtype != torch.float32 or not w.is_contiguous())
+                   for w in (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None)))
+
+    @staticmethod
+    def _weights(data, ei, bu):
+        """(TD, BU) weights checked and laid out as fp32 [E] (or None); a cast copy is kept by the plan that reads it"""
+        return (edge_weight(getattr(data, "edge_weight", None), int(ei.shape[1]), "edge_weight"),
+                edge_weight(getattr(data, "BU_edge_weight", None), int(bu.shape[1]), "BU_edge_weight"))
 
     def step(self, data, b_global=None, node_id_base=0, seed=None, next_data=None):
         """One optimisation step on a device-resident batch; returns the loss (device scalar).
@@ -340,12 +382,11 @@ class FusedTrainer:
         ``cudaGraphLaunch``, and every later step on it is a replay.  The dropout seed of a replay comes
         from the device-side calls counter, so replays draw fresh masks exactly as enqueued steps do."""
         for d in (data, next_data):
-            if d is not None and (getattr(d, "edge_weight", None) is not None or
-                                  getattr(d, "BU_edge_weight", None) is not None):
-                raise L.BigcnError("FusedTrainer does not take edge-weighted batches (data.edge_weight / "
-                                   "data.BU_edge_weight): train them through the modules (BiGCN(data))")
+            if d is not None:
+                self._check_weights(d)
         self._calls += 1
-        use_graph = self.graphs and seed is None and not self.validate
+        # a weight that needs an fp32 copy is read through that copy: a replay would not see the caller's later writes
+        use_graph = self.graphs and seed is None and not self.validate and not self._weights_copied(data)
         pk_any = next_data is not None or (self._prep_buf is not None and any(
             o is not None and o[1]() is data for o in self._prep_owner))
         key = None
@@ -363,7 +404,7 @@ class FusedTrainer:
                 return ent["plan"]["loss"]
         p = self._plan(data, b_global, node_id_base, seed)
         ws_before = self._ws
-        self._workspace(p["dims"], p["dev"])
+        self._workspace(p["dims"], p["dev"], p["weighted"])
         if self._ws is not ws_before:
             self._graphs.clear()               # the workspace moved: every captured pointer into it is stale
         if pk_any:

@@ -24,10 +24,12 @@ def train_GCN(model, forest, train_ids, test_ids, TDdroprate, BUdroprate, lr, we
               batchsize, datasetname="Twitter16", iter=0, fold=0, modelname="BiGCN", seed=0, log=print,
               trainer=None, save=True, checkpoint_dir="checkpoints"):
     """``model``: a bigcn_b200.BiGCN / Net on the device; ``forest``: a DeviceForest holding every tree;
-    ``train_ids`` / ``test_ids``: tree indices of the fold (the reference's x_train / x_test)."""
+    ``train_ids`` / ``test_ids``: tree indices of the fold (the reference's x_train / x_test).  A forest with edge
+    weights trains them (``FusedTrainer(..., edge_weights=True)`` unless ``trainer`` is given) and validates with them."""
     dev = forest.device
     c = model.fc.weight.shape[0]
-    tr = trainer or FusedTrainer(model, lr=lr, weight_decay=weight_decay)
+    tr = trainer or FusedTrainer(model, lr=lr, weight_decay=weight_decay,
+                                 edge_weights=getattr(forest, "edge_weight", None) is not None)
     train_ev, val_ev = EvalCounts(c, dev), EvalCounts(c, dev)
     early_stopping = EarlyStopping(patience=patience, verbose=True)
     rng = np.random.default_rng(seed)

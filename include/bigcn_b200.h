@@ -118,7 +118,8 @@ typedef struct bigcn_batch {
    * bu_edge_index): both convs of that direction then run GCNConv(x, edge_index, edge_weight) -- gcn_norm with weights
    * (a self-loop edge in the list hands its weight to the node's loop, the last one wins; fill 1 otherwise; degree =
    * the weighted sum).  NULL = the unweighted path, unchanged.  Needs a workspace of
-   * bigcn_features_edge_workspace_bytes and no `prepared` buffer. */
+   * bigcn_features_edge_workspace_bytes; a `prepared` buffer must then come from bigcn_batch_prepare on this batch with
+   * these weight pointers (it carries the weighted normalisation), and opts.edge_grad takes none. */
   const float* td_edge_weight;
   const float* bu_edge_weight;
 } bigcn_batch_t;
@@ -372,8 +373,12 @@ int bigcn_features_forward(const bigcn_dims_t* dims, const bigcn_batch_t* batch,
  * right after step i: the HBM-bound pass over the next x then overlaps the latency-bound kernels of the current
  * step (the role of the reference's DataLoader worker processes, BiGCN_Twitter.py:168).  Capturable: fork and join
  * sit on `stream`.  Then pass the buffer as batch->prepared to the three calls of step i+1.  An edge-weighted batch
- * (td_edge_weight / bu_edge_weight set) is refused: the buffer carries no weights. */
+ * (td_edge_weight / bu_edge_weight set) also gets the weighted normalisation of the directions opts.dir_mask selects
+ * (graph prep with the edge ids, loop weights, weighted degrees, normalised weights in both CSR orders), written after
+ * the unweighted layout: its buffer is bigcn_batch_prepare_edge_bytes(dims) bytes, and the weighted step no longer
+ * computes any of it.  A non-finite weight or a negative weighted degree raises BIGCN_FLAG_EDGE_WEIGHT in `flags`. */
 size_t bigcn_batch_prepare_bytes(const bigcn_dims_t* dims);
+size_t bigcn_batch_prepare_edge_bytes(const bigcn_dims_t* dims);
 int bigcn_batch_prepare(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts, int32_t* flags,
                         void* prepared, size_t prepared_bytes, bigcn_stream_t stream);
 int bigcn_batch_prepare_join(bigcn_stream_t stream);
@@ -518,6 +523,33 @@ int bigcn_assemble_batch_dense(const int64_t* node_ptr, const int64_t* edge_ptr,
                                int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch, int64_t* rootindex,
                                int64_t* y, const void* x_all, int64_t K, int32_t elem_bytes, void* ox,
                                bigcn_stream_t stream);
+/* Edge weights through the same assembly: every kept edge's weight lands at the position its edge takes in
+ * edge_index / bu_edge_index (each direction after its own DropEdge subset, in kept order), copied bit for bit in the
+ * launch that places the edges.  td_weight is one weight per tree edge, aligned with edge_src / edge_dst; bu_weight the
+ * same for the BU list (NULL = td_weight: a reply carries one weight seen from either end). */
+typedef struct bigcn_asm_weights {
+  const float* td_weight;   /* [E_all]                             */
+  const float* bu_weight;   /* [E_all] or NULL (= td_weight)       */
+  float* edge_weight;       /* [E_td] out, aligned with edge_index */
+  float* bu_edge_weight;    /* [E_bu] out, aligned with bu_edge_index */
+} bigcn_asm_weights_t;
+/* bigcn_assemble_batch / bigcn_assemble_batch_dense with weights (non-NULL); the same edges, nodes and features. */
+int bigcn_assemble_batch_weighted(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                                  const int32_t* edge_dst, const int64_t* x_ptr, const int32_t* x_col,
+                                  const float* x_val, const int32_t* root_local, const int64_t* y_all,
+                                  const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                                  const int64_t* bu_off, const int64_t* nnz_off, int64_t B, int64_t E_td,
+                                  int64_t E_bu, uint64_t seed, int64_t* edge_index, int64_t* bu_edge_index,
+                                  int64_t* batch, int64_t* rootindex, int64_t* y, int32_t* ox_ptr, int32_t* ox_col,
+                                  float* ox_val, const bigcn_asm_weights_t* weights, bigcn_stream_t stream);
+int bigcn_assemble_batch_dense_weighted(const int64_t* node_ptr, const int64_t* edge_ptr, const int32_t* edge_src,
+                                        const int32_t* edge_dst, const int32_t* root_local, const int64_t* y_all,
+                                        const int64_t* tree_id, const int64_t* node_off, const int64_t* td_off,
+                                        const int64_t* bu_off, int64_t B, int64_t E_td, int64_t E_bu, uint64_t seed,
+                                        int64_t* edge_index, int64_t* bu_edge_index, int64_t* batch,
+                                        int64_t* rootindex, int64_t* y, const void* x_all, int64_t K,
+                                        int32_t elem_bytes, void* ox, const bigcn_asm_weights_t* weights,
+                                        bigcn_stream_t stream);
 
 /* ---- data-parallel optimiser step over peer memory (SURVEY.md 8e) -----------------------------
  * One kernel instead of "NCCL all-reduce of the flat gradient + Adam on every rank": grads[q] /
