@@ -40,7 +40,7 @@ struct SideCtx {
   cudaStream_t bwlo[2];  // the prep streams' priority: the dW2 / db chains (knob 12 bit 0, the default)
   cudaStream_t bw[2];    // one level above (knob 12 = 0): the backward's dW2 / db chains -- nobody waits for them before the optimiser,
                          // so they must not take SM slots from G1 -> T1 -> dW1 (the caller's stream, see ops.step_stream)
-  cudaEvent_t ev[14];
+  cudaEvent_t ev[16];
   bool ok;
 };
 static SideCtx* side_ctx() {
@@ -69,7 +69,7 @@ static SideCtx* side_ctx() {
            cudaStreamCreateWithPriority(&c.bwlo[1], cudaStreamNonBlocking, lo) == cudaSuccess &&
            cudaStreamCreateWithPriority(&c.bw[0], cudaStreamNonBlocking, mid) == cudaSuccess &&
            cudaStreamCreateWithPriority(&c.bw[1], cudaStreamNonBlocking, mid) == cudaSuccess;
-    for (int i = 0; i < 14 && c.ok; ++i) c.ok = cudaEventCreateWithFlags(&c.ev[i], cudaEventDisableTiming) == cudaSuccess;
+    for (int i = 0; i < 16 && c.ok; ++i) c.ok = cudaEventCreateWithFlags(&c.ev[i], cudaEventDisableTiming) == cudaSuccess;
     const char* e = getenv("BIGCN_NO_SIDE_STREAM");
     if (e && e[0] == '1') c.ok = false;
   }
@@ -380,8 +380,6 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   const WFeatWs wf = weighted ? step_wfeat(dm, bt, ws, w.total, o->edge_grad != 0) : WFeatWs{};
   BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total + wf.total, "features_forward: workspace too small (%zu < %zu)",
                   ws_bytes, w.total + wf.total);
-  BIGCN_CHECK_ARG(!weighted || !o->edge_grad || bt->prepared == nullptr,
-                  "features_forward: opts.edge_grad takes no prepared buffer (the edge gradient runs graph prep inline)");
   const bool prepared = bt->prepared != nullptr;   // graph structure, root columns, CSR / CSC of x: already there
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const Dirs dirs = active_dirs(o->dir_mask);
@@ -666,7 +664,6 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
   const bool edge_grad = weighted && o->edge_grad != 0;
   const WFeatWs wf = weighted ? step_wfeat(dm, bt, ws, w.total, edge_grad) : WFeatWs{};
   BIGCN_CHECK_ARG(ws != nullptr && ws_bytes >= w.total + wf.total, "features_backward: workspace too small");
-  BIGCN_CHECK_ARG(!edge_grad || bt->prepared == nullptr, "features_backward: opts.edge_grad takes no prepared buffer");
   const int64_t N = dm->N, B = dm->B, K = dm->K;
   const Dirs dirs = active_dirs(o->dir_mask);
   const int n_out = dirs.n == 2 ? 128 : 64;
@@ -801,6 +798,9 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
                           wf.a_e[d], wf.a_self[d]};
     }
     if (int rc = wfeat_edge_dot(a, dirs.n, st)) return rc;
+    // bigcn_features_edge_grad forks from here: the rest of its chain reads a_e / a_self and the normalisation,
+    // which nothing after this point overwrites
+    if (sc) cudaEventRecord(sc->ev[13], st);
   }
   // 6. T1 = A-hat^T G1, both directions side by side in one [N][n_out] matrix
   {
@@ -963,7 +963,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 106; }
+extern "C" int bigcn_version(void) { return 107; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
@@ -1048,29 +1048,38 @@ extern "C" int bigcn_features_edge_grad(const bigcn_dims_t* dims, const bigcn_ba
   if (int rc = check_common(dims, opts, "features_edge_grad")) return rc;
   BIGCN_CHECK_ARG(batch != nullptr, "features_edge_grad: NULL batch");
   BIGCN_CHECK_ARG(opts->edge_grad != 0, "features_edge_grad: needs opts.edge_grad = 1 in the forward and backward calls");
-  BIGCN_CHECK_ARG(batch->prepared == nullptr, "features_edge_grad: opts.edge_grad takes no prepared buffer");
-  const FeatWs w = carve_features(dims, workspace, workspace_bytes);
-  const WFeatWs wf = carve_wfeat(dims, workspace ? reinterpret_cast<char*>(workspace) + w.total : nullptr, true);
+  // structure and normalisation from the prepared buffer when the batch came prepared; a_e / a_self / ddeg from the
+  // workspace either way
+  const FeatWs w = carve_features(dims, workspace, workspace_bytes, batch->prepared);
+  const WFeatWs wf = step_wfeat(dims, batch, workspace, w.total, true);
   BIGCN_CHECK_ARG(workspace != nullptr && workspace_bytes >= w.total + wf.total,
                   "features_edge_grad: workspace too small (bigcn_features_edge_workspace_bytes(dims, 1))");
   float* out[2] = {d_td_w, d_bu_w};
   const int64_t* ei[2] = {batch->edge_index, batch->bu_edge_index};
   const int64_t E[2] = {dims->E_td, dims->E_bu};
+  WGradArgs a{};
+  a.N = dims->N;
+  a.deg_by_source = opts->deg_by == BIGCN_DEG_BY_SOURCE;
   for (int d = 0; d < 2; ++d) {
     if (out[d] == nullptr) continue;
     BIGCN_CHECK_ARG(dir_edge_weight(batch, d) != nullptr && ((opts->dir_mask >> d) & 1),
                     "features_edge_grad: the %s gradient needs that direction active and its weights in the batch",
                     d == 0 ? "TD" : "BU");
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  for (int d = 0; d < 2; ++d) {
-    if (out[d] == nullptr) continue;
     WGraph G = wf.G[d];
     G.g = w.g[d];
-    if (int rc = wfeat_edge_grad(G, ei[d], E[d], dir_edge_weight(batch, d), dims->N, opts->deg_by, wf.a_e[d],
-                                 wf.a_self[d], wf.ddeg[d], out[d], st))
-      return rc;
+    a.d[d] = WGradDir{G, ei[d], E[d], dir_edge_weight(batch, d), wf.a_e[d], wf.a_self[d], wf.ddeg[d], out[d]};
   }
+  // on the low-priority stream from the event features_backward recorded after the per-edge products: the chain runs
+  // underneath the backward's T1 propagate and dW1 instead of behind them, and joins the caller's stream again here
+  cudaStream_t st = (cudaStream_t)stream;
+  SideCtx* sc = side_ctx();
+  cudaStream_t es = st;
+  if (sc) {
+    cudaStreamWaitEvent(sc->low, sc->ev[13], 0);
+    es = sc->low;
+  }
+  if (int rc = wfeat_edge_grad(a, 2, es)) return rc;
+  if (sc) stream_after(sc, 14, es, st);
   return 0;
 }
 

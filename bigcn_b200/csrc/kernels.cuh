@@ -59,8 +59,12 @@ struct EdgeDotDir { const int64_t* ei; int64_t E; const float* xw; int64_t ldxw;
                     const float* h2; const float* gs; float* a_e; float* a_self; };
 struct EdgeDotArgs { EdgeDotDir d[2]; int64_t N; const int64_t* batch; };
 int wfeat_edge_dot(const EdgeDotArgs& a, int ndir, cudaStream_t st);
-int wfeat_edge_grad(const WGraph& G, const int64_t* ei, int64_t E, const float* w, int64_t N, int32_t deg_by,
-                    const float* a_e, const float* a_self, float* ddeg, float* dw, cudaStream_t st);
+// the chain from dL/dnorm through the normalisation to dL/dw, per direction (dw == NULL: direction skipped); both
+// directions in one launch per kernel (k_w_ddeg, k_w_dweight; the direction index in grid.y)
+struct WGradDir { WGraph G; const int64_t* ei; int64_t E; const float* w; const float* a_e; const float* a_self;
+                  float* ddeg; float* dw; };
+struct WGradArgs { WGradDir d[2]; int64_t N; int32_t deg_by_source; };
+int wfeat_edge_grad(const WGradArgs& a, int ndir, cudaStream_t st);
 struct PropDir { const int32_t* ptr; const int32_t* idx; const float* dis; const float* h; const float* bias; float* out; int64_t ldh, ldo; int32_t* lng; int64_t E; };
 struct PropArgs { PropDir d[2]; int64_t N; int32_t relu; int32_t cb; };
 int propagate_launch(const PropArgs&, int, cudaStream_t, const EntryW* ew = nullptr);

@@ -169,8 +169,14 @@ __global__ void __launch_bounds__(256) k_w_edge_dot(const int64_t* __restrict__ 
 
 // ---- backward: dL/ddeg[j] = -1/2 dis_j^3 * dL/ddis_j,
 //      dL/ddis_j = sum_{e: row=j} (w_e dis[col]) a_e + sum_{e: col=j} (dis[row] w_e) a_e + 2 self_w_j dis_j a_self_j
-__global__ void __launch_bounds__(256) k_w_ddeg(WGraph G, const float* __restrict__ w, const float* __restrict__ a_e,
-                                                const float* __restrict__ a_self, float* __restrict__ ddeg, int64_t N) {
+// direction blockIdx.y of `a` (one launch for both directions of the feature path)
+__global__ void __launch_bounds__(256) k_w_ddeg(WGradArgs a) {
+  const WGradDir& p = a.d[blockIdx.y];
+  if (p.dw == nullptr) return;
+  const WGraph& G = p.G;
+  const float* __restrict__ w = p.w;
+  const float* __restrict__ a_e = p.a_e;
+  const int64_t N = a.N;
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarp = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -183,38 +189,40 @@ __global__ void __launch_bounds__(256) k_w_ddeg(WGraph G, const float* __restric
       const int s = ptr[j], e = ptr[j + 1];
       for (int b = s; b < e; b += 32) {
         const int n = min(32, e - b);
-        float p = 0.f;
+        float q = 0.f;
         if (lane < n) {
           const int ed = eid[b + lane];
-          p = G.dis[idx[b + lane]] * w[ed] * a_e[ed];
+          q = G.dis[idx[b + lane]] * w[ed] * a_e[ed];
         }
-        for (int l = 0; l < n; ++l) acc += __shfl_sync(FULL_MASK, p, l);
+        for (int l = 0; l < n; ++l) acc += __shfl_sync(FULL_MASK, q, l);
       }
     }
     const float dj = G.dis[j];
-    acc += 2.f * G.self_w[j] * dj * a_self[j];
-    if (lane == 0) ddeg[j] = -0.5f * dj * dj * dj * acc;
+    acc += 2.f * G.self_w[j] * dj * p.a_self[j];
+    if (lane == 0) p.ddeg[j] = -0.5f * dj * dj * dj * acc;
   }
 }
 
-// ---- backward: gradient of every edge weight -------------------------------------------------
-__global__ void k_w_dweight(WGraph G, const int64_t* __restrict__ ei, int64_t E, int64_t N, const float* __restrict__ a_e,
-                            const float* __restrict__ a_self, const float* __restrict__ ddeg, int deg_by_source,
-                            float* __restrict__ dw) {
+// ---- backward: gradient of every edge weight (direction blockIdx.y) ---------------------------
+__global__ void k_w_dweight(WGradArgs a) {
+  const WGradDir& p = a.d[blockIdx.y];
+  if (p.dw == nullptr) return;
+  const WGraph& G = p.G;
+  const int64_t N = a.N, E = p.E;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < E; e += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t r = ei[e], c = ei[E + e];
+    const int64_t r = p.ei[e], c = p.ei[E + e];
     float d = 0.f;
     if (r >= 0 && r < N && c >= 0 && c < N) {
       if (r != c) {
-        d = G.dis[r] * G.dis[c] * a_e[e] + ddeg[deg_by_source ? r : c];
+        d = G.dis[r] * G.dis[c] * p.a_e[e] + p.ddeg[a.deg_by_source ? r : c];
       } else {
         // a self-loop edge: its weight became self_w[r].  Autograd of the reference's
         // `loop_weight[row[inv]] = edge_weight[inv]` hands the slot's gradient to EVERY loop edge on
         // the node, also the overwritten ones; mirrored here.
-        d = G.dis[r] * G.dis[r] * a_self[r] + ddeg[r];
+        d = G.dis[r] * G.dis[r] * p.a_self[r] + p.ddeg[r];
       }
     }
-    dw[e] = d;
+    p.dw[e] = d;
   }
 }
 
@@ -441,15 +449,23 @@ int wfeat_edge_dot(const EdgeDotArgs& a, int ndir, cudaStream_t st) {
   return 0;
 }
 
-int wfeat_edge_grad(const WGraph& G, const int64_t* ei, int64_t E, const float* w, int64_t N, int32_t deg_by,
-                    const float* a_e, const float* a_self, float* ddeg, float* dw, cudaStream_t st) {
-  if (E == 0) return 0;
-  if (N > 0) {
-    k_w_ddeg<<<grid_for(N, 8), 256, 0, st>>>(G, w, a_e, a_self, ddeg, N);
+int wfeat_edge_grad(const WGradArgs& a, int ndir, cudaStream_t st) {
+  int64_t emax = 0;
+  bool any = false;
+  for (int q = 0; q < ndir; ++q) {
+    if (a.d[q].dw == nullptr) continue;
+    any = true;
+    if (a.d[q].E > emax) emax = a.d[q].E;
+  }
+  if (!any) return 0;
+  if (a.N > 0) {
+    k_w_ddeg<<<dim3(grid_for(a.N, 8), ndir), 256, 0, st>>>(a);
     BIGCN_CHECK_LAUNCH("k_w_ddeg");
   }
-  k_w_dweight<<<grid_for(E, 256), 256, 0, st>>>(G, ei, E, N, a_e, a_self, ddeg, deg_by == BIGCN_DEG_BY_SOURCE, dw);
-  BIGCN_CHECK_LAUNCH("k_w_dweight");
+  if (emax > 0) {
+    k_w_dweight<<<dim3(grid_for(emax, 256), ndir), 256, 0, st>>>(a);
+    BIGCN_CHECK_LAUNCH("k_w_dweight");
+  }
   return 0;
 }
 
@@ -527,13 +543,10 @@ extern "C" int bigcn_gcnconv_weighted_backward(const float* x, int64_t N, int64_
   if (d_edge_weight != nullptr && N > 0) {
     k_w_edge_dot<<<grid_for(E + N, 16), 256, 0, st>>>(edge_index, E, N, grad_out, cw.xw, cw.a_e, cw.a_self);
     BIGCN_CHECK_LAUNCH("k_w_edge_dot");
-    k_w_ddeg<<<grid_for(N, 8), 256, 0, st>>>(G, edge_weight, cw.a_e, cw.a_self, cw.ddeg, N);
-    BIGCN_CHECK_LAUNCH("k_w_ddeg");
-    if (E > 0) {
-      k_w_dweight<<<grid_for(E, 256), 256, 0, st>>>(G, edge_index, E, N, cw.a_e, cw.a_self, cw.ddeg,
-                                                     deg_by == BIGCN_DEG_BY_SOURCE, d_edge_weight);
-      BIGCN_CHECK_LAUNCH("k_w_dweight");
-    }
+    WGradArgs ga{};
+    ga.d[0] = WGradDir{G, edge_index, E, edge_weight, cw.a_e, cw.a_self, cw.ddeg, d_edge_weight};
+    ga.N = N; ga.deg_by_source = deg_by == BIGCN_DEG_BY_SOURCE;
+    if (int rc = wfeat_edge_grad(ga, 1, st)) return rc;
   } else if (d_edge_weight != nullptr && E > 0) {
     cudaMemsetAsync(d_edge_weight, 0, (size_t)E * sizeof(float), st);
   }

@@ -12,6 +12,7 @@ import ctypes as C
 import weakref
 
 import torch
+import torch.utils.weak
 
 from . import _lib as L
 from ._lib import H, Opts, Params, check, lib
@@ -35,7 +36,7 @@ class FusedTrainer:
 
     def __init__(self, model, lr=5e-4, weight_decay=1e-4, betas=(0.9, 0.999), eps=1e-8,
                  process_group=None, world_size=1, validate=False, comm="auto", graphs="auto", max_graphs=16,
-                 fused_sync=True, dp_push=True, edge_weights=False):
+                 fused_sync=True, dp_push=True, edge_weights=False, edge_grad=False):
         """``comm`` (world_size > 1): "symm" = one fused kernel over NVLink peer memory
         (reduce-scatter of the gradients in rank order + Adam on the owned shard + all-gather of
         the parameters, bigcn_dp_reduce_adam) between two symmetric-memory barriers; "nccl" = two
@@ -48,14 +49,25 @@ class FusedTrainer:
         (release / acquire on signal words in symmetric memory) instead of as two more launches.
         ``edge_weights``: True = ``step`` takes batches that carry ``data.edge_weight`` (TD) and / or
         ``data.BU_edge_weight`` (BU), both convs of a direction weighted as ``GCNConv(x, edge_index, edge_weight)``; their
-        normalisation is prepared a step ahead with the rest of ``next_data``.  The weights get no gradient here (one that
-        requires grad is refused: train it through the modules).  False = such a batch is refused."""
+        normalisation is prepared a step ahead with the rest of ``next_data``.  Unless ``edge_grad`` is set the weights get
+        no gradient here (one that requires grad is refused: train it through the modules).  False = such a batch is
+        refused.
+        ``edge_grad`` (implies ``edge_weights``; single GPU only): a weight that requires grad gets the gradient of the
+        step's loss (the mean nll over ``b_global`` trees), handed to autograd as ``loss.backward()`` would -- a leaf
+        accumulates it into ``.grad``, a non-leaf passes it on to whatever produced it.  A batch prepared a step ahead is
+        matched to its weights by tensor identity and ``_version``: a weight written in place or replaced after it was
+        prepared is prepared again inline."""
         L.require_device()
+        if edge_grad and world_size > 1:
+            raise L.BigcnError("FusedTrainer(edge_grad=True) runs on one GPU: data-parallel edge-weight gradients are not "
+                               "supported")
         self.model = model
         self.lr, self.wd, self.betas, self.eps = lr, weight_decay, betas, eps
         self.pg, self.world = process_group, world_size
         self.validate = validate
-        self.edge_weights = bool(edge_weights)
+        self.edge_grad = bool(edge_grad)
+        self.edge_weights = bool(edge_weights) or self.edge_grad
+        self._wserial, self._wnext = torch.utils.weak.WeakIdKeyDictionary(), 0   # edge_grad: weight tensor -> serial
         self.fused_sync = bool(fused_sync)     # comm="symm": cross-rank barriers inside the optimiser kernel
         self.dp_push = bool(dp_push)           # ... and gradient slices pushed to their owners (peer stores) instead of pulled
         self.raise_priority = False            # enqueued (not replayed) steps without a prepared batch: stay on the caller's stream
@@ -159,8 +171,8 @@ class FusedTrainer:
                 self._stage, self._hst = stage, hst
                 self._stptrs = (C.c_void_p * self.world)(*[int(p) for p in hst.buffer_ptrs])
 
-    def _workspace(self, dims, dev, weighted=False):
-        need = lib().bigcn_features_edge_workspace_bytes(C.byref(dims), 0) if weighted else \
+    def _workspace(self, dims, dev, weighted=False, edge_grad=False):
+        need = lib().bigcn_features_edge_workspace_bytes(C.byref(dims), int(edge_grad)) if weighted else \
             lib().bigcn_features_workspace_bytes(C.byref(dims))
         if self._ws is None or self._ws.numel() < need:
             # head room: captured graphs hold pointers into the workspace, a slightly larger batch should not move it
@@ -177,17 +189,22 @@ class FusedTrainer:
         td = m.TDrumorGCN
         c = m.fc.weight.shape[0]
         ew = self._weights(data, ei, bu)
+        # edge_grad: d loss / d weight of each direction whose weight requires grad (ew keeps the autograd link of a cast)
+        dew = [torch.empty(w.numel(), dtype=torch.float32, device=w.device) if w is not None and w.requires_grad else None
+               for w in ew]
+        eg = self.edge_grad and any(d is not None for d in dew)
         dims, bt, _ = _make_structs(x, ei, bu, batch, root, (None,) * 8, c, node_id_base, xs, ew)
         # seed=None: the module's seed plus the device-side calls counter (step_count[2], advanced by the
         # optimiser kernel) -- the same value whether the step is enqueued or replayed from a CUDA graph
         o = Opts(training=int(m.training), p_drop=float(td.p), seed=int(td.seed if seed is None else seed) & ((1 << 64) - 1),
                  deg_by=L.DEG_BY[td.deg_by], gemm_mode=L.GEMM_MODE[td.resolved_gemm_mode(data.x)], dir_mask=L.DIR_TD | L.DIR_BU,
                  fused_tail=1, seed_dev=self.step_count[2:].data_ptr() if seed is None else None,
-                 dense_roots=int(td.resolved_dense_roots(data.x)))
+                 dense_roots=int(td.resolved_dense_roots(data.x)), edge_grad=int(eg))
         dev = xs.device if xs is not None else x.device
         b = dims.B
         p = {"dims": dims, "bt": bt, "o": o, "b": b, "c": c, "dev": dev, "y": y, "b_global": int(b_global or b),
              "keep": (x, xs, ei, bu, batch, root, y, ew), "weighted": any(w is not None for w in ew),
+             "edge_grad": eg, "ew": ew, "dew": dew,
              "feat": torch.empty(b, 4 * H, dtype=torch.float32, device=dev),
              "logp": torch.empty(b, c, dtype=torch.float32, device=dev),
              "gfeat": torch.empty(b, 4 * H, dtype=torch.float32, device=dev),
@@ -251,6 +268,10 @@ class FusedTrainer:
             check(l.bigcn_adam_step(_p(self.flat), _p(self.grad), _p(self.exp_avg), _p(self.exp_avg_sq), self.n,
                                     _p(self.seg_end), _p(self.seg_lr), self.n_seg, self.betas[0], self.betas[1],
                                     self.eps, self.wd, 1.0, _p(self.step_count), st), "adam_step")
+            if p["edge_grad"]:       # forks from inside the backward (it runs under T1 / dW1), joins here
+                dew = p["dew"]
+                check(l.bigcn_features_edge_grad(C.byref(dims), C.byref(bt), C.byref(o), _p(dew[0]), _p(dew[1]), _p(ws),
+                                                 ws.numel(), st), "features_edge_grad")
         if nxt is not None:          # the next step may start: its batch is prepared
             check(l.bigcn_batch_prepare_join(st), "batch_prepare_join")
 
@@ -266,7 +287,7 @@ class FusedTrainer:
         with torch.cuda.stream(s):
             self._enqueue(p)
         cur.wait_stream(s)
-        for t in (p["feat"], p["logp"], p["gfeat"], p["loss"], p["scr"]):
+        for t in (p["feat"], p["logp"], p["gfeat"], p["loss"], p["scr"], *(d for d in p["dew"] if d is not None)):
             t.record_stream(s)
 
     # ---- batches prepared one step ahead (bigcn_batch_prepare) ---------------------------------------------
@@ -277,7 +298,7 @@ class FusedTrainer:
             (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
         small = tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
                       (data.edge_index, data.BU_edge_index, data.batch, data.rootindex))
-        return (id(data), xk, small, self._weight_key(data), td.deg_by, td.resolved_gemm_mode(data.x))
+        return (id(data), xk, small, self._weight_key(data, True), td.deg_by, td.resolved_gemm_mode(data.x))
 
     def _prep_setup(self, p, data, next_data, node_id_base):
         """Decide which prepared buffer this step reads (or prepares inline) and which one the next batch's
@@ -335,15 +356,27 @@ class FusedTrainer:
             (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
         small = tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
                       (data.edge_index, data.BU_edge_index, data.batch, data.rootindex, data.y))
-        return (id(data), xk, small, self._weight_key(data), b_global, node_id_base, m.training, td.p, td.deg_by,
+        return (id(data), xk, small, self._weight_key(data, False), b_global, node_id_base, m.training, td.p, td.deg_by,
                 td.gemm_mode, td.dense_roots, td.seed)
 
     # ---- edge weights (edge_weights=True) ------------------------------------------------------------------
-    @staticmethod
-    def _weight_key(data):
-        """what a captured step or a prepared buffer read of the batch's weights: the tensors, not their values"""
+    def _weight_key(self, data, prepared):
+        """what a captured step or a prepared buffer read of the batch's weights: the tensors, not their values.  With
+        edge_grad the tensors are told apart by identity (a serial per live tensor, so one at a recycled address is
+        another) and, for a prepared buffer (``prepared``), by ``_version``: learnt weights change between steps, and a
+        normalisation prepared from older values must not be used"""
         ws = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
-        return tuple((w.data_ptr(), tuple(w.shape), w.dtype) if torch.is_tensor(w) else id(w) for w in ws)
+        if not self.edge_grad:
+            return tuple((w.data_ptr(), tuple(w.shape), w.dtype) if torch.is_tensor(w) else id(w) for w in ws)
+        return tuple((w.data_ptr(), self._serial(w), w._version if prepared else None, tuple(w.shape), w.dtype,
+                      w.requires_grad) if torch.is_tensor(w) else id(w) for w in ws)
+
+    def _serial(self, w):
+        s = self._wserial.get(w)
+        if s is None:
+            self._wnext += 1
+            s = self._wserial[w] = self._wnext
+        return s
 
     def _check_weights(self, data):
         ws = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
@@ -352,7 +385,7 @@ class FusedTrainer:
         if not self.edge_weights:
             raise L.BigcnError("FusedTrainer does not take edge-weighted batches (data.edge_weight / data.BU_edge_weight) "
                                "unless built with edge_weights=True; or train them through the modules (BiGCN(data))")
-        if any(torch.is_tensor(w) and w.requires_grad for w in ws):
+        if not self.edge_grad and any(torch.is_tensor(w) and w.requires_grad for w in ws):
             raise L.BigcnError("FusedTrainer forms no edge-weight gradient: a weight that requires grad trains through "
                                "the modules (BiGCN(data)); pass it detached here")
 
@@ -363,9 +396,26 @@ class FusedTrainer:
 
     @staticmethod
     def _weights(data, ei, bu):
-        """(TD, BU) weights checked and laid out as fp32 [E] (or None); a cast copy is kept by the plan that reads it"""
-        return (edge_weight(getattr(data, "edge_weight", None), int(ei.shape[1]), "edge_weight"),
-                edge_weight(getattr(data, "BU_edge_weight", None), int(bu.shape[1]), "BU_edge_weight"))
+        """(TD, BU) weights checked and laid out as fp32 [E] (or None); a cast copy is kept by the plan that reads it
+        (and, for a weight that requires grad, carries the gradient back through the cast)"""
+        with torch.enable_grad():
+            return (edge_weight(getattr(data, "edge_weight", None), int(ei.shape[1]), "edge_weight"),
+                    edge_weight(getattr(data, "BU_edge_weight", None), int(bu.shape[1]), "BU_edge_weight"))
+
+    @staticmethod
+    def _deliver(p):
+        """edge_grad: hand the step's weight gradients to autograd, on the caller's stream.  Clones: ``.grad`` must not
+        alias the plan's buffers, which the next replay overwrites."""
+        roots, grads = [], []
+        for w, g in zip(p["ew"], p["dew"]):
+            if g is None:
+                continue
+            if roots and roots[0] is w:       # one tensor for both directions: the sum of the two
+                grads[0] = grads[0] + g
+            else:
+                roots.append(w)
+                grads.append(g.clone())
+        torch.autograd.backward(roots, grads)
 
     def step(self, data, b_global=None, node_id_base=0, seed=None, next_data=None):
         """One optimisation step on a device-resident batch; returns the loss (device scalar).
@@ -400,11 +450,13 @@ class FusedTrainer:
                 self.graph_replays += 1
                 if pk_any:
                     self._prep_commit(ent["plan"], data, next_data)
+                if ent["plan"]["edge_grad"]:
+                    self._deliver(ent["plan"])
                 self.last_logp = ent["plan"]["logp"]
                 return ent["plan"]["loss"]
         p = self._plan(data, b_global, node_id_base, seed)
         ws_before = self._ws
-        self._workspace(p["dims"], p["dev"], p["weighted"])
+        self._workspace(p["dims"], p["dev"], p["weighted"], p["edge_grad"])
         if self._ws is not ws_before:
             self._graphs.clear()               # the workspace moved: every captured pointer into it is stale
         if pk_any:
@@ -431,6 +483,8 @@ class FusedTrainer:
                 self.graph_replays += 1
         if pk_any:
             self._prep_commit(p, data, next_data)
+        if p["edge_grad"]:
+            self._deliver(p)
         self.last_logp = p["logp"]
         if self.validate:
             raise_on_flags(self.flags)

@@ -119,7 +119,7 @@ typedef struct bigcn_batch {
    * (a self-loop edge in the list hands its weight to the node's loop, the last one wins; fill 1 otherwise; degree =
    * the weighted sum).  NULL = the unweighted path, unchanged.  Needs a workspace of
    * bigcn_features_edge_workspace_bytes; a `prepared` buffer must then come from bigcn_batch_prepare on this batch with
-   * these weight pointers (it carries the weighted normalisation), and opts.edge_grad takes none. */
+   * these weight pointers and values (it carries the weighted normalisation, which opts.edge_grad then also reads). */
   const float* td_edge_weight;
   const float* bu_edge_weight;
 } bigcn_batch_t;
@@ -168,7 +168,8 @@ typedef struct bigcn_opts {
                           instead of walks over each tree's list of positive root columns; needs a dense x.  Same
                           forward sums in the same order either way; 0 suits bag-of-words roots */
   int32_t edge_grad;   /* edge-weighted batch: 1 = features_backward keeps what bigcn_features_edge_grad reads (the
-                          workspace must be bigcn_features_edge_workspace_bytes(dims, 1) bytes); 0 otherwise */
+                          workspace must be bigcn_features_edge_workspace_bytes(dims, 1) bytes), with or without a
+                          prepared buffer; 0 otherwise */
 } bigcn_opts_t;
 
 const char* bigcn_last_error(void);
@@ -397,7 +398,10 @@ size_t bigcn_features_edge_workspace_bytes(const bigcn_dims_t* dims, int32_t edg
  * workspace.  Per direction it sums over conv1 and conv2 dL/dnorm_e = <G1[c], XW[r]> + <G2[c], M[r]> (taken by the
  * backward) and carries it through the normalisation: dis_r dis_c dL/dnorm_e + dL/ddeg of the degree node; a self-loop
  * edge of the list gets its node's loop gradient (every such edge, as autograd of the reference's index_put gives).
- * Deterministic, no floating-point atomics. */
+ * A prepared batch (batch->prepared) reads the normalisation from that buffer, the products from the workspace.
+ * The chain forks onto the library's low-priority stream from the point right after the backward's per-edge products,
+ * so it runs underneath the backward's last propagate and dW1, and joins `stream` before returning; do not enqueue
+ * another features_backward between the two calls.  Deterministic, no floating-point atomics. */
 int bigcn_features_edge_grad(const bigcn_dims_t* dims, const bigcn_batch_t* batch, const bigcn_opts_t* opts,
                              float* d_td_w, float* d_bu_w, void* workspace, size_t workspace_bytes,
                              bigcn_stream_t stream);

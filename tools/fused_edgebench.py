@@ -7,6 +7,10 @@ the first argument when there is one; the profiler trace of `timeline` goes besi
               b  FusedTrainer(edge_weights=True), weighted batches, pipelined and replayed
               c  FusedTrainer(edge_weights=True), weighted batches without next_data: the normalisation runs inline
               d  the module path (BiGCN(data), nll_loss, backward) plus torch.optim.Adam in the reference's lr groups
+              e  FusedTrainer(edge_grad=True), weighted batches whose weights are leaves that require grad (the step
+                 forms d loss / d weight and accumulates it into .grad), pipelined and replayed
+              f  as e without next_data
+              g  as d with weights that require grad (the modules form the edge gradient)
             Cases: Twitter16-shaped 128 trees K = 5000 'sparse' (3 batches of ~625 MB dense x in rotation, > L2);
             PHEME-shaped 24 and 4,096 trees K = 768 in 'auto' (tf32x3 + dense_roots) and 'bf16' (4,096 trees: 3 batches
             of ~125 / 63 MB; 24 trees: 32 batches in rotation, which together still fit in L2).
@@ -14,7 +18,8 @@ the first argument when there is one; the profiler trace of `timeline` goes besi
             ms per step, weighted forest against the same forest without weights, alternated over three repeats.
   asm       torch.profiler, a run of its own: device time of k_asm_edges<false> / <true> per batch.
   timeline  torch.profiler trace of pipelined weighted steps: the stream every kernel ran on, so that the
-            normalisation kernels (k_w_*, k_wf_*) show on the prepare streams and not on the step's chain.
+            normalisation kernels (k_w_*, k_wf_*) show on the prepare streams and not on the step's chain; then a
+            pipelined edge_grad step: where k_w_ddeg / k_w_dweight ran against the T1 propagate and dW1.
   gpu       card name, power limit and max SM clock (nvidia-smi), read in the same call.
 """
 import json
@@ -83,40 +88,54 @@ def ref_adam(m, lr=5e-4, wd=1e-4):
                              {"params": m.BUrumorGCN.conv2.parameters(), "lr": lr / 5}], lr=lr, weight_decay=wd)
 
 
+def with_leaf_weights(d):
+    w = Batch(**{f: getattr(d, f) for f in Batch._tensor_keys})
+    w.edge_weight = d.edge_weight.detach().clone().requires_grad_()
+    w.BU_edge_weight = d.BU_edge_weight.detach().clone().requires_grad_()
+    return w
+
+
 def step_case(dev, name, batches, k, mode):
     r = len(batches)
     plain = [unweighted(d) for d in batches]
+    learnt = [with_leaf_weights(d) for d in batches]
     models = {}
-    for v in "abcd":
+    for v in "abcdefg":
         torch.manual_seed(0)
         models[v] = bigcn_b200.BiGCN(k, 64, 64, dev, gemm_mode=mode, validate="off").to(dev).train()
-    trs = {v: bigcn_b200.FusedTrainer(models[v], lr=5e-4, weight_decay=1e-4, edge_weights=v != "a", max_graphs=2 * r + 2)
-           for v in "abc"}
-    opt = ref_adam(models["d"])
+    trs = {v: bigcn_b200.FusedTrainer(models[v], lr=5e-4, weight_decay=1e-4, edge_weights=v != "a", edge_grad=v in "ef",
+                                      max_graphs=2 * r + 2)
+           for v in "abcef"}
+    opts = {v: ref_adam(models[v]) for v in "dg"}
 
     def fused(v, data, pipelined):
         tr = trs[v]
         return lambda i: tr.step(data[i % r], next_data=data[(i + 1) % r] if pipelined else None)
 
-    def module(i):
-        m, d = models["d"], batches[i % r]
-        opt.zero_grad(set_to_none=True)
-        F.nll_loss(m(d), d.y).backward()
-        opt.step()
+    def module(v, data):
+        def run(i):
+            m, d, opt = models[v], data[i % r], opts[v]
+            opt.zero_grad(set_to_none=True)
+            F.nll_loss(m(d), d.y).backward()
+            opt.step()
+        return run
 
-    runs = {"a": fused("a", plain, True), "b": fused("b", batches, True), "c": fused("c", batches, False), "d": module}
+    runs = {"a": fused("a", plain, True), "b": fused("b", batches, True), "c": fused("c", batches, False),
+            "d": module("d", batches), "e": fused("e", learnt, True), "f": fused("f", learnt, False),
+            "g": module("g", learnt)}
     iters = max(30, 3 * r)
     res = {v: [] for v in runs}
     for rep in range(3):
         for v, fn in runs.items():
             res[v].append(timed(fn, iters, warm=2 * r + 4 if rep == 0 else r))
-    for v in "abc":
+    for v in trs:
         trs[v].check_inputs()
+    assert all(d.edge_weight.grad is not None and d.BU_edge_weight.grad is not None for d in learnt)
     nodes = [int(d.batch.numel()) for d in batches]
     x_mb = [round(d.x.numel() * d.x.element_size() / 2 ** 20, 1) for d in batches]
     for v in runs:
         s = sorted(res[v])
-        extra = {} if v == "d" else {"graph_replays": trs[v].graph_replays}
+        extra = {"graph_replays": trs[v].graph_replays} if v in trs else {}
         out(part="step", case=name, K=k, mode=mode, variant=v, ms_runs=[round(a, 4) for a in res[v]],
             ms_median=round(s[len(s) // 2], 4), spread=round(s[-1] - s[0], 4), iters=iters, batches_in_rotation=r,
             nodes_per_batch_mean=round(float(np.mean(nodes)), 1), x_mb_per_batch_mean=round(float(np.mean(x_mb)), 1),
@@ -196,6 +215,42 @@ def timeline(dev, trace_path):
     out(part="timeline", steps=1, step_chain_streams=sorted(step_streams), normalisation_streams=norm,
         normalisation_on_step_chain=any(set(v) & step_streams for v in norm.values()),
         all_kernel_streams={k: sorted(v) for k, v in sorted(streams.items())}, trace=os.path.basename(trace_path))
+    # edge_grad: the chain through the normalisation forks after k_wf_edge_dot; where it ran against T1 and dW1
+    learnt = [with_leaf_weights(d) for d in batches]
+    torch.manual_seed(0)
+    m = bigcn_b200.BiGCN(5000, 64, 64, dev, gemm_mode="sparse", validate="off").to(dev).train()
+    tr = bigcn_b200.FusedTrainer(m, lr=5e-4, weight_decay=1e-4, edge_grad=True, graphs=False)
+    for i in range(4):
+        tr.step(learnt[i % 3], next_data=learnt[(i + 1) % 3])
+    torch.cuda.synchronize()
+    eg_path = trace_path.replace("timeline", "timeline_edge_grad")
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        tr.step(learnt[1], next_data=learnt[2])
+        torch.cuda.synchronize()
+    prof.export_chrome_trace(eg_path)
+    with open(eg_path) as fh:
+        kern = sorted((e for e in json.load(fh)["traceEvents"] if e.get("cat") == "kernel"), key=lambda e: e["ts"])
+
+    def short(e):
+        return e["name"].split("(")[0].replace("void ", "").replace("bigcn::", "").split("<")[0]
+
+    t0 = kern[0]["ts"]
+    dot = next(e for e in kern if short(e) == "k_wf_edge_dot")
+    chain = dot.get("args", {}).get("stream", dot.get("tid"))
+    after = [e for e in kern if e["ts"] >= dot["ts"] + dot["dur"]]
+    t1 = next(e for e in after if short(e) == "k_propagate_w" and e.get("args", {}).get("stream", e.get("tid")) == chain)
+    dw1 = next(e for e in after if short(e) == "k_dw_sweep")
+    adam = next(e for e in after if "adam" in short(e))
+
+    def span(e):
+        return {"stream": e.get("args", {}).get("stream", e.get("tid")), "start_us": round(e["ts"] - t0, 2),
+                "end_us": round(e["ts"] + e["dur"] - t0, 2)}
+    eg = {short(e): span(e) for e in kern if short(e) in ("k_w_ddeg", "k_w_dweight")}
+    eg_end = max(v["end_us"] for v in eg.values())
+    out(part="timeline_edge_grad", step_chain_stream=chain, k_wf_edge_dot=span(dot), t1_propagate=span(t1),
+        dw1=span(dw1), adam=span(adam), edge_chain=eg, edge_chain_ends_before_dw1_ends=eg_end <= span(dw1)["end_us"],
+        adam_start_after_dw1_end_us=round(span(adam)["start_us"] - span(dw1)["end_us"], 2),
+        trace=os.path.basename(eg_path))
 
 
 def main():
@@ -213,7 +268,7 @@ def main():
             torch.cuda.empty_cache()
     forest_case(dev)
     torch.cuda.empty_cache()
-    trace = os.path.join(os.path.dirname(os.path.abspath(dest)) if dest else tempfile.gettempdir(), "r08_timeline.pt.trace.json")
+    trace = os.path.join(os.path.dirname(os.path.abspath(dest)) if dest else tempfile.gettempdir(), "r09_timeline.pt.trace.json")
     os.makedirs(os.path.dirname(trace), exist_ok=True)
     timeline(dev, trace)
     if dest:
