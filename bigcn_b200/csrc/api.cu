@@ -36,10 +36,9 @@ struct SideCtx {
   cudaStream_t side2;  // high priority, a second short chain beside the first (root columns; dW2b)
   cudaStream_t low;    // lowest priority: work nobody waits for until much later (column sort of X)
   cudaStream_t prep[2];  // lowest priority: bigcn_batch_prepare of the NEXT batch, beside the whole current step
-  cudaStream_t tail;     // the step stream's priority: the last two launches of the column sort (knob 12 bit 1)
-  cudaStream_t bwlo[2];  // the prep streams' priority: the dW2 / db chains (knob 12 bit 0, the default)
-  cudaStream_t bw[2];    // one level above (knob 12 = 0): the backward's dW2 / db chains -- nobody waits for them before the optimiser,
-                         // so they must not take SM slots from G1 -> T1 -> dW1 (the caller's stream, see ops.step_stream)
+  cudaStream_t bw[2];    // lowest priority: the backward's dW2 / db chains -- nobody waits for them before the optimiser, so they
+                         // must not take SM slots from G1 -> T1 -> dW1 (the caller's stream, see ops.step_stream) nor from this
+                         // step's column sort, which the dW1 sweep waits for
   cudaEvent_t ev[16];
   bool ok;
 };
@@ -57,18 +56,15 @@ static SideCtx* side_ctx() {
     //   hi      side / side2   short chains the main chain is about to wait for (graph prep inline, root columns)
     //   lo - 2  [the caller's step stream: bigcn_b200.ops.step_stream]
     //   lo - 1  low            this step's column sort of x: the dW1 sweep at the end of the chain waits for it
-    //   lo      prep / bwlo    the NEXT batch's preparation; this step's dW2 / db chains (only the optimiser waits for them)
+    //   lo      prep / bw      the NEXT batch's preparation; this step's dW2 / db chains (only the optimiser waits for them)
     const int mid = lo - 1 < hi ? hi : lo - 1;
     c.ok = cudaStreamCreateWithPriority(&c.s.side, cudaStreamNonBlocking, hi) == cudaSuccess &&
            cudaStreamCreateWithPriority(&c.side2, cudaStreamNonBlocking, hi) == cudaSuccess &&
            cudaStreamCreateWithPriority(&c.low, cudaStreamNonBlocking, mid) == cudaSuccess &&
            cudaStreamCreateWithPriority(&c.prep[0], cudaStreamNonBlocking, lo) == cudaSuccess &&
            cudaStreamCreateWithPriority(&c.prep[1], cudaStreamNonBlocking, lo) == cudaSuccess &&
-           cudaStreamCreateWithPriority(&c.tail, cudaStreamNonBlocking, lo - 2 < hi ? hi : lo - 2) == cudaSuccess &&
-           cudaStreamCreateWithPriority(&c.bwlo[0], cudaStreamNonBlocking, lo) == cudaSuccess &&
-           cudaStreamCreateWithPriority(&c.bwlo[1], cudaStreamNonBlocking, lo) == cudaSuccess &&
-           cudaStreamCreateWithPriority(&c.bw[0], cudaStreamNonBlocking, mid) == cudaSuccess &&
-           cudaStreamCreateWithPriority(&c.bw[1], cudaStreamNonBlocking, mid) == cudaSuccess;
+           cudaStreamCreateWithPriority(&c.bw[0], cudaStreamNonBlocking, lo) == cudaSuccess &&
+           cudaStreamCreateWithPriority(&c.bw[1], cudaStreamNonBlocking, lo) == cudaSuccess;
     for (int i = 0; i < 16 && c.ok; ++i) c.ok = cudaEventCreateWithFlags(&c.ev[i], cudaEventDisableTiming) == cudaSuccess;
     const char* e = getenv("BIGCN_NO_SIDE_STREAM");
     if (e && e[0] == '1') c.ok = false;
@@ -117,7 +113,6 @@ struct FeatWs {
   int32_t* node_ptr;
   float* w1T;               // [K][128]  (TD cols 0..63, BU cols 64..127) | hi/lo split [4][64][K]
   float* w2aT[2];           // [64][64]
-  float* w2a_split;         // [2][4][64][64] hi / lo of W2a and W2a^T (tcgen05 mix kernels)
   float* xw_part;           // split-K partials of the tcgen05 X * W on small batches
   float* w2bT[2];           // [K][64]
   int32_t* rnz_cnt; int32_t* rnz_col; float* rnz_val;
@@ -198,7 +193,6 @@ static FeatWs carve_features(const bigcn_dims_t* dm, void* ws, size_t bytes, voi
     w.w2aT[d] = c.take<float>(H * H);
     w.w2bT[d] = c.take<float>((size_t)K * H);
   }
-  w.w2a_split = c.take<float>(mix_tc_scratch_floats());
   w.xw_part = c.take<float>(xw_tc_partial_floats());
   const size_t nh = (size_t)(N > 0 ? N : 1) * H;
   for (int d = 0; d < 2; ++d) w.P[d] = c.take<float>((size_t)(B > 0 ? B : 1) * H);
@@ -453,10 +447,6 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     } else {
       if (int rc = root_nz_launch(a, s2)) return rc;
     }
-    if (mix_tc_available() && !o->skip_wgrad_prep && debug_knob(8) != 1) {   // hi / lo split of W2a, W2a^T for the tensor-core 64 x 64 products (knob 8 = 1, the default: FFMA forms, no split needed)
-      const float* w2[2] = {dir_w2(pr, dirs.id[0]), dirs.n == 2 ? dir_w2(pr, dirs.id[1]) : nullptr};
-      if (int rc = mix_tc_split_weights(w2, dirs.n, H + K, w.w2a_split, s2)) return rc;
-    }
     if (!dropping) {
       RootProjArgs pa{};
       pa.cnt = w.rnz_cnt; pa.col = w.rnz_col; pa.val = w.rnz_val; pa.B = B; pa.K = K;
@@ -486,15 +476,14 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     if (!prepared) stream_after(sc, 1, ss, st);
     stream_after(sc, 7, s2, st);
   }
-  bool side_busy = false, sort_tail = false;
+  bool side_busy = false;
   if (sparse && prepared && N > 0 && !o->skip_wgrad_prep) {   // the CSR came prepared; sort it by column beside the rest of this step
     if (sc) stream_after(sc, 2, st, sc->low);
     w.xs.flags = flags;
-    sort_tail = sc && (debug_knob(12) & 2);
     if (csr_in) {
-      if (int rc = xs_sort_csc(w.xs, sc ? sc->low : st, sort_tail)) return rc;
+      if (int rc = xs_sort_csc(w.xs, sc ? sc->low : st)) return rc;
     } else {
-      if (int rc = xs_build_csc(w.xs, bt->x, true, sc ? sc->low : st, sort_tail)) return rc;
+      if (int rc = xs_build_csc(w.xs, bt->x, true, sc ? sc->low : st)) return rc;
     }
     side_busy = sc != nullptr;
   }
@@ -530,13 +519,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
     }
     a.root_splits = root_splits;
     for (int q = 0; q < dirs.n; ++q) a.root_r[q] = root_splits > 1 ? w.rootR[dirs.id[q]] : w.z[dirs.id[q]];
-    // the tcgen05 form of the forward product (sweep + activate, then k_h64_tc) is measured slower than the fused
-    // sweep at these sizes (DESIGN.md): kept behind a knob for the A/B
-    if (mix_tc_available() && !dense_roots && !weighted && (debug_knob(8) == 2 || debug_knob(8) == 3)) {
-      if (int rc = mix_tc_forward(a, dirs.n, w.w2a_split, st)) return rc;
-    } else {
-      if (int rc = prop1_mix_launch(a, dirs.n, st, weighted ? &ew_in : nullptr)) return rc;
-    }
+    if (int rc = prop1_mix_launch(a, dirs.n, st, weighted ? &ew_in : nullptr)) return rc;
   }
   // 6. conv2 propagate + bias + relu
   {
@@ -564,13 +547,7 @@ int features_forward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const bigc
   }
   // the column sort keeps running on the low-priority stream: features_backward waits for it
   // right before the sweep that needs it (event 3)
-  if (side_busy && sort_tail) {   // the passes fill gaps at low priority; the last two launches must not queue behind the dW2 chains
-    stream_after(sc, 12, sc->low, sc->tail);
-    if (int rc = xs_sort_finish(w.xs, sc->tail)) return rc;
-    cudaEventRecord(sc->ev[3], sc->tail);
-  } else if (side_busy) {
-    cudaEventRecord(sc->ev[3], sc->low);
-  }
+  if (side_busy) cudaEventRecord(sc->ev[3], sc->low);
   return 0;
 }
 
@@ -685,9 +662,8 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
   // scratch is Z (G1, consumed by the propagate before it) and H1 (dead since the forward), not T2)
   const bool join_late = phase == 0;
   SideCtx* sc = side_ctx();
-  const bool bw_lo = debug_knob(12) & 1;
-  cudaStream_t ss = sc ? (debug_knob(7) ? sc->s.side : bw_lo ? sc->bwlo[0] : sc->bw[0]) : st;
-  cudaStream_t s2 = sc ? (debug_knob(7) ? sc->side2 : bw_lo ? sc->bwlo[1] : sc->bw[1]) : st;
+  cudaStream_t ss = sc ? sc->bw[0] : st;
+  cudaStream_t s2 = sc ? sc->bw[1] : st;
   if (phase == 2) goto dw1_only;
   // 1. per-tree scaled gradient gs = grad_feat / n_b and db2 (from the readout's positive counts)
   {
@@ -778,11 +754,7 @@ int features_backward(const bigcn_dims_t* dm, const bigcn_batch_t* bt, const big
       a.d[q] = BwdMixDir{t2[d], w.a1[d], dir_w2(pr, d), g1[d], w.cs_part1[d], make_drop(o, d)};   // A1 stands in for (H1, mask)
       c.part[q] = w.cs_part1[d]; c.out[q] = gdir_b1(gr, d);
     }
-    if (mix_tc_available() && (debug_knob(8) == 0 || debug_knob(8) == 2)) {   // tensor cores (tcgen05, TMEM)
-      if (int rc = mix_tc_backward(a, dirs.n, w.w2a_split, st)) return rc;
-    } else {
-      if (int rc = bwd_mix_launch(a, dirs.n, st)) return rc;
-    }
+    if (int rc = bwd_mix_launch(a, dirs.n, st)) return rc;
     if (sc) stream_after(sc, 2, st, ss);           // db1: ordered sum of the partials, beside T1
     if (int rc = colsum_reduce_launch(c, dirs.n, ss)) return rc;
   }
@@ -908,37 +880,20 @@ int colsum64_launch(const float* g, int64_t N, float* part, float* out, cudaStre
 
 using namespace bigcn;
 
-// tuning knobs for tools/stepbench.py (0 = the shipped configuration); not part of the documented ABI
+// Two switches for tests and measurements, read at enqueue time; not part of the documented ABI.  0 is the shipped
+// value of both, and every other key is ignored.
+//   key 10: 9 = the LDG form of the background capture pass over x (x_capture), anything else = the TMA-fed form.
+//           bench.py times the LDG form through it (its "unpaced" capture entry); tools/stepbench.py and
+//           tools/capture_check.py compare the two forms.
+//   key 15: 1 = one column split of the dense-root product (rootdense.cu) at every batch size, for the tests that
+//           compare a fixed summation order (tests/test_gpu_bf16.py, tests/test_gpu_parity.py).
 namespace bigcn {
-static int g_knob[16];
-static bool g_knob_init = false;
-static void knob_defaults() {
-  if (g_knob_init) return;
-  g_knob_init = true;
-  // knob 8: which form of the 64 x 64 products runs.  1 (default) = the fused FFMA kernels (k_prop1_mix, k_bwd_mix);
-  // 0 = backward on the tensor cores (k_h64_tc<bwd>); 2 = forward and backward; 3 = forward only.  Measured at the
-  // bench configuration (tools/stepbench.py 8:0,1,2,3, DESIGN.md section 8): 0.3706 / 0.3697 / 0.3744 / 0.3719 ms per step.
-  g_knob[8] = 1;
-  // knob 12: bit 0 = the backward's dW2 / db chains run at the prep streams' priority (below this step's column sort,
-  // which then no longer queues behind them); bit 1 = the sort's last two launches at the step stream's priority.
-  // tools/stepbench.py 12:0,1,2,3 -> 0.3347 / 0.3319 / 0.3347 / 0.3328 ms per step.
-  g_knob[12] = 1;
-  // knob 13: 2 = two bf16 terms of the small operand in gemm_mode BF16 instead of three (the A/B of tools/bf16bench.py;
-  // three are shipped, DESIGN.md section 8)
-  if (const char* e = getenv("BIGCN_MIX_TC")) {
-    if (e[0] == 'b' && e[1] == 'w') g_knob[8] = 0;        // "bwd"
-    else if (e[0] == 'b') g_knob[8] = 2;                  // "both"
-    else if (e[0] == 'f') g_knob[8] = 3;                  // "fwd"
-  }
-}
-int debug_knob(int key) {
-  knob_defaults();
-  return key >= 0 && key < 16 ? g_knob[key] : 0;
-}
+static int g_knob10 = 0, g_knob15 = 0;
+int debug_knob(int key) { return key == 10 ? g_knob10 : key == 15 ? g_knob15 : 0; }
 }  // namespace bigcn
 extern "C" void bigcn_debug_set(int key, int value) {
-  bigcn::knob_defaults();
-  if (key >= 0 && key < 16) bigcn::g_knob[key] = value;
+  if (key == 10) bigcn::g_knob10 = value;
+  else if (key == 15) bigcn::g_knob15 = value;
 }
 extern "C" const char* bigcn_last_error(void) { return g_err; }
 // `stream` waits for everything the library still has in flight on its internal streams
@@ -951,7 +906,7 @@ extern "C" int bigcn_join_internal_streams(bigcn_stream_t stream) {
   cudaStreamWaitEvent((cudaStream_t)stream, sc->ev[2], 0);
   cudaEventRecord(sc->ev[6], sc->side2);
   cudaStreamWaitEvent((cudaStream_t)stream, sc->ev[6], 0);
-  for (cudaStream_t s : {sc->bw[0], sc->bw[1], sc->bwlo[0], sc->bwlo[1], sc->tail}) {
+  for (cudaStream_t s : {sc->bw[0], sc->bw[1]}) {
     cudaEventRecord(sc->ev[11], s);
     cudaStreamWaitEvent((cudaStream_t)stream, sc->ev[11], 0);
   }

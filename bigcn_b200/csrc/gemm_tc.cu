@@ -610,8 +610,8 @@ int dw_tc(const float* x, int64_t N, int64_t K, const float* t, int64_t ldt, int
 // only rounding left is in the small operand (W forward, T backward): it is split into NT bf16 terms
 //   t0 = bf16(v), t1 = bf16(v - t0), t2 = bf16(v - t0 - t1)
 // (each difference exact in fp32) and every term takes one kind::f16 MMA against the same x tile into one fp32 TMEM
-// accumulator.  Three terms carry 24 significant bits, as many as fp32; two carry 16.  DESIGN.md section 8 has the
-// measurements behind the term count (knob 13 = 2 selects two terms for the A/B).
+// accumulator.  Three terms carry 24 significant bits, as many as fp32; two carry 16 and fail the fp64 bars (DESIGN.md
+// section 8 has the measurements behind the term count).
 template <int NT>
 __device__ __forceinline__ void bf16_terms(float v, __nv_bfloat16 (&t)[NT]) {
   float r = v;
@@ -621,7 +621,7 @@ __device__ __forceinline__ void bf16_terms(float v, __nv_bfloat16 (&t)[NT]) {
     r -= __bfloat162float(t[i]);
   }
 }
-static int bf16_nterms() { return debug_knob(13) == 2 ? 2 : 3; }
+constexpr int BF_NT = 3;   // bf16 terms of the small operand
 
 // terms of the [64, K] weight w (row pitch ldw) of direction d: out[t][d * 64 + r][k], [NT][n_out][K] bf16
 template <int NT>
@@ -640,21 +640,20 @@ __global__ void k_split_w_bf16(const float* __restrict__ w, int64_t ldw, int64_t
 // ---- forward  Y[N, n_out] = X[N, K] * W^T  with X bf16 -------------------------------------------------------------
 // Same warp roles, 256-row tiles (two M = 128 accumulators sharing every B tile), split-K and epilogue as k_xw_tc.
 // K blocks of 32 elements = one 64 B row of the SWIZZLE_64B layout: a stage is 16 KB of X plus NT x 8 KB of W terms
-// (40 KB at NT = 3: five stages; 32 KB at NT = 2: six).  With 64-element blocks and the 128B swizzle a stage would be
+// (40 KB at NT = 3: five stages).  With 64-element blocks and the 128B swizzle a stage would be
 // 80 KB and only two would fit.
 constexpr int BF_BLOCK_K = 32;
 constexpr int BF_UMMA_K = 16;
 constexpr int BF_A_BYTES = TC_BLOCK_M * 64;   // 16 KB
 constexpr int BF_B_BYTES = 128 * 64;          // 8 KB: one W term, up to 128 output rows
+constexpr int BF_XW_STAGES = 5;
 template <int NT>
-constexpr int bf_xw_stages() { return NT == 3 ? 5 : 6; }
-template <int NT>
-constexpr int bf_xw_smem() { return bf_xw_stages<NT>() * (BF_A_BYTES + NT * BF_B_BYTES) + 1024; }
+constexpr int bf_xw_smem() { return BF_XW_STAGES * (BF_A_BYTES + NT * BF_B_BYTES) + 1024; }
 
 template <int NT>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_xw_bf16(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const TcParams p) {
-  constexpr int STAGES = bf_xw_stages<NT>();
+  constexpr int STAGES = BF_XW_STAGES;
   constexpr int STAGE_BYTES = BF_A_BYTES + NT * BF_B_BYTES;
   extern __shared__ __align__(1024) uint8_t tc_smem[];
   __shared__ __align__(8) uint64_t bar_full[STAGES];
@@ -755,16 +754,14 @@ static int xw_bf16(const void* x, int64_t N, int64_t K, const float* const* w, i
   BIGCN_CHECK_ARG(K % 8 == 0, "xw (bf16): in_feats must be a multiple of 8 for TMA (16 B rows), got %lld", (long long)K);
   BIGCN_CHECK_ARG((reinterpret_cast<uintptr_t>(x) & 15) == 0, "xw (bf16): x must be 16-byte aligned");
   BIGCN_CHECK_ARG(scratch != nullptr, "xw (bf16): needs the weight scratch");
-  const int nt = bf16_nterms();
   __nv_bfloat16* terms = reinterpret_cast<__nv_bfloat16*>(scratch);
   for (int d = 0; d < n_out / 64; ++d) {
-    if (nt == 3) k_split_w_bf16<3><<<num_sms() * 2, 256, 0, st>>>(w[d], ldw, K, n_out, d, terms);
-    else k_split_w_bf16<2><<<num_sms() * 2, 256, 0, st>>>(w[d], ldw, K, n_out, d, terms);
+    k_split_w_bf16<BF_NT><<<num_sms() * 2, 256, 0, st>>>(w[d], ldw, K, n_out, d, terms);
     BIGCN_CHECK_LAUNCH("k_split_w_bf16");
   }
   CUtensorMap mx, mw;
   if (int rc = make_map_bf16(&mx, x, N, K, K, BF_BLOCK_K, TC_BLOCK_M, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
-  if (int rc = make_map_bf16(&mw, terms, (int64_t)nt * n_out, K, K, BF_BLOCK_K, n_out, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
+  if (int rc = make_map_bf16(&mw, terms, (int64_t)BF_NT * n_out, K, K, BF_BLOCK_K, n_out, CU_TENSOR_MAP_SWIZZLE_64B)) return rc;
   TcParams p;
   p.y = y; p.ldy = ldy; p.N = N; p.K = K; p.n_out = n_out;
   p.num_tiles = (int)ceil_div(N, TC_BLOCK_M);
@@ -773,13 +770,11 @@ static int xw_bf16(const void* x, int64_t N, int64_t K, const float* const* w, i
   const int nsplit = xw_split_k(p, partial);
   static bool attr = false;
   if (!attr) {
-    cudaFuncSetAttribute(k_xw_bf16<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_xw_smem<3>());
-    cudaFuncSetAttribute(k_xw_bf16<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_xw_smem<2>());
+    cudaFuncSetAttribute(k_xw_bf16<BF_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_xw_smem<BF_NT>());
     attr = true;
   }
   const dim3 grid(grid_x, nsplit);
-  if (nt == 3) k_xw_bf16<3><<<grid, TC_THREADS, bf_xw_smem<3>(), st>>>(mx, mw, p);
-  else k_xw_bf16<2><<<grid, TC_THREADS, bf_xw_smem<2>(), st>>>(mx, mw, p);
+  k_xw_bf16<BF_NT><<<grid, TC_THREADS, bf_xw_smem<BF_NT>(), st>>>(mx, mw, p);
   BIGCN_CHECK_LAUNCH("k_xw_bf16");
   if (nsplit > 1) {
     int rb = (int)ceil_div(N * (n_out / 4), 256);
@@ -797,10 +792,9 @@ static int xw_bf16(const void* x, int64_t N, int64_t K, const float* const* w, i
 constexpr int DWB_BK = 32;
 constexpr int DWB_A_BYTES = 2 * DWB_BK * 128;   // one T term: 128 outputs = 2 blocks of 64
 constexpr int DWB_B_BYTES = 4 * DWB_BK * 128;   // 256 columns of X = 4 blocks of 64
+constexpr int BF_DW_STAGES = 5;
 template <int NT>
-constexpr int bf_dw_stages() { return NT == 3 ? 5 : 6; }
-template <int NT>
-constexpr int bf_dw_smem() { return bf_dw_stages<NT>() * (NT * DWB_A_BYTES + DWB_B_BYTES) + 1024; }
+constexpr int bf_dw_smem() { return BF_DW_STAGES * (NT * DWB_A_BYTES + DWB_B_BYTES) + 1024; }
 __host__ __device__ constexpr uint32_t make_idesc_bf16_mn(int m, int n) {
   return make_idesc_bf16(m, n) | (1u << 15) | (1u << 16);   // a_major = b_major = MN
 }
@@ -810,7 +804,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
 k_dw_bf16(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_t0,
           const __grid_constant__ CUtensorMap map_t1, const __grid_constant__ CUtensorMap map_t2, const DwtParams p) {
   static_assert(DWB_BK == DWT_BK, "dw_tc's node splits are multiples of DWT_BK");
-  constexpr int STAGES = bf_dw_stages<NT>();
+  constexpr int STAGES = BF_DW_STAGES;
   constexpr int STAGE_BYTES = NT * DWB_A_BYTES + DWB_B_BYTES;   // [T0 | T1 | (T2) | X]
   extern __shared__ __align__(1024) uint8_t tc_smem[];
   __shared__ __align__(8) uint64_t bar_full[STAGES];
@@ -929,11 +923,9 @@ static int dw_bf16(const void* x, int64_t N, int64_t K, const float* t, int n_ou
   } else {
     int64_t rps = 0;
     nsplit = dw_node_splits(N, tiles, &rps);
-    const int nt = bf16_nterms();
     __nv_bfloat16* t01 = reinterpret_cast<__nv_bfloat16*>(scratch01);
     __nv_bfloat16* t2 = reinterpret_cast<__nv_bfloat16*>(scratch2);
-    if (nt == 3) k_split_rows_bf16<3><<<num_sms() * 4, 256, 0, st>>>(t, N * n_out, t01, t2);
-    else k_split_rows_bf16<2><<<num_sms() * 4, 256, 0, st>>>(t, N * n_out, t01, t2);
+    k_split_rows_bf16<BF_NT><<<num_sms() * 4, 256, 0, st>>>(t, N * n_out, t01, t2);
     BIGCN_CHECK_LAUNCH("k_split_rows_bf16");
     CUtensorMap mx, m0, m1, m2;
     if (int rc = make_map_bf16(&mx, x, N, K, K, 64, DWB_BK, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
@@ -944,12 +936,10 @@ static int dw_bf16(const void* x, int64_t N, int64_t K, const float* t, int n_ou
     p.partial = partial; p.N = N; p.K = K; p.n_out = n_out; p.rows_per_split = (int)rps;
     static bool attr = false;
     if (!attr) {
-      cudaFuncSetAttribute(k_dw_bf16<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_dw_smem<3>());
-      cudaFuncSetAttribute(k_dw_bf16<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_dw_smem<2>());
+      cudaFuncSetAttribute(k_dw_bf16<BF_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, bf_dw_smem<BF_NT>());
       attr = true;
     }
-    if (nt == 3) k_dw_bf16<3><<<dim3(tiles, nsplit), TC_THREADS, bf_dw_smem<3>(), st>>>(mx, m0, m1, m2, p);
-    else k_dw_bf16<2><<<dim3(tiles, nsplit), TC_THREADS, bf_dw_smem<2>(), st>>>(mx, m0, m1, m2, p);
+    k_dw_bf16<BF_NT><<<dim3(tiles, nsplit), TC_THREADS, bf_dw_smem<BF_NT>(), st>>>(mx, m0, m1, m2, p);
     BIGCN_CHECK_LAUNCH("k_dw_bf16");
   }
   return dw_reduce_launch(partial, nsplit, K, n_out, dw_a, ldw_a, k0_a, dw_b, ldw_b, k0_b, st);

@@ -80,11 +80,6 @@ struct MixArgs { MixDir d[2]; int64_t N, K, ldxw; int32_t cb; int64_t node_id_ba
                                             partial sums root_r[d] + s * N * 64, added in order; the list walk is skipped */
                  const float* root_r[2]; };
 int prop1_mix_launch(const MixArgs&, int, cudaStream_t, const EntryW* ew = nullptr);
-// tcgen05 form (mix_tc.cu): sweep + activate, then the 64 x 64 product on the tensor cores with the root part in the epilogue
-bool mix_tc_available();
-size_t mix_tc_scratch_floats();
-int mix_tc_split_weights(const float* const* w2, int ndir, int64_t ldw2, float* scratch, cudaStream_t);
-int mix_tc_forward(const MixArgs&, int ndir, float* scratch, cudaStream_t);
 constexpr int RO_SLICE = 512;  // rows per readout slice
 struct ReadoutArgs { const float* h2[2]; const float* h1[2]; float* pos[2]; int feat_base[2]; int ndir; const int32_t* node_ptr; const int64_t* rootindex; float* feat; int64_t ldfeat; int64_t N, B; int32_t* flags; float* scratch; int64_t nitems; };
 int readout_launch(const ReadoutArgs&, cudaStream_t, bool with_final = true);
@@ -142,7 +137,6 @@ int colsum_reduce_launch(const ColsumArgs&, int, cudaStream_t);
 struct BwdMixDir { const float* t2; const float* h1 /* A1 = dropout(relu(H1)): > 0 where kept and positive */; const float* w2; float* g1; float* part; DropSpec drop; };
 struct BwdMixArgs { BwdMixDir d[2]; int64_t N, ldw2, node_id_base; };
 int bwd_mix_launch(const BwdMixArgs&, int, cudaStream_t);
-int mix_tc_backward(const BwdMixArgs&, int ndir, const float* scratch, cudaStream_t);
 struct OuterArgs { const float* u[2]; const float* v[2]; float* part[2]; int64_t N; };
 struct OuterReduceArgs { const float* part[2]; float* dst[2]; int64_t ld; int nchunk; };
 int outer64_launch(const OuterArgs&, const OuterReduceArgs&, int, cudaStream_t);
@@ -214,11 +208,9 @@ struct XSparse {
 int debug_knob(int key);
 int64_t xs_capacity(int64_t N, int64_t K);
 XSparse xs_carve(Carver& c, int64_t N, int64_t K);
-// st_tail: leave the last two launches (xs_sort_finish) to the caller
-int xs_build_csc(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st, bool st_tail = false);
+int xs_build_csc(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st);
 int xs_build_csr(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st);
-int xs_sort_csc(const XSparse& x, cudaStream_t st, bool st_tail = false);
-int xs_sort_finish(const XSparse& x, cudaStream_t st);
+int xs_sort_csc(const XSparse& x, cudaStream_t st);
 int dw_sparse(const XSparse& x, const float* t, int64_t ldt, int n_out, float* dw_a, float* dw_b, int64_t ldw,
               cudaStream_t st);
 int xw_fp32_capture(const float*, int64_t, int64_t, const float*, int, float*, int64_t, const XSparse&, cudaStream_t);

@@ -975,45 +975,31 @@ int root_proj_launch(const RootProjArgs& a, int ndir, cudaStream_t st) {
   BIGCN_CHECK_LAUNCH("k_root_proj");
   return 0;
 }
-template <int R, int Q, int MINB>
-static int mix_launch(const MixArgs& a0, int ndir, cudaStream_t st) {
-  constexpr int smem = SweepSmem<R, Q>::kBytes;
-  static bool attr = false;
-  if (!attr) {
-    sweep_attr(k_prop1_mix<R, Q, MINB>, smem);
-    attr = true;
-  }
-  MixArgs a = a0;
-  const int max_ctas = num_sms() * MINB;
-  a.cb = sweep_cb(a.N, R, max_ctas);
-  k_prop1_mix<R, Q, MINB><<<dim3(sweep_grid(a.N, R, a.cb, max_ctas), ndir), 256, smem, st>>>(a);
-  BIGCN_CHECK_LAUNCH("k_prop1_mix");
-  return 0;
-}
 int prop1_mix_launch(const MixArgs& a, int ndir, cudaStream_t st, const EntryW* ew) {
   if (a.N == 0) return 0;
-  if (ew) {   // one configuration, the default one
-    constexpr int smem = SweepSmem<MIX_R, MIX_Q>::kBytes;
+  constexpr int smem = SweepSmem<MIX_R, MIX_Q>::kBytes;
+  MixArgs m = a;
+  const int max_ctas = num_sms() * 4;
+  m.cb = sweep_cb(m.N, MIX_R, max_ctas);
+  const dim3 grid(sweep_grid(m.N, MIX_R, m.cb, max_ctas), ndir);
+  if (ew) {
     static bool attr = false;
     if (!attr) {
       sweep_attr(k_prop1_mix_w, smem);
       attr = true;
     }
-    MixArgs m = a;
-    const int max_ctas = num_sms() * 4;
-    m.cb = sweep_cb(m.N, MIX_R, max_ctas);
-    k_prop1_mix_w<<<dim3(sweep_grid(m.N, MIX_R, m.cb, max_ctas), ndir), 256, smem, st>>>(m, *ew);
+    k_prop1_mix_w<<<grid, 256, smem, st>>>(m, *ew);
     BIGCN_CHECK_LAUNCH("k_prop1_mix_w");
     return 0;
   }
-  switch (debug_knob(2)) {
-    case 1: return mix_launch<4, 4, 4>(a, ndir, st);
-    case 2: return mix_launch<2, 8, 4>(a, ndir, st);
-    case 3: return mix_launch<2, 4, 5>(a, ndir, st);
-    case 4: return mix_launch<8, 8, 2>(a, ndir, st);
-    case 5: return mix_launch<4, 8, 3>(a, ndir, st);
-    default: return mix_launch<MIX_R, MIX_Q, 4>(a, ndir, st);
+  static bool attr = false;
+  if (!attr) {
+    sweep_attr(k_prop1_mix<MIX_R, MIX_Q, 4>, smem);
+    attr = true;
   }
+  k_prop1_mix<MIX_R, MIX_Q, 4><<<grid, 256, smem, st>>>(m);
+  BIGCN_CHECK_LAUNCH("k_prop1_mix");
+  return 0;
 }
 size_t readout_scratch_floats(int64_t N, int64_t B, int ndir) {
   return (size_t)ndir * (size_t)(ceil_div(N > 0 ? N : 1, RO_SLICE) + B) * 2 * H;

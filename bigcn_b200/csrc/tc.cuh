@@ -1,5 +1,4 @@
-// tcgen05 / TMA / TMEM building blocks shared by the tensor-core kernels (gemm_tc.cu: X * W^T and dW1;
-// mix_tc.cu: the 64 x 64 contractions of conv2.lin and its backward).  sm_100a only.
+// tcgen05 / TMA / TMEM building blocks of the tensor-core kernels (gemm_tc.cu: X * W^T, dW1 and dX).  sm_100a only.
 #pragma once
 #include <cuda.h>
 

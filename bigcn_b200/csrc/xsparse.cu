@@ -372,7 +372,7 @@ int xs_build_csr(const XSparse& x, const float* x_dense, bool from_capture, cuda
 }
 
 // CSR -> column-sorted CSC (stable LSD radix sort of the column keys) + hub-column lists
-int xs_sort_csc(const XSparse& x, cudaStream_t st, bool st_tail) {
+int xs_sort_csc(const XSparse& x, cudaStream_t st) {
   const int nblk = (int)xs_nblk(x.cap);
   const int passes = radix_passes_for(x.K);
   cudaMemsetAsync(x.hist + (int64_t)256 * nblk, 0, 4 * 256 * sizeof(int32_t), st);   // digit totals
@@ -385,13 +385,7 @@ int xs_sort_csc(const XSparse& x, cudaStream_t st, bool st_tail) {
     k_xs_scatter<<<grid_keys, RSX_THREADS, 0, st>>>(x, p & 1, 8 * p, nblk);
     BIGCN_CHECK_LAUNCH("k_xs_scatter");
   }
-  return st_tail ? 0 : xs_sort_finish(x, st);
-}
-
-// the last two launches of the column sort (on their own so that a caller can give them a more urgent stream)
-int xs_sort_finish(const XSparse& x, cudaStream_t st) {
   const int cap_ctas = num_sms() * 4;
-  const int passes = radix_passes_for(x.K);
   int gf = (int)ceil_div(x.cap, 256);
   if (gf > cap_ctas) gf = cap_ctas;
   k_xs_finish<<<gf, 256, 0, st>>>(x, passes & 1);
@@ -403,9 +397,9 @@ int xs_sort_finish(const XSparse& x, cudaStream_t st) {
 }
 
 // everything between the row capture / a caller's CSR and the column-sorted copy
-int xs_build_csc(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st, bool st_tail) {
+int xs_build_csc(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st) {
   if (int rc = xs_build_csr(x, x_dense, from_capture, st)) return rc;
-  return xs_sort_csc(x, st, st_tail);
+  return xs_sort_csc(x, st);
 }
 
 // ---- dW1[o, k] = sum_{(i,v) in column k} v * T[i, o]: CSR sweep over the columns ------------
@@ -474,15 +468,7 @@ int dw_sparse(const XSparse& x, const float* t, int64_t ldt, int n_out, float* d
   if (x.K == 0) return 0;
   DwSweepArgs a{};
   a.x = x; a.t = t; a.ldt = ldt; a.dw[0] = dw_a; a.dw[1] = dw_b; a.ldw = ldw;
-  switch (debug_knob(1)) {
-    case 1: return dw_sweep_launch<2, 8, 4>(a, n_out, st);
-    case 2: return dw_sweep_launch<1, 8, 4>(a, n_out, st);
-    case 3: return dw_sweep_launch<4, 8, 3>(a, n_out, st);
-    case 4: return dw_sweep_launch<2, 8, 5>(a, n_out, st);
-    case 5: return dw_sweep_launch<1, 16, 3>(a, n_out, st);
-    case 6: return dw_sweep_launch<1, 4, 6>(a, n_out, st);
-    default: return dw_sweep_launch<DW_R, DW_Q, 3>(a, n_out, st);
-  }
+  return dw_sweep_launch<DW_R, DW_Q, 3>(a, n_out, st);
 }
 
 }  // namespace bigcn

@@ -21,12 +21,12 @@ constexpr int XW_U = 8;
 // CAPTURE: lane 0 also records every non-zero (column, value) in the row's ELL slots and the
 // exact count (xsparse.cu turns that into the CSR / CSC the sparse weight gradient sweeps).
 // PRODUCT = false: capture only (bigcn_batch_prepare: the weights of the step that will use the batch do not exist yet).
-template <int NOUT, bool VEC4, bool CAPTURE, int MINB = 1, bool PRODUCT = true>
-__global__ void __launch_bounds__(256, MINB) k_xw_scan(const float* __restrict__ x, int64_t N, int64_t K,
-                                                 const float* __restrict__ wt,
-                                                 float* __restrict__ y, int64_t ldy,
-                                                 int32_t* __restrict__ xs_cnt, int32_t* __restrict__ xs_col,
-                                                 float* __restrict__ xs_val, int pace_ns = 0) {
+template <int NOUT, bool VEC4, bool CAPTURE, bool PRODUCT = true>
+__global__ void __launch_bounds__(256, 1) k_xw_scan(const float* __restrict__ x, int64_t N, int64_t K,
+                                              const float* __restrict__ wt,
+                                              float* __restrict__ y, int64_t ldy,
+                                              int32_t* __restrict__ xs_cnt, int32_t* __restrict__ xs_col,
+                                              float* __restrict__ xs_val) {
   constexpr int V = NOUT / 32;
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -94,11 +94,10 @@ __global__ void __launch_bounds__(256, MINB) k_xw_scan(const float* __restrict__
         *reinterpret_cast<float2*>(yr) = make_float2(acc[0], acc[1]);
     }
     if (CAPTURE && lane == 0) xs_cnt[row] = nz;
-    if (!PRODUCT && pace_ns > 0) __nanosleep(pace_ns);   // background pass: leave HBM headroom for the step's own kernels
   }
 }
 
-template <bool CAPTURE, int MINB = 1>
+template <bool CAPTURE>
 static int xw_scan_launch(const float* x, int64_t N, int64_t K, const float* wt, int n_out, float* y, int64_t ldy,
                           int32_t* xs_cnt, int32_t* xs_col, float* xs_val, int ctas_per_sm, cudaStream_t st) {
   if (N == 0) return 0;
@@ -107,11 +106,11 @@ static int xw_scan_launch(const float* x, int64_t N, int64_t K, const float* wt,
   const int cap = num_sms() * ctas_per_sm;
   if (blocks > cap) blocks = cap;
   if (n_out == 128) {
-    if (vec4) k_xw_scan<128, true, CAPTURE, MINB><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
-    else k_xw_scan<128, false, CAPTURE, MINB><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
+    if (vec4) k_xw_scan<128, true, CAPTURE><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
+    else k_xw_scan<128, false, CAPTURE><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
   } else {
-    if (vec4) k_xw_scan<64, true, CAPTURE, MINB><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
-    else k_xw_scan<64, false, CAPTURE, MINB><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
+    if (vec4) k_xw_scan<64, true, CAPTURE><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
+    else k_xw_scan<64, false, CAPTURE><<<blocks, 256, 0, st>>>(x, N, K, wt, y, ldy, xs_cnt, xs_col, xs_val);
   }
   BIGCN_CHECK_LAUNCH("k_xw_scan");
   return 0;
@@ -125,19 +124,7 @@ int xw_fp32(const float* x, int64_t N, int64_t K, const float* wt, int n_out, fl
 // for the short kernels of the side stream to run beside it
 int xw_fp32_capture(const float* x, int64_t N, int64_t K, const float* wt, int n_out, float* y, int64_t ldy,
                     const XSparse& xs, cudaStream_t st) {
-  switch (debug_knob(3)) {
-    case 1: return xw_scan_launch<true, 6>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 6, st);
-    case 2: return xw_scan_launch<true, 8>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 8, st);
-    case 3: return xw_scan_launch<true, 1>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 8, st);
-    case 4: return xw_scan_launch<true, 1>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 4, st);
-    case 5: return xw_scan_launch<true, 1>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 3, st);
-    case 6: return xw_scan_launch<true, 1>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 2, st);
-    case 7: return xw_scan_launch<true, 3>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 3, st);
-    case 8: return xw_scan_launch<true, 4>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 4, st);
-    case 9: return xw_scan_launch<true, 4>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 8, st);
-    case 10: return xw_scan_launch<true, 5>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 5, st);
-    default: return xw_scan_launch<true, 1>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 6, st);
-  }
+  return xw_scan_launch<true>(x, N, K, wt, n_out, y, ldy, xs.cnt, xs.ell_col, xs.ell_val, 6, st);
 }
 
 // ---- the background pass over x (bigcn_batch_prepare): capture only, fed by the TMA engine -----------------------------
@@ -145,14 +132,14 @@ int xw_fp32_capture(const float* x, int64_t N, int64_t K, const float* wt, int n
 // memory with cp.async.bulk (4 KB chunks = the 1024-column blocks of the fused scan, L2 evict-first); every lane owns 32
 // consecutive floats of a chunk, builds a bit mask of its non-zeros, and two warp scans place them in the row's ELL slots in
 // exactly the slot order of k_xw_scan (same ELL contents; tools/capture_check.py).  The point is the footprint: 4 warps x 3
-// stages by default -- 128 threads, 42 registers, 48 KB of shared memory per SM and at most CAPW * CAPS * 4 KB in flight per
+// stages -- 128 threads, 50 registers, 48 KB of shared memory per SM and at most CAPW * CAPS * 4 KB in flight per
 // SM -- so the pass runs the whole length of a step without taking slots or registers from the step's own latency-bound
 // kernels (DESIGN.md section 4: the chain feels the footprint of the pass, not its HBM traffic).
 constexpr int CAP_CHUNK = 1024;   // floats per chunk
 template <int CAPW, int CAPS>
 __global__ void __launch_bounds__(32 * CAPW) k_x_capture_tma(const float* __restrict__ x, int64_t N, int64_t K,
                                                              int32_t* __restrict__ xs_cnt, int32_t* __restrict__ xs_col,
-                                                             float* __restrict__ xs_val, int no_fence, int row_mod) {
+                                                             float* __restrict__ xs_val) {
   extern __shared__ __align__(128) float cap_smem[];
   float (*buf)[CAPS][CAP_CHUNK] = reinterpret_cast<float (*)[CAPS][CAP_CHUNK]>(cap_smem);
   __shared__ __align__(8) uint64_t full[CAPW][CAPS];
@@ -176,10 +163,7 @@ __global__ void __launch_bounds__(32 * CAPW) k_x_capture_tma(const float* __rest
     const int nfl = (int)min((int64_t)CAP_CHUNK, K - (int64_t)pc * CAP_CHUNK);
     const uint32_t fb = smem_u32(&full[warp][s]);
     mbar_expect_tx(fb, (uint32_t)nfl * 4);
-    // row_mod: timing experiment only (tools/stepbench.py set:14=64): every row reads one of the first row_mod rows, i.e.
-    // the pass runs out of L2 -- same footprint and instruction stream, no HBM traffic
-    const int64_t srow = row_mod > 0 ? prow % row_mod : prow;
-    bulk_g2s_hint(smem_u32(&buf[warp][s][0]), x + srow * K + (int64_t)pc * CAP_CHUNK, (uint32_t)nfl * 4, fb, pol);
+    bulk_g2s_hint(smem_u32(&buf[warp][s][0]), x + prow * K + (int64_t)pc * CAP_CHUNK, (uint32_t)nfl * 4, fb, pol);
     if (++pc == nchunk) { pc = 0; prow += stride; }
   };
   if (lane == 0)
@@ -246,7 +230,7 @@ __global__ void __launch_bounds__(32 * CAPW) k_x_capture_tma(const float* __rest
       // the stage is read: hand it back to the TMA engine (generic-proxy reads before the async-proxy write)
       __syncwarp();
       if (lane == 0) {
-        if (!no_fence) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         issue(s);
       }
       if (++s == CAPS) { s = 0; ph ^= 1; }
@@ -257,53 +241,26 @@ __global__ void __launch_bounds__(32 * CAPW) k_x_capture_tma(const float* __rest
 
 // The LDG form of the same pass (k_xw_scan<..., capture, no product>): launched as MANY SHORT CTAs (8 rows each, one per warp,
 // ~160 KB of x) so that slots free up every few microseconds and the block scheduler hands them to the step's own
-// (higher-priority) kernels first.  Used when x is not 16-byte addressable, and for the A/B (tools/stepbench.py knob 10).
+// (higher-priority) kernels first.  Used when x is not 16-byte addressable, and for the A/B (debug key 10 = 9:
+// tools/stepbench.py, bench.py's unpaced capture entry).
 int x_capture(const float* x, int64_t N, int64_t K, const XSparse& xs, cudaStream_t st) {
   if (N == 0) return 0;
   const bool vec4 = (K % 4 == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
-  if (vec4 && debug_knob(10) != 9) {   // TMA-fed persistent form (knob 10: consumer warps / stages; 9 = the LDG form below)
-    const int grid = (int)min((int64_t)num_sms(), ceil_div(N, 4));
-#define CAP_LAUNCH(W_, S_)                                                                                           \
-  do {                                                                                                               \
-    static bool attr = false;                                                                                        \
-    constexpr int smem = W_ * S_ * CAP_CHUNK * 4;                                                                    \
-    if (!attr) {                                                                                                     \
-      cudaFuncSetAttribute(k_x_capture_tma<W_, S_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);              \
-      attr = true;                                                                                                   \
-    }                                                                                                                \
-    k_x_capture_tma<W_, S_><<<grid, 32 * W_, smem, st>>>(x, N, K, xs.cnt, xs.ell_col, xs.ell_val, debug_knob(13), debug_knob(14)); \
-  } while (0)
-    switch (debug_knob(10)) {
-      case 1: CAP_LAUNCH(4, 2); break;
-      case 2: CAP_LAUNCH(6, 2); break;
-      case 3: CAP_LAUNCH(8, 2); break;
-      case 4: CAP_LAUNCH(4, 4); break;
-      case 5: CAP_LAUNCH(6, 3); break;
-      case 6: CAP_LAUNCH(8, 3); break;
-      case 7: CAP_LAUNCH(7, 2); break;
-      case 8: CAP_LAUNCH(2, 6); break;
-      case 10: CAP_LAUNCH(3, 4); break;
-      case 11: CAP_LAUNCH(2, 4); break;
-      case 12: CAP_LAUNCH(2, 8); break;
-      case 13: CAP_LAUNCH(1, 12); break;
-      default: CAP_LAUNCH(4, 3); break;
+  if (vec4 && debug_knob(10) != 9) {   // TMA-fed persistent form
+    constexpr int CAPW = 4, CAPS = 3, smem = CAPW * CAPS * CAP_CHUNK * 4;
+    static bool attr = false;
+    if (!attr) {
+      cudaFuncSetAttribute(k_x_capture_tma<CAPW, CAPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+      attr = true;
     }
-#undef CAP_LAUNCH
+    const int grid = (int)min((int64_t)num_sms(), ceil_div(N, 4));
+    k_x_capture_tma<CAPW, CAPS><<<grid, 32 * CAPW, smem, st>>>(x, N, K, xs.cnt, xs.ell_col, xs.ell_val);
     BIGCN_CHECK_LAUNCH("k_x_capture_tma");
     return 0;
   }
-  int blocks = (int)ceil_div(N, 8), threads = 256;
-  switch (debug_knob(5)) {   // tools/stepbench.py: grid shape of the background pass
-    case 1: blocks = min(blocks, num_sms() * 2); break;
-    case 2: blocks = min(blocks, num_sms()); break;
-    case 3: threads = 128; blocks = min((int)ceil_div(N, 4), num_sms()); break;
-    case 4: threads = 128; blocks = (int)ceil_div(N, 4); break;
-    case 5: threads = 64; blocks = min((int)ceil_div(N, 2), num_sms() * 2); break;
-    default: break;
-  }
-  const int pace = debug_knob(6) * 100;
-  if (vec4) k_xw_scan<64, true, true, 1, false><<<blocks, threads, 0, st>>>(x, N, K, nullptr, nullptr, 0, xs.cnt, xs.ell_col, xs.ell_val, pace);
-  else k_xw_scan<64, false, true, 1, false><<<blocks, threads, 0, st>>>(x, N, K, nullptr, nullptr, 0, xs.cnt, xs.ell_col, xs.ell_val, pace);
+  const int blocks = (int)ceil_div(N, 8);
+  if (vec4) k_xw_scan<64, true, true, false><<<blocks, 256, 0, st>>>(x, N, K, nullptr, nullptr, 0, xs.cnt, xs.ell_col, xs.ell_val);
+  else k_xw_scan<64, false, true, false><<<blocks, 256, 0, st>>>(x, N, K, nullptr, nullptr, 0, xs.cnt, xs.ell_col, xs.ell_val);
   BIGCN_CHECK_LAUNCH("k_xw_scan (capture only)");
   return 0;
 }

@@ -612,8 +612,7 @@ def launches_per_step(n_nodes: int, n_dirs: int = 2, training: bool = True, gemm
     if sparse:      # row scan x2 + compaction (or CSR ingest), radix passes over the column keys, finish, hub columns
         kbits = max(1, (in_feats - 1).bit_length())
         csc = (1 if sparse_input else 3) + 3 * ((kbits + 7) // 8) + 2
-    # transposes, prep, root_nz, [root_proj], xw, [csc build], mix, prop2, readout x2  (the W2a hi/lo split is only launched
-    # when the tcgen05 forms of the 64 x 64 products are selected: BIGCN_MIX_TC)
+    # transposes, prep, root_nz, [root_proj], xw, [csc build], mix, prop2, readout x2
     fwd = 1 + prep + 1 + (0 if training else 1) + xw + csc + 1 + 1 + 2
     head = 1 + 1 + 3                           # head fwd, nll, head bwd (feat, w partial, w reduce)
     if sparse:

@@ -108,45 +108,34 @@ def make_dev(b, dev):
     return Batch(**{k: getattr(b, k).to(dev) for k in Batch._tensor_keys})
 
 
-@pytest.mark.parametrize("knob", [0, 2, 3])
-def test_mix_products_on_tensor_cores(dev, knob):
-    """The tcgen05 form of conv2.lin / its backward (csrc/mix_tc.cu: k_prop1_act + k_h64_tc) against the oracle, at
-    the bars of the FFMA kernels it can stand in for: train-mode log-probs 1e-5 with the kernel's Philox mask injected,
-    all ten gradients 1e-4.  knob 0 = backward, 2 = both, 3 = forward on the tensor cores."""
-    import ctypes as C
+def test_ffma_mix_kernels_match_oracle(dev):
+    """The FFMA kernels of conv2.lin and its backward (k_prop1_mix, k_bwd_mix) against the oracle: train-mode log-probs
+    1e-5 with the kernel's Philox mask injected, all ten gradients 1e-4, then eval mode."""
     import bigcn_b200
-    from bigcn_b200 import _lib as L
     from oracle import gcn_oracle
-    lib = L.lib()
-    lib.bigcn_debug_set.argtypes = [C.c_int, C.c_int]
-    lib.bigcn_debug_set.restype = None
-    lib.bigcn_debug_set(8, knob)
-    try:
-        for shape, k, trees in (("twitter15", 5000, 9), ("pheme", 768, 40)):
-            b = make_batch(shape, trees, seed=21, train=True, in_feats=k)
-            n = b.x.shape[0]
-            torch.manual_seed(8)
-            ref = bigcn_oracle.BiGCN(k, 64, 64).train()
-            with torch.no_grad():
-                for p in ref.parameters():
-                    if p.dim() == 1:
-                        p.uniform_(-0.1, 0.1)
-            m = bigcn_b200.BiGCN(k, 64, 64, dev).to(dev).train()
-            m.load_state_dict(ref.state_dict())
-            got = m(make_dev(b, dev))
-            m.check_inputs()
-            seed = m.TDrumorGCN.last_seed
-            ktd = torch.from_numpy(gcn_oracle.dropout_keep_mask(seed, 0, np.arange(n), 64 + k, 0.5))
-            kbu = torch.from_numpy(gcn_oracle.dropout_keep_mask(seed, 1, np.arange(n), 64 + k, 0.5))
-            want = ref(b, keep_td=ktd, keep_bu=kbu)
-            assert rel_err(got, want) < (1e-5 if k == 5000 else 2.2e-5), shape
-            torch.nn.functional.nll_loss(want, b.y).backward()
-            torch.nn.functional.nll_loss(got, b.y.to(dev)).backward()
-            for (name, p), (_, q) in zip(m.named_parameters(), ref.named_parameters()):
-                e = rel_err(p.grad, q.grad)
-                assert e < 1e-4, f"knob {knob} {shape} {name}: {e:.3e}"
-            # eval mode: the root projection P is added in the epilogue instead
-            m.eval(); ref.eval()
-            assert rel_err(m(make_dev(b, dev)), ref(b)) < (1e-5 if k == 5000 else 2.2e-5)
-    finally:
-        lib.bigcn_debug_set(8, 1)
+    for shape, k, trees in (("twitter15", 5000, 9), ("pheme", 768, 40)):
+        b = make_batch(shape, trees, seed=21, train=True, in_feats=k)
+        n = b.x.shape[0]
+        torch.manual_seed(8)
+        ref = bigcn_oracle.BiGCN(k, 64, 64).train()
+        with torch.no_grad():
+            for p in ref.parameters():
+                if p.dim() == 1:
+                    p.uniform_(-0.1, 0.1)
+        m = bigcn_b200.BiGCN(k, 64, 64, dev).to(dev).train()
+        m.load_state_dict(ref.state_dict())
+        got = m(make_dev(b, dev))
+        m.check_inputs()
+        seed = m.TDrumorGCN.last_seed
+        ktd = torch.from_numpy(gcn_oracle.dropout_keep_mask(seed, 0, np.arange(n), 64 + k, 0.5))
+        kbu = torch.from_numpy(gcn_oracle.dropout_keep_mask(seed, 1, np.arange(n), 64 + k, 0.5))
+        want = ref(b, keep_td=ktd, keep_bu=kbu)
+        assert rel_err(got, want) < (1e-5 if k == 5000 else 2.2e-5), shape
+        torch.nn.functional.nll_loss(want, b.y).backward()
+        torch.nn.functional.nll_loss(got, b.y.to(dev)).backward()
+        for (name, p), (_, q) in zip(m.named_parameters(), ref.named_parameters()):
+            e = rel_err(p.grad, q.grad)
+            assert e < 1e-4, f"{shape} {name}: {e:.3e}"
+        # eval mode: the root projection P is added instead
+        m.eval(); ref.eval()
+        assert rel_err(m(make_dev(b, dev)), ref(b)) < (1e-5 if k == 5000 else 2.2e-5)

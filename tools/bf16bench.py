@@ -2,8 +2,8 @@
 """gemm_mode='bf16' against the fp32-x tensor-core modes, in one GPU call (prints JSON lines):
 
   kernel  X * W (both directions, n_out = 128) and dW1 = T^T X alone on a Twitter-sized dense matrix (31 k x 5000,
-          bag-of-words counts) and on PHEME at 4096 trees (41 k x 768): tf32 / tf32x3 on fp32 x, bf16 on bf16 x with
-          two and three weight terms (knob 13).  Inputs rotate over enough copies to exceed the 126 MB L2.  ms per call
+          bag-of-words counts) and on PHEME at 4096 trees (41 k x 768): tf32 / tf32x3 on fp32 x, bf16 on bf16 x (three
+          weight terms).  Inputs rotate over enough copies to exceed the 126 MB L2.  ms per call
           (CUDA events), algorithmic bytes (x read once + y / dW written), fraction of the copy peak measured in the
           same call, tensor TFLOP/s of the MMAs issued, and the error against fp64.
   step    whole steps replayed from CUDA graphs (FusedTrainer with next_data for training), three rotating batches,
@@ -11,7 +11,6 @@
           fp32 x against bf16), Weibo training at 128 trees, and PHEME v1 width (in_feats = 196,608) at 24 trees.
   gpu     card name, power limit and max SM clock (nvidia-smi), read in the same call.
 """
-import ctypes as C
 import json
 import os
 import subprocess
@@ -29,13 +28,6 @@ L2_BYTES = 126 << 20
 
 def out(**kw):
     print(json.dumps(kw), flush=True)
-
-
-def set_terms(nt):
-    lib = L.lib()
-    lib.bigcn_debug_set.argtypes = [C.c_int, C.c_int]
-    lib.bigcn_debug_set.restype = None
-    lib.bigcn_debug_set(13, nt)
 
 
 def timed(fn, iters, warm=3):
@@ -76,10 +68,8 @@ def kernels(dev, peak):
         ref_dw = t.double().t() @ x16.double()                              # [128, K]
         ref_y32 = (x32.double() @ torch.cat(w).double().t())
         ref_dw32 = t.double().t() @ x32.double()
-        for mode, nt in (("tf32", 1), ("tf32x3", 3), ("bf16", 2), ("bf16", 3)):
+        for mode, terms in (("tf32", 1), ("tf32x3", 3), ("bf16", 3)):
             xb = x16 if mode == "bf16" else x32
-            if mode == "bf16":
-                set_terms(nt)
             copies = max(2, -(-2 * L2_BYTES // (xb.numel() * xb.element_size())))
             xs = [xb] + [xb.clone() for _ in range(copies - 1)]
             y = torch.empty(n, 128, device=dev)
@@ -97,7 +87,6 @@ def kernels(dev, peak):
                 L.check(lib.bigcn_xw_wgrad(xs[i % copies].data_ptr(), n, k, t.data_ptr(), 2, dw[0].data_ptr(),
                                            dw[1].data_ptr(), k, m, scr_d.data_ptr(), st), "xw_wgrad")
             xbytes = xb.numel() * xb.element_size()
-            terms = nt if mode != "tf32x3" else 3
             for op, fn, ybytes, ref in (("xw", fwd, n * 128 * 4, ref_y if mode == "bf16" else ref_y32),
                                         ("dw1", bwd, n * 128 * 4 + k * 128 * 4, ref_dw if mode == "bf16" else ref_dw32)):
                 ms = timed(fn, 20)
@@ -109,18 +98,16 @@ def kernels(dev, peak):
                     tensor_tflops=round(2 * n * k * 128 * terms / (ms * 1e-3) / 1e12, 1), rel_err_fp64=float(f"{err:.3e}"),
                     x_copies_rotated=copies)
             del xs
-    set_terms(0)
 
 
 def steps(dev):
     # PHEME's fp32 baseline is 'auto' (tf32x3 with dense_roots on, what a user gets for dense features; an explicit
     # 'tf32x3' leaves dense_roots off); bf16 turns dense_roots on by its own probe
-    pheme = [("auto", "auto", 0), ("bf16x3", "bf16", 3), ("bf16x2", "bf16", 2)]
-    cases = [  # (shape, trees, in_feats, phases, [(label, gemm_mode, terms)])
+    pheme = [("auto", "auto"), ("bf16x3", "bf16")]
+    cases = [  # (shape, trees, in_feats, phases, [(label, gemm_mode)])
         ("pheme", 24, 768, ("infer", "train"), pheme),
         ("pheme", 4096, 768, ("infer", "train"), pheme),
-        ("weibo", 128, 5000, ("train",), [("sparse", "sparse", 0), ("tf32", "tf32", 0), ("tf32x3", "tf32x3", 0),
-                                          ("bf16x3", "bf16", 3), ("bf16x2", "bf16", 2)]),
+        ("weibo", 128, 5000, ("train",), [("sparse", "sparse"), ("tf32", "tf32"), ("tf32x3", "tf32x3"), ("bf16x3", "bf16")]),
         ("pheme", 24, 196608, ("infer", "train"), pheme),
     ]
     for shape, trees, k, phases, modes in cases:
@@ -139,7 +126,7 @@ def steps(dev):
         nodes = [int(b.x.shape[0]) for b in b32]
         for phase in phases:
             runners = {}
-            for label, mode, nt in modes:
+            for label, mode in modes:
                 torch.manual_seed(0)
                 m = bigcn_b200.BiGCN(k, 64, 64, dev, num_classes=cfg["num_classes"], gemm_mode=mode, validate="off",
                                      graphs=True).to(dev)
@@ -152,15 +139,12 @@ def steps(dev):
                         return tr.step(data[i % 3], next_data=data[(i + 1) % 3])
                     with torch.no_grad():
                         return m(data[i % 3])
-                runners[label] = (one, nt)
-            res = {label: [] for label, _, _ in modes}
+                runners[label] = one
+            res = {label: [] for label, _ in modes}
             for rep in range(3):
-                for label, _, _ in modes:
-                    one, nt = runners[label]
-                    set_terms(nt)
-                    res[label].append(timed(one, 30, warm=24 if rep == 0 else 6))
-            set_terms(0)
-            for label, mode, nt in modes:
+                for label, _ in modes:
+                    res[label].append(timed(runners[label], 30, warm=24 if rep == 0 else 6))
+            for label, mode in modes:
                 v = sorted(res[label])
                 out(part="step", shape=shape, trees=trees, K=k, phase=phase, mode=label, ms_runs=[round(a, 4) for a in res[label]],
                     ms_median=round(v[1], 4), spread=round(v[-1] - v[0], 4), nodes_per_batch=nodes,

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """bigcn_x_capture (the TMA-fed pass over x of bigcn_batch_prepare) against torch.to_sparse_csr, several shapes
-(run on the GPU box): the same entries per row, and -- between the kernel variants knob 10 selects, 9 being the LDG
-scan whose slot order the product is defined by -- the same slot order.  `python tools/capture_check.py 9 0 2 8`."""
+(needs the GPU): the same entries per row, and -- between the two forms bigcn_debug_set key 10 selects, 9 being the
+LDG scan whose slot order the product is defined by, 0 the TMA-fed pass -- the same slot order.
+`python tools/capture_check.py 9 0`."""
 import ctypes as C
 import os
 import sys
@@ -37,7 +38,7 @@ def main():
     lib.bigcn_debug_set.restype = None
     bad = 0
     first = {}
-    for knob in [int(a) for a in sys.argv[1:]] or [0]:
+    for knob in [int(a) for a in sys.argv[1:]] or [9, 0]:
         lib.bigcn_debug_set(10, knob)
         g = torch.Generator(device="cpu").manual_seed(3)      # every variant sees the same matrices
         for n, k, per_row in ((1, 4, 2), (37, 24, 3), (300, 1000, 11), (2000, 5000, 20), (513, 5000, 1), (64, 4096, 20), (100, 1028, 5)):

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Per-kernel SASS opcode counts of the tensor-core objects (cuobjdump -sass; runs on the CPU box after a build):
-the evidence that k_xw_tc / k_dw_tc / k_h64_tc are tcgen05 (UTCHMMA), TMA (UTMALDG) and TMEM (LDTM) kernels.
+the evidence that k_xw_tc / k_dw_tc are tcgen05 (UTCHMMA), TMA (UTMALDG) and TMEM (LDTM) kernels.
 Usage: python tools/sass_listing.py > profiles/sass_tc.txt"""
 import collections
 import os
@@ -15,7 +15,7 @@ def main():
     print("# SASS evidence for the tcgen05 / TMA / TMEM kernels (cuobjdump -sass of the objects linked into libbigcn_b200.so, sm_100a).")
     print("# UTCHMMA = tcgen05.mma (kind::tf32 here), UTMALDG = TMA tensor load (cp.async.bulk.tensor), LDTM = tcgen05.ld (TMEM -> registers),")
     print("# UTCBAR = tcgen05.commit -> mbarrier, UTCATOMSWS = TMEM allocation, SYNCS = mbarrier ops, FENCE = fence.proxy.async / tcgen05 fences.")
-    for obj in ("bigcn_b200/csrc/gemm_tc.o", "bigcn_b200/csrc/mix_tc.o"):
+    for obj in ("bigcn_b200/csrc/gemm_tc.o",):
         txt = subprocess.run(["cuobjdump", "-sass", os.path.join(ROOT, obj)], capture_output=True, text=True).stdout
         cur, cnt = None, collections.OrderedDict()
         for line in txt.splitlines():

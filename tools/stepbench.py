@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Step-level A/B of kernel configurations through the bigcn_debug_set knobs (run on the GPU box):
-times FusedTrainer.step on three resident Twitter16-shaped batches with CUDA events."""
+"""Step-level A/B through the bigcn_debug_set keys (needs the GPU): times FusedTrainer.step on three resident
+Twitter16-shaped batches with CUDA events.  `python tools/stepbench.py 10:0,9` compares the two forms of the background
+capture pass over x (0 = TMA-fed, the shipped one; 9 = LDG)."""
 import ctypes as C
 import os
 import sys
@@ -41,17 +42,17 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / steps
-    for a in [a for a in sys.argv[1:] if a.startswith("set:")]:      # "set:13=1": holds for the whole run (combinations)
+    for a in [a for a in sys.argv[1:] if a.startswith("set:")]:      # "set:15=1": holds for the whole run (combinations)
         key, v = a[4:].split("=")
         lib.bigcn_debug_set(int(key), int(v))
-    spec = [a for a in sys.argv[1:] if not a.startswith("set:")] or ["1:0,1,2,3,4,5,6", "2:0,1,2,3,4,5", "3:0,1,2,3,4"]
+    spec = [a for a in sys.argv[1:] if not a.startswith("set:")] or ["10:0,9"]
     print(f"baseline {run():.4f} ms/step", flush=True)
     for s in spec:
         key, vals = s.split(":")
         for v in vals.split(","):
             lib.bigcn_debug_set(int(key), int(v))
             print(f"knob {key} = {v}: {run():.4f} ms/step", flush=True)
-        lib.bigcn_debug_set(int(key), 0)
+        lib.bigcn_debug_set(int(key), 0)      # 0: the shipped value of every key
     tr.check_inputs()
 
 

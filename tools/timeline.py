@@ -28,7 +28,7 @@ def main():
     lib = L.lib()
     lib.bigcn_debug_set.argtypes = [C.c_int, C.c_int]
     lib.bigcn_debug_set.restype = None
-    for spec in sys.argv[1:]:               # "knob:value" pairs (bigcn_debug_set), e.g. 4:1
+    for spec in sys.argv[1:]:               # "key:value" pairs (bigcn_debug_set), e.g. 10:9
         k, v = spec.split(":")
         lib.bigcn_debug_set(int(k), int(v))
     batches = []
