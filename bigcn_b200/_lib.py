@@ -58,6 +58,15 @@ class AsmWeights(C.Structure):
     _fields_ = [(n, c_ptr) for n in ("td_weight", "bu_weight", "edge_weight", "bu_edge_weight")]
 
 
+class Ebgcn(C.Structure):
+    _fields_ = [("N", C.c_int64), ("B", C.c_int64), ("K", C.c_int64), ("E", C.c_int64),
+                ("h1", c_ptr), ("x", c_ptr), ("edge_index", c_ptr), ("edge_weight", c_ptr), ("batch", c_ptr),
+                ("rootindex", c_ptr), ("node_ptr", c_ptr), ("bn_weight", c_ptr), ("bn_bias", c_ptr),
+                ("running_mean", c_ptr), ("running_var", c_ptr), ("num_batches_tracked", c_ptr),
+                ("momentum", C.c_float), ("eps", C.c_float), ("training", C.c_int32), ("deg_by", C.c_int32),
+                ("w2", c_ptr), ("b2", c_ptr)]
+
+
 class BigcnError(RuntimeError):
     pass
 
@@ -141,6 +150,10 @@ _SIGS = {
     "bigcn_gcnconv_weighted_backward": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, C.c_int64, c_ptr, c_ptr, c_ptr,
                                                   c_ptr, c_ptr, c_ptr, c_ptr, C.c_int32, C.c_int32, c_ptr, C.c_size_t,
                                                   c_ptr]),
+    "bigcn_ebgcn_conv2_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int64, C.c_int64]),
+    "bigcn_ebgcn_conv2_forward": (C.c_int, [C.POINTER(Ebgcn), c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
+    "bigcn_ebgcn_conv2_backward": (C.c_int, [C.POINTER(Ebgcn), c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                             c_ptr, C.c_size_t, c_ptr]),
     "bigcn_dense_row_counts": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr]),
     "bigcn_dense_row_counts_bf16": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, c_ptr]),
     "bigcn_dense_rows_to_csr": (C.c_int, [c_ptr, C.c_int64, C.c_int64, c_ptr, C.c_int64, c_ptr, c_ptr, c_ptr, C.c_int64,

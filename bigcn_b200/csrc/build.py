@@ -6,7 +6,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["api.cu", "graph_prep.cu", "xw.cu", "xsparse.cu", "gemm_tc.cu", "propagate.cu", "rootdense.cu", "head.cu", "loader.cu", "weighted.cu", "feeder.cu"]
+SOURCES = ["api.cu", "graph_prep.cu", "xw.cu", "xsparse.cu", "gemm_tc.cu", "propagate.cu", "rootdense.cu", "head.cu", "loader.cu", "weighted.cu", "feeder.cu", "ebgcn.cu"]
 HOST_SOURCES = ["host_compact.cpp"]      # host-only C++ (g++), linked into the same library
 HEADERS = ["common.cuh", "kernels.cuh", "gather.cuh", "tc.cuh", os.path.join("..", "..", "include", "bigcn_b200.h")]
 LIB = os.path.join(HERE, "..", "libbigcn_b200.so")

@@ -65,6 +65,16 @@ struct WGradDir { WGraph G; const int64_t* ei; int64_t E; const float* w; const 
                   float* ddeg; float* dw; };
 struct WGradArgs { WGradDir d[2]; int64_t N; int32_t deg_by_source; };
 int wfeat_edge_grad(const WGradArgs& a, int ndir, cudaStream_t st);
+// the generic weighted GCNConv's kernels (weighted.cu) for one direction, [N,64] operands with row pitch 64:
+// out = relu?(sum over the CSR row of norm_e[eid] h[idx] + norm_self h + bias); a_e / a_self = <g[col], h[row]>
+int w_propagate_launch(const int32_t* ptr, const int32_t* idx, const int32_t* eid, const float* norm_e,
+                       const float* norm_self, const float* h, const float* bias, float* out, int64_t N, bool relu,
+                       cudaStream_t st);
+int w_edge_dot_launch(const int64_t* ei, int64_t E, int64_t N, const float* g, const float* h, float* a_e, float* a_self,
+                      cudaStream_t st);
+int xw_dispatch(const float* x, int64_t N, int64_t K, const float* const* w, int n_w, int64_t ldw, float* scratch,
+                float* y, int64_t ldy, int mode, cudaStream_t st);
+int colsum64_launch(const float* g, int64_t N, float* part, float* out, cudaStream_t st);
 struct PropDir { const int32_t* ptr; const int32_t* idx; const float* dis; const float* h; const float* bias; float* out; int64_t ldh, ldo; int32_t* lng; int64_t E; };
 struct PropArgs { PropDir d[2]; int64_t N; int32_t relu; int32_t cb; };
 int propagate_launch(const PropArgs&, int, cudaStream_t, const EntryW* ew = nullptr);

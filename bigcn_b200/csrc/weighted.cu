@@ -78,7 +78,8 @@ __global__ void k_w_norm(WGraph G, const int64_t* __restrict__ ei, const float* 
 
 // ---- propagate: out[i] = sum_entries norm[eid] * h[idx] (+ norm_self[i] h[i]) (+ bias) -------
 // warp per row, lane owns 2 of the 64 columns; (index, norm) pairs of 32 entries per coalesced load,
-// rows gathered four at a time, accumulated strictly in entry order.
+// rows gathered four at a time, accumulated strictly in entry order.  RELU: relu of the sum (EBGCN's conv2, ebgcn.cu).
+template <bool RELU>
 __global__ void __launch_bounds__(256) k_w_propagate(const int32_t* __restrict__ ptr, const int32_t* __restrict__ idx,
                                                      const int32_t* __restrict__ eid, const float* __restrict__ norm_e,
                                                      const float* __restrict__ norm_self, const float* __restrict__ h,
@@ -129,6 +130,10 @@ __global__ void __launch_bounds__(256) k_w_propagate(const int32_t* __restrict__
     if (bias != nullptr) {
       acc.x = __fadd_rn(acc.x, bias[2 * lane]);
       acc.y = __fadd_rn(acc.y, bias[2 * lane + 1]);
+    }
+    if (RELU) {
+      acc.x = fmaxf(acc.x, 0.f);
+      acc.y = fmaxf(acc.y, 0.f);
     }
     *reinterpret_cast<float2*>(out + i * ldo + 2 * lane) = acc;
   }
@@ -469,9 +474,23 @@ int wfeat_edge_grad(const WGradArgs& a, int ndir, cudaStream_t st) {
   return 0;
 }
 
-int xw_dispatch(const float* x, int64_t N, int64_t K, const float* const* w, int n_w, int64_t ldw, float* scratch,
-                float* y, int64_t ldy, int mode, cudaStream_t st);
-int colsum64_launch(const float* g, int64_t N, float* part, float* out, cudaStream_t st);
+int w_propagate_launch(const int32_t* ptr, const int32_t* idx, const int32_t* eid, const float* norm_e,
+                       const float* norm_self, const float* h, const float* bias, float* out, int64_t N, bool relu,
+                       cudaStream_t st) {
+  if (N == 0) return 0;
+  if (relu) k_w_propagate<true><<<grid_for(N, 8), 256, 0, st>>>(ptr, idx, eid, norm_e, norm_self, h, H, bias, out, H, N);
+  else k_w_propagate<false><<<grid_for(N, 8), 256, 0, st>>>(ptr, idx, eid, norm_e, norm_self, h, H, bias, out, H, N);
+  BIGCN_CHECK_LAUNCH("k_w_propagate");
+  return 0;
+}
+
+int w_edge_dot_launch(const int64_t* ei, int64_t E, int64_t N, const float* g, const float* h, float* a_e, float* a_self,
+                      cudaStream_t st) {
+  if (N == 0) return 0;
+  k_w_edge_dot<<<grid_for(E + N, 16), 256, 0, st>>>(ei, E, N, g, h, a_e, a_self);
+  BIGCN_CHECK_LAUNCH("k_w_edge_dot");
+  return 0;
+}
 
 }  // namespace bigcn
 
@@ -516,7 +535,7 @@ extern "C" int bigcn_gcnconv_weighted_forward(const float* x, int64_t N, int64_t
   const float* ws1[1] = {w};
   if (int rc = xw_dispatch(x, N, K, ws1, 1, K, cw.wT, cw.xw, H, gemm_mode, st)) return rc;
   const WGraph& G = cw.n.G;
-  k_w_propagate<<<grid_for(N, 8), 256, 0, st>>>(G.g.in_ptr, G.g.in_idx, G.in_eid, G.norm_e, G.norm_self, cw.xw, H, bias,
+  k_w_propagate<false><<<grid_for(N, 8), 256, 0, st>>>(G.g.in_ptr, G.g.in_idx, G.in_eid, G.norm_e, G.norm_self, cw.xw, H, bias,
                                                 out, H, N);
   BIGCN_CHECK_LAUNCH("k_w_propagate");
   return 0;
@@ -536,7 +555,7 @@ extern "C" int bigcn_gcnconv_weighted_backward(const float* x, int64_t N, int64_
   if (int rc = colsum64_launch(grad_out, N, cw.cs_part, db, st)) return rc;
   if (N > 0) {
     // T = A-hat^T grad_out: the by-source CSR with the same per-edge norms
-    k_w_propagate<<<grid_for(N, 8), 256, 0, st>>>(G.g.out_ptr, G.g.out_idx, G.out_eid, G.norm_e, G.norm_self, grad_out,
+    k_w_propagate<false><<<grid_for(N, 8), 256, 0, st>>>(G.g.out_ptr, G.g.out_idx, G.out_eid, G.norm_e, G.norm_self, grad_out,
                                                   H, nullptr, cw.t, H, N);
     BIGCN_CHECK_LAUNCH("k_w_propagate");
   }

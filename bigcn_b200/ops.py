@@ -551,6 +551,86 @@ class GCNConvWeightedFunction(torch.autograd.Function):
         return dx, None, dew, dw, db, None, None
 
 
+def ebgcn_x(x):
+    """EBGCN's data.x for :class:`EBGCNConv2Function`: dense, widened to contiguous fp32 as the reference's ``.float()``
+    does.  A sparse x, or one that requires grad, raises: the op reads x only at the tree roots and forms no gradient
+    for it."""
+    if not torch.is_tensor(x) or x.layout != torch.strided:
+        raise L.BigcnError("EBGCN takes a dense data.x (a sparse x is not supported: its bn1 statistics are formed from "
+                           "the dense root rows); pass x.to_dense()")
+    if x.requires_grad:
+        raise L.BigcnError("EBGCN forms no gradient w.r.t. data.x: pass data.x.detach() (a data.x that requires grad "
+                           "is not supported)")
+    if x.dim() != 2:
+        raise L.BigcnError(f"EBGCN: data.x must be [N, input_features], got shape {tuple(x.shape)}")
+    return _f32(x)
+
+
+class EBGCNConv2Function(torch.autograd.Function):
+    """EBGCN's ``relu(conv2(relu(bn1(cat(h1, x[rootindex[batch]]))), edge_index, edge_weight))`` for one direction
+    (EBGCN.py:71-85) without the N x (64 + K) concatenation (bigcn_ebgcn_conv2_*, csrc/ebgcn.cu).  ``bn`` is the
+    module's ``torch.nn.BatchNorm1d(64 + K)``: the op reads its parameters and buffers (updating the running statistics
+    and ``num_batches_tracked`` in training, as its forward would) and does not run it.  Gradients for h1, edge_weight,
+    bn.weight, bn.bias, w2 and b2; ``x`` is data.  ``node_ptr`` ([B+1] int32) receives the tree offsets."""
+
+    @staticmethod
+    def forward(ctx, h1, edge_weight_, bn_weight, bn_bias, w2, b2, x, edge_index, batch, rootindex, bn, deg_by, node_ptr,
+                flags):
+        L.require_device()
+        h1, w2, b2 = _f32(h1), _f32(w2), _f32(b2)
+        ei, batch, rootindex = _i64(edge_index), _i64(batch), _i64(rootindex)
+        n, k = x.shape
+        e, b = int(ei.shape[1]), int(rootindex.numel())
+        ew = edge_weight(edge_weight_, e, "edge_weight")
+        _need_cuda(h1, x, ei, batch, rootindex, w2, b2)
+        if tuple(h1.shape) != (n, H):
+            raise L.BigcnError(f"EBGCN: conv1's output must be [{n},{H}], got {tuple(h1.shape)}")
+        if tuple(w2.shape) != (H, H + k) or tuple(b2.shape) != (H,):
+            raise L.BigcnError(f"EBGCN: conv2 must be GCNConv({H + k}, {H}), got weight {tuple(w2.shape)}")
+        if bn.num_features != H + k:
+            raise L.BigcnError(f"EBGCN: bn1 must be BatchNorm1d({H + k}), got {bn.num_features}")
+        gw = None if bn_weight is None else _f32(bn_weight)
+        gb = None if bn_bias is None else _f32(bn_bias)
+        rm, rv, nbt = bn.running_mean, bn.running_var, bn.num_batches_tracked
+        for t in (rm, rv):
+            if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda):
+                raise L.BigcnError("EBGCN: bn1's running statistics must be contiguous fp32 CUDA tensors")
+        a = L.Ebgcn(N=n, B=b, K=k, E=e, h1=_p(h1), x=_p(x), edge_index=_p(ei), edge_weight=_p(ew), batch=_p(batch),
+                    rootindex=_p(rootindex), node_ptr=_p(node_ptr), bn_weight=_p(gw), bn_bias=_p(gb), running_mean=_p(rm),
+                    running_var=_p(rv), num_batches_tracked=_p(nbt),
+                    momentum=-1.0 if bn.momentum is None else float(bn.momentum), eps=float(bn.eps),
+                    training=int(bn.training), deg_by=L.DEG_BY[deg_by], w2=_p(w2), b2=_p(b2))
+        ws_bytes = lib().bigcn_ebgcn_conv2_workspace_bytes(n, b, k, e)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        out = torch.empty(n, H, dtype=torch.float32, device=x.device)
+        check(lib().bigcn_ebgcn_conv2_forward(C.byref(a), _p(out), _p(flags), _p(ws), ws_bytes, _stream()),
+              "ebgcn_conv2_forward")
+        # the backward reads the same arguments: keep every tensor they point at
+        ctx.save_for_backward(h1, x, ei, batch, rootindex, node_ptr, w2, b2, ws, out,
+                              *[t for t in (ew, gw, gb) if t is not None])
+        ctx.a, ctx.has = a, (ew is not None, gw is not None, gb is not None)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        saved = ctx.saved_tensors
+        ws, out = saved[8], saved[9]
+        a = ctx.a
+        n, k, e = a.N, a.K, a.E
+        dev = out.device
+        g = _f32(grad_out)
+        dh1 = torch.empty(n, H, dtype=torch.float32, device=dev)
+        dw2 = torch.empty(H, H + k, dtype=torch.float32, device=dev)
+        db2 = torch.empty(H, dtype=torch.float32, device=dev)
+        bn_on = n != 1          # EBGCN.py:79: bn1 is skipped for a one-node batch
+        dgw = torch.empty(H + k, dtype=torch.float32, device=dev) if bn_on and ctx.needs_input_grad[2] else None
+        dgb = torch.empty(H + k, dtype=torch.float32, device=dev) if bn_on and ctx.needs_input_grad[3] else None
+        dew = torch.empty(e, dtype=torch.float32, device=dev) if ctx.has[0] and ctx.needs_input_grad[1] else None
+        check(lib().bigcn_ebgcn_conv2_backward(C.byref(a), _p(out), _p(g), _p(dh1), _p(dgw), _p(dgb), _p(dw2), _p(db2),
+                                               _p(dew), _p(ws), ws.numel(), _stream()), "ebgcn_conv2_backward")
+        return (dh1, dew, dgw, dgb, dw2, db2) + (None,) * 8
+
+
 def gcn_norm(edge_index, edge_weight=None, num_nodes=None, improved=False, add_self_loops=True, deg_by="target"):
     """``torch_geometric.nn.conv.gcn_conv.gcn_norm`` as explain_PHEME.py:62-63 calls it
     (``gcn_norm(edge_index, edge_weight, N, False, True)``): returns (edge_index', norm) with

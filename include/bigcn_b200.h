@@ -357,6 +357,44 @@ int bigcn_gcnconv_weighted_backward(const float* x, int64_t N, int64_t K, const 
                                     float* dx /*[N,K] or NULL*/, int32_t deg_by, int32_t gemm_mode,
                                     void* workspace, size_t workspace_bytes, bigcn_stream_t stream);
 
+/* ---- EBGCN's second conv (model/Twitter/EBGCN.py:71-85, BU twin :168-182) -------------------
+ * out = relu(conv2(relu(bn1(cat(h1, x[rootindex[batch]]))), edge_index, edge_weight)) for one direction, without
+ * forming the N x (64 + K) concatenation: every row of the root half in tree b is x[rootindex[b]], so bn1's
+ * statistics over those K columns are count-weighted statistics over B root rows, the normalised root half is one row
+ * R_b per tree, and its conv2 product one row Y_b = R_b W2b^T per tree.  bn1 follows torch.nn.BatchNorm1d: batch
+ * statistics (biased variance, two passes) when training or without running statistics; in training the running
+ * statistics move by `momentum` (< 0: the cumulative average of momentum=None) with the unbiased variance, and
+ * num_batches_tracked is incremented; otherwise the running statistics normalise.  N == 1 skips bn1 (EBGCN.py:79).
+ * x is dense fp32 [N,K] and gets no gradient; edge_weight NULL = every weight 1; bn_weight / bn_bias NULL = no affine;
+ * running_mean / running_var / num_batches_tracked NULL = no running statistics.  node_ptr [B+1] (out) receives the
+ * tree offsets of the sorted batch vector.  Deterministic, no floating-point atomics.
+ *   backward: grad_out [N,64] at `out`; dh1 [N,64] (the gradient reaching conv1's output), d_bn_weight / d_bn_bias
+ *   [64+K] (NULL skips; not written when N == 1), dw2 [64,64+K], db2 [64], d_edge_weight [E] or NULL.  Takes the
+ *   forward's workspace and the same arguments. */
+typedef struct {
+  int64_t N, B, K, E;
+  const float* h1;                       /* [N,64] conv1 output */
+  const float* x;                        /* [N,K] */
+  const int64_t* edge_index;             /* [2,E] */
+  const float* edge_weight;              /* [E] or NULL */
+  const int64_t* batch;                  /* [N], sorted */
+  const int64_t* rootindex;              /* [B] */
+  int32_t* node_ptr;                     /* [B+1], written by the forward */
+  const float* bn_weight; const float* bn_bias;   /* [64+K] or NULL */
+  float* running_mean; float* running_var;        /* [64+K] or NULL */
+  int64_t* num_batches_tracked;                   /* [1] or NULL */
+  float momentum, eps;
+  int32_t training, deg_by;
+  const float* w2;                       /* conv2.lin.weight [64, 64+K] */
+  const float* b2;                       /* conv2.bias [64] */
+} bigcn_ebgcn_t;
+size_t bigcn_ebgcn_conv2_workspace_bytes(int64_t N, int64_t B, int64_t K, int64_t E);
+int bigcn_ebgcn_conv2_forward(const bigcn_ebgcn_t* a, float* out /*[N,64]*/, int32_t* flags, void* workspace,
+                              size_t workspace_bytes, bigcn_stream_t stream);
+int bigcn_ebgcn_conv2_backward(const bigcn_ebgcn_t* a, const float* out, const float* grad_out, float* dh1,
+                               float* d_bn_weight, float* d_bn_bias, float* dw2, float* db2, float* d_edge_weight,
+                               void* workspace, size_t workspace_bytes, bigcn_stream_t stream);
+
 /* ---- the two-direction feature path ------------------------------------
  * Replaces TDrumorGCN.forward / BUrumorGCN.forward (BiGCN_Twitter.py:26-67,
  * 77-114): conv1, root-extend, relu, dropout, conv2, relu, root-extend,
