@@ -18,11 +18,10 @@ import torch
 
 from . import _lib as L
 import ctypes as C
-import weakref
 
-from .ops import (FeaturesFunction, GCNConvFunction, GCNConvWeightedFunction, HeadFunction, raise_on_flags,
-                  capture_graph, pick_gemm_mode, bf16_features_dense, edge_weight, x_val, _as_x, _i64, _make_structs, _p,
-                  _stream)
+from .ops import (FeaturesFunction, GCNConvFunction, GCNConvWeightedFunction, GraphCache, HeadFunction, raise_on_flags,
+                  pick_gemm_mode, bf16_features_dense, batch_args, batch_key, edge_weight_key, features_workspace_bytes,
+                  x_val, _p, _stream)
 
 H = L.H
 
@@ -170,8 +169,7 @@ class BiGCN(torch.nn.Module):
         self.validate = validate            # "lazy": check the previous call's flags; "sync"; "off"
         self.last_flags = None
         self.graphs = bool(graphs)          # inference under torch.no_grad(): replay a CUDA graph for a batch seen before
-        self.max_graphs = int(max_graphs)
-        self._graphs, self._seen = {}, {}
+        self._graphs = GraphCache(max_graphs, 4096)
 
     @property
     def gemm_mode(self):
@@ -212,30 +210,20 @@ class BiGCN(torch.nn.Module):
         L.require_device()
         td, bu = self.TDrumorGCN, self.BUrumorGCN
         mode = td.resolved_gemm_mode(data.x)
-        x, xs = _as_x(data.x, mode)
-        ei, bue, batch, root = _i64(data.edge_index), _i64(data.BU_edge_index), _i64(data.batch), _i64(data.rootindex)
-        params = tuple(p.detach() for p in td._conv_params() + bu._conv_params())
-        for t in (x, ei, bue, batch, root) + params:
-            if t is not None and not t.is_cuda:
-                raise L.BigcnError("bigcn_b200 ops take CUDA tensors only (no CPU fallback)")
         c = self.fc.weight.shape[0]
-        if xs is not None and mode != "sparse":
-            raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
-        ew = (edge_weight(getattr(data, "edge_weight", None), int(ei.shape[1]), "edge_weight"),
-              edge_weight(getattr(data, "BU_edge_weight", None), int(bue.shape[1]), "BU_edge_weight"))
-        dims, bt, pr = _make_structs(x, ei, bue, batch, root, params, c, td.node_id_base, xs, ew)
+        params = tuple(p.detach() for p in td._conv_params() + bu._conv_params())
+        a = batch_args(data.x, data.edge_index, data.BU_edge_index, data.batch, data.rootindex,
+                       getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None), gemm_mode=mode,
+                       num_classes=c, node_id_base=td.node_id_base, params=params)
         opts = td._opts(L.DIR_TD | L.DIR_BU, data.x)
         o = L.Opts(training=int(self.training), p_drop=float(td.p), seed=int(opts["seed"]), deg_by=L.DEG_BY[td.deg_by],
                    gemm_mode=L.GEMM_MODE[mode], dir_mask=L.DIR_TD | L.DIR_BU, skip_wgrad_prep=1)
-        dev = xs.device if xs is not None else x.device
-        nbytes = L.lib().bigcn_features_workspace_bytes(C.byref(dims)) if ew == (None, None) else \
-            L.lib().bigcn_features_edge_workspace_bytes(C.byref(dims), 0)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        return {"dims": dims, "bt": bt, "pr": pr, "o": o, "ws": ws, "c": c,
-                "keep": (x, xs, ei, bue, batch, root, params, ew, self.fc.weight, self.fc.bias),
-                "flags": torch.zeros(1, dtype=torch.int32, device=dev),
-                "feat": torch.empty(dims.B, 4 * H, dtype=torch.float32, device=dev),
-                "logp": torch.empty(dims.B, c, dtype=torch.float32, device=dev)}
+        ws = torch.empty(features_workspace_bytes(a.dims, a.weighted), dtype=torch.uint8, device=a.dev)
+        return {"dims": a.dims, "bt": a.bt, "pr": a.pr, "o": o, "ws": ws, "c": c,
+                "keep": (a, params, self.fc.weight, self.fc.bias),
+                "flags": torch.zeros(1, dtype=torch.int32, device=a.dev),
+                "feat": torch.empty(a.dims.B, 4 * H, dtype=torch.float32, device=a.dev),
+                "logp": torch.empty(a.dims.B, c, dtype=torch.float32, device=a.dev)}
 
     def _infer_enqueue(self, p):
         l, st = L.lib(), _stream()
@@ -246,36 +234,17 @@ class BiGCN(torch.nn.Module):
 
     def _forward_nograd(self, data):
         use_graph = self.graphs and not (self.training and self.TDrumorGCN.p > 0)   # train-mode masks need a fresh seed
-        if not use_graph:
+        p = key = None
+        if use_graph:
+            key = batch_key(data) + (edge_weight_key(data), tuple(q.data_ptr() for q in self.parameters()),
+                                     self.training, self.TDrumorGCN.deg_by, self.TDrumorGCN.gemm_mode)
+            p = self._graphs.replay(key)
+        if p is None:
             p = self._infer_plan(data)
-            self._infer_enqueue(p)
-        else:
-            x = data.x
-            xk = (x.ptr.data_ptr(), x.col.data_ptr(), x.val.data_ptr(), x.shape) if hasattr(x, "ptr") else \
-                (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
-            ews = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
-            key = (id(data), xk, tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
-                             (data.edge_index, data.BU_edge_index, data.batch, data.rootindex)),
-                   tuple(None if t is None else (t.data_ptr(), tuple(t.shape), t.dtype) for t in ews),
-                   tuple(q.data_ptr() for q in self.parameters()), self.training, self.TDrumorGCN.deg_by,
-                   self.TDrumorGCN.gemm_mode)
-            p = self._graphs.get(key)
-            if p is not None:
-                p["graph"].replay()
-            elif self._seen.get(key) is None or self._seen[key]() is not data:   # first sighting of this batch object
-                if len(self._seen) >= 4096:
-                    self._seen.clear()
-                self._seen[key] = weakref.ref(data)
-                p = self._infer_plan(data)
+            if not use_graph or self._graphs.first_sighting(key, data):
                 self._infer_enqueue(p)
-            else:                               # seen before: capture, then replay
-                p = self._infer_plan(data)
-                g = capture_graph(lambda: self._infer_enqueue(p))
-                p["graph"], p["data"] = g, data        # the strong reference pins id(data)
-                while len(self._graphs) >= self.max_graphs:
-                    self._graphs.pop(next(iter(self._graphs)))
-                self._graphs[key] = p
-                g.replay()
+            else:
+                self._graphs.capture(key, lambda: self._infer_enqueue(p), p, data=data)
         self.last_flags = p["flags"]
         if self.validate == "sync":
             self.check_inputs()

@@ -3,6 +3,9 @@ autograd plumbing; every arithmetic step runs in libbigcn_b200.so."""
 from __future__ import annotations
 
 import ctypes as C
+import operator
+import weakref
+from types import SimpleNamespace
 
 import torch
 
@@ -24,19 +27,23 @@ _capture_streams = {}
 _step_streams = {}
 
 
-def step_stream(device=None):
-    """A stream two priority levels above the default one (the library's own levels are listed in csrc/api.cu), per device: FusedTrainer runs (and captures) its steps
-    on it so that bigcn_batch_prepare's lowest-priority streams -- the next batch's preparation -- really yield
-    to the step's own kernels (the caller's default stream already has the lowest priority there is)."""
-    dev = torch.cuda.current_device() if device is None else torch.device(device).index
-    s = _step_streams.get(dev)
+def _priority_stream(table, dev):
+    """``table``'s stream on device ``dev``, two priority levels above the default one (levels: csrc/api.cu)"""
+    s = table.get(dev)
     if s is None:
         try:
             lo, hi = torch.cuda.Stream.priority_range()
         except Exception:  # noqa: BLE001
             lo, hi = 0, -1
-        s = _step_streams[dev] = torch.cuda.Stream(device=dev, priority=max(hi, lo - 2) if hi < lo else lo)
+        s = table[dev] = torch.cuda.Stream(device=dev, priority=max(hi, lo - 2) if hi < lo else lo)
     return s
+
+
+def step_stream(device=None):
+    """A stream two priority levels above the default one, per device: FusedTrainer runs (and captures) its steps
+    on it so that bigcn_batch_prepare's lowest-priority streams -- the next batch's preparation -- really yield
+    to the step's own kernels (the caller's default stream already has the lowest priority there is)."""
+    return _priority_stream(_step_streams, torch.cuda.current_device() if device is None else torch.device(device).index)
 
 
 def capture_graph(enqueue):
@@ -44,14 +51,8 @@ def capture_graph(enqueue):
     torch.cuda.CUDAGraph on a side stream.  The bare capture_begin / capture_end pair instead of the
     ``torch.cuda.graph`` context manager: no device synchronise, gc.collect or empty_cache per capture, so a
     capture costs about one enqueue plus the instantiation."""
-    dev = torch.cuda.current_device()
-    s = _capture_streams.get(dev)
-    if s is None:       # kernel nodes inherit the capturing stream's priority: the step stream's level
-        try:
-            lo, hi = torch.cuda.Stream.priority_range()
-        except Exception:  # noqa: BLE001
-            lo, hi = 0, -1
-        s = _capture_streams[dev] = torch.cuda.Stream(device=dev, priority=max(hi, lo - 2) if hi < lo else lo)
+    # kernel nodes inherit the capturing stream's priority: the step stream's level
+    s = _priority_stream(_capture_streams, torch.cuda.current_device())
     cur = torch.cuda.current_stream()
     s.wait_stream(cur)
     g = torch.cuda.CUDAGraph()
@@ -63,6 +64,52 @@ def capture_graph(enqueue):
             g.capture_end()
     cur.wait_stream(s)
     return g
+
+
+class GraphCache:
+    """CUDA graphs by batch key: a batch object's first sighting is enqueued (which also warms the library's lazy
+    state), its second is captured, later ones replay.  Keeps at most ``max_graphs`` captures (the oldest goes first)
+    and ``max_seen`` first sightings; ``clear()`` drops the captures only."""
+
+    def __init__(self, max_graphs, max_seen, capture=capture_graph):
+        self.max_graphs, self.max_seen, self._capture = int(max_graphs), int(max_seen), capture
+        self._entries, self._seen = {}, {}     # key -> (graph, plan, pins, batch); key -> weakref to the batch
+        self.captures = self.replays = 0
+
+    def __len__(self):
+        return len(self._entries)
+
+    def clear(self):
+        self._entries.clear()
+
+    def replay(self, key, pins=()):
+        """Replay ``key``'s capture and return its plan if ``pins`` are the objects they were at capture, else None"""
+        e = self._entries.get(key)
+        if e is None or len(e[2]) != len(pins) or not all(map(operator.is_, e[2], pins)):
+            return None
+        e[0].replay()
+        self.replays += 1
+        return e[1]
+
+    def first_sighting(self, key, data):
+        """True (and remembered, weakly) the first time ``data`` comes under ``key``"""
+        ref = self._seen.get(key)
+        if ref is not None and ref() is data:
+            return False
+        if len(self._seen) >= self.max_seen:
+            self._seen.clear()
+        self._seen[key] = weakref.ref(data)
+        return True
+
+    def capture(self, key, enqueue, plan, pins=(), data=None):
+        """Capture ``enqueue()`` as the graph of ``key`` and replay it.  The entry keeps ``plan`` (what the launches
+        point at) and ``data``: the strong reference pins id(data)."""
+        g = self._capture(enqueue)
+        while len(self._entries) >= self.max_graphs:
+            self._entries.pop(next(iter(self._entries)))
+        self._entries[key] = (g, plan, tuple(pins), data)
+        self.captures += 1
+        self.replay(key, pins)
 
 
 def _need_cuda(*ts):
@@ -685,15 +732,64 @@ def _make_structs(x, ei, bu_ei, batch, rootindex, params, num_classes, node_id_b
     n, k = xs.shape if xs is not None else x.shape
     dims = Dims(N=n, B=int(rootindex.numel()), K=k, C=num_classes, E_td=int(ei.shape[1]),
                 E_bu=int(bu_ei.shape[1]))
-    bt = BatchPtrs(x=_p(x), edge_index=_p(ei), bu_edge_index=_p(bu_ei), batch=_p(batch),
-                   rootindex=_p(rootindex), node_id_base=int(node_id_base))
+    bt = BatchPtrs(x=_p(x), edge_index=_p(ei), bu_edge_index=_p(bu_ei), batch=_p(batch), rootindex=_p(rootindex),
+                   node_id_base=int(node_id_base), td_edge_weight=_p(ew[0]), bu_edge_weight=_p(ew[1]))
     if xs is not None:
         bt.x_ptr, bt.x_col, bt.x_val = _p(xs.ptr), _p(xs.col), _p(xs.val)
-    bt.td_edge_weight, bt.bu_edge_weight = _p(ew[0]), _p(ew[1])
     pr = Params()
     for name, t in zip(_PNAMES, params):
+        if t is not None:
+            want = {"w1": (H, k), "b1": (H,), "w2": (H, H + k), "b2": (H,)}[name[3:]]
+            if tuple(t.shape) != want:
+                raise L.BigcnError(f"{name}: expected shape {want} (hid_feats = out_feats = 64), got {tuple(t.shape)}")
         setattr(pr, name, _p(t))
     return dims, bt, pr
+
+
+def batch_args(x, edge_index, bu_edge_index, batch, rootindex, td_ew=None, bu_ew=None, *, gemm_mode, num_classes=0,
+               node_id_base=0, params=()):
+    """Check a batch and lay it out for the feature path: data.x as ``gemm_mode`` reads it, the index tensors as
+    int64, the edge weights as fp32 [E], all on a CUDA device; ``params`` (``_PNAMES`` order, None for a direction
+    left out) shape-checked.  Returns the structs ``dims``, ``bt``, ``pr`` (null pointers without params), the tensors
+    they point at, which the caller keeps until the launches are done (``x`` or ``xs`` (SparseX), ``ei``, ``bu``,
+    ``batch``, ``root``, ``ew`` = (TD, BU)), ``dev`` and ``weighted``."""
+    x, xs = _as_x(x, gemm_mode)
+    if xs is not None and gemm_mode != "sparse":
+        raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
+    ei, bu, batch, root = _i64(edge_index), _i64(bu_edge_index), _i64(batch), _i64(rootindex)
+    _need_cuda(x, ei, bu, batch, root, *params)
+    if xs is not None:
+        _need_cuda(xs.ptr, xs.col, xs.val)
+    ew = (edge_weight(td_ew, int(ei.shape[1]), "edge_weight"), edge_weight(bu_ew, int(bu.shape[1]), "BU_edge_weight"))
+    dims, bt, pr = _make_structs(x, ei, bu, batch, root, params, num_classes, node_id_base, xs, ew)
+    return SimpleNamespace(dims=dims, bt=bt, pr=pr, x=x, xs=xs, ei=ei, bu=bu, batch=batch, root=root, ew=ew,
+                           dev=xs.device if xs is not None else x.device, weighted=any(w is not None for w in ew))
+
+
+def features_workspace_bytes(dims, weighted, edge_grad=False):
+    return lib().bigcn_features_edge_workspace_bytes(C.byref(dims), int(edge_grad)) if weighted else \
+        lib().bigcn_features_workspace_bytes(C.byref(dims))
+
+
+def batch_prepare_bytes(dims, weighted):
+    return (lib().bigcn_batch_prepare_edge_bytes if weighted else lib().bigcn_batch_prepare_bytes)(C.byref(dims))
+
+
+def batch_key(data, *extra):
+    """What a captured CUDA graph or a prepared buffer read of a batch: the object, and where its tensors (data.x, the
+    two edge indices, batch, rootindex, then ``extra``) live, with their shapes and dtypes -- not their values"""
+    x = data.x
+    xk = (x.ptr.data_ptr(), x.col.data_ptr(), x.val.data_ptr(), x.shape) if hasattr(x, "ptr") else \
+        (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
+    # built on every replayed step: a list comprehension costs less host time than a generator here
+    return (id(data), xk, tuple([(t.data_ptr(), tuple(t.shape), t.dtype) for t in
+                                 (data.edge_index, data.BU_edge_index, data.batch, data.rootindex, *extra)]))
+
+
+def edge_weight_key(data):
+    """batch_key's counterpart for the batch's edge weights (data.edge_weight, data.BU_edge_weight)"""
+    return tuple([(w.data_ptr(), tuple(w.shape), w.dtype) if torch.is_tensor(w) else id(w)
+                  for w in (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))])
 
 
 def x_val(x):
@@ -725,41 +821,24 @@ class FeaturesFunction(torch.autograd.Function):
             ctx.x_pattern = (x.indices(),) if x.layout == torch.sparse_coo else (x.crow_indices(), x.col_indices())
         elif ctx.needs_input_grad[0] and x.layout != torch.strided:
             raise L.BigcnError(f"a gradient w.r.t. a {x.layout} data.x is not produced: pass it as sparse COO or CSR")
-        x, xs = _as_x(x, opts["gemm_mode"])
-        if xs is not None and opts["gemm_mode"] != "sparse":
-            raise L.BigcnError("a sparse data.x needs gemm_mode='sparse'")
-        ei, bu_ei, batch, rootindex = _i64(ei), _i64(bu_ei), _i64(batch), _i64(rootindex)
         params = tuple(None if p is None else _f32(p) for p in params)
-        _need_cuda(x, ei, bu_ei, batch, rootindex, *params)
-        if xs is not None:
-            _need_cuda(xs.ptr, xs.col, xs.val)
-        k = xs.shape[1] if xs is not None else x.shape[1]
-        dev = xs.device if xs is not None else x.device
-        for name, p in zip(_PNAMES, params):
-            if p is None:
-                continue
-            want = {"w1": (H, k), "b1": (H,), "w2": (H, H + k), "b2": (H,)}[name[3:]]
-            if tuple(p.shape) != want:
-                raise L.BigcnError(f"{name}: expected shape {want} (hid_feats = out_feats = 64), got {tuple(p.shape)}")
-        ew = (edge_weight(td_ew, int(ei.shape[1]), "edge_weight"), edge_weight(bu_ew, int(bu_ei.shape[1]), "BU_edge_weight"))
+        a = batch_args(x, ei, bu_ei, batch, rootindex, td_ew, bu_ew, gemm_mode=opts["gemm_mode"],
+                       node_id_base=opts["node_id_base"], params=params)
+        x, xs, dims, dev = a.x, a.xs, a.dims, a.dev
         want_grad = opts.get("want_grad", True)
         edge_grad = want_grad and (ctx.needs_input_grad[6] or ctx.needs_input_grad[7])
-        dims, bt, pr = _make_structs(x, ei, bu_ei, batch, rootindex, params, 0, opts["node_id_base"], xs, ew)
         o = Opts(training=int(opts["training"]), p_drop=float(opts["p"]), seed=int(opts["seed"]),
                  deg_by=L.DEG_BY[opts["deg_by"]], gemm_mode=L.GEMM_MODE[opts["gemm_mode"]],
                  dir_mask=int(opts["dir_mask"]), dense_roots=int(bool(opts.get("dense_roots", False))),
                  # inference (torch.no_grad() or no parameter wants a gradient): no column sort of x
                  skip_wgrad_prep=int(not (want_grad and any(ctx.needs_input_grad))), edge_grad=int(edge_grad))
-        if ew == (None, None):
-            ws_bytes = lib().bigcn_features_workspace_bytes(C.byref(dims))
-        else:
-            ws_bytes = lib().bigcn_features_edge_workspace_bytes(C.byref(dims), o.edge_grad)
+        ws_bytes = features_workspace_bytes(dims, a.weighted, o.edge_grad)
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         flags = opts.get("flags")
         if flags is None:
             flags = torch.zeros(1, dtype=torch.int32, device=dev)
         feat = torch.empty(dims.B, 4 * H, dtype=torch.float32, device=dev)
-        check(lib().bigcn_features_forward(C.byref(dims), C.byref(bt), C.byref(pr), C.byref(o), _p(feat),
+        check(lib().bigcn_features_forward(C.byref(dims), C.byref(a.bt), C.byref(a.pr), C.byref(o), _p(feat),
                                            _p(flags), _p(ws), ws_bytes, _stream()), "features_forward")
         if o.gemm_mode == L.GEMM_MODE["sparse"] and not o.skip_wgrad_prep:
             # the column sort of x is still running on the library's low-priority stream: keep the
@@ -771,25 +850,26 @@ class FeaturesFunction(torch.autograd.Function):
                     t.record_stream(side)
         xt = (x,) if xs is None else (xs.ptr, xs.col, xs.val)
         ctx.x_sparse_shape = None if xs is None else xs.shape
-        ctx.save_for_backward(*xt, ei, bu_ei, batch, rootindex, ws, *[p for p in params if p is not None])
+        # the backward reuses the structs: the saved tensors are the ones they point at
+        ctx.save_for_backward(*xt, a.ei, a.bu, a.batch, a.root, ws, *[p for p in params if p is not None])
         ctx.present = [p is not None for p in params]
         ctx.o = o
-        ctx.ew = ew
-        ctx.node_id_base = opts["node_id_base"]
+        ctx.ew = a.ew
+        ctx.structs = (dims, a.bt, a.pr)
         ctx.flags = flags
         return feat
 
     @staticmethod
     def backward(ctx, grad_feat):
-        saved = ctx.saved_tensors
+        saved = ctx.saved_tensors      # unpacked all the same: autograd's check that none was modified in place
         x, xs = saved[0], None
         if ctx.x_sparse_shape is not None:
             x, xs = None, SparseX(saved[0], saved[1], saved[2], ctx.x_sparse_shape)
             saved = saved[2:]
-        ei, bu_ei, batch, rootindex, ws = saved[1:6]
+        ws = saved[5]
         it = iter(saved[6:])
         params = tuple(next(it) if pres else None for pres in ctx.present)
-        dims, bt, pr = _make_structs(x, ei, bu_ei, batch, rootindex, params, 0, ctx.node_id_base, xs, ctx.ew)
+        dims, bt, pr = ctx.structs
         grads = tuple(None if p is None else torch.empty_like(p) for p in params)
         gs = Params()
         for name, t in zip(_PNAMES, grads):

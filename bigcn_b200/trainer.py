@@ -16,7 +16,8 @@ import torch.utils.weak
 
 from . import _lib as L
 from ._lib import H, Opts, Params, check, lib
-from .ops import _make_structs, _p, _stream, _i64, _f32, _as_x, capture_graph, edge_weight, raise_on_flags, step_stream
+from .ops import (GraphCache, _p, _stream, _i64, batch_args, batch_key, batch_prepare_bytes, edge_weight_key,
+                  features_workspace_bytes, raise_on_flags, step_stream)
 
 # flat layout: the two conv1 weights (the gradients the second X stream produces LAST) first, so
 # the gradient splits into two contiguous all-reduce buckets: [W1_td | W1_bu] and [everything else]
@@ -124,10 +125,11 @@ class FusedTrainer:
         self._calls = 0
         self.launches_per_step = None
         self.graphs = (self.comm in ("single", "symm")) if graphs == "auto" else bool(graphs)
-        self.max_graphs = int(max_graphs)
-        self._graphs, self._seen = {}, {}   # captured steps by batch identity; batch identities seen once
+        self._graphs = GraphCache(max_graphs, 256)   # captured steps by batch key
         self._prep_buf, self._prep_owner = None, [None, None]   # two prepared-batch buffers and what they hold
-        self.graph_captures = self.graph_replays = 0
+
+    graph_captures = property(lambda self: self._graphs.captures)
+    graph_replays = property(lambda self: self._graphs.replays)
 
     # -------------------------------------------------------------------------------
     def _setup_symm(self, dev):
@@ -172,45 +174,46 @@ class FusedTrainer:
                 self._stptrs = (C.c_void_p * self.world)(*[int(p) for p in hst.buffer_ptrs])
 
     def _workspace(self, dims, dev, weighted=False, edge_grad=False):
-        need = lib().bigcn_features_edge_workspace_bytes(C.byref(dims), int(edge_grad)) if weighted else \
-            lib().bigcn_features_workspace_bytes(C.byref(dims))
+        need = features_workspace_bytes(dims, weighted, edge_grad)
         if self._ws is None or self._ws.numel() < need:
             # head room: captured graphs hold pointers into the workspace, a slightly larger batch should not move it
             self._ws = torch.empty(need + need // 4 if self.graphs else need, dtype=torch.uint8, device=dev)
-        return self._ws
+            self._graphs.clear()               # the workspace moved: every captured pointer into it is stale
+
+    def _batch_args(self, data, num_classes, node_id_base):
+        # grad mode on: a weight that requires grad keeps its autograd link through the fp32 cast (edge_grad)
+        with torch.enable_grad():
+            return batch_args(data.x, data.edge_index, data.BU_edge_index, data.batch, data.rootindex,
+                              getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None),
+                              gemm_mode=self.model.TDrumorGCN.resolved_gemm_mode(data.x), num_classes=num_classes,
+                              node_id_base=node_id_base)
 
     def _plan(self, data, b_global, node_id_base, seed):
         """Everything one step needs besides the launches: argument structs, output buffers, workspace."""
         m = self.model
-        x, xs = _as_x(data.x, m.TDrumorGCN.resolved_gemm_mode(data.x))
-        ei, bu, batch, root = _i64(data.edge_index), _i64(data.BU_edge_index), _i64(data.batch), \
-            _i64(data.rootindex)
-        y = _i64(data.y)
         td = m.TDrumorGCN
         c = m.fc.weight.shape[0]
-        ew = self._weights(data, ei, bu)
+        a = self._batch_args(data, c, node_id_base)
+        y = _i64(data.y)
         # edge_grad: d loss / d weight of each direction whose weight requires grad (ew keeps the autograd link of a cast)
         dew = [torch.empty(w.numel(), dtype=torch.float32, device=w.device) if w is not None and w.requires_grad else None
-               for w in ew]
+               for w in a.ew]
         eg = self.edge_grad and any(d is not None for d in dew)
-        dims, bt, _ = _make_structs(x, ei, bu, batch, root, (None,) * 8, c, node_id_base, xs, ew)
         # seed=None: the module's seed plus the device-side calls counter (step_count[2], advanced by the
         # optimiser kernel) -- the same value whether the step is enqueued or replayed from a CUDA graph
         o = Opts(training=int(m.training), p_drop=float(td.p), seed=int(td.seed if seed is None else seed) & ((1 << 64) - 1),
                  deg_by=L.DEG_BY[td.deg_by], gemm_mode=L.GEMM_MODE[td.resolved_gemm_mode(data.x)], dir_mask=L.DIR_TD | L.DIR_BU,
                  fused_tail=1, seed_dev=self.step_count[2:].data_ptr() if seed is None else None,
                  dense_roots=int(td.resolved_dense_roots(data.x)), edge_grad=int(eg))
-        dev = xs.device if xs is not None else x.device
-        b = dims.B
-        p = {"dims": dims, "bt": bt, "o": o, "b": b, "c": c, "dev": dev, "y": y, "b_global": int(b_global or b),
-             "keep": (x, xs, ei, bu, batch, root, y, ew), "weighted": any(w is not None for w in ew),
-             "edge_grad": eg, "ew": ew, "dew": dew,
-             "feat": torch.empty(b, 4 * H, dtype=torch.float32, device=dev),
-             "logp": torch.empty(b, c, dtype=torch.float32, device=dev),
-             "gfeat": torch.empty(b, 4 * H, dtype=torch.float32, device=dev),
-             "loss": torch.empty(1, dtype=torch.float32, device=dev)}
+        b = a.dims.B
+        p = {"dims": a.dims, "bt": a.bt, "o": o, "b": b, "c": c, "dev": a.dev, "y": y, "b_global": int(b_global or b),
+             "keep": a, "weighted": a.weighted, "edge_grad": eg, "ew": a.ew, "dew": dew,
+             "feat": torch.empty(b, 4 * H, dtype=torch.float32, device=a.dev),
+             "logp": torch.empty(b, c, dtype=torch.float32, device=a.dev),
+             "gfeat": torch.empty(b, 4 * H, dtype=torch.float32, device=a.dev),
+             "loss": torch.empty(1, dtype=torch.float32, device=a.dev)}
         p["nscr"] = lib().bigcn_head_train_scratch_floats(b, c)
-        p["scr"] = torch.empty(p["nscr"], dtype=torch.float32, device=dev)
+        p["scr"] = torch.empty(p["nscr"], dtype=torch.float32, device=a.dev)
         return p
 
     def _enqueue(self, p):
@@ -293,55 +296,32 @@ class FusedTrainer:
     # ---- batches prepared one step ahead (bigcn_batch_prepare) ---------------------------------------------
     def _prep_key(self, data):
         td = self.model.TDrumorGCN
-        x = data.x
-        xk = (x.ptr.data_ptr(), x.col.data_ptr(), x.val.data_ptr(), x.shape) if hasattr(x, "ptr") else \
-            (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
-        small = tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
-                      (data.edge_index, data.BU_edge_index, data.batch, data.rootindex))
-        return (id(data), xk, small, self._weight_key(data, True), td.deg_by, td.resolved_gemm_mode(data.x))
+        return batch_key(data) + (self._weight_key(data, True), td.deg_by, td.resolved_gemm_mode(data.x))
 
     def _prep_setup(self, p, data, next_data, node_id_base):
         """Decide which prepared buffer this step reads (or prepares inline) and which one the next batch's
         preparation writes; returns the part of the CUDA-graph key that pins those decisions."""
-        l = lib()
-        pk = self._prep_key(data)
-
-        def prep_bytes(dims, weighted):
-            return (l.bigcn_batch_prepare_edge_bytes if weighted else l.bigcn_batch_prepare_bytes)(C.byref(dims))
-        need = prep_bytes(p["dims"], p["weighted"])
-        nxt = None
+        need = batch_prepare_bytes(p["dims"], p["weighted"])
         if next_data is not None:
-            nx, nxs = _as_x(next_data.x, self.model.TDrumorGCN.resolved_gemm_mode(next_data.x))
-            nei, nbu = _i64(next_data.edge_index), _i64(next_data.BU_edge_index)
-            new = self._weights(next_data, nei, nbu)
-            nd, nbt, _ = _make_structs(nx, nei, nbu, _i64(next_data.batch), _i64(next_data.rootindex), (None,) * 8, p["c"],
-                                       0, nxs, new)
-            need = max(need, prep_bytes(nd, any(w is not None for w in new)))
-            nxt = {"dims": nd, "bt": nbt, "keep": (nx, nxs, nei, nbu, new, next_data), "key": self._prep_key(next_data)}
+            na = self._batch_args(next_data, p["c"], 0)
+            need = max(need, batch_prepare_bytes(na.dims, na.weighted))
         if self._prep_buf is None or self._prep_buf[0].numel() < need:
             self._prep_buf = [torch.empty(need + need // 4, dtype=torch.uint8, device=p["dev"]) for _ in range(2)]
             self._prep_owner = [None, None]
             self._graphs.clear()               # captured pointers into the old buffers are stale
-        slot = next((i for i in (0, 1) if self._prep_owner[i] is not None and self._prep_owner[i][0] == pk
-                     and self._prep_owner[i][1]() is data), None)
-        p["prep_inline"] = slot is None
-        if slot is None:
-            slot = 0
+        pkey = self._prep_peek(data, next_data)
+        slot, p["prep_inline"], nkey = pkey
         p["slot"] = slot
         p["bt"].prepared = self._prep_buf[slot].data_ptr()
-        if nxt is not None:
-            nxt["slot"] = 1 - slot
-            p["next"] = nxt
-        return (slot, p["prep_inline"], None if nxt is None else nxt["key"])
+        if next_data is not None:
+            p["next"] = {"dims": na.dims, "bt": na.bt, "keep": (na, next_data), "key": nkey, "slot": 1 - slot}
+        return pkey
 
     def _prep_peek(self, data, next_data):
-        """(slot, inline, key of the next batch) as _prep_setup would decide them, without building anything."""
-        slot = None
-        if self._prep_buf is not None:
-            pk = self._prep_key(data)
-            slot = next((i for i in (0, 1) if self._prep_owner[i] is not None and self._prep_owner[i][0] == pk
-                         and self._prep_owner[i][1]() is data), None)
-        return (0 if slot is None else slot, slot is None, None if next_data is None else self._prep_key(next_data))
+        """(slot, inline, key of the next batch): the prepared buffer holding ``data`` as it is now, else (0, True)"""
+        pk = self._prep_key(data)
+        slot = next((i for i, o in enumerate(self._prep_owner) if o is not None and o[0] == pk and o[1]() is data), None)
+        return (slot or 0, slot is None, None if next_data is None else self._prep_key(next_data))
 
     def _prep_commit(self, p, data, next_data):
         """Host-side record of what the prepared buffers hold after this step (enqueued or replayed)."""
@@ -351,13 +331,8 @@ class FusedTrainer:
 
     def _graph_key(self, data, b_global, node_id_base):
         m, td = self.model, self.model.TDrumorGCN
-        x = data.x
-        xk = (x.ptr.data_ptr(), x.col.data_ptr(), x.val.data_ptr(), x.shape) if hasattr(x, "ptr") else \
-            (x.data_ptr(), tuple(x.shape), x.dtype, x.layout)
-        small = tuple((t.data_ptr(), tuple(t.shape), t.dtype) for t in
-                      (data.edge_index, data.BU_edge_index, data.batch, data.rootindex, data.y))
-        return (id(data), xk, small, self._weight_key(data, False), b_global, node_id_base, m.training, td.p, td.deg_by,
-                td.gemm_mode, td.dense_roots, td.seed)
+        return batch_key(data, data.y) + (self._weight_key(data, False), b_global, node_id_base, m.training, td.p,
+                                          td.deg_by, td.gemm_mode, td.dense_roots, td.seed)
 
     # ---- edge weights (edge_weights=True) ------------------------------------------------------------------
     def _weight_key(self, data, prepared):
@@ -365,9 +340,9 @@ class FusedTrainer:
         edge_grad the tensors are told apart by identity (a serial per live tensor, so one at a recycled address is
         another) and, for a prepared buffer (``prepared``), by ``_version``: learnt weights change between steps, and a
         normalisation prepared from older values must not be used"""
-        ws = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
         if not self.edge_grad:
-            return tuple((w.data_ptr(), tuple(w.shape), w.dtype) if torch.is_tensor(w) else id(w) for w in ws)
+            return edge_weight_key(data)
+        ws = (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None))
         return tuple((w.data_ptr(), self._serial(w), w._version if prepared else None, tuple(w.shape), w.dtype,
                       w.requires_grad) if torch.is_tensor(w) else id(w) for w in ws)
 
@@ -393,14 +368,6 @@ class FusedTrainer:
     def _weights_copied(data):
         return any(torch.is_tensor(w) and (w.dtype != torch.float32 or not w.is_contiguous())
                    for w in (getattr(data, "edge_weight", None), getattr(data, "BU_edge_weight", None)))
-
-    @staticmethod
-    def _weights(data, ei, bu):
-        """(TD, BU) weights checked and laid out as fp32 [E] (or None); a cast copy is kept by the plan that reads it
-        (and, for a weight that requires grad, carries the gradient back through the cast)"""
-        with torch.enable_grad():
-            return (edge_weight(getattr(data, "edge_weight", None), int(ei.shape[1]), "edge_weight"),
-                    edge_weight(getattr(data, "BU_edge_weight", None), int(bu.shape[1]), "BU_edge_weight"))
 
     @staticmethod
     def _deliver(p):
@@ -437,50 +404,32 @@ class FusedTrainer:
         self._calls += 1
         # a weight that needs an fp32 copy is read through that copy: a replay would not see the caller's later writes
         use_graph = self.graphs and seed is None and not self.validate and not self._weights_copied(data)
-        pk_any = next_data is not None or (self._prep_buf is not None and any(
-            o is not None and o[1]() is data for o in self._prep_owner))
+        pk_any = next_data is not None or any(o is not None and o[1]() is data for o in self._prep_owner)
         key = None
         if use_graph:
             key = self._graph_key(data, b_global, node_id_base)
             if pk_any:                          # which prepared buffer holds this batch, what the next batch is
                 key = key + self._prep_peek(data, next_data)
-            ent = self._graphs.get(key)
-            if ent is not None and ent["ws"] is self._ws and (not pk_any or ent["prep"] is self._prep_buf):
-                ent["graph"].replay()
-                self.graph_replays += 1
+            # a capture reads the workspace and, with pk_any, the prepared buffers: valid while they are the same
+            p = self._graphs.replay(key, (self._ws, self._prep_buf) if pk_any else (self._ws,))
+            if p is not None:
                 if pk_any:
-                    self._prep_commit(ent["plan"], data, next_data)
-                if ent["plan"]["edge_grad"]:
-                    self._deliver(ent["plan"])
-                self.last_logp = ent["plan"]["logp"]
-                return ent["plan"]["loss"]
+                    self._prep_commit(p, data, next_data)
+                if p["edge_grad"]:
+                    self._deliver(p)
+                self.last_logp = p["logp"]
+                return p["loss"]
         p = self._plan(data, b_global, node_id_base, seed)
-        ws_before = self._ws
         self._workspace(p["dims"], p["dev"], p["weighted"], p["edge_grad"])
-        if self._ws is not ws_before:
-            self._graphs.clear()               # the workspace moved: every captured pointer into it is stale
         if pk_any:
             pkey = self._prep_setup(p, data, next_data, node_id_base)
             if use_graph:
                 key = self._graph_key(data, b_global, node_id_base) + pkey   # (the buffers may just have moved)
-        if not use_graph:
+        if not use_graph or self._graphs.first_sighting(key, data):
             self._enqueue_prio(p, pk_any)
         else:
-            ref = self._seen.get(key)
-            if ref is None or ref() is not data:   # first sighting: enqueue (also warms the library's lazy state)
-                if len(self._seen) >= 256:
-                    self._seen.clear()
-                self._seen[key] = weakref.ref(data)
-                self._enqueue_prio(p, pk_any)
-            else:                                   # seen before: capture, then replay
-                g = capture_graph(lambda: self._enqueue(p))
-                while len(self._graphs) >= self.max_graphs:
-                    self._graphs.pop(next(iter(self._graphs)))
-                self._graphs[key] = {"ws": self._ws, "prep": self._prep_buf, "graph": g, "plan": p,
-                                     "data": (data, next_data)}   # the strong references pin id(data)
-                self.graph_captures += 1
-                g.replay()
-                self.graph_replays += 1
+            self._graphs.capture(key, lambda: self._enqueue(p), p, (self._ws, self._prep_buf) if pk_any else (self._ws,),
+                                 (data, next_data))
         if pk_any:
             self._prep_commit(p, data, next_data)
         if p["edge_grad"]:

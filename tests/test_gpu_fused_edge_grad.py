@@ -346,42 +346,41 @@ def test_no_edge_work_without_grad(dev):
 def _abi_edge_grad(d, m, prepared):
     """bigcn_batch_prepare (optional) -> features_forward -> features_backward -> features_edge_grad, directly."""
     from bigcn_b200 import _lib as L
-    from bigcn_b200.ops import _PNAMES, _as_x, _i64, _make_structs, _p, _stream, edge_weight
+    from bigcn_b200.ops import _PNAMES, _p, _stream, batch_args, batch_prepare_bytes, features_workspace_bytes
     lib = L.lib()
-    x, xs = _as_x(d.x, "sparse")
-    ei, bu, batch, root = _i64(d.edge_index), _i64(d.BU_edge_index), _i64(d.batch), _i64(d.rootindex)
-    ew = (edge_weight(d.edge_weight, ei.shape[1], "edge_weight"), edge_weight(d.BU_edge_weight, bu.shape[1], "BU"))
     mods = {"td": m.TDrumorGCN, "bu": m.BUrumorGCN}
     params = []
     for n in _PNAMES:
         conv = getattr(mods[n[:2]], "conv" + n[4])
         params.append((conv.lin.weight if n[3] == "w" else conv.bias).detach())
-    dims, bt, pr = _make_structs(x, ei, bu, batch, root, params, 0, 0, xs, ew)
+    a = batch_args(d.x, d.edge_index, d.BU_edge_index, d.batch, d.rootindex, d.edge_weight, d.BU_edge_weight,
+                   gemm_mode="sparse", params=params)
+    dims, bt, pr, dev = a.dims, a.bt, a.pr, a.dev
     o = L.Opts(training=1, p_drop=0.2, seed=9, deg_by=L.DEG_BY["target"], gemm_mode=L.GEMM_MODE["sparse"],
                dir_mask=L.DIR_TD | L.DIR_BU, edge_grad=1)
     st = _stream()
-    flags = torch.zeros(1, dtype=torch.int32, device=x.device)
+    flags = torch.zeros(1, dtype=torch.int32, device=dev)
     keep = []
     if prepared:
-        nb = lib.bigcn_batch_prepare_edge_bytes(C.byref(dims))
-        buf = torch.empty(nb, dtype=torch.uint8, device=x.device)
+        nb = batch_prepare_bytes(dims, True)
+        buf = torch.empty(nb, dtype=torch.uint8, device=dev)
         keep.append(buf)
         bt.prepared = buf.data_ptr()
         L.check(lib.bigcn_batch_prepare(C.byref(dims), C.byref(bt), C.byref(o), _p(flags), _p(buf), nb, st), "prepare")
         L.check(lib.bigcn_batch_prepare_join(st), "prepare_join")
-    nws = lib.bigcn_features_edge_workspace_bytes(C.byref(dims), 1)
-    ws = torch.empty(nws, dtype=torch.uint8, device=x.device)
-    feat = torch.empty(dims.B, 256, device=x.device)
+    nws = features_workspace_bytes(dims, True, True)
+    ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+    feat = torch.empty(dims.B, 256, device=dev)
     L.check(lib.bigcn_features_forward(C.byref(dims), C.byref(bt), C.byref(pr), C.byref(o), _p(feat), _p(flags), _p(ws),
                                        nws, st), "forward")
-    gfeat = torch.randn(dims.B, 256, generator=torch.Generator().manual_seed(3)).to(x.device)
+    gfeat = torch.randn(dims.B, 256, generator=torch.Generator().manual_seed(3)).to(dev)
     grads = [torch.empty_like(p) for p in params]
     gr = L.Params()
     for n, t in zip(_PNAMES, grads):
         setattr(gr, n, _p(t))
     L.check(lib.bigcn_features_backward(C.byref(dims), C.byref(bt), C.byref(pr), C.byref(o), _p(gfeat), C.byref(gr),
                                         _p(ws), nws, st), "backward")
-    dew = [torch.empty(dims.E_td, device=x.device), torch.empty(dims.E_bu, device=x.device)]
+    dew = [torch.empty(dims.E_td, device=dev), torch.empty(dims.E_bu, device=dev)]
     L.check(lib.bigcn_features_edge_grad(C.byref(dims), C.byref(bt), C.byref(o), _p(dew[0]), _p(dew[1]), _p(ws), nws,
                                          st), "edge_grad")
     torch.cuda.synchronize()

@@ -12,6 +12,7 @@ import torch  # noqa: E402
 import bigcn_b200  # noqa: E402
 from bigcn_b200 import _lib as L  # noqa: E402
 from bigcn_b200.data import Batch, make_batch_shard  # noqa: E402
+from bigcn_b200.ops import GraphCache  # noqa: E402
 
 
 def main():
@@ -30,8 +31,8 @@ def main():
     nxt = lambda i: batches[(i + 1) % 3] if prefetch else None  # noqa: E731
 
     def run(steps=60):
-        tr._graphs.clear()                   # knobs are read at enqueue / capture time
-        tr._seen.clear()
+        # knobs are read at enqueue / capture time: start from no captures and no sightings
+        tr._graphs = GraphCache(tr._graphs.max_graphs, tr._graphs.max_seen)
         for i in range(18):
             tr.step(batches[i % 3], next_data=nxt(i))
         torch.cuda.synchronize()
