@@ -60,7 +60,8 @@ class AsmWeights(C.Structure):
 
 class Ebgcn(C.Structure):
     _fields_ = [("N", C.c_int64), ("B", C.c_int64), ("K", C.c_int64), ("E", C.c_int64),
-                ("h1", c_ptr), ("x", c_ptr), ("edge_index", c_ptr), ("edge_weight", c_ptr), ("batch", c_ptr),
+                ("h1", c_ptr), ("x", c_ptr), ("x_ptr", c_ptr), ("x_col", c_ptr), ("x_val", c_ptr),
+                ("edge_index", c_ptr), ("edge_weight", c_ptr), ("batch", c_ptr),
                 ("rootindex", c_ptr), ("node_ptr", c_ptr), ("bn_weight", c_ptr), ("bn_bias", c_ptr),
                 ("running_mean", c_ptr), ("running_var", c_ptr), ("num_batches_tracked", c_ptr),
                 ("momentum", C.c_float), ("eps", C.c_float), ("training", C.c_int32), ("deg_by", C.c_int32),
@@ -111,6 +112,12 @@ _SIGS = {
                                         C.c_int32, C.c_int32, c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "bigcn_gcnconv_backward": (C.c_int, [c_ptr, C.c_int64, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr,
                                          C.c_int32, c_ptr, C.c_size_t, c_ptr]),
+    "bigcn_gcnconv_csr_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int64]),
+    "bigcn_gcnconv_csr_scratch_bytes": (C.c_size_t, [C.c_int64, C.c_int64]),
+    "bigcn_gcnconv_csr_forward": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int64, C.c_int64, c_ptr, C.c_int64, c_ptr, c_ptr,
+                                            C.c_int32, c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr, C.c_size_t, c_ptr]),
+    "bigcn_gcnconv_csr_backward": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int64, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr,
+                                             c_ptr, C.c_size_t, c_ptr, C.c_size_t, c_ptr]),
     "bigcn_features_workspace_bytes": (C.c_size_t, [C.POINTER(Dims)]),
     "bigcn_batch_prepare_bytes": (C.c_size_t, [C.POINTER(Dims)]),
     "bigcn_batch_prepare_edge_bytes": (C.c_size_t, [C.POINTER(Dims)]),
@@ -151,6 +158,7 @@ _SIGS = {
                                                   c_ptr, c_ptr, c_ptr, c_ptr, C.c_int32, C.c_int32, c_ptr, C.c_size_t,
                                                   c_ptr]),
     "bigcn_ebgcn_conv2_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int64, C.c_int64]),
+    "bigcn_ebgcn_conv2_csr_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int64, C.c_int64]),
     "bigcn_ebgcn_conv2_forward": (C.c_int, [C.POINTER(Ebgcn), c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "bigcn_ebgcn_conv2_backward": (C.c_int, [C.POINTER(Ebgcn), c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
                                              c_ptr, C.c_size_t, c_ptr]),

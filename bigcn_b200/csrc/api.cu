@@ -918,7 +918,7 @@ extern "C" void* bigcn_internal_stream(void) {
   SideCtx* sc = side_ctx();
   return sc ? (void*)sc->low : nullptr;
 }
-extern "C" int bigcn_version(void) { return 108; }
+extern "C" int bigcn_version(void) { return 109; }
 extern "C" int bigcn_device_ok(void) {
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
@@ -1209,6 +1209,131 @@ extern "C" int bigcn_gcnconv_backward(const float* x, int64_t N, int64_t K, int6
   if (gemm_mode == BIGCN_GEMM_FP32) return dw_fp32(x, N, K, cw.xw, H, 64, cw.dw_part, dw, K, 0, nullptr, 0, 0, st);
   return dw_tc(x, N, K, cw.xw, H, 64, cw.split, cw.split + (size_t)(N > 0 ? N : 1) * H, cw.dw_part, dw, K, 0,
                nullptr, 0, 0, gemm_mode, st);
+}
+
+// ---- GCNConv on a CSR x: BiGCN's sparse-input conv1 kernels for one direction ------------------------------------
+// The workspace the forward hands to the backward holds the structure, W^T and X W^T (then T): nothing N x K and
+// nothing per non-zero.  The per-non-zero buffers (sort keys, column-sorted copy, hub-column lists; BiGCN's capacity
+// N * min(K, 48)) are a scratch of each call: the forward checks the columns and the capacity with k_xs_from_csr, the
+// backward runs it again (no flags) and sorts by column for the dW sweep.
+struct ConvCsrWs {
+  bigcn_graph_t g;
+  float* wT;      // [K][64]
+  float* xw;      // [N][64]  (backward: T)
+  float* cs_part;
+  void* prep_ws; size_t prep_bytes;
+  size_t total;
+};
+static ConvCsrWs carve_conv_csr(int64_t N, int64_t E, int64_t K, void* ws, size_t bytes) {
+  ConvCsrWs w{};
+  Carver c(ws, bytes);
+  w.g.in_ptr = c.take<int32_t>(N + 1);
+  w.g.out_ptr = c.take<int32_t>(N + 1);
+  w.g.in_idx = c.take<int32_t>(E > 0 ? E : 1);
+  w.g.out_idx = c.take<int32_t>(E > 0 ? E : 1);
+  w.g.deg = c.take<int32_t>(N > 0 ? N : 1);
+  w.g.dis = c.take<float>(N > 0 ? N : 1);
+  w.g.rowsum = nullptr;
+  w.g.in_long = c.take<int32_t>(long_ws_ints(E));
+  w.g.out_long = c.take<int32_t>(long_ws_ints(E));
+  w.wT = c.take<float>((size_t)K * H);
+  w.xw = c.take<float>((size_t)(N > 0 ? N : 1) * H);
+  w.cs_part = c.take<float>((size_t)cs_chunks(N) * H);
+  w.prep_bytes = graph_prep_ws_bytes(N, E, 1);
+  w.prep_ws = c.take<char>(w.prep_bytes);
+  w.total = align_up(c.off, 256);
+  return w;
+}
+
+struct ConvCsrScratch {
+  XSparse xs;
+  size_t total;
+};
+static ConvCsrScratch carve_conv_csr_scratch(int64_t N, int64_t K, void* ws, size_t bytes) {
+  ConvCsrScratch w{};
+  Carver c(ws, bytes);
+  w.xs = xs_carve_csr(c, N, K);
+  w.total = align_up(c.off, 256);
+  return w;
+}
+
+// the caller's CSR in the scratch's view, the keys / row ids / capacity state written (k_xs_from_csr)
+static int conv_csr_keys(ConvCsrScratch& sc, const int32_t* ptr, const int32_t* col, const float* val, int32_t* flags,
+                         cudaStream_t st) {
+  sc.xs.ptr = const_cast<int32_t*>(ptr);
+  sc.xs.col = const_cast<int32_t*>(col);
+  sc.xs.val = const_cast<float*>(val);
+  sc.xs.flags = flags;
+  return xs_build_csr(sc.xs, nullptr, false, st);
+}
+
+extern "C" size_t bigcn_gcnconv_csr_workspace_bytes(int64_t N, int64_t E, int64_t K) {
+  return carve_conv_csr(N, E, K, nullptr, 0).total;
+}
+
+extern "C" size_t bigcn_gcnconv_csr_scratch_bytes(int64_t N, int64_t K) {
+  return carve_conv_csr_scratch(N, K, nullptr, 0).total;
+}
+
+extern "C" int bigcn_gcnconv_csr_forward(const int32_t* ptr, const int32_t* col, const float* val, int64_t N, int64_t K,
+                                         const int64_t* edge_index, int64_t E, const float* w, const float* bias,
+                                         int32_t deg_by, float* out, int32_t* flags, void* workspace,
+                                         size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                                         bigcn_stream_t stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  BIGCN_CHECK_ARG(N >= 0 && K > 0 && E >= 0, "gcnconv_csr_forward: bad dims");
+  BIGCN_CHECK_ARG(w && flags && (N == 0 || (ptr && out)), "gcnconv_csr_forward: NULL argument");
+  ConvCsrWs cw = carve_conv_csr(N, E, K, workspace, workspace_bytes);
+  BIGCN_CHECK_ARG(workspace && workspace_bytes >= cw.total, "gcnconv_csr_forward: workspace too small");
+  ConvCsrScratch sc = carve_conv_csr_scratch(N, K, scratch, scratch_bytes);
+  BIGCN_CHECK_ARG(scratch && scratch_bytes >= sc.total, "gcnconv_csr_forward: scratch too small");
+  const int64_t* ei[1] = {edge_index};
+  const int64_t Es[1] = {E};
+  if (int rc = graph_prep_impl(1, ei, Es, N, nullptr, 0, deg_by, &cw.g, nullptr, flags, cw.prep_ws, cw.prep_bytes, st))
+    return rc;
+  if (N == 0) return 0;
+  TransposeJobs js{};
+  js.job[js.n++] = TransposeJob{w, K, 0, K, cw.wT, H, 0};
+  if (int rc = transpose_jobs_launch(js, st)) return rc;
+  if (int rc = conv_csr_keys(sc, ptr, col, val, flags, st)) return rc;   // column range, capacity
+  if (int rc = xw_csr(sc.xs, cw.wT, H, cw.xw, H, st)) return rc;
+  PropArgs a{};
+  a.N = N; a.relu = 0;
+  a.d[0] = PropDir{cw.g.in_ptr, cw.g.in_idx, cw.g.dis, cw.xw, bias, out, H, H, cw.g.in_long, E};
+  return propagate_launch(a, 1, st);
+}
+
+extern "C" int bigcn_gcnconv_csr_backward(const int32_t* ptr, const int32_t* col, const float* val, int64_t N,
+                                          int64_t K, int64_t E, const float* grad_out, float* dw, float* db,
+                                          void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                                          bigcn_stream_t stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  BIGCN_CHECK_ARG(N >= 0 && K > 0 && E >= 0 && dw && db && (N == 0 || (ptr && grad_out)),
+                  "gcnconv_csr_backward: bad arguments");
+  ConvCsrWs cw = carve_conv_csr(N, E, K, workspace, workspace_bytes);
+  BIGCN_CHECK_ARG(workspace && workspace_bytes >= cw.total, "gcnconv_csr_backward: workspace too small");
+  ConvCsrScratch sc = carve_conv_csr_scratch(N, K, scratch, scratch_bytes);
+  BIGCN_CHECK_ARG(scratch && scratch_bytes >= sc.total, "gcnconv_csr_backward: scratch too small");
+  if (N == 0) {
+    cudaMemsetAsync(dw, 0, (size_t)H * K * sizeof(float), st);
+    cudaMemsetAsync(db, 0, H * sizeof(float), st);
+    return 0;
+  }
+  k_colsum_part<<<cs_chunks(N), 256, 0, st>>>(grad_out, N, cw.cs_part);
+  BIGCN_CHECK_LAUNCH("k_colsum_part");
+  ColsumArgs c{};
+  c.nchunk = cs_chunks(N); c.part[0] = cw.cs_part; c.out[0] = db;
+  if (int rc = colsum_reduce_launch(c, 1, st)) return rc;
+  // T = A-hat^T grad_out
+  PropArgs a{};
+  a.N = N; a.relu = 0;
+  a.d[0] = PropDir{cw.g.out_ptr, cw.g.out_idx, cw.g.dis, grad_out, nullptr, cw.xw, H, H, cw.g.out_long, E};
+  if (int rc = propagate_launch(a, 1, st)) return rc;
+  // dw = T^T x: the sort keys again (the forward raised the flags), the column-sorted copy, the column sweep (NaN past
+  // the capacity)
+  if (int rc = conv_csr_keys(sc, ptr, col, val, nullptr, st)) return rc;
+  if (int rc = xs_sort_csc(sc.xs, st)) return rc;
+  return dw_sparse(sc.xs, cw.xw, H, H, dw, nullptr, K, st);
 }
 
 // ---- X * W^T with the row-sparse capture, and its weight gradient, on their own -------------

@@ -15,6 +15,8 @@
 // dW2b = S^T R (the dW scan of xw.cu over R), dR = (S W2b) [R > 0] -> dbeta_k = sum_b dR_bk, dgamma_k = sum_b dR_bk xhat_bk
 // (k_eb_root_bwd), and for the 64 h1 columns an ordinary BatchNorm backward over N rows (k_eb_hbwd1 / k_eb_hbwd2).
 // d edge_weight: the chain of weighted.cu (k_w_edge_dot with Z as the propagated operand, k_w_ddeg, k_w_dweight).
+// A CSR x (bigcn_ebgcn_t.x == NULL) is read at the roots only: k_eb_root_csr fills a dense block Xr [B,K] of the B root
+// rows and a tree-local root map, and the kernels below run unchanged on Xr with that map (r_b = b).
 // Every reduction runs in a fixed order (row / tree segments combined in index order): deterministic, no atomics on
 // floats.  bn1's sums over N rows (statistics, dbeta, dgamma) accumulate in fp64: BatchNorm's output is centred, so a
 // shift of the mean by a few fp32 ulps of its partial sums enters every row's term of dW2 = T^T A with the same sign.
@@ -57,6 +59,31 @@ __global__ void k_eb_roots(const int64_t* __restrict__ rootindex, const int32_t*
   const bool ok = r >= 0 && r < N;
   if (nonempty && !ok) atomicOr(flags, BIGCN_FLAG_ROOT_RANGE);
   root[b] = nonempty && ok ? (int32_t)r : -1;
+}
+
+// CSR x: Xr[b] = x[r_b] as a dense row (zeroed, then the row's entries added in CSR order; a column outside [0, K) is
+// skipped and flagged), rmap[b] = b, or -1 where root[b] is -1 (Xr[b] then stays zero).  CTA per tree.
+__global__ void __launch_bounds__(128) k_eb_root_csr(const int32_t* __restrict__ root, const int32_t* __restrict__ ptr,
+                                                     const int32_t* __restrict__ col, const float* __restrict__ val,
+                                                     int64_t K, float* __restrict__ Xr, int32_t* __restrict__ rmap,
+                                                     int32_t* flags) {
+  const int64_t b = blockIdx.x;
+  const int32_t r = root[b];
+  float* row = Xr + b * K;
+  for (int64_t k = threadIdx.x; k < K; k += blockDim.x) row[k] = 0.f;
+  if (threadIdx.x == 0) rmap[b] = r >= 0 ? (int32_t)b : -1;
+  if (r < 0) return;   // the same for the whole CTA
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  const int p1 = ptr[r + 1];
+  for (int p = ptr[r]; p < p1; ++p) {
+    const int k = col[p];
+    if (k < 0 || k >= K) {
+      atomicOr(flags, BIGCN_FLAG_X_CSR_RANGE);
+      continue;
+    }
+    row[k] += val[p];
+  }
 }
 
 // ---- bn1 statistics: PASS 0 sums the values, PASS 1 the squared deviations from the mean of PASS 0 -----------------
@@ -345,11 +372,13 @@ struct EbWs {
   float* dwpart;
   float* cspart;
   double* dgb;                 // [2][64]
+  float* Xr;                   // [B][K] CSR x only: the root rows
+  int32_t* rmap;               // [B]    CSR x only: b, or -1 for a tree without a root
   int32_t nh, nseg;
   size_t total;
 };
 
-static EbWs carve_eb(int64_t N, int64_t B, int64_t K, int64_t E, void* ws, size_t bytes) {
+static EbWs carve_eb(int64_t N, int64_t B, int64_t K, int64_t E, bool csr, void* ws, size_t bytes) {
   EbWs w{};
   Carver c(ws, bytes);
   const size_t n1 = (size_t)(N > 0 ? N : 1), e1 = (size_t)(E > 0 ? E : 1), b1 = (size_t)(B > 0 ? B : 1);
@@ -397,6 +426,10 @@ static EbWs carve_eb(int64_t N, int64_t B, int64_t K, int64_t E, void* ws, size_
   w.dwpart = c.take<float>(dw_partial_floats(B, K, H));
   w.cspart = c.take<float>((size_t)cs_chunks(N) * H);
   w.dgb = c.take<double>(2 * H);
+  if (csr) {
+    w.Xr = c.take<float>(b1 * K);
+    w.rmap = c.take<int32_t>(b1);
+  }
   w.total = align_up(c.off, 256);
   return w;
 }
@@ -410,7 +443,9 @@ static int eb_mode(const bigcn_ebgcn_t* a) {
 static Eb eb_args(const bigcn_ebgcn_t* a, const EbWs& w) {
   Eb e{};
   e.N = a->N; e.B = a->B; e.K = a->K; e.ld = H + a->K;
-  e.h1 = a->h1; e.x = a->x; e.batch = a->batch; e.root = w.root; e.node_ptr = a->node_ptr;
+  e.h1 = a->h1; e.batch = a->batch; e.node_ptr = a->node_ptr;
+  e.x = a->x != nullptr ? a->x : w.Xr;
+  e.root = a->x != nullptr ? w.root : w.rmap;
   const bool bn = eb_mode(a) != 3;
   e.gamma = bn ? a->bn_weight : nullptr;
   e.beta = bn ? a->bn_bias : nullptr;
@@ -425,7 +460,8 @@ static Eb eb_args(const bigcn_ebgcn_t* a, const EbWs& w) {
 
 static int eb_check(const bigcn_ebgcn_t* a, size_t workspace_bytes, const void* workspace, EbWs& w) {
   BIGCN_CHECK_ARG(a != nullptr && a->N >= 0 && a->B >= 0 && a->K > 0 && a->E >= 0, "ebgcn_conv2: bad dimensions");
-  BIGCN_CHECK_ARG(a->N == 0 || (a->h1 && a->x && a->batch && a->w2), "ebgcn_conv2: NULL h1, x, batch or w2");
+  BIGCN_CHECK_ARG(a->N == 0 || (a->h1 && (a->x || a->x_ptr) && a->batch && a->w2),
+                  "ebgcn_conv2: NULL h1, x (and x_ptr), batch or w2");
   BIGCN_CHECK_ARG(a->B == 0 || (a->rootindex && a->node_ptr), "ebgcn_conv2: NULL rootindex or node_ptr");
   BIGCN_CHECK_ARG(a->E == 0 || a->edge_index, "ebgcn_conv2: NULL edge_index");
   BIGCN_CHECK_ARG((a->bn_weight == nullptr) == (a->bn_bias == nullptr), "ebgcn_conv2: bn_weight and bn_bias go together");
@@ -433,10 +469,11 @@ static int eb_check(const bigcn_ebgcn_t* a, size_t workspace_bytes, const void* 
                   "ebgcn_conv2: running_mean and running_var go together");
   BIGCN_CHECK_ARG(!(a->training && a->running_mean && a->momentum < 0.f && !a->num_batches_tracked),
                   "ebgcn_conv2: momentum=None needs num_batches_tracked");
-  w = carve_eb(a->N, a->B, a->K, a->E, nullptr, 0);
+  const bool csr = a->x == nullptr;
+  w = carve_eb(a->N, a->B, a->K, a->E, csr, nullptr, 0);
   BIGCN_CHECK_ARG(workspace && workspace_bytes >= w.total, "ebgcn_conv2: workspace too small (%zu < %zu)", workspace_bytes,
                   w.total);
-  w = carve_eb(a->N, a->B, a->K, a->E, const_cast<void*>(workspace), workspace_bytes);
+  w = carve_eb(a->N, a->B, a->K, a->E, csr, const_cast<void*>(workspace), workspace_bytes);
   return 0;
 }
 
@@ -445,7 +482,11 @@ static int eb_check(const bigcn_ebgcn_t* a, size_t workspace_bytes, const void* 
 using namespace bigcn;
 
 extern "C" size_t bigcn_ebgcn_conv2_workspace_bytes(int64_t N, int64_t B, int64_t K, int64_t E) {
-  return carve_eb(N, B, K, E, nullptr, 0).total;
+  return carve_eb(N, B, K, E, false, nullptr, 0).total;
+}
+
+extern "C" size_t bigcn_ebgcn_conv2_csr_workspace_bytes(int64_t N, int64_t B, int64_t K, int64_t E) {
+  return carve_eb(N, B, K, E, true, nullptr, 0).total;
 }
 
 extern "C" int bigcn_ebgcn_conv2_forward(const bigcn_ebgcn_t* a, float* out, int32_t* flags, void* workspace,
@@ -472,6 +513,10 @@ extern "C" int bigcn_ebgcn_conv2_forward(const bigcn_ebgcn_t* a, float* out, int
   if (B > 0) {
     k_eb_roots<<<(unsigned)ceil_div(B, 256), 256, 0, st>>>(a->rootindex, a->node_ptr, B, N, w.root, flags);
     BIGCN_CHECK_LAUNCH("k_eb_roots");
+    if (a->x == nullptr) {
+      k_eb_root_csr<<<(unsigned)B, 128, 0, st>>>(w.root, a->x_ptr, a->x_col, a->x_val, K, w.Xr, w.rmap, flags);
+      BIGCN_CHECK_LAUNCH("k_eb_root_csr");
+    }
   }
   Eb e = eb_args(a, w);
   const int mode = eb_mode(a);

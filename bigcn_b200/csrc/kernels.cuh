@@ -218,6 +218,7 @@ struct XSparse {
 int debug_knob(int key);
 int64_t xs_capacity(int64_t N, int64_t K);
 XSparse xs_carve(Carver& c, int64_t N, int64_t K);
+XSparse xs_carve_csr(Carver& c, int64_t N, int64_t K);   // caller's CSR: ptr / col / val / cnt / ELL left unset
 int xs_build_csc(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st);
 int xs_build_csr(const XSparse& x, const float* x_dense, bool from_capture, cudaStream_t st);
 int xs_sort_csc(const XSparse& x, cudaStream_t st);

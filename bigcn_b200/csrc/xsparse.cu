@@ -53,6 +53,27 @@ XSparse xs_carve(Carver& c, int64_t N, int64_t K) {
   return x;
 }
 
+// The same view for a caller's CSR (ptr / col / val are the caller's; no capture, so no row counts, ELL slots or scan
+// partials): what k_xs_from_csr, the column sort and the column sweep touch, at the same capacity.
+XSparse xs_carve_csr(Carver& c, int64_t N, int64_t K) {
+  XSparse x{};
+  x.N = N;
+  x.K = K;
+  x.cap = xs_capacity(N, K);
+  x.state = c.take<int32_t>(4);
+  x.row = c.take<int32_t>(x.cap);
+  x.keys[0] = c.take<int32_t>(x.cap);
+  x.keys[1] = c.take<int32_t>(x.cap);
+  x.perm[0] = c.take<int32_t>(x.cap);
+  x.perm[1] = c.take<int32_t>(x.cap);
+  x.hist = c.take<int32_t>((size_t)256 * xs_nblk(x.cap) + 4 * 256);
+  x.cptr = c.take<int32_t>(K + 1);
+  x.crow = c.take<int32_t>(x.cap);
+  x.cval = c.take<float>(x.cap);
+  for (int d = 0; d < 2; ++d) x.clong[d] = c.take<int32_t>(long_ws_ints(x.cap));
+  return x;
+}
+
 // ---- exclusive scan of the row counts -> ptr[N+1] -------------------------------------------
 __device__ __forceinline__ int block_excl_scan256(int v, int* total) {
   __shared__ int warp_tot[8];

@@ -18,8 +18,10 @@ What runs where:
   generator, so the random stream is the reference's).
 
 ``bn1`` is a real ``torch.nn.BatchNorm1d(hidden + input)``: its parameters, buffers, ``train()`` / ``eval()`` and
-momentum behave as users expect; the op reads and updates them as its forward would.  data.x must be dense (it is
-widened to fp32); a sparse data.x, or one that requires grad, raises BigcnError.
+momentum behave as users expect; the op reads and updates them as its forward would.  data.x is dense (widened to
+fp32) or a ``SparseX``, as ``DeviceForest`` batches and ``forest_from_raw`` forests hand it over: conv1 then runs on
+the CSR and conv2's op reads the root rows from it, so nothing N x K is formed.  A torch sparse data.x, or one that
+requires grad, raises BigcnError.
 """
 from __future__ import annotations
 
@@ -69,9 +71,10 @@ class _EdgeRumorGCN(torch.nn.Module):
         self.last_flags = None
 
     def check_inputs(self):
-        """Raise if the last forward saw an invalid graph (synchronises)."""
-        if self.last_flags is not None:
-            flags, self.last_flags = self.last_flags, None
+        """Raise if the last forward saw an invalid graph, or a SparseX x that conv1 flagged (synchronises)."""
+        pending = [f for f in (self.conv1.last_flags, self.last_flags) if f is not None]
+        self.conv1.last_flags = self.last_flags = None
+        for flags in pending:
             raise_on_flags(flags)
 
     def forward(self, data):

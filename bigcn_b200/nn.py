@@ -19,9 +19,9 @@ import torch
 from . import _lib as L
 import ctypes as C
 
-from .ops import (FeaturesFunction, GCNConvFunction, GCNConvWeightedFunction, GraphCache, HeadFunction, raise_on_flags,
-                  pick_gemm_mode, bf16_features_dense, batch_args, batch_key, edge_weight_key, features_workspace_bytes,
-                  x_val, _p, _stream)
+from .ops import (FeaturesFunction, GCNConvCSRFunction, GCNConvFunction, GCNConvWeightedFunction, GraphCache,
+                  HeadFunction, SparseX, raise_on_flags, pick_gemm_mode, bf16_features_dense, batch_args, batch_key,
+                  edge_weight_key, features_workspace_bytes, sparse_x, x_val, _p, _stream)
 
 H = L.H
 
@@ -39,7 +39,12 @@ class _Lin(torch.nn.Module):
 
 class GCNConv(torch.nn.Module):
     """GCNConv(in, 64): state_dict keys ``lin.weight`` [64,in] and ``bias`` [64] (PyG 2.x);
-    PyG-1.3.2 checkpoints (``weight`` [in,64]) are accepted on load."""
+    PyG-1.3.2 checkpoints (``weight`` [in,64]) are accepted on load.
+
+    ``x`` may be a :class:`~bigcn_b200.SparseX` (bag-of-words rows as CSR, never densified): the product then runs
+    from the CSR and dW as a sweep over x's columns, with ``gemm_mode`` 'auto' or 'sparse' and no ``edge_weight``.
+    Its violation word (an out-of-range column, more non-zeros than N*min(K,48)) is ``last_flags``; pass it to
+    ``ops.raise_on_flags`` to check."""
 
     def __init__(self, in_channels, out_channels, deg_by="target", gemm_mode="auto"):
         super().__init__()
@@ -51,6 +56,7 @@ class GCNConv(torch.nn.Module):
         self.bias = torch.nn.Parameter(torch.zeros(out_channels))
         self.deg_by, self.gemm_mode = deg_by, gemm_mode
         self._auto_mode = None
+        self.last_flags = None
 
     def _mode(self, x):
         if self.gemm_mode != "auto":
@@ -60,6 +66,17 @@ class GCNConv(torch.nn.Module):
         return self._auto_mode
 
     def forward(self, x, edge_index, edge_weight=None):
+        if isinstance(x, SparseX):
+            if edge_weight is not None:
+                raise L.BigcnError("GCNConv: edge_weight is not supported with a SparseX x (the edge-weighted conv has "
+                                   "no CSR form); pass a dense x")
+            if self.gemm_mode not in ("auto", "sparse"):
+                raise L.BigcnError(f"a sparse data.x needs gemm_mode='sparse' (or 'auto'), got {self.gemm_mode!r}")
+            xs = sparse_x(x, "GCNConv")
+            self.last_flags = torch.zeros(1, dtype=torch.int32, device=xs.device)
+            return GCNConvCSRFunction.apply(xs.val, xs.ptr, xs.col, xs.shape, edge_index, self.lin.weight, self.bias,
+                                            self.deg_by, self.last_flags)
+        self.last_flags = None             # the dense paths report nothing here: no stale flags from a SparseX batch
         if edge_weight is None and torch.is_tensor(x) and x.requires_grad:
             # x is an activation (EBGCN's conv2 input is batch-normalised): the generic form returns dx
             edge_weight = torch.ones(edge_index.shape[1], dtype=torch.float32, device=x.device)

@@ -200,6 +200,27 @@ def host_dense_to_csr(x, n_threads=0, out=None, cap=None):
     return SparseX(ptr[:n + 1], col[:nnz], val[:nnz], (n, k))
 
 
+def sparse_x(xs, who):
+    """A :class:`SparseX` checked for the CSR ops (GCNConv on a SparseX, EBGCN): on a CUDA device, int32 ``ptr [N+1]``,
+    int32 ``col`` and fp32 ``val`` of one length, shape (N, K); returned with contiguous buffers.  These ops form no
+    gradient for x, so a ``val`` that requires grad raises."""
+    n, k = xs.shape
+    _need_cuda(xs.ptr, xs.col, xs.val)
+    if not xs.ptr.device == xs.col.device == xs.val.device:
+        raise L.BigcnError(f"{who}: a SparseX's ptr, col and val must be on one device, got {xs.ptr.device}, "
+                           f"{xs.col.device}, {xs.val.device}")
+    if xs.ptr.dtype != torch.int32 or xs.col.dtype != torch.int32 or xs.val.dtype != torch.float32:
+        raise L.BigcnError(f"{who}: a SparseX needs int32 ptr, int32 col and fp32 val, got {xs.ptr.dtype}, "
+                           f"{xs.col.dtype}, {xs.val.dtype}")
+    if n < 0 or k < 1 or tuple(xs.ptr.shape) != (n + 1,) or xs.col.dim() != 1 or xs.col.shape != xs.val.shape:
+        raise L.BigcnError(f"{who}: a SparseX of shape {xs.shape} needs ptr [{n + 1}] and col / val of one length, got "
+                           f"ptr {tuple(xs.ptr.shape)}, col {tuple(xs.col.shape)}, val {tuple(xs.val.shape)}")
+    if xs.val.requires_grad:
+        raise L.BigcnError(f"{who} forms no gradient w.r.t. data.x: pass SparseX(ptr, col, val.detach(), shape) (a "
+                           "SparseX whose val requires grad is not supported)")
+    return SparseX(xs.ptr.contiguous(), xs.col.contiguous(), xs.val.contiguous(), xs.shape)
+
+
 def check_bf16_width(k):
     """bf16 features reach the tensor cores through TMA, which needs 16-byte rows"""
     if k % 8:
@@ -511,7 +532,8 @@ def raise_on_flags(flags: torch.Tensor):
         msgs.append("sparse data.x has a column index outside [0, in_feats)")
     if v & L.FLAG_X_NOT_SPARSE:
         msgs.append("gemm_mode='sparse' needs at most N*min(K,48) non-zeros in data.x (the conv1 weight "
-                    "gradient of this batch is NaN): use 'tf32x3' / 'fp32' for dense features")
+                    "gradient of this batch is NaN): use 'tf32x3' / 'fp32' for dense features; a SparseX data.x "
+                    "that dense (EBGCN, GCNConv) is better passed dense (x.to_dense())")
     raise IndexError("bigcn_b200: invalid graph input: " + "; ".join(msgs))
 
 
@@ -552,6 +574,53 @@ class GCNConvFunction(torch.autograd.Function):
         check(lib().bigcn_gcnconv_backward(_p(x), n, k, e, _p(g), _p(dw), _p(db), L.GEMM_MODE[ctx.gemm_mode],
                                            _p(ws), ws.numel(), _stream()), "gcnconv_backward")
         return None, None, dw, db, None, None
+
+
+def _csr_scratch(n, k, device):
+    # dropped when the call returns: the caching allocator hands it out again only behind this stream's queued work
+    return torch.empty(lib().bigcn_gcnconv_csr_scratch_bytes(n, k), dtype=torch.uint8, device=device)
+
+
+class GCNConvCSRFunction(torch.autograd.Function):
+    """conv(x, edge_index) -> [N,64] for a SparseX x (bigcn_gcnconv_csr_*, given as its ``val``, ``ptr``, ``col`` and
+    ``shape``): the CSR product forward, dW as a sweep over x's columns; gradients for weight and bias.  ``flags``
+    receives an out-of-range column and a batch past the sparse capacity (its dW is then NaN).  Only the structure,
+    W^T and X W^T are kept for the backward; each call allocates the per-non-zero scratch it needs and drops it."""
+
+    @staticmethod
+    def forward(ctx, val, ptr, col, shape, edge_index, weight, bias, deg_by, flags):
+        L.require_device()
+        weight, bias = _f32(weight), _f32(bias)
+        ei = _i64(edge_index)
+        _need_cuda(val, ei, weight, bias)
+        if weight.device != val.device:
+            raise L.BigcnError(f"GCNConv: the SparseX x is on {val.device}, the conv's weight on {weight.device}")
+        n, k = shape
+        e = int(ei.shape[1])
+        if weight.shape != (H, k):
+            raise L.BigcnError(f"GCNConv: out_channels must be {H} and weight [64,{k}], got {tuple(weight.shape)}")
+        ws_bytes = lib().bigcn_gcnconv_csr_workspace_bytes(n, e, k)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=val.device)
+        out = torch.empty(n, H, dtype=torch.float32, device=val.device)
+        sc = _csr_scratch(n, k, val.device)
+        check(lib().bigcn_gcnconv_csr_forward(_p(ptr), _p(col), _p(val), n, k, _p(ei), e, _p(weight), _p(bias),
+                                              L.DEG_BY[deg_by], _p(out), _p(flags), _p(ws), ws_bytes, _p(sc), sc.numel(),
+                                              _stream()), "gcnconv_csr_forward")
+        ctx.save_for_backward(ptr, col, val, ws)
+        ctx.dims = (n, k, e)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        ptr, col, val, ws = ctx.saved_tensors
+        n, k, e = ctx.dims
+        g = _f32(grad_out)
+        dw = torch.empty(H, k, dtype=torch.float32, device=val.device)
+        db = torch.empty(H, dtype=torch.float32, device=val.device)
+        sc = _csr_scratch(n, k, val.device)
+        check(lib().bigcn_gcnconv_csr_backward(_p(ptr), _p(col), _p(val), n, k, e, _p(g), _p(dw), _p(db), _p(ws),
+                                               ws.numel(), _p(sc), sc.numel(), _stream()), "gcnconv_csr_backward")
+        return None, None, None, None, None, dw, db, None, None
 
 
 class GCNConvWeightedFunction(torch.autograd.Function):
@@ -600,11 +669,14 @@ class GCNConvWeightedFunction(torch.autograd.Function):
 
 def ebgcn_x(x):
     """EBGCN's data.x for :class:`EBGCNConv2Function`: dense, widened to contiguous fp32 as the reference's ``.float()``
-    does.  A sparse x, or one that requires grad, raises: the op reads x only at the tree roots and forms no gradient
-    for it."""
+    does, or a :class:`SparseX` (checked by :func:`sparse_x`; conv1 then runs on the CSR and conv2's op reads the root
+    rows from it).  A torch sparse tensor, or an x that requires grad, raises: the op reads x only at the tree roots
+    and forms no gradient for it."""
+    if isinstance(x, SparseX):
+        return sparse_x(x, "EBGCN")
     if not torch.is_tensor(x) or x.layout != torch.strided:
-        raise L.BigcnError("EBGCN takes a dense data.x (a sparse x is not supported: its bn1 statistics are formed from "
-                           "the dense root rows); pass x.to_dense()")
+        raise L.BigcnError("EBGCN takes a dense data.x or a bigcn_b200.SparseX (a torch sparse x is not supported); "
+                           "pass bigcn_b200.SparseX.from_torch_csr(x)")
     if x.requires_grad:
         raise L.BigcnError("EBGCN forms no gradient w.r.t. data.x: pass data.x.detach() (a data.x that requires grad "
                            "is not supported)")
@@ -618,7 +690,8 @@ class EBGCNConv2Function(torch.autograd.Function):
     (EBGCN.py:71-85) without the N x (64 + K) concatenation (bigcn_ebgcn_conv2_*, csrc/ebgcn.cu).  ``bn`` is the
     module's ``torch.nn.BatchNorm1d(64 + K)``: the op reads its parameters and buffers (updating the running statistics
     and ``num_batches_tracked`` in training, as its forward would) and does not run it.  Gradients for h1, edge_weight,
-    bn.weight, bn.bias, w2 and b2; ``x`` is data.  ``node_ptr`` ([B+1] int32) receives the tree offsets."""
+    bn.weight, bn.bias, w2 and b2; ``x`` (dense fp32 or a :class:`SparseX`) is data.  ``node_ptr`` ([B+1] int32)
+    receives the tree offsets."""
 
     @staticmethod
     def forward(ctx, h1, edge_weight_, bn_weight, bn_bias, w2, b2, x, edge_index, batch, rootindex, bn, deg_by, node_ptr,
@@ -626,10 +699,14 @@ class EBGCNConv2Function(torch.autograd.Function):
         L.require_device()
         h1, w2, b2 = _f32(h1), _f32(w2), _f32(b2)
         ei, batch, rootindex = _i64(edge_index), _i64(batch), _i64(rootindex)
+        xs = x if isinstance(x, SparseX) else None
+        xd = None if xs is not None else x
         n, k = x.shape
         e, b = int(ei.shape[1]), int(rootindex.numel())
         ew = edge_weight(edge_weight_, e, "edge_weight")
-        _need_cuda(h1, x, ei, batch, rootindex, w2, b2)
+        _need_cuda(h1, xd, ei, batch, rootindex, w2, b2, *((xs.ptr, xs.col, xs.val) if xs is not None else ()))
+        if xs is not None and xs.val.device != h1.device:
+            raise L.BigcnError(f"EBGCN: the SparseX x is on {xs.val.device}, the model on {h1.device}")
         if tuple(h1.shape) != (n, H):
             raise L.BigcnError(f"EBGCN: conv1's output must be [{n},{H}], got {tuple(h1.shape)}")
         if tuple(w2.shape) != (H, H + k) or tuple(b2.shape) != (H,):
@@ -642,19 +719,22 @@ class EBGCNConv2Function(torch.autograd.Function):
         for t in (rm, rv):
             if t is not None and (t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda):
                 raise L.BigcnError("EBGCN: bn1's running statistics must be contiguous fp32 CUDA tensors")
-        a = L.Ebgcn(N=n, B=b, K=k, E=e, h1=_p(h1), x=_p(x), edge_index=_p(ei), edge_weight=_p(ew), batch=_p(batch),
+        a = L.Ebgcn(N=n, B=b, K=k, E=e, h1=_p(h1), x=_p(xd), edge_index=_p(ei), edge_weight=_p(ew), batch=_p(batch),
                     rootindex=_p(rootindex), node_ptr=_p(node_ptr), bn_weight=_p(gw), bn_bias=_p(gb), running_mean=_p(rm),
                     running_var=_p(rv), num_batches_tracked=_p(nbt),
                     momentum=-1.0 if bn.momentum is None else float(bn.momentum), eps=float(bn.eps),
                     training=int(bn.training), deg_by=L.DEG_BY[deg_by], w2=_p(w2), b2=_p(b2))
-        ws_bytes = lib().bigcn_ebgcn_conv2_workspace_bytes(n, b, k, e)
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
-        out = torch.empty(n, H, dtype=torch.float32, device=x.device)
+        if xs is not None:
+            a.x_ptr, a.x_col, a.x_val = _p(xs.ptr), _p(xs.col), _p(xs.val)
+        ws_bytes = (lib().bigcn_ebgcn_conv2_workspace_bytes if xs is None else
+                    lib().bigcn_ebgcn_conv2_csr_workspace_bytes)(n, b, k, e)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=h1.device)
+        out = torch.empty(n, H, dtype=torch.float32, device=h1.device)
         check(lib().bigcn_ebgcn_conv2_forward(C.byref(a), _p(out), _p(flags), _p(ws), ws_bytes, _stream()),
               "ebgcn_conv2_forward")
         # the backward reads the same arguments: keep every tensor they point at
-        ctx.save_for_backward(h1, x, ei, batch, rootindex, node_ptr, w2, b2, ws, out,
-                              *[t for t in (ew, gw, gb) if t is not None])
+        ctx.save_for_backward(h1, xd if xs is None else xs.val, ei, batch, rootindex, node_ptr, w2, b2, ws, out,
+                              *[t for t in (ew, gw, gb) if t is not None], *((xs.ptr, xs.col) if xs is not None else ()))
         ctx.a, ctx.has = a, (ew is not None, gw is not None, gb is not None)
         return out
 

@@ -327,6 +327,26 @@ int bigcn_gcnconv_backward(const float* x, int64_t N, int64_t K, int64_t E,
                            const float* grad_out /*[N,64]*/, float* dw /*[64,K]*/, float* db /*[64]*/,
                            int32_t gemm_mode, void* workspace /* the forward's */, size_t workspace_bytes,
                            bigcn_stream_t stream);
+/* The same conv on a CSR x (ptr [N+1], col [ptr[N]] int32, val [ptr[N]] fp32; col / val may be NULL when ptr[N] = 0):
+ * BiGCN's sparse-input conv1 for one direction.  Forward: the exact fp32 product from the CSR (row entries in CSR
+ * order), the propagate and the bias; a column outside [0,K) is ignored and raises BIGCN_FLAG_X_CSR_RANGE.  Backward:
+ * db, T = A-hat^T grad_out, the column-sorted copy of the CSR and dw = T^T x as a sweep over x's columns (rows
+ * ascending; deterministic).  The sort holds N*min(K,48) entries, as BIGCN_GEMM_SPARSE does: with more,
+ * BIGCN_FLAG_X_NOT_SPARSE is raised and dw is NaN (the forward output is still exact).  No N x K buffer.
+ *   workspace (bigcn_gcnconv_csr_workspace_bytes): the structure, W^T and X W^T; the backward takes the forward's, with
+ *   the same ptr / col / val.  scratch (bigcn_gcnconv_csr_scratch_bytes): the per-non-zero buffers of one call (sort
+ *   keys, column-sorted copy, hub-column lists), needed only until that call's work on `stream` is done -- it does not
+ *   have to live from the forward to the backward. */
+size_t bigcn_gcnconv_csr_workspace_bytes(int64_t N, int64_t E, int64_t K);
+size_t bigcn_gcnconv_csr_scratch_bytes(int64_t N, int64_t K);
+int bigcn_gcnconv_csr_forward(const int32_t* ptr, const int32_t* col, const float* val, int64_t N, int64_t K,
+                              const int64_t* edge_index, int64_t E, const float* w, const float* bias, int32_t deg_by,
+                              float* out, int32_t* flags, void* workspace, size_t workspace_bytes, void* scratch,
+                              size_t scratch_bytes, bigcn_stream_t stream);
+int bigcn_gcnconv_csr_backward(const int32_t* ptr, const int32_t* col, const float* val, int64_t N, int64_t K,
+                               int64_t E, const float* grad_out /*[N,64]*/, float* dw /*[64,K]*/, float* db /*[64]*/,
+                               void* workspace /* the forward's */, size_t workspace_bytes, void* scratch,
+                               size_t scratch_bytes, bigcn_stream_t stream);
 
 /* ---- edge-weighted GCNConv (SURVEY.md 8f N3) -----------------------------
  * conv(x, edge_index, edge_weight) as EBGCN calls it (model/Twitter/EBGCN.py:84,181:
@@ -365,7 +385,10 @@ int bigcn_gcnconv_weighted_backward(const float* x, int64_t N, int64_t K, const 
  * statistics (biased variance, two passes) when training or without running statistics; in training the running
  * statistics move by `momentum` (< 0: the cumulative average of momentum=None) with the unbiased variance, and
  * num_batches_tracked is incremented; otherwise the running statistics normalise.  N == 1 skips bn1 (EBGCN.py:79).
- * x is dense fp32 [N,K] and gets no gradient; edge_weight NULL = every weight 1; bn_weight / bn_bias NULL = no affine;
+ * x is dense fp32 [N,K], or (x == NULL) CSR: x_ptr [N+1], x_col / x_val [x_ptr[N]] (NULL allowed when x_ptr[N] = 0), read
+ * at the roots only -- the forward forms the B root rows as a dense [B,K] block in the workspace (a column outside [0,K)
+ * is skipped and raises BIGCN_FLAG_X_CSR_RANGE), the same arithmetic then runs on it, and a CSR x needs a workspace of
+ * bigcn_ebgcn_conv2_csr_workspace_bytes (B*K floats and B ints more).  x gets no gradient; edge_weight NULL = every weight 1; bn_weight / bn_bias NULL = no affine;
  * running_mean / running_var / num_batches_tracked NULL = no running statistics.  node_ptr [B+1] (out) receives the
  * tree offsets of the sorted batch vector.  Deterministic, no floating-point atomics.
  *   backward: grad_out [N,64] at `out`; dh1 [N,64] (the gradient reaching conv1's output), d_bn_weight / d_bn_bias
@@ -374,7 +397,10 @@ int bigcn_gcnconv_weighted_backward(const float* x, int64_t N, int64_t K, const 
 typedef struct {
   int64_t N, B, K, E;
   const float* h1;                       /* [N,64] conv1 output */
-  const float* x;                        /* [N,K] */
+  const float* x;                        /* [N,K], or NULL for a CSR x */
+  const int32_t* x_ptr;                  /* [N+1]      CSR x (x == NULL) */
+  const int32_t* x_col;                  /* [x_ptr[N]] */
+  const float* x_val;                    /* [x_ptr[N]] */
   const int64_t* edge_index;             /* [2,E] */
   const float* edge_weight;              /* [E] or NULL */
   const int64_t* batch;                  /* [N], sorted */
@@ -389,6 +415,7 @@ typedef struct {
   const float* b2;                       /* conv2.bias [64] */
 } bigcn_ebgcn_t;
 size_t bigcn_ebgcn_conv2_workspace_bytes(int64_t N, int64_t B, int64_t K, int64_t E);
+size_t bigcn_ebgcn_conv2_csr_workspace_bytes(int64_t N, int64_t B, int64_t K, int64_t E);
 int bigcn_ebgcn_conv2_forward(const bigcn_ebgcn_t* a, float* out /*[N,64]*/, int32_t* flags, void* workspace,
                               size_t workspace_bytes, bigcn_stream_t stream);
 int bigcn_ebgcn_conv2_backward(const bigcn_ebgcn_t* a, const float* out, const float* grad_out, float* dh1,

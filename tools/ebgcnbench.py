@@ -11,8 +11,11 @@ lines, and writes them to the file given with --out.
   gpu    card name, power limit and max SM clock (nvidia-smi), read in the same call.
 
 Cases: Twitter16-shaped 128 trees with K = 5000 (bag-of-words), PHEME-shaped 24 and 4,096 trees with K = 768 (dense
-tanh features).  --tiny runs every path once at a toy size (a rehearsal, not a measurement)."""
+tanh features).  --sparse instead alternates two library models with the same weights, one fed data.x dense and one
+fed the same batch as a SparseX (CSR, what DeviceForest and forest_from_raw hand over): Twitter16- and Twitter15-shaped
+128 trees at K = 5000.  --tiny runs every path once at a toy size (a rehearsal, not a measurement)."""
 import argparse
+import copy
 import json
 import os
 import subprocess
@@ -56,31 +59,36 @@ def peak_above(m, bd):
     return torch.cuda.max_memory_allocated() - base
 
 
-def run_case(name, shape, n_trees, k, infer, steps, warmup):
+def run_case(name, shape, n_trees, k, infer, steps, warmup, sparse=False):
     dev = torch.device("cuda:0")
     args = SimpleNamespace(input_features=k, hidden_features=64, output_features=64, edge_num=2, dropout=0.5,
                            num_class=4, edge_infer_td=infer, edge_infer_bu=infer, device=dev)
     torch.manual_seed(0)
-    ref = ebgcn_harness.EBGCN(args).to(dev).train()
+    ref = (bigcn_b200.EBGCN if sparse else ebgcn_harness.EBGCN)(args).to(dev).train()
     new = bigcn_b200.EBGCN(args).to(dev).train()
     new.load_state_dict(ref.state_dict())
     bd = make_batch(shape, n_trees, seed=1, train=True, in_feats=k).to(dev)
     n = int(bd.x.shape[0])
-    models = {"library": new, "harness": ref}
+    if sparse:
+        sb = copy.copy(bd)
+        sb.x = bigcn_b200.SparseX.from_torch_csr(bd.x.to_sparse_csr())
+        models = {"sparse_x": (new, sb), "dense_x": (ref, bd)}
+    else:
+        models = {"library": (new, bd), "harness": (ref, bd)}
     for _ in range(warmup):
-        for m in models.values():
+        for m, b in models.values():
             m.zero_grad(set_to_none=True)
-            step(m, bd)
+            step(m, b)
     times = {key: [] for key in models}
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     for i in range(steps):
         order = list(models) if i % 2 == 0 else list(models)[::-1]
         for key in order:
-            m = models[key]
+            m, b = models[key]
             m.zero_grad(set_to_none=True)
             torch.cuda.synchronize()
             ev[0].record()
-            step(m, bd)
+            step(m, b)
             ev[1].record()
             torch.cuda.synchronize()
             times[key].append(ev[0].elapsed_time(ev[1]))
@@ -89,10 +97,11 @@ def run_case(name, shape, n_trees, k, infer, steps, warmup):
         emit(kind="step", case=name, edge_infer=infer, model=key, N=n, B=n_trees, K=k, E=int(bd.edge_index.shape[1]),
              ms_median=t[len(t) // 2], ms_min=t[0], ms_max=t[-1], steps=steps)
     if not infer:
-        for key, m in models.items():
-            p = peak_above(m, bd)
+        for key, (m, b) in models.items():
+            p = peak_above(m, b)
+            extra = {"x_csr_mib": b.x.nbytes() / 2**20} if key == "sparse_x" else {}
             emit(kind="mem", case=name, model=key, N=n, B=n_trees, K=k, peak_above_inputs_mib=p / 2**20,
-                 x_fp32_mib=n * k * 4 / 2**20, ratio_to_x=p / (n * k * 4))
+                 x_fp32_mib=n * k * 4 / 2**20, ratio_to_x=p / (n * k * 4), **extra)
     del ref, new, models
     torch.cuda.empty_cache()
 
@@ -102,21 +111,25 @@ def main():
     ap.add_argument("--steps", type=int, default=30)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--tiny", action="store_true")
+    ap.add_argument("--sparse", action="store_true")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                          capture_output=True, text=True).stdout.strip().splitlines()
     emit(kind="gpu", nvidia_smi=smi[0] if smi else None, torch_name=torch.cuda.get_device_name(0))
     if a.tiny:
-        cases = [("tiny", "twitter15", 4, 40), ("tiny-dense", "pheme", 6, 96)]
+        cases = [("tiny", "twitter15", 4, 40)] if a.sparse else [("tiny", "twitter15", 4, 40), ("tiny-dense", "pheme", 6, 96)]
         steps, warmup = 2, 1
+    elif a.sparse:
+        cases = [("twitter16-128-K5000", "twitter16", 128, 5000), ("twitter15-128-K5000", "twitter15", 128, 5000)]
+        steps, warmup = a.steps, a.warmup
     else:
         cases = [("twitter16-128-K5000", "twitter16", 128, 5000), ("pheme-24-K768", "pheme", 24, 768),
                  ("pheme-4096-K768", "pheme", 4096, 768)]
         steps, warmup = a.steps, a.warmup
     for infer in (False, True):
         for name, shape, b, k in cases:
-            run_case(name, shape, b, k, infer, steps, warmup)
+            run_case(name, shape, b, k, infer, steps, warmup, a.sparse)
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "w") as f:
